@@ -13,6 +13,7 @@ Contract (one JSON line on rank 0):
 torch_geometric / lightning, which are not in this image and there is no network).
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -56,6 +57,8 @@ ALG = {
 }
 
 
+DUMP_LIMIT = 64 << 20                      # bytes written by --dump-outputs at most
+
 TRAFFIC_FILE = "r2_dominant_traffic.json"   # ncu DRAM bytes of THIS round's kernels (tools/launch_traffic.py); keyed by kernel kind
 
 
@@ -96,6 +99,7 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "20",
                                        "-i", str(gpu_index)], stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.p.kill)              # a run that fails before stop() must not leave the sampler running
         except Exception:
             self.p = None
 
@@ -125,6 +129,21 @@ class ClockSampler:
         if sm:
             out.update(sm_mhz=statistics.median(sm), sm_max_mhz=mx, reasons=sorted(reasons), samples=len(sm))
         return out
+
+
+def dump_outputs(path, arrays):
+    """Writes each tensor as <path>/<name>.npy (float64 stays float64, everything else becomes float32).  Above DUMP_LIMIT
+    bytes in all, every array is replaced by the same share of its elements at fixed, seeded positions (flattened)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().cpu() if v.dtype == torch.float64 else v.detach().float().cpu() for k, v in arrays.items()}
+    total = sum(v.numel() * v.element_size() for v in arrays.values())
+    for i, (name, v) in enumerate(arrays.items()):
+        if total > DUMP_LIMIT:
+            keep = max(1, v.numel() * DUMP_LIMIT // total)
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(i))[:keep].sort().values
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), v.numpy())
 
 
 def oracle_train_rate(B, steps, warmup, dtype=torch.float64, threads=None):
@@ -196,7 +215,13 @@ def main():
     ap.add_argument("--skip-e2e", action="store_true")
     ap.add_argument("--skip-extra", action="store_true", help="skip the short runs of the other BASELINE.json configs")
     ap.add_argument("--skip-strong", action="store_true", help="skip the strong-scaling block (16384 graphs global)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed train step and the last timed inference "
+                    "step returned to the caller as DIR/<name>.npy (same arguments -> same inputs: compares two builds)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to the native implementation")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -263,9 +288,18 @@ def main():
     for _ in range(W):
         trainer.train_step(resident)
     sampler = ClockSampler(local_rank) if rank == 0 else None
+    last = {}
+
+    def train_step():
+        last["loss"] = trainer.train_step(resident)
+
     n0 = N.launch_count()
-    train_ms = timed(lambda: trainer.train_step(resident), K)
+    train_ms = timed(train_step, K)
     launches = N.launch_count() - n0
+    # after the last timed step its caller holds the returned loss and the parameters it updated in place (views of the flat
+    # buffer); the flat gradient that update used is kept as well.  Copied now: the steps below change all three.
+    dumped = {"train_loss": last["loss"].clone(), "train_params": trainer.model._flat.clone(),
+              "train_grads": trainer.grads.clone()} if args.dump_outputs else None
 
     # ---------------- per-kernel times (same steps, events around every launch) ----------------
     N.profile_enable(True)
@@ -276,7 +310,13 @@ def main():
     # ---------------- inference, device resident ----------------
     for _ in range(W):
         trainer.infer(resident)
-    infer_ms = timed(lambda: trainer.infer(resident), K)
+
+    def infer_step():
+        last["infer"] = trainer.infer(resident)
+
+    infer_ms = timed(infer_step, K)
+    if dumped is not None:
+        dumped["infer_out"] = last["infer"].clone()
     clocks = sampler.stop() if sampler else {}          # sampled across the three device-resident timed regions above
 
     # ---------------- strong scaling: BASELINE.json configs[2] as written = 16384 graphs GLOBAL over the N GPUs ----------------
@@ -482,6 +522,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
 
     # ---------------- roofline of the dominant kernel ----------------
     pk = peaks()

@@ -1,12 +1,12 @@
 """TEST INFRASTRUCTURE ONLY - runs the reference's UNMODIFIED model files on the CPU.
 
-The reference's model classes (``/root/reference/src/ms_hgnn/lightning_py/hgnn*.py``) import four names from
-``torch_geometric.nn`` and nothing else outside torch / yaml.  With ``oracle/pyg_shim`` first on ``sys.path`` they
+The reference's model classes (``src/ms_hgnn/lightning_py/hgnn*.py`` of the MorphSym-HGNN repository) import four names
+from ``torch_geometric.nn`` and nothing else outside torch / yaml.  With ``oracle/pyg_shim`` first on ``sys.path`` they
 import and run as they are: this module loads them from where they lie (nothing is copied), builds the class a
-``synthetic.Config`` names with the reference's own yaml (``/root/reference/cfg/*.yaml``), and returns fp64 outputs,
-loss and every parameter gradient.  ``tests/test_reference_pin.py`` compares the oracle with that, live in this
-container and through the fixtures ``tools/make_golden.py`` stores under ``tests/golden/`` for the GPU box
-(``/root/reference`` does not exist there).
+``synthetic.Config`` names with the reference's own yaml (``cfg/*.yaml``), and returns fp64 outputs, loss and every
+parameter gradient.  The reference is found through the environment variable ``MSHGNN_REFERENCE`` (the directory of a
+checkout of that repository).  ``tests/test_reference_pin.py`` compares the oracle with it live when it is set, and
+always through the fixtures ``tools/make_golden.py`` stores under ``tests/golden/``.
 """
 from __future__ import annotations
 
@@ -19,7 +19,7 @@ from typing import Dict
 
 import torch
 
-REF_ROOT = "/root/reference"
+REF_ROOT = os.environ.get("MSHGNN_REFERENCE", "")          # checkout of the reference repository; unset: live checks skip
 REF_MODELS = os.path.join(REF_ROOT, "src", "ms_hgnn", "lightning_py")
 SHIM = os.path.join(os.path.dirname(os.path.abspath(__file__)), "pyg_shim")
 
@@ -31,7 +31,7 @@ REF_FILE = {
 
 
 def available() -> bool:
-    return os.path.isdir(REF_MODELS)
+    return bool(REF_ROOT) and os.path.isdir(REF_MODELS)
 
 
 def load_reference_class(name: str):

@@ -1,4 +1,4 @@
-"""Generates tests/golden/* in THIS container (where /root/reference exists).
+"""Generates tests/golden/* from a checkout of the reference repository (MSHGNN_REFERENCE=<its directory>).
 
 1. mi_grf_ckpt.pt  - from the reference's shipped checkpoint tests/test_models/epoch=48-val_MSE_loss=6.33834.ckpt:
    its embedded 20-graph batch (x, edge_index, y), the weights rounded to float32 (5.3 MB instead of 10.6 MB),
@@ -6,9 +6,10 @@
 2. seeded.pt       - oracle outputs / losses / gradient norms of every model class on seeded synthetic batches
    (weights and inputs are regenerated from the seeds by the tests; only the expected numbers are stored).
 3. reference_models.pt - outputs, loss and per-tensor gradient digests of the reference's UNMODIFIED model files
-   (/root/reference/src/ms_hgnn/lightning_py/hgnn*.py, imported against oracle/pyg_shim by oracle/reference_pin.py) for
+   (src/ms_hgnn/lightning_py/hgnn*.py, imported against oracle/pyg_shim by oracle/reference_pin.py) for
    every CONFIGS entry at L = 8 on a seeded 5-graph batch with seeded weights - the pin of the MS-HGNN-specific oracle
    semantics (sign tables, base_transform + residual, mean relations, output decoders) and of all gradients.
+4. reference_cfg.json - the reference's group tables (cfg/*.yaml), parsed.
 """
 import os
 import sys
@@ -19,16 +20,19 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in ("morphsym-hgnn_b200", "oracle", "tests"):
     sys.path.insert(0, os.path.join(ROOT, p))
 import mshgnn_oracle as O  # noqa: E402
+import reference_pin as RP  # noqa: E402
 from helpers import oracle_model, oracle_run  # noqa: E402
 from ms_hgnn.synthetic import CONFIGS, make_batch  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
-CKPT = "/root/reference/tests/test_models/epoch=48-val_MSE_loss=6.33834.ckpt"
+CKPT = os.path.join(RP.REF_ROOT, "tests", "test_models", "epoch=48-val_MSE_loss=6.33834.ckpt")
 SEEDED_CASES = [(n, 3, 2) for n in CONFIGS]   # (config, B, layers)
 RP_B, RP_LAYERS, RP_BATCH_SEED, RP_WEIGHT_SEED = 5, 8, 11, 4
 
 
 def main():
+    if not RP.available():
+        raise SystemExit("set MSHGNN_REFERENCE to the directory of a checkout of the reference repository")
     os.makedirs(GOLD, exist_ok=True)
     torch.set_default_dtype(torch.float64)
     sd, hp, batch = O.load_reference_checkpoint(CKPT)
@@ -60,7 +64,6 @@ def main():
                         "x_checksum": {k: v.double().sum().item() for k, v in b.x_dict.items()},
                         "w_checksum": sum(p.double().sum().item() for p in om.parameters())}
     torch.save(seeded, os.path.join(GOLD, "seeded.pt"))
-    import reference_pin as RP
     from helpers import oracle_loss
     ref = {}
     for name, cfg in CONFIGS.items():
@@ -74,8 +77,14 @@ def main():
                      "out": o, "loss": l, "grad_digest": RP.grad_digest(g),
                      "grad_is_none": sorted(n for n, p in rm.named_parameters() if p.grad is None)}
         print("reference", name, tuple(o.shape), float(l))
-    torch.save({"cases": ref, "source": "unmodified /root/reference/src/ms_hgnn/lightning_py/hgnn*.py @ 9e55c68 run against "
+    torch.save({"cases": ref, "source": "unmodified src/ms_hgnn/lightning_py/hgnn*.py of the reference @ 9e55c68 run against "
                 "oracle/pyg_shim (torch_geometric 2.5.0 semantics), fp64, CPU"}, os.path.join(GOLD, "reference_models.pt"))
+    import glob
+    import json
+    import yaml
+    tables = {os.path.basename(p)[:-5]: yaml.safe_load(open(p)) for p in sorted(glob.glob(os.path.join(RP.REF_ROOT, "cfg", "*.yaml")))}
+    with open(os.path.join(GOLD, "reference_cfg.json"), "w") as f:
+        f.write(json.dumps(tables, sort_keys=True) + "\n")
     for f in os.listdir(GOLD):
         print(f, os.path.getsize(os.path.join(GOLD, f)))
 
