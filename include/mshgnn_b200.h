@@ -126,6 +126,8 @@ int mshgnn_loss(const mshgnn_plan* plan, int64_t B, int32_t loss_kind,
 
 /* Backward of mshgnn_forward(train=1) on the same workspace: writes d(loss)/d(params)
  * (every element, zeros for structurally dead branches) into grads[param_count].
+ * grads == NULL runs the input-only backward of a frozen model: the decoder backward and the dX chain through the
+ * layers (everything mshgnn_input_grad reads), without any weight-gradient launch or partial reduction.
  * Replaces: torch autograd through PyG (SURVEY 3.1 "loss.backward()"). */
 int mshgnn_backward(const mshgnn_plan* plan, int64_t B,
                     const void* const* x, int32_t x_dtype,
@@ -142,6 +144,15 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B,
                            const float* params, const float* dout, float* grads,
                            void* workspace, int64_t workspace_bytes,
                            int32_t mode, void* stream, void* layers_ready_event);
+
+/* Input gradient: after mshgnn_backward / mshgnn_backward_staged (with or without grads) on the same workspace and
+ * before the next mshgnn_forward on it, writes d(loss)/d(x[t]) into dx[t] - fp32 [B*nodes_per_graph[t], in_width[t]],
+ * graph-major like x[t] - for every type whose dx[t] is not NULL.  Every element is written (rows of node slots that
+ * cannot reach the output get exact zeros), so dx[t] may be uninitialised memory.  The result does not depend on x_dtype
+ * of the forward: cast it to the features' type if needed.  params: the flat parameters of that forward.
+ * Replaces: torch autograd into the node features through the encoder and apply_symmetry (hgnn_k4.py:L159-160, L198-237). */
+int mshgnn_input_grad(const mshgnn_plan* plan, int64_t B, const float* params, float* const* dx,
+                      void* workspace, int64_t workspace_bytes, int32_t mode, void* stream);
 
 /* Fused Adam on flat buffers (torch.optim.Adam defaults semantics, gnnLightning.py:L258-265):
  * step is the 1-based step count after this update. */
@@ -208,9 +219,9 @@ int64_t mshgnn_plan_describe(const mshgnn_plan* plan, char* buf, int64_t cap);
 /* ---- per-kernel timing (CUDA events on the launching stream) -----------------------------
  * While enabled, every kernel launch of this library is bracketed by a pair of CUDA events on the
  * stream it is launched on.  mshgnn_profile_read synchronises those events, adds the elapsed
- * milliseconds and launch counts per kernel kind into ms_out / launches_out (n entries each, n >=
- * MSHGNN_NUM_KERNEL_KINDS) and clears the record.  Used by bench.py for the roofline figures. */
-#define MSHGNN_NUM_KERNEL_KINDS 19
+ * milliseconds and launch counts per kernel kind into ms_out / launches_out (n entries each, n >= 19: the first n
+ * kinds) and clears the record.  Used by bench.py for the roofline figures. */
+#define MSHGNN_NUM_KERNEL_KINDS 20     /* n = 19 (the kinds before "dx_encoder") is accepted too */
 int mshgnn_profile_enable(int32_t on);
 int mshgnn_profile_read(double* ms_out, int64_t* launches_out, int32_t n);
 const char* mshgnn_kernel_kind_name(int32_t kind);

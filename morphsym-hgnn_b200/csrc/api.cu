@@ -13,6 +13,7 @@
 #include "kernels_simt.cuh"
 #include "kernels_tc.cuh"
 #include "kernels_enc.cuh"
+#include "kernels_dx.cuh"
 #include "kernels_stack.cuh"
 #include "kernels_stack2.cuh"
 #include "plan.cuh"
@@ -47,12 +48,13 @@ int fail(int code, const char* fmt, ...) {
 
 // ---- per-kernel event profiling ----
 enum Kind : int { K_DERIVE = 0, K_ENC_FWD, K_CONV_FWD, K_MLP_FWD, K_DEC_FWD, K_LOSS, K_DEC_BWD, K_MLP_BWD, K_DX_BWD,
-                  K_DW_LAYER, K_DW_ENC, K_REDUCE, K_OPTIM, K_MEMSET, K_WINDOWS, K_METRICS, K_STACK_FWD, K_STACK_BWD, K_EDGES, K_NKINDS };
+                  K_DW_LAYER, K_DW_ENC, K_REDUCE, K_OPTIM, K_MEMSET, K_WINDOWS, K_METRICS, K_STACK_FWD, K_STACK_BWD, K_EDGES, K_DX_ENC, K_NKINDS };
 static_assert(K_NKINDS == MSHGNN_NUM_KERNEL_KINDS, "kernel kind table out of sync with the header");
+constexpr int K_NKINDS_V1 = 19;      // kinds before dx_encoder: mshgnn_profile_read still accepts n = 19 from callers built against that header
 const char* const kKindNames[MSHGNN_NUM_KERNEL_KINDS] = {
     "derive_weights", "encoder_fwd", "conv_fwd", "base_mlp_fwd", "decoder_fwd", "loss",
     "decoder_bwd", "base_mlp_bwd", "dx_bwd", "dw_layers", "dw_encoder",
-    "reduce_partials", "optimizer", "memset", "window_builder", "step_metrics", "stack_fwd", "stack_bwd", "check_edges"};
+    "reduce_partials", "optimizer", "memset", "window_builder", "step_metrics", "stack_fwd", "stack_bwd", "check_edges", "dx_encoder"};
 struct ProfRec { int kind; cudaEvent_t a, b; };
 std::mutex g_prof_mu;
 bool g_prof_on = false;
@@ -118,6 +120,7 @@ int ensure_uploaded(const Plan& p) {
     if ((rc = upload(p.signs, &p.d_signs))) return rc;
     if ((rc = upload(p.enc_units, &p.d_enc_units))) return rc;
     if ((rc = upload(p.enc_groups, &p.d_enc_groups))) return rc;
+    if ((rc = upload(p.dx_units, &p.d_dx_units))) return rc;
     p.device = dev;
     p.uploaded = true;
     return 0;
@@ -207,7 +210,9 @@ int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, in
 
 // The caller's fp32 feature tensor x[B * nodes, K] of one node type as a (K, nodes, B) tensor, box = 64 columns x 1 node x 128 graphs:
 // one TMA request fetches the 256-byte fragments of a K block of 128 consecutive graphs of one node slot (k_tc_encoder_stream).
-int make_map_x3d(CUtensorMap* m, const void* base, int64_t B, int nodes, int K, int box_rows = 128) {
+// The input gradient (k_tc_encoder_dx) stores through the same view: box 32 columns x 1 x 128 graphs, SWIZZLE_128B.
+int make_map_x3d(CUtensorMap* m, const void* base, int64_t B, int nodes, int K, int box_rows = 128, int box_cols = 64,
+                 CUtensorMapSwizzle sw = CU_TENSOR_MAP_SWIZZLE_NONE) {
     EncodeTiledFn enc;
     int rc = get_encode_fn(&enc);
     if (rc) return rc;
@@ -215,10 +220,10 @@ int make_map_x3d(CUtensorMap* m, const void* base, int64_t B, int nodes, int K, 
     if (!ctx_bound) { CUDA_TRY(cudaFree(0)); ctx_bound = true; }
     cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)nodes, (cuuint64_t)B};
     cuuint64_t strides[2] = {(cuuint64_t)K * 4, (cuuint64_t)nodes * K * 4};
-    cuuint32_t box[3] = {64, 1, (cuuint32_t)box_rows};
+    cuuint32_t box[3] = {(cuuint32_t)box_cols, 1, (cuuint32_t)box_rows};
     cuuint32_t estr[3] = {1, 1, 1};
     CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                     sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(MSHGNN_ERR_CUDA, "cuTensorMapEncodeTiled (features) failed with CUresult %d", (int)r);
     return 0;
 }
@@ -570,6 +575,7 @@ void mshgnn_plan_destroy(mshgnn_plan* plan) {
     if (p.uploaded) {
         cudaFree(p.d_tiles); cudaFree(p.d_stack_items); cudaFree(p.d_edge_tpl); cudaFree(p.d_rtasks); cudaFree(p.d_rpairs);
         cudaFree(p.d_groups); cudaFree(p.d_derive); cudaFree(p.d_derive16); cudaFree(p.d_signs); cudaFree(p.d_enc_units); cudaFree(p.d_enc_groups);
+        cudaFree(p.d_dx_units);
     }
     delete plan;
 }
@@ -763,7 +769,8 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
     const Plan& p = plan->p;
     if (mode != MSHGNN_MODE_FP32 && mode != MSHGNN_MODE_TC && mode != MSHGNN_MODE_TC_1X) return fail(MSHGNN_ERR_ARG, "unknown mode %d", mode);
     if (x_dtype != MSHGNN_F32 && x_dtype != MSHGNN_F64 && x_dtype != MSHGNN_F16) return fail(MSHGNN_ERR_ARG, "x_dtype must be F32, F64 or F16");
-    if (!x || !params || !dout || !grads) return fail(MSHGNN_ERR_ARG, "NULL argument");
+    if (!x || !params || !dout) return fail(MSHGNN_ERR_ARG, "NULL argument");
+    const bool want_dw = grads != nullptr;      // NULL: input-only backward (the dX chain for mshgnn_input_grad, no weight gradient)
     const WsLayout w = ws_layout(p, B, 1, mode);
     int rc = check_common(plan, B, workspace, workspace_bytes, w);
     if (rc) return rc;
@@ -792,7 +799,9 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
     float G = 1.f;
     if (tc) { int e = 0; std::frexp((double)(B * p.dec.n_dec), &e); G = (float)std::ldexp(1.0, e - 1); }
 
-    if (tc && w.stack && (reinterpret_cast<uintptr_t>(grads) & 15) == 0) {
+    if (!want_dw) {
+        if (tc && (rc = stack_sync_reset(w, ws, st))) return rc;
+    } else if (tc && w.stack && (reinterpret_cast<uintptr_t>(grads) & 15) == 0) {
         ProfScope ps(K_MEMSET, st);
         const int64_t n4 = p.n_params / 4;
         k_bwd_prologue<<<296, 256, 0, st>>>((float4*)grads, n4, grads + n4 * 4, (int)(p.n_params - n4 * 4), (uint32_t*)(ws + w.stack_sync), w.stack_sync_bytes / 4);
@@ -821,11 +830,13 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         if (p.dec.C <= 2) MSHGNN_DEC_BWD(2); else if (p.dec.C <= 4) MSHGNN_DEC_BWD(4); else MSHGNN_DEC_BWD(8);
 #undef MSHGNN_DEC_BWD
         LAUNCH_CHECK();
-        k_decoder_bwd_reduce<<<p.dec.C * H + p.dec.C, 256, 0, st>>>(p.dec, dec_part, DEC_BLOCKS, grads, 1.f / G);
-        LAUNCH_CHECK();
+        if (want_dw) {
+            k_decoder_bwd_reduce<<<p.dec.C * H + p.dec.C, 256, 0, st>>>(p.dec, dec_part, DEC_BLOCKS, grads, 1.f / G);
+            LAUNCH_CHECK();
+        }
     }
     auto launch_dw = [&](int kind, const Launch& L) -> int {
-        if (L.count == 0) return 0;
+        if (L.count == 0 || !want_dw) return 0;
         ProfScope ps(kind, st);
         dim3 grid((unsigned)L.count, (unsigned)w.n_splits);
         k_reducegemm<<<grid, 256, 0, st>>>(p.d_rtasks, p.d_rpairs, L.begin, bt, B, w.Bp, xf64, w.n_splits, part_w, part_b);
@@ -836,12 +847,12 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         // the whole dX chain (with the base_transform backward chained on chip) in one launch over per-layer dh / dc / du
         // images, then the weight gradients of every layer (they only read what the chain and the forward pass stored)
         if ((rc = launch_stack(K_STACK_BWD, p, p.stack_bwd, w, bt, br, wm, ws, B, split, st))) return rc;
-        if (w.dw_merged) {
+        if (want_dw && w.dw_merged) {
             // tasks are laid out layer L-1 first, contiguously: one launch covers them all (ws_layout fitted one split count)
             Launch all{p.dw_layer[p.L - 1].begin, 0};
             for (int l = 0; l < p.L; ++l) all.count += p.dw_layer[l].count;
             if ((rc = launch_tc_dw(K_DW_LAYER, p, p.L - 1, all, w, br, wm, B, split, part_w, part_b, st))) return rc;
-        } else {
+        } else if (want_dw) {
             for (int l = p.L - 1; l >= 0; --l)
                 if ((rc = launch_tc_dw(K_DW_LAYER, p, l, p.dw_layer[l], w, br, wm, B, split, part_w, part_b, st))) return rc;
         }
@@ -850,7 +861,7 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         if (tc) {
             if ((rc = launch_tc_rowgemm(K_MLP_BWD, p, p.bwd_m1[l], bt, br, wm, B, w.Bp, split, st))) return rc;
             if ((rc = launch_tc_rowgemm(K_MLP_BWD, p, p.bwd_m2[l], bt, br, wm, B, w.Bp, split, st))) return rc;
-            if ((rc = launch_tc_dw(K_DW_LAYER, p, l, p.dw_layer[l], w, br, wm, B, split, part_w, part_b, st))) return rc;
+            if (want_dw && (rc = launch_tc_dw(K_DW_LAYER, p, l, p.dw_layer[l], w, br, wm, B, split, part_w, part_b, st))) return rc;
             if ((rc = launch_tc_rowgemm(K_DX_BWD, p, p.bwd_dx[l], bt, br, wm, B, w.Bp, split, st))) return rc;
         } else {
             if ((rc = launch_rowgemm(K_MLP_BWD, p, p.bwd_m1[l], bt, B, w.Bp, 0, st))) return rc;
@@ -862,7 +873,7 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
     // layer-stack groups were produced with the split count of the kernel that ran them, encoder groups with the SIMT one
     const int ngl = p.n_groups_layers, nge = (int)p.groups.size() - ngl;
     auto reduce_layers = [&]() -> int {
-        if (ngl > 0) {
+        if (ngl > 0 && want_dw) {
             // 64 blocks per group = one element per thread: the groups of the shared base_transform weights sum up to 16 tasks x
             // 16..64 splits per element, and that serial chain (not the 117 MB of partials) sets the launch time.  (Four lanes per
             // element over the splits of a task, combined through shared memory, was measured: 2x SLOWER - the chain that matters is
@@ -879,7 +890,7 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         // even started: the caller's event lets a data-parallel trainer all-reduce that 7.5 MB segment underneath it.
         if ((rc = reduce_layers())) return rc;
         if (layers_ready_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)layers_ready_event, st));
-        if (!p.enc_units.empty()) {
+        if (!p.enc_units.empty() && want_dw) {
             static std::atomic<bool> attr_set[64];
             if (first_on_device(attr_set)) {
                 CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder_dw<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, EDW_SMEM_BYTES));
@@ -919,7 +930,7 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         }
     } else if ((rc = launch_dw(K_DW_ENC, p.dw_enc))) return rc;
     if (!tc && (rc = reduce_layers())) return rc;
-    if (nge > 0 && !tc) {
+    if (nge > 0 && !tc && want_dw) {
         dim3 grid((unsigned)nge, 32);
         ProfScope ps(K_REDUCE, st);
         k_reduce_partials<<<grid, 256, 0, st>>>(p.d_groups + ngl, part_w, part_b, w.segs, grads, 1.f / G);
@@ -929,7 +940,68 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
     return 0;
 }
 
-int mshgnn_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, int64_t step,
+int mshgnn_input_grad(const mshgnn_plan* plan, int64_t B, const float* params, float* const* dx, void* workspace, int64_t workspace_bytes,
+                      int32_t mode, void* stream) {
+    if (!plan) return fail(MSHGNN_ERR_ARG, "plan is NULL");
+    const Plan& p = plan->p;
+    if (mode != MSHGNN_MODE_FP32 && mode != MSHGNN_MODE_TC && mode != MSHGNN_MODE_TC_1X) return fail(MSHGNN_ERR_ARG, "unknown mode %d", mode);
+    if (!params || !dx) return fail(MSHGNN_ERR_ARG, "NULL argument");
+    if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1 (got %lld)", (long long)B);
+    const WsLayout w = ws_layout(p, B, 1, mode);
+    int rc = check_common(plan, B, workspace, workspace_bytes, w);
+    if (rc) return rc;
+    DxOut o;
+    memset(&o, 0, sizeof o);
+    unsigned n_kb = 1;
+    bool any = false;
+    for (int t = 0; t < p.n_types; ++t) {
+        if (dx[t] && (reinterpret_cast<uintptr_t>(dx[t]) & 3)) return fail(MSHGNN_ERR_ARG, "dx[%d] must be 4-byte aligned", t);
+        o.p[t] = dx[t]; o.nodes[t] = p.nodes[t]; o.w_off[t] = p.off_enc_w[t];
+        n_kb = std::max(n_kb, (unsigned)((p.in_w[t] + 63) / 64));
+        any = any || dx[t];
+    }
+    if (!any) return 0;
+    if ((rc = ensure_uploaded(p))) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    char* ws = (char*)workspace;
+    const unsigned n_units = (unsigned)p.dx_units.size();
+    if (mode == MSHGNN_MODE_FP32) {
+        BufTable bt;
+        fill_bufs(p, w, ws, bt);
+        ProfScope ps(K_DX_ENC, st);
+        k_encoder_dx<<<dim3((unsigned)((B + 15) / 16), n_units, n_kb), 256, 0, st>>>(p.d_dx_units, o, (const float*)bt.p[BUF_DCL0 - 1], params, p.d_signs, B, w.Bp);
+        LAUNCH_CHECK();
+        return 0;
+    }
+    // tensor-core modes: dpre0 as (hi, lo) images, the encoder weight image of the forward prologue (x 2^8), G of the backward
+    static std::atomic<bool> attr_set[64];
+    if (first_on_device(attr_set)) CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder_dx, cudaFuncAttributeMaxDynamicSharedMemorySize, DX_SMEM_BYTES));
+    WsMaps wm;
+    if ((rc = make_ws_maps(&wm, workspace, w))) return rc;
+    BufRows br;
+    fill_rows16(p, w, br);
+    DxMaps maps;
+    maps.a = wm.tc.o;
+    if ((rc = make_map_2d(&maps.w_hi, ws + w.wenc16[0], (int64_t)p.n_types * H, p.enc_kmax, 64, 64, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+    if ((rc = make_map_2d(&maps.w_lo, ws + w.wenc16[1], (int64_t)p.n_types * H, p.enc_kmax, 64, 64, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+    for (int t = 0; t < 4; ++t) {
+        maps.x[t] = wm.tc.o;
+        if (t < p.n_types && dx[t] && enq_rows_ok(dx[t], p.in_w[t], -1)) {
+            if ((rc = make_map_x3d(&maps.x[t], dx[t], B, p.nodes[t], p.in_w[t], 128, 32, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+            o.tma |= 1 << t;
+        }
+    }
+    int e = 0;
+    std::frexp((double)(B * p.dec.n_dec), &e);
+    const float scale = (float)std::ldexp(1.0, -(e - 1)) * TC_W_UNSCALE;      // 1 / (G 2^8)
+    ProfScope ps(K_DX_ENC, st);
+    k_tc_encoder_dx<<<dim3((unsigned)(w.Bp / TILE_M), n_units), DX_THREADS, DX_SMEM_BYTES, st>>>(maps, p.d_dx_units, o, p.d_signs, br.hi[BUF_DC1_ID],
+                                                                                               br.lo[BUF_DC1_ID], B, w.Bp, mode == MSHGNN_MODE_TC, scale);
+    LAUNCH_CHECK();
+    return 0;
+}
+
+int mshgnn_adam_step(float* params,const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, int64_t step,
                      float lr, float beta1, float beta2, float eps, float weight_decay, void* stream) {
     if (!params || !grads || !exp_avg || !exp_avg_sq || n < 1 || step < 1) return fail(MSHGNN_ERR_ARG, "bad argument");
     const float bc1 = 1.f - (float)std::pow((double)beta1, (double)step);
@@ -1047,7 +1119,7 @@ int mshgnn_profile_enable(int32_t on) {
 }
 
 int mshgnn_profile_read(double* ms_out, int64_t* launches_out, int32_t n) {
-    if (!ms_out || !launches_out || n < MSHGNN_NUM_KERNEL_KINDS) return fail(MSHGNN_ERR_ARG, "bad argument");
+    if (!ms_out || !launches_out || n < K_NKINDS_V1) return fail(MSHGNN_ERR_ARG, "bad argument");
     std::vector<ProfRec> recs;
     {
         std::lock_guard<std::mutex> lk(g_prof_mu);
@@ -1058,7 +1130,7 @@ int mshgnn_profile_read(double* ms_out, int64_t* launches_out, int32_t n) {
         CUDA_TRY(cudaEventSynchronize(r.b));
         float ms = 0.f;
         CUDA_TRY(cudaEventElapsedTime(&ms, r.a, r.b));
-        ms_out[r.kind] += ms; launches_out[r.kind] += 1;
+        if (r.kind < n) { ms_out[r.kind] += ms; launches_out[r.kind] += 1; }
     }
     std::lock_guard<std::mutex> lk(g_prof_mu);
     for (auto& r : recs) { g_prof_pool.push_back(r.a); g_prof_pool.push_back(r.b); }

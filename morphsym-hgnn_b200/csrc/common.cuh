@@ -174,6 +174,23 @@ struct EncDwGroup {
     int pad;
 };
 
+// One node slot of the input gradient dx[t][g * nodes + node, :] = sign[slot] * (dpre0[slot][g] W_enc[t]) (k_tc_encoder_dx,
+// k_encoder_dx): every slot of every type has one, in slot order.  A dead slot (need[0][slot] == 0) has no dpre0: its rows are zeros.
+struct DxUnit {
+    int type, slot, node;          // node type, slab slot, local node inside a graph
+    int K, n_kb;                   // in-width of the type, 64-column blocks
+    int sign_off;                  // BUF_SIGNS offset of the [K] +-1 vector or -1
+    int live;                      // need[0][slot]
+    int pad;
+};
+// the caller's input-gradient tensors dx[t] (NULL: type not requested), graph-major like x[t]
+struct DxOut {
+    float* p[4];
+    int nodes[4];
+    int64_t w_off[4];              // flat parameter offset of W_enc[t] (the fp32 kernel)
+    int tma;                       // bit t: dx[t] is stored through a tensor map (16-byte rows, tensor-core kernel)
+};
+
 struct DecoderDesc {
     int n_dec;                        // decoded nodes per graph
     int C;                            // output channels

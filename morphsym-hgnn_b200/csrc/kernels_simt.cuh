@@ -7,6 +7,7 @@
 //                (hgnn_k4.py:L170-186), base_transform, and the dX half of the backward pass.
 //  k_reducegemm: dW[128, K] = sum_pairs dC[rows,128]^T * A[rows, K]  split over row ranges,
 //                + column sums of dC (bias gradients); deterministic two-stage reduction.
+//  k_encoder_dx: dx[rows, K] = sign * (dpre0[rows, 128] W_enc[128, K]): the input gradient (mshgnn_input_grad).
 //  k_decoder_* : Linear(H, C) on the decoded node type + output signs (hgnn_c2.py:L184-189,
 //                hgnn_k4_com.py:L157-165) and its backward.
 //  k_loss_*    : MSE / per-row 2-way CE heads (gnnLightning.py:L124-139, customMetrics.py:L6-25).
@@ -579,6 +580,49 @@ k_decoder_bwd_reduce(const DecoderDesc dd, const float* __restrict__ part, const
     if (threadIdx.x == 0) {
         const float r = sh[0] * scale;
         if (e < dd.C * H) grads[dd.w_off + e] = r; else grads[dd.b_off + (e - dd.C * H)] = r;
+    }
+}
+
+// ------------------------------------------------------------------------------------------
+// input gradient of the encoder (MSHGNN_MODE_FP32, mshgnn_input_grad):
+//   dx[t][g * nodes + n, k] = sign[slot][k] * sum_c dpre0[slot][g][c] * W_enc[t][c, k]        (hgnn_k4.py:L159-160, L198-237)
+// one CTA = 16 graphs x 64 columns of one node slot (blockIdx.y = DxUnit); dead slots write exact zeros and read nothing
+// ------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+k_encoder_dx(const DxUnit* __restrict__ units, const DxOut out, const float* __restrict__ dpre, const float* __restrict__ params,
+             const float* __restrict__ signs, const int64_t B, const int64_t Bp) {
+    __shared__ float D[16][H + 1];
+    __shared__ float W[H][64];
+    const DxUnit u = units[blockIdx.y];
+    float* dx = out.p[u.type];
+    const int64_t g0 = (int64_t)blockIdx.x * 16;
+    const int k0 = blockIdx.z * 64, K = u.K;
+    if (!dx || k0 >= K || g0 >= B) return;
+    const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
+    float acc[4] = {0.f, 0.f, 0.f, 0.f};
+    if (u.live) {
+        const float* dp = dpre + ((int64_t)u.slot * Bp + g0) * H;      // rows up to Bp exist
+        for (int e = tid; e < 16 * H; e += 256) D[e / H][e % H] = dp[e];
+        const float* w = params + out.w_off[u.type];
+        for (int e = tid; e < H * 64; e += 256) {
+            const int c = e / 64, kk = e % 64;
+            W[c][kk] = k0 + kk < K ? w[(int64_t)c * K + k0 + kk] : 0.f;
+        }
+        __syncthreads();
+#pragma unroll 4
+        for (int c = 0; c < H; ++c) {
+            const float d = D[ty][c];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) acc[i] = fmaf(d, W[c][tx + 16 * i], acc[i]);
+        }
+    }
+    const int64_t g = g0 + ty;
+    if (g >= B) return;
+    float* row = dx + (g * out.nodes[u.type] + u.node) * K;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int k = k0 + tx + 16 * i;
+        if (k < K) row[k] = u.live ? (u.sign_off >= 0 ? acc[i] * signs[u.sign_off + k] : acc[i]) : 0.f;
     }
 }
 

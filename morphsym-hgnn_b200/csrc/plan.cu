@@ -621,6 +621,15 @@ std::string build_plan(const mshgnn_desc* d, Plan& p) {
             p.enc_groups.push_back(g);
         }
     }
+    // ---- input-gradient units: one per node slot ----
+    for (int t = 0; t < p.n_types; ++t)
+        for (int n = 0; n < p.nodes[t]; ++n) {
+            const int s = p.slot_of(t, n);
+            DxUnit u{};
+            u.type = t; u.slot = s; u.node = n; u.K = p.in_w[t]; u.n_kb = (p.in_w[t] + 63) / 64;
+            u.sign_off = p.sign_off_slot[s]; u.live = p.need[0][s] ? 1 : 0;
+            p.dx_units.push_back(u);
+        }
     { std::string e = build_stack_programs(p); if (!e.empty()) return e; }
     return "";
 }

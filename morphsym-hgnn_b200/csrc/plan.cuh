@@ -89,6 +89,7 @@ struct Plan {
     std::vector<EncDwUnit> enc_units;
     std::vector<EncDwGroup> enc_groups;
     int n_groups_layers = 0;           // groups [0, n_groups_layers) belong to the layer stack, the rest to the encoder
+    std::vector<DxUnit> dx_units;      // input gradient: one per node slot (mshgnn_input_grad)
     DecoderDesc dec;
 
     // ---- device copies (lazy) ----
@@ -106,6 +107,7 @@ struct Plan {
     mutable float* d_signs = nullptr;
     mutable EncDwUnit* d_enc_units = nullptr;
     mutable EncDwGroup* d_enc_groups = nullptr;
+    mutable DxUnit* d_dx_units = nullptr;
 
     int slot_of(int type, int local) const { return type_base[type] + local; }
 };

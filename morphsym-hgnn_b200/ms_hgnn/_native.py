@@ -30,7 +30,7 @@ EXPORTS = (
     "mshgnn_last_error", "mshgnn_version", "mshgnn_profile_enable", "mshgnn_profile_read", "mshgnn_kernel_kind_name",
     "mshgnn_relu_mask_offset", "mshgnn_build_windows", "mshgnn_step_metrics", "mshgnn_dw_layout",
     "mshgnn_check_edges", "mshgnn_set_option", "mshgnn_get_option", "mshgnn_stack_status", "mshgnn_stack_timing_offset",
-    "mshgnn_backward_staged",
+    "mshgnn_backward_staged", "mshgnn_input_grad",
 )
 
 
@@ -109,6 +109,8 @@ def lib() -> C.CDLL:
     L.mshgnn_loss.argtypes = [vp, i64, i32, vp, vp, i32, f32, vp, vp, vp, i64, vp]; L.mshgnn_loss.restype = C.c_int
     L.mshgnn_backward.argtypes = [vp, i64, C.POINTER(vp), i32, vp, vp, vp, vp, i64, i32, vp]; L.mshgnn_backward.restype = C.c_int
     L.mshgnn_backward_staged.argtypes = [vp, i64, C.POINTER(vp), i32, vp, vp, vp, vp, i64, i32, vp, vp]; L.mshgnn_backward_staged.restype = C.c_int
+    if hasattr(L, "mshgnn_input_grad"):          # absent from builds before it (MSHGNN_LIB A/B runs against an older commit)
+        L.mshgnn_input_grad.argtypes = [vp, i64, vp, C.POINTER(vp), vp, i64, i32, vp]; L.mshgnn_input_grad.restype = C.c_int
     L.mshgnn_adam_step.argtypes = [vp, vp, vp, vp, i64, i64, f32, f32, f32, f32, f32, vp]; L.mshgnn_adam_step.restype = C.c_int
     L.mshgnn_sgd_step.argtypes = [vp, vp, i64, f32, vp]; L.mshgnn_sgd_step.restype = C.c_int
     L.mshgnn_plan_describe.argtypes = [vp, C.c_char_p, i64]; L.mshgnn_plan_describe.restype = i64
@@ -137,7 +139,7 @@ def check(rc: int, what: str) -> None:
         raise RuntimeError(f"{what} failed (code {rc}): {lib().mshgnn_last_error().decode()}")
 
 
-NUM_KERNEL_KINDS = 19
+NUM_KERNEL_KINDS = 20
 
 
 def profile_enable(on: bool) -> None:
@@ -276,9 +278,15 @@ class NativePlan:
                                 ws_ptr, ws_bytes, stream), "mshgnn_loss")
 
     def backward(self, B, x_ptrs, x_dtype, params_ptr, dout_ptr, grads_ptr, ws_ptr, ws_bytes, mode, stream, layers_ready_event=None):
+        """grads_ptr None: input-only backward (dX chain for input_grad, no weight gradient)."""
         arr = (C.c_void_p * len(x_ptrs))(*x_ptrs)
         check(lib().mshgnn_backward_staged(self.handle, B, arr, x_dtype, params_ptr, dout_ptr, grads_ptr, ws_ptr, ws_bytes, mode, stream,
                                            layers_ready_event), "mshgnn_backward")
+
+    def input_grad(self, B, params_ptr, dx_ptrs, ws_ptr, ws_bytes, mode, stream):
+        """d loss / d x[t] into the fp32 buffers dx_ptrs[t] (None: skip type t), after backward on the same workspace."""
+        arr = (C.c_void_p * len(dx_ptrs))(*dx_ptrs)
+        check(lib().mshgnn_input_grad(self.handle, B, params_ptr, arr, ws_ptr, ws_bytes, mode, stream), "mshgnn_input_grad")
 
 
 METRIC_SLOTS, METRIC_SCRATCH = 32, 296 * 32

@@ -156,7 +156,9 @@ class Engine:
         return min(o for (name, o, _) in self.param_layout() if not name.startswith("encoder."))
 
     def backward(self, dout: torch.Tensor, flat_params: torch.Tensor, grads: Optional[torch.Tensor] = None,
-                 layers_ready: Optional[torch.cuda.Event] = None) -> torch.Tensor:
+                 layers_ready: Optional[torch.cuda.Event] = None, param_grads: bool = True) -> Optional[torch.Tensor]:
+        """d loss / d params into ``grads`` (allocated when None) and returned.  ``param_grads=False`` runs the input-only
+        backward of a frozen model: no weight gradient is computed and None is returned; input_grad() may follow."""
         if self._train_ctx is None:
             raise RuntimeError("backward() needs a preceding forward(train=True) on the same engine")
         B, x, xd = self._train_ctx
@@ -166,7 +168,9 @@ class Engine:
             dout = dout.float()
         if dout.numel() != self.plan.out_rows(B) * self.spec["out_channels"]:
             raise ValueError("dout has the wrong number of elements")
-        if grads is None:
+        if not param_grads:
+            grads = None
+        elif grads is None:
             grads = torch.empty(self.n_params, dtype=torch.float32, device=dev)
         ws = self.workspace(B, True, dev)
         stream = torch.cuda.current_stream(dev).cuda_stream
@@ -175,7 +179,23 @@ class Engine:
                 # torch creates the CUDA event lazily at its first record(): make sure the handle exists
                 if layers_ready.cuda_event == 0:
                     layers_ready.record(torch.cuda.current_stream(dev))
-            self.plan.backward(B, [t.data_ptr() for t in x], xd, flat_params.data_ptr(), dout.data_ptr(), grads.data_ptr(),
+            self.plan.backward(B, [t.data_ptr() for t in x], xd, flat_params.data_ptr(), dout.data_ptr(),
+                               grads.data_ptr() if grads is not None else None,
                                ws.data_ptr(), ws.numel(), self.mode, stream,
                                layers_ready.cuda_event if layers_ready is not None else None)
         return grads
+
+    def input_grad(self, which: Sequence[bool], flat_params: torch.Tensor) -> List[Optional[torch.Tensor]]:
+        """d loss / d x[t] (fp32, the shape of x[t]) for every node type t with which[t] true, None for the others.  Runs after
+        backward() of the last train-mode forward, on the same workspace."""
+        if self._train_ctx is None:
+            raise RuntimeError("input_grad() needs a preceding forward(train=True) and backward() on the same engine")
+        B, x, _ = self._train_ctx
+        dev = x[0].device
+        out = [torch.empty(t.shape, dtype=torch.float32, device=dev) if w else None for t, w in zip(x, which)]
+        ws = self.workspace(B, True, dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        with torch.cuda.device(dev):
+            self.plan.input_grad(B, flat_params.data_ptr(), [t.data_ptr() if t is not None else None for t in out], ws.data_ptr(),
+                                 ws.numel(), self.mode, stream)
+        return out

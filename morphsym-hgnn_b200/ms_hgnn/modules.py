@@ -106,6 +106,7 @@ class _HGNNFn(torch.autograd.Function):
         out = engine.forward(x, model._flat, train=True)
         ctx.model, ctx.engine = model, engine
         ctx.n_x = n_x
+        ctx.x_dtype = x[0].dtype
         ctx.token = model._fwd_token = object()
         return out
 
@@ -115,9 +116,17 @@ class _HGNNFn(torch.autograd.Function):
         if model._fwd_token is not ctx.token:
             raise RuntimeError("the native workspace was overwritten by a later forward(); "
                                "call backward() before the next training forward of this model")
-        g = engine.backward(dout, model._flat)
-        grads = [g[o:o + n].view(s) for (o, n, s) in model._views]
-        return (None, None, None) + (None,) * ctx.n_x + tuple(grads)
+        n_x = ctx.n_x
+        want_x = list(ctx.needs_input_grad[3:3 + n_x])
+        # a frozen model runs the input-only backward; without input gradients the launches are those of a plain training step
+        want_p = any(ctx.needs_input_grad[3 + n_x:]) or not any(want_x)
+        g = engine.backward(dout, model._flat, param_grads=want_p)
+        grads = [g[o:o + n].view(s) for (o, n, s) in model._views] if want_p else [None] * len(model._views)
+        dx = [None] * n_x
+        if any(want_x):
+            dx = engine.input_grad(want_x, model._flat)
+            dx = [d if (d is None or d.dtype == ctx.x_dtype) else d.to(ctx.x_dtype) for d in dx]
+        return (None, None, None) + tuple(dx) + tuple(grads)
 
 
 class NativeHGNN(nn.Module):
@@ -411,7 +420,7 @@ class NativeHGNN(nn.Module):
         self._last_engine = eng
         self._ensure_flat(x0.device)
         xs = [x_dict[t] for t in self.node_types]          # never mutated (the reference mutates its input dict)
-        need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in self._flat_params)
+        need_grad = torch.is_grad_enabled() and (any(p.requires_grad for p in self._flat_params) or any(t.requires_grad for t in xs))
         if need_grad:
             out = _HGNNFn.apply(self, eng, len(xs), *xs, *self._flat_params)
         else:
