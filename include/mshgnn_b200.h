@@ -78,7 +78,7 @@ typedef struct mshgnn_desc {
     int32_t edge_count[MSHGNN_MAX_EDGE_TYPES];           /* edges per graph                                  */
     const int32_t* edge_src[MSHGNN_MAX_EDGE_TYPES];      /* per-graph local source node index, [edge_count]  */
     const int32_t* edge_dst[MSHGNN_MAX_EDGE_TYPES];      /* per-graph local destination node index           */
-    int32_t hidden;                                      /* H; this build supports 128                       */
+    int32_t hidden;                                      /* H: 128; 1..128 with MSHGNN_PLAN_PAD_HIDDEN       */
     int32_t num_layers;                                  /* L >= 1                                           */
     int32_t morph_sym;                                   /* 1: MS-HGNN (shared base MLP + residual), 0: MI-HGNN (ReLU only) */
     int32_t mlp_type;                                    /* node type that goes through base_transform (morph_sym only) */
@@ -89,12 +89,21 @@ typedef struct mshgnn_desc {
 } mshgnn_desc;
 
 /* ---- plan ------------------------------------------------------------------------- */
+/* The kernels are 128 channels wide: mshgnn_plan_create takes hidden == 128 only. */
 int  mshgnn_plan_create(const mshgnn_desc* desc, mshgnn_plan** plan_out);
+/* flags = 0: the same as mshgnn_plan_create.  MSHGNN_PLAN_PAD_HIDDEN: hidden may be 1..128.  Such a model runs on the
+ * 128-wide kernels as the model whose weights are its zero-padded copy, and gives bit for bit that model's outputs, loss,
+ * input gradients and (the matching sub-blocks of its) parameter gradients.  params / grads stay in the model's own layout
+ * ([H, in], [H], [H, H], [C, H] tensors, reported by mshgnn_param_count / mshgnn_param_offset).  For hidden < 128 every
+ * forward first copies params into a 128-wide internal buffer in the workspace, and the backward copies the gradients back
+ * out of another one: mshgnn_workspace_bytes includes both.  hidden == 128 with the flag is exactly mshgnn_plan_create. */
+#define MSHGNN_PLAN_PAD_HIDDEN 1
+int  mshgnn_plan_create_ex(const mshgnn_desc* desc, int32_t flags, mshgnn_plan** plan_out);
 void mshgnn_plan_destroy(mshgnn_plan* plan);
 
 /* number of fp32 elements of the flat parameter (and gradient) buffer */
 int64_t mshgnn_param_count(const mshgnn_plan* plan);
-/* offset/numel of one parameter tensor inside the flat buffer */
+/* offset/numel of one parameter tensor inside the flat buffer (at the model's hidden width) */
 int  mshgnn_param_offset(const mshgnn_plan* plan, int32_t kind, int32_t layer, int32_t idx,
                          int64_t* offset_out, int64_t* numel_out);
 
@@ -126,6 +135,7 @@ int mshgnn_loss(const mshgnn_plan* plan, int64_t B, int32_t loss_kind,
 
 /* Backward of mshgnn_forward(train=1) on the same workspace: writes d(loss)/d(params)
  * (every element, zeros for structurally dead branches) into grads[param_count].
+ * A padded plan (hidden < 128) reads the parameters that forward copied into the workspace, not `params`.
  * grads == NULL runs the input-only backward of a frozen model: the decoder backward and the dX chain through the
  * layers (everything mshgnn_input_grad reads), without any weight-gradient launch or partial reduction.
  * Replaces: torch autograd through PyG (SURVEY 3.1 "loss.backward()"). */
@@ -221,7 +231,7 @@ int64_t mshgnn_plan_describe(const mshgnn_plan* plan, char* buf, int64_t cap);
  * stream it is launched on.  mshgnn_profile_read synchronises those events, adds the elapsed
  * milliseconds and launch counts per kernel kind into ms_out / launches_out (n entries each, n >= 19: the first n
  * kinds) and clears the record.  Used by bench.py for the roofline figures. */
-#define MSHGNN_NUM_KERNEL_KINDS 20     /* n = 19 (the kinds before "dx_encoder") is accepted too */
+#define MSHGNN_NUM_KERNEL_KINDS 21     /* n = 19 and 20 (the kinds before "dx_encoder" / "pad_params") are accepted too */
 int mshgnn_profile_enable(int32_t on);
 int mshgnn_profile_read(double* ms_out, int64_t* launches_out, int32_t n);
 const char* mshgnn_kernel_kind_name(int32_t kind);
@@ -231,7 +241,8 @@ const char* mshgnn_kernel_kind_name(int32_t kind);
  * layer = -1: encoder output; layer = l (0..L-1): slots [0, S) = ReLU of the HeteroConv output of node slot s
  * (hgnn_k4.py:L175-186), slots [S, S + n_mlp) = hidden ReLU of base_transform (hgnn_k4.py:L133-137) of MLP-type node n.
  * Layout at workspace + *byte_off: uint32 [n_slots][*rows_padded][4]; bit (c % 32) of word (c / 32) <=> pre-activation
- * of hidden channel c > 0.  Slots whose value cannot reach the output are never written. */
+ * of hidden channel c > 0.  Slots whose value cannot reach the output are never written.  Rows are 128 bits whatever the
+ * plan's hidden width: bits c >= hidden of a padded plan are always 0. */
 int mshgnn_relu_mask_offset(const mshgnn_plan* plan, int64_t B, int32_t mode, int32_t layer,
                             int64_t* byte_off, int64_t* n_slots, int64_t* rows_padded);
 

@@ -16,6 +16,7 @@
 #include "kernels_dx.cuh"
 #include "kernels_stack.cuh"
 #include "kernels_stack2.cuh"
+#include "kernels_pad.cuh"
 #include "plan.cuh"
 #include "windows.cuh"
 #include "metrics.cuh"
@@ -48,13 +49,13 @@ int fail(int code, const char* fmt, ...) {
 
 // ---- per-kernel event profiling ----
 enum Kind : int { K_DERIVE = 0, K_ENC_FWD, K_CONV_FWD, K_MLP_FWD, K_DEC_FWD, K_LOSS, K_DEC_BWD, K_MLP_BWD, K_DX_BWD,
-                  K_DW_LAYER, K_DW_ENC, K_REDUCE, K_OPTIM, K_MEMSET, K_WINDOWS, K_METRICS, K_STACK_FWD, K_STACK_BWD, K_EDGES, K_DX_ENC, K_NKINDS };
+                  K_DW_LAYER, K_DW_ENC, K_REDUCE, K_OPTIM, K_MEMSET, K_WINDOWS, K_METRICS, K_STACK_FWD, K_STACK_BWD, K_EDGES, K_DX_ENC, K_PAD, K_NKINDS };
 static_assert(K_NKINDS == MSHGNN_NUM_KERNEL_KINDS, "kernel kind table out of sync with the header");
-constexpr int K_NKINDS_V1 = 19;      // kinds before dx_encoder: mshgnn_profile_read still accepts n = 19 from callers built against that header
+constexpr int K_NKINDS_V1 = 19;      // kinds before dx_encoder: mshgnn_profile_read still accepts n = 19 (and 20) from callers built against older headers
 const char* const kKindNames[MSHGNN_NUM_KERNEL_KINDS] = {
     "derive_weights", "encoder_fwd", "conv_fwd", "base_mlp_fwd", "decoder_fwd", "loss",
     "decoder_bwd", "base_mlp_bwd", "dx_bwd", "dw_layers", "dw_encoder",
-    "reduce_partials", "optimizer", "memset", "window_builder", "step_metrics", "stack_fwd", "stack_bwd", "check_edges", "dx_encoder"};
+    "reduce_partials", "optimizer", "memset", "window_builder", "step_metrics", "stack_fwd", "stack_bwd", "check_edges", "dx_encoder", "pad_params"};
 struct ProfRec { int kind; cudaEvent_t a, b; };
 std::mutex g_prof_mu;
 bool g_prof_on = false;
@@ -121,6 +122,7 @@ int ensure_uploaded(const Plan& p) {
     if ((rc = upload(p.enc_units, &p.d_enc_units))) return rc;
     if ((rc = upload(p.enc_groups, &p.d_enc_groups))) return rc;
     if ((rc = upload(p.dx_units, &p.d_dx_units))) return rc;
+    if ((rc = upload(p.pad_segs, &p.d_pad_segs))) return rc;
     p.device = dev;
     p.uploaded = true;
     return 0;
@@ -545,6 +547,15 @@ int launch_stack(int kind, const Plan& p, const Plan::Stack& sp, const WsLayout&
     return 0;
 }
 
+// padded plans: caller's gradients of the tensors segs [first, first + count) from the internal 128-wide gradient buffer
+int compact_grads(const Plan& p, int first, int count, const float* in, float* ext, cudaStream_t st) {
+    if (count == 0) return 0;
+    ProfScope ps(K_PAD, st);
+    k_compact_grads<<<dim3(PAD_BLOCKS_X, (unsigned)count), 256, 0, st>>>(p.d_pad_segs + first, in, ext);
+    LAUNCH_CHECK();
+    return 0;
+}
+
 int check_common(const mshgnn_plan* plan, int64_t B, const void* ws, int64_t ws_bytes, const WsLayout& w) {
     if (!plan) return fail(MSHGNN_ERR_ARG, "plan is NULL");
     if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1 (got %lld)", (long long)B);
@@ -558,16 +569,18 @@ int check_common(const mshgnn_plan* plan, int64_t B, const void* ws, int64_t ws_
 
 extern "C" {
 
-int mshgnn_plan_create(const mshgnn_desc* desc, mshgnn_plan** plan_out) {
+int mshgnn_plan_create_ex(const mshgnn_desc* desc, int32_t flags, mshgnn_plan** plan_out) {
     if (!plan_out) return fail(MSHGNN_ERR_ARG, "plan_out is NULL");
     *plan_out = nullptr;
     mshgnn_plan* pl = new (std::nothrow) mshgnn_plan();
     if (!pl) return fail(MSHGNN_ERR_ARG, "out of host memory");
-    std::string e = build_plan(desc, pl->p);
+    std::string e = build_plan(desc, flags, pl->p);
     if (!e.empty()) { delete pl; return fail(MSHGNN_ERR_ARG, "%s", e.c_str()); }
     *plan_out = pl;
     return 0;
 }
+
+int mshgnn_plan_create(const mshgnn_desc* desc, mshgnn_plan** plan_out) { return mshgnn_plan_create_ex(desc, 0, plan_out); }
 
 void mshgnn_plan_destroy(mshgnn_plan* plan) {
     if (!plan) return;
@@ -575,27 +588,29 @@ void mshgnn_plan_destroy(mshgnn_plan* plan) {
     if (p.uploaded) {
         cudaFree(p.d_tiles); cudaFree(p.d_stack_items); cudaFree(p.d_edge_tpl); cudaFree(p.d_rtasks); cudaFree(p.d_rpairs);
         cudaFree(p.d_groups); cudaFree(p.d_derive); cudaFree(p.d_derive16); cudaFree(p.d_signs); cudaFree(p.d_enc_units); cudaFree(p.d_enc_groups);
-        cudaFree(p.d_dx_units);
+        cudaFree(p.d_dx_units); cudaFree(p.d_pad_segs);
     }
     delete plan;
 }
 
-int64_t mshgnn_param_count(const mshgnn_plan* plan) { return plan ? plan->p.n_params : -1; }
+int64_t mshgnn_param_count(const mshgnn_plan* plan) { return plan ? plan->p.ext.n : -1; }
 
 int mshgnn_param_offset(const mshgnn_plan* plan, int32_t kind, int32_t layer, int32_t idx, int64_t* off, int64_t* numel) {
     if (!plan || !off || !numel) return fail(MSHGNN_ERR_ARG, "NULL argument");
     const Plan& p = plan->p;
+    const ParamLayout& y = p.ext;      // the caller's layout, at the model's width h
+    const int64_t h = p.hidden;
     auto lay_ok = [&]() { return layer >= 0 && layer < p.L && idx >= 0 && idx < p.n_etypes; };
     switch (kind) {
-        case MSHGNN_P_ENC_W: if (idx < 0 || idx >= p.n_types) break; *off = p.off_enc_w[idx]; *numel = (int64_t)H * p.in_w[idx]; return 0;
-        case MSHGNN_P_ENC_B: if (idx < 0 || idx >= p.n_types) break; *off = p.off_enc_b[idx]; *numel = H; return 0;
-        case MSHGNN_P_REL_W: if (!lay_ok()) break; *off = p.off_rel_w[layer * p.n_etypes + idx]; *numel = H * H; return 0;
-        case MSHGNN_P_REL_B: if (!lay_ok()) break; *off = p.off_rel_b[layer * p.n_etypes + idx]; *numel = H; return 0;
-        case MSHGNN_P_ROOT_W: if (!lay_ok()) break; *off = p.off_root_w[layer * p.n_etypes + idx]; *numel = H * H; return 0;
-        case MSHGNN_P_MLP_W: if (!p.morph_sym || idx < 0 || idx > 1) break; *off = p.off_mlp_w[idx]; *numel = H * H; return 0;
-        case MSHGNN_P_MLP_B: if (!p.morph_sym || idx < 0 || idx > 1) break; *off = p.off_mlp_b[idx]; *numel = H; return 0;
-        case MSHGNN_P_DEC_W: *off = p.off_dec_w; *numel = (int64_t)p.C * H; return 0;
-        case MSHGNN_P_DEC_B: *off = p.off_dec_b; *numel = p.C; return 0;
+        case MSHGNN_P_ENC_W: if (idx < 0 || idx >= p.n_types) break; *off = y.enc_w[idx]; *numel = h * p.in_w[idx]; return 0;
+        case MSHGNN_P_ENC_B: if (idx < 0 || idx >= p.n_types) break; *off = y.enc_b[idx]; *numel = h; return 0;
+        case MSHGNN_P_REL_W: if (!lay_ok()) break; *off = y.rel_w[layer * p.n_etypes + idx]; *numel = h * h; return 0;
+        case MSHGNN_P_REL_B: if (!lay_ok()) break; *off = y.rel_b[layer * p.n_etypes + idx]; *numel = h; return 0;
+        case MSHGNN_P_ROOT_W: if (!lay_ok()) break; *off = y.root_w[layer * p.n_etypes + idx]; *numel = h * h; return 0;
+        case MSHGNN_P_MLP_W: if (!p.morph_sym || idx < 0 || idx > 1) break; *off = y.mlp_w[idx]; *numel = h * h; return 0;
+        case MSHGNN_P_MLP_B: if (!p.morph_sym || idx < 0 || idx > 1) break; *off = y.mlp_b[idx]; *numel = h; return 0;
+        case MSHGNN_P_DEC_W: *off = y.dec_w; *numel = p.C * h; return 0;
+        case MSHGNN_P_DEC_B: *off = y.dec_b; *numel = p.C; return 0;
         default: break;
     }
     return fail(MSHGNN_ERR_ARG, "no such parameter (kind=%d layer=%d idx=%d)", kind, layer, idx);
@@ -655,6 +670,13 @@ int mshgnn_forward(const mshgnn_plan* plan, int64_t B, const void* const* x, int
         if (!x[t]) return fail(MSHGNN_ERR_ARG, "x[%d] is NULL", t);
     if ((rc = ensure_uploaded(p))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
+    if (p.padded) {     // every kernel below reads the 128-wide zero-padded copy
+        float* in = (float*)((char*)workspace + w.pad_params);
+        ProfScope ps(K_PAD, st);
+        k_pad_params<<<dim3(PAD_BLOCKS_X, (unsigned)p.pad_segs.size()), 256, 0, st>>>(p.d_pad_segs, params, in);
+        LAUNCH_CHECK();
+        params = in;
+    }
     BufTable bt;
     fill_bufs(p, w, (char*)workspace, bt);
     bt.p[BUF_PARAMS] = (void*)params;
@@ -776,6 +798,11 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
     if (rc) return rc;
     if ((rc = ensure_uploaded(p))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
+    float* const grads_out = grads;
+    if (p.padded) {     // the forward's 128-wide parameter copy; gradients go to the 128-wide buffer, then compacted into grads_out
+        params = (const float*)((char*)workspace + w.pad_params);
+        if (grads) grads = (float*)((char*)workspace + w.pad_grads);
+    }
     BufTable bt;
     fill_bufs(p, w, (char*)workspace, bt);
     bt.p[BUF_PARAMS] = (void*)params;
@@ -889,6 +916,7 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         // Every gradient outside the encoder is final here - before the encoder weight gradient, the last 8 % of the step, has
         // even started: the caller's event lets a data-parallel trainer all-reduce that 7.5 MB segment underneath it.
         if ((rc = reduce_layers())) return rc;
+        if (p.padded && want_dw && (rc = compact_grads(p, p.n_pad_enc, (int)p.pad_segs.size() - p.n_pad_enc, grads, grads_out, st))) return rc;
         if (layers_ready_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)layers_ready_event, st));
         if (!p.enc_units.empty() && want_dw) {
             static std::atomic<bool> attr_set[64];
@@ -928,6 +956,7 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
                 LAUNCH_CHECK();
             }
         }
+        if (p.padded && want_dw && (rc = compact_grads(p, 0, p.n_pad_enc, grads, grads_out, st))) return rc;
     } else if ((rc = launch_dw(K_DW_ENC, p.dw_enc))) return rc;
     if (!tc && (rc = reduce_layers())) return rc;
     if (nge > 0 && !tc && want_dw) {
@@ -936,6 +965,7 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         k_reduce_partials<<<grid, 256, 0, st>>>(p.d_groups + ngl, part_w, part_b, w.segs, grads, 1.f / G);
         LAUNCH_CHECK();
     }
+    if (!tc && p.padded && want_dw && (rc = compact_grads(p, 0, (int)p.pad_segs.size(), grads, grads_out, st))) return rc;
     if (!tc && layers_ready_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)layers_ready_event, st));
     return 0;
 }
@@ -966,6 +996,7 @@ int mshgnn_input_grad(const mshgnn_plan* plan, int64_t B, const float* params, f
     char* ws = (char*)workspace;
     const unsigned n_units = (unsigned)p.dx_units.size();
     if (mode == MSHGNN_MODE_FP32) {
+        if (p.padded) params = (const float*)(ws + w.pad_params);      // the forward's 128-wide copy (o.w_off is in that layout)
         BufTable bt;
         fill_bufs(p, w, ws, bt);
         ProfScope ps(K_DX_ENC, st);

@@ -191,6 +191,14 @@ struct DxOut {
     int tma;                       // bit t: dx[t] is stored through a tensor map (16-byte rows, tensor-core kernel)
 };
 
+// One parameter tensor of a padded plan (kernels_pad.cuh): [rows, cols] row-major at ext_off of the caller's flat buffer
+// (the model's own width) is the top-left block of [rows_i, cols_i] at int_off of the 128-wide internal buffer; the rest
+// of the internal tensor is zero.
+struct PadSeg {
+    int64_t ext_off, int_off;
+    int rows, cols, rows_i, cols_i;
+};
+
 struct DecoderDesc {
     int n_dec;                        // decoded nodes per graph
     int C;                            // output channels

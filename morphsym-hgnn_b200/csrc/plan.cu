@@ -239,10 +239,35 @@ static std::string build_stack_programs(Plan& p) {
     return "";
 }
 
-std::string build_plan(const mshgnn_desc* d, Plan& p) {
+// Offsets of every parameter tensor at hidden width `h` (reference named_parameters() order).
+static ParamLayout param_layout(const Plan& p, int64_t h) {
+    ParamLayout y;
+    int64_t o = 0;
+    for (int t = 0; t < p.n_types; ++t) { y.enc_w[t] = o; o += h * p.in_w[t]; y.enc_b[t] = o; o += h; }
+    y.rel_w.assign(p.L * p.n_etypes, 0); y.rel_b = y.rel_w; y.root_w = y.rel_w;
+    for (int l = 0; l < p.L; ++l)
+        for (int e = 0; e < p.n_etypes; ++e) {
+            const int i = l * p.n_etypes + e;
+            y.rel_w[i] = o; o += h * h; y.rel_b[i] = o; o += h; y.root_w[i] = o; o += h * h;
+        }
+    if (p.morph_sym)
+        for (int i = 0; i < 2; ++i) { y.mlp_w[i] = o; o += h * h; y.mlp_b[i] = o; o += h; }
+    y.dec_w = o; o += p.C * h; y.dec_b = o; o += p.C;
+    y.n = o;
+    return y;
+}
+
+std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p) {
     char err[256];
     if (!d) return "desc is NULL";
-    if (d->hidden != H) { snprintf(err, sizeof err, "hidden=%d unsupported: this build is specialised for H=128", d->hidden); return err; }
+    if (flags & ~MSHGNN_PLAN_PAD_HIDDEN) { snprintf(err, sizeof err, "unknown plan flags 0x%x", (unsigned)flags); return err; }
+    if (!(flags & MSHGNN_PLAN_PAD_HIDDEN) && d->hidden != H) {
+        snprintf(err, sizeof err, "hidden=%d unsupported: this build is specialised for H=128 (MSHGNN_PLAN_PAD_HIDDEN runs 1..128)", d->hidden);
+        return err;
+    }
+    if (d->hidden < 1 || d->hidden > H) { snprintf(err, sizeof err, "hidden=%d unsupported: padded plans take 1..128 hidden channels", d->hidden); return err; }
+    p.hidden = d->hidden;
+    p.padded = p.hidden != H;
     if (d->n_node_types < 1 || d->n_node_types > MSHGNN_MAX_NODE_TYPES) return "n_node_types out of range";
     if (d->n_edge_types < 1 || d->n_edge_types > MSHGNN_MAX_EDGE_TYPES) return "n_edge_types out of range";
     if (d->num_layers < 1 || d->num_layers > MAX_LAYERS) return "num_layers out of range (1..15)";
@@ -291,19 +316,35 @@ std::string build_plan(const mshgnn_desc* d, Plan& p) {
         if (!has_in[t]) return "every node type must be the destination of at least one edge type";
 
     // ---------------- parameter layout: reference named_parameters() order ----------------
-    int64_t o = 0;
-    for (int t = 0; t < p.n_types; ++t) { p.off_enc_w[t] = o; o += (int64_t)H * p.in_w[t]; p.off_enc_b[t] = o; o += H; }
-    p.off_rel_w.assign(p.L * p.n_etypes, 0); p.off_rel_b = p.off_rel_w; p.off_root_w = p.off_rel_w;
-    for (int l = 0; l < p.L; ++l)
-        for (int e = 0; e < p.n_etypes; ++e) {
-            const int i = l * p.n_etypes + e;
-            p.off_rel_w[i] = o; o += H * H; p.off_rel_b[i] = o; o += H; p.off_root_w[i] = o; o += H * H;
+    {
+        const ParamLayout in = param_layout(p, H);
+        for (int t = 0; t < p.n_types; ++t) { p.off_enc_w[t] = in.enc_w[t]; p.off_enc_b[t] = in.enc_b[t]; }
+        p.off_rel_w = in.rel_w; p.off_rel_b = in.rel_b; p.off_root_w = in.root_w;
+        for (int i = 0; i < 2; ++i) { p.off_mlp_w[i] = in.mlp_w[i]; p.off_mlp_b[i] = in.mlp_b[i]; }
+        p.off_dec_w = in.dec_w; p.off_dec_b = in.dec_b;
+        p.n_params = in.n;
+        if (in.n > (int64_t)1 << 30) return "parameter count too large";
+        p.ext = p.padded ? param_layout(p, p.hidden) : in;
+    }
+    if (p.padded) {
+        // the caller's [h, in], [h], [h, h], [C, h] tensors are the top-left blocks of the 128-wide ones
+        const int h = p.hidden;
+        auto seg = [&](int64_t e, int64_t i, int rows, int cols, int rows_i, int cols_i) { p.pad_segs.push_back(PadSeg{e, i, rows, cols, rows_i, cols_i}); };
+        for (int t = 0; t < p.n_types; ++t) {
+            seg(p.ext.enc_w[t], p.off_enc_w[t], h, p.in_w[t], H, p.in_w[t]);
+            seg(p.ext.enc_b[t], p.off_enc_b[t], 1, h, 1, H);
         }
-    if (p.morph_sym)
-        for (int i = 0; i < 2; ++i) { p.off_mlp_w[i] = o; o += H * H; p.off_mlp_b[i] = o; o += H; }
-    p.off_dec_w = o; o += (int64_t)p.C * H; p.off_dec_b = o; o += p.C;
-    p.n_params = o;
-    if (o > (int64_t)1 << 30) return "parameter count too large";
+        p.n_pad_enc = (int)p.pad_segs.size();
+        for (int i = 0; i < p.L * p.n_etypes; ++i) {
+            seg(p.ext.rel_w[i], p.off_rel_w[i], h, h, H, H);
+            seg(p.ext.rel_b[i], p.off_rel_b[i], 1, h, 1, H);
+            seg(p.ext.root_w[i], p.off_root_w[i], h, h, H, H);
+        }
+        if (p.morph_sym)
+            for (int i = 0; i < 2; ++i) { seg(p.ext.mlp_w[i], p.off_mlp_w[i], h, h, H, H); seg(p.ext.mlp_b[i], p.off_mlp_b[i], 1, h, 1, H); }
+        seg(p.ext.dec_w, p.off_dec_w, p.C, h, p.C, H);
+        seg(p.ext.dec_b, p.off_dec_b, 1, p.C, 1, p.C);
+    }
 
     // ---------------- derived weights ----------------
     int64_t q = 0;
@@ -846,14 +887,18 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode) {
         w.stack_sync = take(w.stack_sync_bytes);
         w.stack_timing = take(256 * 16 * 8);
     }
-    w.loss_part = take(LOSS_BLOCKS * 8);
+    if (p.padded) {
+        w.pad_params = take(p.n_params * 4);
+        if (train) w.pad_grads = take(p.n_params * 4);
+    }
+    w.loss_part = take(LOSS_BLOCKS * 8);      // last: mshgnn_loss finds its partials at the end of the caller's workspace
     w.total = o;
     return w;
 }
 
 std::string describe_plan(const Plan& p) {
     std::ostringstream os;
-    os << "{\"S\":" << p.S << ",\"L\":" << p.L << ",\"n_params\":" << p.n_params << ",\"n_derived\":" << p.n_derived
+    os << "{\"S\":" << p.S << ",\"L\":" << p.L << ",\"hidden\":" << p.hidden << ",\"kernel_hidden\":" << H << ",\"n_params\":" << p.ext.n << ",\"n_derived\":" << p.n_derived
        << ",\"n_tiles\":" << p.tiles.size() << ",\"n_rtasks\":" << p.rtasks.size() << ",\"n_rpairs\":" << p.rpairs.size()
        << ",\"n_groups\":" << p.groups.size() << ",\"need\":[";
     for (int l = 0; l <= p.L; ++l) {

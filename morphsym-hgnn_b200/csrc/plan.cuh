@@ -31,9 +31,26 @@ static_assert(BUF_DCL0 - 1 == 80, "kernels_tc.cuh BUF_DC1_ID names the encoder d
 
 struct Launch { int begin = 0, count = 0; };
 
+// flat parameter layout at one hidden width, reference named_parameters() order
+struct ParamLayout {
+    int64_t n = 0;
+    int64_t enc_w[MSHGNN_MAX_NODE_TYPES] = {0}, enc_b[MSHGNN_MAX_NODE_TYPES] = {0};
+    std::vector<int64_t> rel_w, rel_b, root_w;   // [l * n_etypes + e]
+    int64_t mlp_w[2] = {-1, -1}, mlp_b[2] = {-1, -1};
+    int64_t dec_w = 0, dec_b = 0;
+};
+
 struct Plan {
     // ---- description (deep copy) ----
     int n_types = 0, n_etypes = 0, L = 0, morph_sym = 0, mlp_type = -1, dec_type = 0, C = 0;
+    // Hidden width of the model.  The kernels are H = 128 wide: a padded plan (hidden < H, MSHGNN_PLAN_PAD_HIDDEN) runs the
+    // model as the 128-wide one whose weights are its zero-padded copy.  Every table below except `ext` refers to that
+    // 128-wide internal layout; the caller's params / grads are in `ext`, copied by k_pad_params / k_compact_grads.
+    int hidden = H;
+    bool padded = false;
+    ParamLayout ext;
+    std::vector<PadSeg> pad_segs;      // one per parameter tensor, in flat order
+    int n_pad_enc = 0;                 // segments [0, n_pad_enc) are the encoder block
     int nodes[MSHGNN_MAX_NODE_TYPES] = {0}, in_w[MSHGNN_MAX_NODE_TYPES] = {0};
     int e_src_t[MSHGNN_MAX_EDGE_TYPES] = {0}, e_dst_t[MSHGNN_MAX_EDGE_TYPES] = {0}, e_mean[MSHGNN_MAX_EDGE_TYPES] = {0};
     std::vector<int> e_src[MSHGNN_MAX_EDGE_TYPES], e_dst[MSHGNN_MAX_EDGE_TYPES];
@@ -44,7 +61,7 @@ struct Plan {
     std::vector<int> slot_type, slot_local;
     int nm = 0;                        // nodes of the MLP type
 
-    // ---- flat parameter layout (reference named_parameters order) ----
+    // ---- flat parameter layout of the kernels (reference named_parameters order, 128 wide) ----
     int64_t n_params = 0;
     int64_t off_enc_w[MSHGNN_MAX_NODE_TYPES], off_enc_b[MSHGNN_MAX_NODE_TYPES];
     std::vector<int64_t> off_rel_w, off_rel_b, off_root_w;   // [l * n_etypes + e]
@@ -108,6 +125,7 @@ struct Plan {
     mutable EncDwUnit* d_enc_units = nullptr;
     mutable EncDwGroup* d_enc_groups = nullptr;
     mutable DxUnit* d_dx_units = nullptr;
+    mutable PadSeg* d_pad_segs = nullptr;
 
     int slot_of(int type, int local) const { return type_base[type] + local; }
 };
@@ -141,13 +159,14 @@ struct WsLayout {
     int64_t stack_sync = -1;           // dependency counters of the stack kernel (uint32 [phases][row tiles]) + error word
     int64_t stack_sync_bytes = 0;
     int64_t stack_timing = -1;         // diagnostic cycle counters of the TIMING instantiation: [CTA][8] uint64
+    int64_t pad_params = -1, pad_grads = -1;   // padded plans: 128-wide fp32 parameters (every call) / gradients (training)
     int64_t total = 0;
 };
 
 constexpr int DEC_BLOCKS = 1184;     // 148 SMs x 8 resident CTAs of the 2-channel instantiation (48 registers, 8 KB of shared memory; the 8-channel one: 2 per SM): one load in flight per warp, so latency is hidden by warps
 constexpr int LOSS_BLOCKS = 592;
 
-std::string build_plan(const mshgnn_desc* d, Plan& p);            // returns error text ("" = ok)
+std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p);   // returns error text ("" = ok)
 WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode);
 bool stack_enabled();                 // cross-layer stack kernel on (default) / off (MSHGNN_STACK=0 or mshgnn_set_option)
 void set_stack_enabled(int on);

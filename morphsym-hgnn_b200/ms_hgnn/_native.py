@@ -19,6 +19,7 @@ MAX_EDGE_TYPES = 16
 
 F32, F64, I64, F16 = 0, 1, 2, 3
 MODE_FP32, MODE_TC, MODE_TC_1X = 0, 1, 2
+PLAN_PAD_HIDDEN = 1
 LOSS_MSE, LOSS_CE2 = 0, 1
 P_ENC_W, P_ENC_B, P_REL_W, P_REL_B, P_ROOT_W, P_MLP_W, P_MLP_B, P_DEC_W, P_DEC_B = range(9)
 
@@ -30,7 +31,7 @@ EXPORTS = (
     "mshgnn_last_error", "mshgnn_version", "mshgnn_profile_enable", "mshgnn_profile_read", "mshgnn_kernel_kind_name",
     "mshgnn_relu_mask_offset", "mshgnn_build_windows", "mshgnn_step_metrics", "mshgnn_dw_layout",
     "mshgnn_check_edges", "mshgnn_set_option", "mshgnn_get_option", "mshgnn_stack_status", "mshgnn_stack_timing_offset",
-    "mshgnn_backward_staged", "mshgnn_input_grad",
+    "mshgnn_backward_staged", "mshgnn_input_grad", "mshgnn_plan_create_ex",
 )
 
 
@@ -99,6 +100,8 @@ def lib() -> C.CDLL:
     L = C.CDLL(path)
     vp, i32, i64, f32 = C.c_void_p, C.c_int32, C.c_int64, C.c_float
     L.mshgnn_plan_create.argtypes = [C.POINTER(Desc), C.POINTER(vp)]; L.mshgnn_plan_create.restype = C.c_int
+    if hasattr(L, "mshgnn_plan_create_ex"):      # absent from builds before it (MSHGNN_LIB A/B runs against an older commit)
+        L.mshgnn_plan_create_ex.argtypes = [C.POINTER(Desc), i32, C.POINTER(vp)]; L.mshgnn_plan_create_ex.restype = C.c_int
     L.mshgnn_plan_destroy.argtypes = [vp]; L.mshgnn_plan_destroy.restype = None
     L.mshgnn_param_count.argtypes = [vp]; L.mshgnn_param_count.restype = i64
     L.mshgnn_param_offset.argtypes = [vp, i32, i32, i32, C.POINTER(i64), C.POINTER(i64)]; L.mshgnn_param_offset.restype = C.c_int
@@ -139,7 +142,7 @@ def check(rc: int, what: str) -> None:
         raise RuntimeError(f"{what} failed (code {rc}): {lib().mshgnn_last_error().decode()}")
 
 
-NUM_KERNEL_KINDS = 20
+NUM_KERNEL_KINDS = 21
 
 
 def profile_enable(on: bool) -> None:
@@ -174,7 +177,8 @@ def get_option(name: str) -> int:
 
 
 class NativePlan:
-    """Owns a mshgnn_plan*.  ``spec`` is a plain dict (see engine.build_spec)."""
+    """Owns a mshgnn_plan*.  ``spec`` is a plain dict (see engine.build_spec); ``spec["pad_hidden"]`` true creates the plan
+    with MSHGNN_PLAN_PAD_HIDDEN (hidden 1..128, run zero-padded on the 128-wide kernels)."""
 
     def __init__(self, spec: dict):
         L = lib()
@@ -205,7 +209,10 @@ class NativePlan:
             self._keep.append(arr)
             d.out_sign = C.cast(arr, C.POINTER(C.c_float))
         h = C.c_void_p()
-        check(L.mshgnn_plan_create(C.byref(d), C.byref(h)), "mshgnn_plan_create")
+        if spec.get("pad_hidden") and hasattr(L, "mshgnn_plan_create_ex"):     # older builds (MSHGNN_LIB): 128 wide only
+            check(L.mshgnn_plan_create_ex(C.byref(d), PLAN_PAD_HIDDEN, C.byref(h)), "mshgnn_plan_create_ex")
+        else:
+            check(L.mshgnn_plan_create(C.byref(d), C.byref(h)), "mshgnn_plan_create")
         self.handle = h
         self.spec = spec
         self.n_params = int(L.mshgnn_param_count(h))

@@ -19,9 +19,11 @@ def build_spec(node_types: Sequence[str], nodes_per_graph: Dict[str, int], in_wi
                edge_types: Sequence[EdgeType], edges: Dict[EdgeType, Tuple[List[int], List[int]]],
                mean_relations: Sequence[str], hidden: int, num_layers: int, morph_sym: bool, mlp_type: Optional[str],
                decode_type: str, out_channels: int, in_sign: Dict[str, Optional[List[float]]],
-               out_sign: Optional[List[float]]) -> dict:
+               out_sign: Optional[List[float]], pad_hidden: bool = False) -> dict:
+    """Plain-dict model description for NativePlan.  ``pad_hidden``: accept hidden widths 1..128 (the model runs zero-padded
+    on the 128-wide kernels; parameters and gradients stay in its own layout)."""
     ti = {t: i for i, t in enumerate(node_types)}
-    return {
+    spec = {
         "node_types": list(node_types),
         "edge_types": [tuple(e) for e in edge_types],
         "nodes_per_graph": [int(nodes_per_graph[t]) for t in node_types],
@@ -33,6 +35,9 @@ def build_spec(node_types: Sequence[str], nodes_per_graph: Dict[str, int], in_wi
         "decode_type": ti[decode_type], "out_channels": out_channels,
         "in_sign": [in_sign.get(t) for t in node_types], "out_sign": out_sign,
     }
+    if pad_hidden:
+        spec["pad_hidden"] = True
+    return spec
 
 
 def _dtype_code(t: torch.Tensor) -> int:

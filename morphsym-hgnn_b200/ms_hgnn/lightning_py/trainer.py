@@ -156,9 +156,9 @@ def train_model(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dat
     model_type = fmts[0]
     if model_type not in _HGNN_FORMATS:
         raise ValueError("Invalid model type.")
-    if hidden_size != 128:
-        # the signature keeps the reference's default (10); the native plan is compiled for 128 hidden channels only
-        raise ValueError(f"hidden_size={hidden_size}: the B200-native path supports hidden_size=128 only (pass hidden_size=128)")
+    if not 1 <= hidden_size <= 128:
+        # narrower models run zero-padded on the 128-channel kernels; wider ones have no kernels
+        raise ValueError(f"hidden_size={hidden_size}: the B200-native path supports hidden_size 1..128")
     if devices != 1:
         raise ValueError("train_model drives one GPU; launch one process per GPU and pass a process group to FusedTrainer for data parallelism")
     data_metadata = train_dataset.dataset.get_data_metadata()

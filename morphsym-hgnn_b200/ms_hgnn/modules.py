@@ -401,7 +401,7 @@ class NativeHGNN(nn.Module):
         if eng is None:
             spec = build_spec(self.node_types, npg, in_dims, self.edge_types, edges, self.mean_relations,
                               self.hidden_channels, self.num_layers, self.morph_sym, "base" if self.morph_sym else None,
-                              self.decode_node, self._out_channels, self._in_sign(in_dims), self._out_sign())
+                              self.decode_node, self._out_channels, self._in_sign(in_dims), self._out_sign(), pad_hidden=True)
             eng = Engine(spec, self.mode)
             eng._edges = edges
             eng._npg = npg
