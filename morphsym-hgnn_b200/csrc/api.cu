@@ -88,10 +88,11 @@ struct ProfScope {
     } while (0)
 
 template <typename T>
-int upload(const std::vector<T>& v, T** d) {
+int upload(const Plan& p, const std::vector<T>& v, T** d) {
     *d = nullptr;
     if (v.empty()) return 0;
     CUDA_TRY(cudaMalloc((void**)d, v.size() * sizeof(T)));
+    p.d_allocs.push_back(*d);
     CUDA_TRY(cudaMemcpy(*d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
     return 0;
 }
@@ -105,67 +106,50 @@ int ensure_uploaded(const Plan& p) {
         return 0;
     }
     int rc;
-    if ((rc = upload(p.tiles, &p.d_tiles))) return rc;
-    if ((rc = upload(p.stack_items, &p.d_stack_items))) return rc;
+    if ((rc = upload(p, p.tiles, &p.d_tiles))) return rc;
+    if ((rc = upload(p, p.stack_items, &p.d_stack_items))) return rc;
     {
         std::vector<int> tpl;
         for (int e = 0; e < p.n_etypes; ++e) { tpl.insert(tpl.end(), p.e_src[e].begin(), p.e_src[e].end()); tpl.insert(tpl.end(), p.e_dst[e].begin(), p.e_dst[e].end()); }
         if (tpl.empty()) tpl.push_back(0);
-        if ((rc = upload(tpl, &p.d_edge_tpl))) return rc;
+        if ((rc = upload(p, tpl, &p.d_edge_tpl))) return rc;
     }
-    if ((rc = upload(p.rtasks, &p.d_rtasks))) return rc;
-    if ((rc = upload(p.rpairs, &p.d_rpairs))) return rc;
-    if ((rc = upload(p.groups, &p.d_groups))) return rc;
-    if ((rc = upload(p.derive_ops, &p.d_derive))) return rc;
-    if ((rc = upload(p.derive16_ops, &p.d_derive16))) return rc;
-    if ((rc = upload(p.signs, &p.d_signs))) return rc;
-    if ((rc = upload(p.enc_units, &p.d_enc_units))) return rc;
-    if ((rc = upload(p.enc_groups, &p.d_enc_groups))) return rc;
-    if ((rc = upload(p.dx_units, &p.d_dx_units))) return rc;
-    if ((rc = upload(p.pad_segs, &p.d_pad_segs))) return rc;
+    if ((rc = upload(p, p.rtasks, &p.d_rtasks))) return rc;
+    if ((rc = upload(p, p.rpairs, &p.d_rpairs))) return rc;
+    if ((rc = upload(p, p.groups, &p.d_groups))) return rc;
+    if ((rc = upload(p, p.derive_ops, &p.d_derive))) return rc;
+    if ((rc = upload(p, p.derive16_ops, &p.d_derive16))) return rc;
+    if ((rc = upload(p, p.signs, &p.d_signs))) return rc;
+    if ((rc = upload(p, p.enc_units, &p.d_enc_units))) return rc;
+    if ((rc = upload(p, p.enc_groups, &p.d_enc_groups))) return rc;
+    if ((rc = upload(p, p.dx_units, &p.d_dx_units))) return rc;
+    if ((rc = upload(p, p.pad_segs, &p.d_pad_segs))) return rc;
     p.device = dev;
     p.uploaded = true;
     return 0;
 }
 
+// device pointers of the workspace buffers (ws_layout placed them); params, grads and the feature tensors are the caller's
 void fill_bufs(const Plan& p, const WsLayout& w, char* ws, BufTable& bt) {
-    memset(&bt, 0, sizeof bt);
-    bt.p[BUF_DERIVED] = ws + w.derived;
+    for (int id = 0; id < MAX_BUFS; ++id) bt.p[id] = w.buf[id] < 0 ? nullptr : ws + w.buf[id];
     bt.p[BUF_SIGNS] = p.d_signs;
-    auto at = [&](int64_t off) -> void* { return off < 0 ? nullptr : (void*)(ws + off); };
-    // per-layer backward ids alias the two ping-pong slabs (fp32 SIMT mode; the tensor-core modes carry fp16 images only)
-    for (int l = 0; l <= p.L; ++l) bt.p[BUF_DHL0 + l] = at(w.dh[l & 1]);
-    for (int l = -1; l < p.L; ++l) bt.p[BUF_DCL0 + l] = at(w.dc[(l + 2) & 1]);
-    for (int l = 0; l < p.L; ++l) bt.p[BUF_DUL0 + l] = at(w.du);
-    bt.p[BUF_MASKE] = at(w.maske);
-    for (int l = 0; l <= p.L; ++l) bt.p[BUF_H0 + l] = at(w.h[l]);
-    for (int l = 0; l < p.L; ++l) { bt.p[BUF_CT0 + l] = at(w.ct[l]); bt.p[BUF_MASK0 + l] = at(w.mask[l]); }
 }
 
-void fill_bufs16(const Plan& p, const WsLayout& w, char* ws, BufTable16& bh) {
-    memset(&bh, 0, sizeof bh);
-    auto at = [&](int64_t off) -> __half* { return off < 0 ? nullptr : (__half*)(ws + off); };
-    for (int l = 0; l <= p.L; ++l) {
-        bh.hi[BUF_DHL0 + l] = at(w.stack ? w.dhL16[l][0] : w.dh16[l & 1][0]); bh.lo[BUF_DHL0 + l] = at(w.stack ? w.dhL16[l][1] : w.dh16[l & 1][1]);
-    }
-    for (int l = -1; l < p.L; ++l) {
-        bh.hi[BUF_DCL0 + l] = at(w.stack ? w.dcL16[l + 1][0] : w.dc16[(l + 2) & 1][0]); bh.lo[BUF_DCL0 + l] = at(w.stack ? w.dcL16[l + 1][1] : w.dc16[(l + 2) & 1][1]);
-    }
-    for (int l = 0; l < p.L; ++l) {
-        bh.hi[BUF_DUL0 + l] = at(w.stack ? w.duL16[l][0] : w.du16[0]); bh.lo[BUF_DUL0 + l] = at(w.stack ? w.duL16[l][1] : w.du16[1]);
-    }
-    for (int l = 0; l <= p.L; ++l) { bh.hi[BUF_H0 + l] = at(w.h16[l][0]); bh.lo[BUF_H0 + l] = at(w.h16[l][1]); }
-    for (int l = 0; l < p.L; ++l) { bh.hi[BUF_CT0 + l] = at(w.ct16[l][0]); bh.lo[BUF_CT0 + l] = at(w.ct16[l][1]); }
+// first 256-byte row of every fp16 image relative to the workspace base (one TMA map then covers all of them)
+void fill_rows16(const WsLayout& w, BufRows& br) {
+    auto row = [](int64_t off) { return off < 0 ? 0 : (int)(off / 256); };
+    for (int id = 0; id < MAX_BUFS; ++id) { br.hi[id] = row(w.buf16[id][0]); br.lo[id] = row(w.buf16[id][1]); }
+    br.w_hi = row(w.w16[0]); br.w_lo = row(w.w16[1]);
 }
 
-int launch_rowgemm(int kind, const Plan& p, const Launch& L, const BufTable& bt, int64_t B, int64_t Bp, int x_f64, cudaStream_t st,
-                   const BufTable16* bh = nullptr) {
+// image i (0 = hi, 1 = lo) of a buffer id, NULL when the layout has none
+__half* image16(char* ws, const WsLayout& w, int id, int i) { return w.buf16[id][i] < 0 ? nullptr : (__half*)(ws + w.buf16[id][i]); }
+
+int launch_rowgemm(int kind, const Plan& p, const Launch& L, const BufTable& bt, int64_t B, int64_t Bp, int x_f64, cudaStream_t st) {
     if (L.count == 0) return 0;
     ProfScope ps(kind, st);
     dim3 grid((unsigned)(Bp / TILE_M), (unsigned)L.count);
-    BufTable16 none;
-    if (!bh) memset(&none, 0, sizeof none);
-    k_rowgemm<<<grid, 256, 0, st>>>(p.d_tiles + L.begin, bt, B, Bp, x_f64, bh ? *bh : none, bh ? 1 : 0);
+    k_rowgemm<<<grid, 256, 0, st>>>(p.d_tiles + L.begin, bt, B, Bp, x_f64);
     LAUNCH_CHECK();
     return 0;
 }
@@ -175,39 +159,37 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-int get_encode_fn(EncodeTiledFn* out) {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
+// cuTensorMapEncodeTiled with unit element strides; `what` names the tensor in the error text
+int encode_map(CUtensorMap* m, CUtensorMapDataType type, cuuint32_t rank, const void* base, const cuuint64_t* dims, const cuuint64_t* strides,
+               const cuuint32_t* box, CUtensorMapSwizzle sw, const char* what) {
+    static EncodeTiledFn enc = nullptr;
+    if (!enc) {
         void* ptr = nullptr;
         cudaDriverEntryPointQueryResult qres;
         CUDA_TRY(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres));
         if (qres != cudaDriverEntryPointSuccess || !ptr) return fail(MSHGNN_ERR_CUDA, "cuTensorMapEncodeTiled is not available in this driver");
-        fn = (EncodeTiledFn)ptr;
+        enc = (EncodeTiledFn)ptr;
     }
-    *out = fn;
-    return 0;
-}
-
-// [rows, cols] fp16 row-major tensor viewed through a (box_cols x box_rows) box with the given swizzle
-int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int box_cols, int box_rows, CUtensorMapSwizzle sw) {
-    EncodeTiledFn enc;
-    int rc = get_encode_fn(&enc);
-    if (rc) return rc;
     // cuTensorMapEncodeTiled is a driver call and needs a context current on THIS thread.  The runtime binds the primary
     // context lazily: a thread that has not yet made a context-binding runtime call - PyTorch's autograd worker when the
     // caching allocator serves every allocation of its first backward from cached blocks - fails here with
     // CUDA_ERROR_INVALID_CONTEXT (201).  cudaFree(0) binds it; once per thread.
     static thread_local bool ctx_bound = false;
     if (!ctx_bound) { CUDA_TRY(cudaFree(0)); ctx_bound = true; }
-    if (!base || rows < 1) return fail(MSHGNN_ERR_ARG, "internal: bad fp16 tensor for a TMA map");
-    cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)cols * 2};
-    cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    const cuuint32_t estr[3] = {1, 1, 1};
+    CUresult r = enc(m, type, rank, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(MSHGNN_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
+    if (r != CUDA_SUCCESS) return fail(MSHGNN_ERR_CUDA, "cuTensorMapEncodeTiled%s failed with CUresult %d", what, (int)r);
     return 0;
+}
+
+// [rows, cols] fp16 row-major tensor viewed through a (box_cols x box_rows) box with the given swizzle
+int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int box_cols, int box_rows, CUtensorMapSwizzle sw) {
+    if (!base || rows < 1) return fail(MSHGNN_ERR_ARG, "internal: bad fp16 tensor for a TMA map");
+    const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+    const cuuint64_t strides[1] = {(cuuint64_t)cols * 2};
+    const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+    return encode_map(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, base, dims, strides, box, sw, "");
 }
 
 // The caller's fp32 feature tensor x[B * nodes, K] of one node type as a (K, nodes, B) tensor, box = 64 columns x 1 node x 128 graphs:
@@ -215,19 +197,10 @@ int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, in
 // The input gradient (k_tc_encoder_dx) stores through the same view: box 32 columns x 1 x 128 graphs, SWIZZLE_128B.
 int make_map_x3d(CUtensorMap* m, const void* base, int64_t B, int nodes, int K, int box_rows = 128, int box_cols = 64,
                  CUtensorMapSwizzle sw = CU_TENSOR_MAP_SWIZZLE_NONE) {
-    EncodeTiledFn enc;
-    int rc = get_encode_fn(&enc);
-    if (rc) return rc;
-    static thread_local bool ctx_bound = false;
-    if (!ctx_bound) { CUDA_TRY(cudaFree(0)); ctx_bound = true; }
-    cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)nodes, (cuuint64_t)B};
-    cuuint64_t strides[2] = {(cuuint64_t)K * 4, (cuuint64_t)nodes * K * 4};
-    cuuint32_t box[3] = {(cuuint32_t)box_cols, 1, (cuuint32_t)box_rows};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(MSHGNN_ERR_CUDA, "cuTensorMapEncodeTiled (features) failed with CUresult %d", (int)r);
-    return 0;
+    const cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)nodes, (cuuint64_t)B};
+    const cuuint64_t strides[2] = {(cuuint64_t)K * 4, (cuuint64_t)nodes * K * 4};
+    const cuuint32_t box[3] = {(cuuint32_t)box_cols, 1, (cuuint32_t)box_rows};
+    return encode_map(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, base, dims, strides, box, sw, " (features)");
 }
 
 // The whole workspace as one [total/256 rows][128 fp16] tensor: every (hi, lo) image of every buffer (and the 128x128
@@ -369,24 +342,6 @@ int launch_tc_rowgemm(int kind, const Plan& p, const Launch& L, const BufTable& 
     }
     LAUNCH_CHECK();
     return 0;
-}
-
-// first 256-byte row of every fp16 image relative to the workspace base (one TMA map then covers all of them)
-void fill_rows16(const Plan& p, const WsLayout& w, BufRows& br) {
-    for (int i = 0; i < MAX_BUFS; ++i) br.hi[i] = br.lo[i] = 0;
-    auto at = [&](int64_t off) -> int { return off < 0 ? 0 : (int)(off / 256); };
-    for (int l = 0; l <= p.L; ++l) {
-        br.hi[BUF_DHL0 + l] = at(w.stack ? w.dhL16[l][0] : w.dh16[l & 1][0]); br.lo[BUF_DHL0 + l] = at(w.stack ? w.dhL16[l][1] : w.dh16[l & 1][1]);
-    }
-    for (int l = -1; l < p.L; ++l) {
-        br.hi[BUF_DCL0 + l] = at(w.stack ? w.dcL16[l + 1][0] : w.dc16[(l + 2) & 1][0]); br.lo[BUF_DCL0 + l] = at(w.stack ? w.dcL16[l + 1][1] : w.dc16[(l + 2) & 1][1]);
-    }
-    for (int l = 0; l < p.L; ++l) {
-        br.hi[BUF_DUL0 + l] = at(w.stack ? w.duL16[l][0] : w.du16[0]); br.lo[BUF_DUL0 + l] = at(w.stack ? w.duL16[l][1] : w.du16[1]);
-    }
-    for (int l = 0; l <= p.L; ++l) { br.hi[BUF_H0 + l] = at(w.h16[l][0]); br.lo[BUF_H0 + l] = at(w.h16[l][1]); }
-    for (int l = 0; l < p.L; ++l) { br.hi[BUF_CT0 + l] = at(w.ct16[l][0]); br.lo[BUF_CT0 + l] = at(w.ct16[l][1]); }
-    br.w_hi = at(w.w16[0]); br.w_lo = at(w.w16[1]);
 }
 
 int launch_tc_dw(int kind, const Plan& p, int layer, const Launch& L, const WsLayout& w, const BufRows& br, const WsMaps& wm, int64_t B, int split,
@@ -556,12 +511,116 @@ int compact_grads(const Plan& p, int first, int count, const float* in, float* e
     return 0;
 }
 
-int check_common(const mshgnn_plan* plan, int64_t B, const void* ws, int64_t ws_bytes, const WsLayout& w) {
+// Tensor-core modes carry every backward quantity multiplied by a power of two G ~ #output rows so that the fp16 (hi, lo)
+// images of dL/dh stay in the normal range; the weight-gradient reductions and the input gradient multiply by 1/G (exact).
+float grad_scale(const Plan& p, int64_t B) {
+    int e = 0;
+    std::frexp((double)(B * p.dec.n_dec), &e);
+    return (float)std::ldexp(1.0, e - 1);
+}
+
+int check_plan_mode(const mshgnn_plan* plan, int32_t mode) {
     if (!plan) return fail(MSHGNN_ERR_ARG, "plan is NULL");
-    if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1 (got %lld)", (long long)B);
+    if (mode != MSHGNN_MODE_FP32 && mode != MSHGNN_MODE_TC && mode != MSHGNN_MODE_TC_1X) return fail(MSHGNN_ERR_ARG, "unknown mode %d", mode);
+    return 0;
+}
+
+// What forward, backward and input_grad share for one call on a workspace.  open_call checks the workspace and lays it out;
+// bind_call, after the entry point's own checks, uploads the plan and resolves every buffer the kernels address.
+struct Call {
+    const Plan* p = nullptr;
+    WsLayout w;
+    char* ws = nullptr;
+    bool tc = false;
+    int split = 0;                     // MSHGNN_MODE_TC: (hi, lo) products; MSHGNN_MODE_TC_1X: hi products only
+    float G = 1.f;                     // grad_scale in the tensor-core modes
+    const float* params = nullptr;     // the kernels' parameters and gradients: a padded plan's 128-wide workspace buffers
+    float* grads = nullptr;
+    BufTable bt;
+    BufRows br;
+    WsMaps wm;                         // tensor-core modes
+};
+
+int open_call(Call& c, const mshgnn_plan* plan, int64_t B, int train, int32_t mode, void* ws, int64_t ws_bytes) {
+    if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1 (got %lld)", (long long)B);      // before ws_layout, which needs B >= 1
+    const Plan& p = plan->p;
+    c.p = &p;
+    c.w = ws_layout(p, B, train, mode);
     if (!ws) return fail(MSHGNN_ERR_ARG, "workspace is NULL");
-    if (ws_bytes < w.total) return fail(MSHGNN_ERR_WORKSPACE, "workspace too small: %lld < %lld bytes", (long long)ws_bytes, (long long)w.total);
+    if (ws_bytes < c.w.total) return fail(MSHGNN_ERR_WORKSPACE, "workspace too small: %lld < %lld bytes", (long long)ws_bytes, (long long)c.w.total);
     if (reinterpret_cast<uintptr_t>(ws) & 255) return fail(MSHGNN_ERR_ARG, "workspace must be 256-byte aligned");
+    c.ws = (char*)ws;
+    c.tc = mode != MSHGNN_MODE_FP32;
+    c.split = mode == MSHGNN_MODE_TC;
+    c.G = c.tc ? grad_scale(p, B) : 1.f;
+    return 0;
+}
+
+// x: the caller's feature tensors (NULL: the call reads none)
+int bind_call(Call& c, const float* params, float* grads, const void* const* x) {
+    const Plan& p = *c.p;
+    int rc;
+    if ((rc = ensure_uploaded(p))) return rc;
+    if (p.padded) {     // the forward's 128-wide zero-padded parameter copy; gradients go to the 128-wide buffer, then compacted
+        params = (const float*)(c.ws + c.w.pad_params);
+        if (grads) grads = (float*)(c.ws + c.w.pad_grads);
+    }
+    c.params = params;
+    c.grads = grads;
+    fill_bufs(p, c.w, c.ws, c.bt);
+    c.bt.p[BUF_PARAMS] = (void*)params;
+    c.bt.p[BUF_GRADS] = grads;
+    for (int t = 0; x && t < p.n_types; ++t) {
+        if (!x[t]) return fail(MSHGNN_ERR_ARG, "x[%d] is NULL", t);
+        c.bt.p[BUF_X0 + t] = (void*)x[t];
+    }
+    fill_rows16(c.w, c.br);
+    if (c.tc && (rc = make_ws_maps(&c.wm, c.ws, c.w))) return rc;
+    return 0;
+}
+
+// tensor-core encoder weight gradient: split partials of every unit, then their reduction into the gradient buffer
+int launch_tc_encoder_dw(const Call& c, int64_t B, int xf64, cudaStream_t st) {
+    const Plan& p = *c.p;
+    const WsLayout& w = c.w;
+    const BufTable& bt = c.bt;
+    static std::atomic<bool> attr_set[64];
+    if (first_on_device(attr_set)) {
+        CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder_dw<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, EDW_SMEM_BYTES));
+        CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder_dw<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, EDW_SMEM_BYTES));
+    }
+    // x rows by TMA (raw fp32 into the X operand area, converted in place) when every feature tensor allows it: fp32, 16-byte rows
+    // (measured, same box: 0.258-0.270 ms against 0.246-0.251 ms for the register-staged loaders - here the loads of a step are issued
+    // BEFORE its stage is free and nothing is pipelined across register sets, so the scoreboard effect of kernels_enc.cuh costs
+    // little, while a landing zone inside the stage serialises copy -> conversion -> MMA per stage.  Off unless MSHGNN_ENC_DW=tma.)
+    static const bool want_xt = [] { const char* e = getenv("MSHGNN_ENC_DW"); return e && !strcmp(e, "tma"); }();
+    bool xt = xf64 == 0 && (g_encoder_dw_tma.load() >= 0 ? g_encoder_dw_tma.load() != 0 : want_xt);
+    for (const EncDwUnit& eu : p.enc_units)
+        if (xt) xt = eu.x_buf >= BUF_X0 && eu.x_buf < BUF_X0 + p.n_types && enq_rows_ok(bt.p[eu.x_buf], eu.K, 0);
+    EncXMaps xm;
+    int rc;
+    for (int t = 0; t < 4; ++t) {
+        if (xt && t < p.n_types && p.in_w[t] % 4 == 0 && (reinterpret_cast<uintptr_t>(bt.p[BUF_X0 + t]) & 15) == 0) {
+            if ((rc = make_map_x3d(&xm.x[t], bt.p[BUF_X0 + t], B, p.nodes[t], p.in_w[t], 64))) return rc;
+        } else xm.x[t] = c.wm.dw;
+    }
+    float* pe_w = (float*)(c.ws + w.part_enc_w);
+    float* pe_b = (float*)(c.ws + w.part_enc_b);
+    {
+        ProfScope ps(K_DW_ENC, st);
+        dim3 grid((unsigned)p.enc_units.size(), (unsigned)w.n_splits_enc);
+        if (xt) k_tc_encoder_dw<true><<<grid, ENC_THREADS, EDW_SMEM_BYTES, st>>>(c.wm.dw, xm, (int)BUF_X0, p.d_enc_units, bt, c.br, B, w.Bp, w.rows_per_enc, w.n_splits_enc, xf64,
+                                                                                 c.split, pe_w, pe_b);
+        else k_tc_encoder_dw<false><<<grid, ENC_THREADS, EDW_SMEM_BYTES, st>>>(c.wm.dw, xm, (int)BUF_X0, p.d_enc_units, bt, c.br, B, w.Bp, w.rows_per_enc, w.n_splits_enc, xf64,
+                                                                               c.split, pe_w, pe_b);
+        LAUNCH_CHECK();
+    }
+    {
+        ProfScope ps(K_REDUCE, st);
+        dim3 grid((unsigned)p.enc_groups.size(), 48);
+        k_reduce_enc<<<grid, 256, 0, st>>>(p.d_enc_groups, pe_w, pe_b, w.n_splits_enc, c.grads, 1.f / c.G);
+        LAUNCH_CHECK();
+    }
     return 0;
 }
 
@@ -585,11 +644,7 @@ int mshgnn_plan_create(const mshgnn_desc* desc, mshgnn_plan** plan_out) { return
 void mshgnn_plan_destroy(mshgnn_plan* plan) {
     if (!plan) return;
     Plan& p = plan->p;
-    if (p.uploaded) {
-        cudaFree(p.d_tiles); cudaFree(p.d_stack_items); cudaFree(p.d_edge_tpl); cudaFree(p.d_rtasks); cudaFree(p.d_rpairs);
-        cudaFree(p.d_groups); cudaFree(p.d_derive); cudaFree(p.d_derive16); cudaFree(p.d_signs); cudaFree(p.d_enc_units); cudaFree(p.d_enc_groups);
-        cudaFree(p.d_dx_units); cudaFree(p.d_pad_segs);
-    }
+    for (void* d : p.d_allocs) cudaFree(d);
     delete plan;
 }
 
@@ -658,41 +713,37 @@ int64_t mshgnn_plan_describe(const mshgnn_plan* plan, char* buf, int64_t cap) {
 
 int mshgnn_forward(const mshgnn_plan* plan, int64_t B, const void* const* x, int32_t x_dtype, const float* params,
                    float* out, void* workspace, int64_t workspace_bytes, int32_t train, int32_t mode, void* stream) {
-    if (!plan) return fail(MSHGNN_ERR_ARG, "plan is NULL");
+    int rc;
+    if ((rc = check_plan_mode(plan, mode))) return rc;
     const Plan& p = plan->p;
-    if (mode != MSHGNN_MODE_FP32 && mode != MSHGNN_MODE_TC && mode != MSHGNN_MODE_TC_1X) return fail(MSHGNN_ERR_ARG, "unknown mode %d", mode);
     if (x_dtype != MSHGNN_F32 && x_dtype != MSHGNN_F64 && x_dtype != MSHGNN_F16) return fail(MSHGNN_ERR_ARG, "x_dtype must be F32, F64 or F16");
     if (!x || !params || !out) return fail(MSHGNN_ERR_ARG, "NULL argument");
-    const WsLayout w = ws_layout(p, B, train, mode);
-    int rc = check_common(plan, B, workspace, workspace_bytes, w);
-    if (rc) return rc;
-    for (int t = 0; t < p.n_types; ++t)
+    Call c;
+    if ((rc = open_call(c, plan, B, train, mode, workspace, workspace_bytes))) return rc;
+    for (int t = 0; t < p.n_types; ++t)      // before the device is touched
         if (!x[t]) return fail(MSHGNN_ERR_ARG, "x[%d] is NULL", t);
-    if ((rc = ensure_uploaded(p))) return rc;
+    if ((rc = bind_call(c, params, nullptr, x))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
+    const WsLayout& w = c.w;
+    const BufTable& bt = c.bt;
     if (p.padded) {     // every kernel below reads the 128-wide zero-padded copy
-        float* in = (float*)((char*)workspace + w.pad_params);
         ProfScope ps(K_PAD, st);
-        k_pad_params<<<dim3(PAD_BLOCKS_X, (unsigned)p.pad_segs.size()), 256, 0, st>>>(p.d_pad_segs, params, in);
+        k_pad_params<<<dim3(PAD_BLOCKS_X, (unsigned)p.pad_segs.size()), 256, 0, st>>>(p.d_pad_segs, params, (float*)c.params);
         LAUNCH_CHECK();
-        params = in;
     }
-    BufTable bt;
-    fill_bufs(p, w, (char*)workspace, bt);
-    bt.p[BUF_PARAMS] = (void*)params;
-    for (int t = 0; t < p.n_types; ++t) bt.p[BUF_X0 + t] = (void*)x[t];
+    params = c.params;
     const int xf64 = x_dtype == MSHGNN_F64 ? 1 : (x_dtype == MSHGNN_F16 ? 2 : 0);      // element-type code of the kernels (ld_x)
 
-    if (mode == MSHGNN_MODE_FP32) {   // derived weights (transposes, root sums, bias sums) from the current parameters
-        ProfScope ps(K_DERIVE, st);
-        const unsigned n_ops = (unsigned)p.derive_ops.size();
-        if (n_ops > 0) {
-            dim3 grid(16, n_ops);
-            k_derive<<<grid, 256, 0, st>>>(p.d_derive, params, (float*)bt.p[BUF_DERIVED]);
-            LAUNCH_CHECK();
+    if (!c.tc) {
+        {   // derived weights (transposes, root sums, bias sums) from the current parameters
+            ProfScope ps(K_DERIVE, st);
+            const unsigned n_ops = (unsigned)p.derive_ops.size();
+            if (n_ops > 0) {
+                dim3 grid(16, n_ops);
+                k_derive<<<grid, 256, 0, st>>>(p.d_derive, params, (float*)bt.p[BUF_DERIVED]);
+                LAUNCH_CHECK();
+            }
         }
-    }
-    if (mode == MSHGNN_MODE_FP32) {
         if ((rc = launch_rowgemm(K_ENC_FWD, p, train ? p.enc_train : p.enc_launch, bt, B, w.Bp, xf64, st))) return rc;
         for (int l = 0; l < p.L; ++l) {
             if ((rc = launch_rowgemm(K_CONV_FWD, p, train ? p.conv_train[l] : p.conv_infer[l], bt, B, w.Bp, 0, st))) return rc;
@@ -701,13 +752,11 @@ int mshgnn_forward(const mshgnn_plan* plan, int64_t B, const void* const* x, int
         }
     } else {
         // tensor-core path: every activation lives as a (hi, lo) fp16 image pair only; TMA in, TMA out
-        BufRows br;
-        fill_rows16(p, w, br);
-        WsMaps wm;
-        if ((rc = make_ws_maps(&wm, workspace, w))) return rc;
+        const BufRows& br = c.br;
+        const WsMaps& wm = c.wm;
         __half* w_hi = (__half*)((char*)workspace + w.w16[0]);
         __half* w_lo = (__half*)((char*)workspace + w.w16[1]);
-        const int split = mode == MSHGNN_MODE_TC;
+        const int split = c.split;
         {   // bias sums, (hi, lo) weight images, encoder weight image, stack counters: one launch (k_fwd_prologue)
             ProfScope ps(K_DERIVE, st);
             FwdPrologue fp;
@@ -741,11 +790,8 @@ int mshgnn_forward(const mshgnn_plan* plan, int64_t B, const void* const* x, int
         int blocks = (int)((rows + 7) / 8);
         if (blocks > 148 * 8) blocks = 148 * 8;
         ProfScope ps(K_DEC_FWD, st);
-        const bool tcm = mode != MSHGNN_MODE_FP32;
-        const char* wsb = (const char*)workspace;
-#define MSHGNN_DEC_FWD(CM) k_decoder_fwd<CM><<<blocks, 256, 0, st>>>(p.dec, tcm ? nullptr : (const float*)bt.p[BUF_H0 + p.L], \
-                                              tcm ? (const __half*)(wsb + w.h16[p.L][0]) : nullptr, tcm ? (const __half*)(wsb + w.h16[p.L][1]) : nullptr, \
-                                              params, p.d_signs, out, B, w.Bp)
+#define MSHGNN_DEC_FWD(CM) k_decoder_fwd<CM><<<blocks, 256, 0, st>>>(p.dec, (const float*)bt.p[BUF_H0 + p.L], image16(c.ws, w, BUF_H0 + p.L, 0), \
+                                              image16(c.ws, w, BUF_H0 + p.L, 1), params, p.d_signs, out, B, w.Bp)
         if (p.dec.C <= 2) MSHGNN_DEC_FWD(2); else if (p.dec.C <= 4) MSHGNN_DEC_FWD(4); else MSHGNN_DEC_FWD(8);
 #undef MSHGNN_DEC_FWD
         LAUNCH_CHECK();
@@ -787,114 +833,64 @@ int mshgnn_backward(const mshgnn_plan* plan, int64_t B, const void* const* x, in
 int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const* x, int32_t x_dtype, const float* params,
                            const float* dout, float* grads, void* workspace, int64_t workspace_bytes, int32_t mode, void* stream,
                            void* layers_ready_event) {
-    if (!plan) return fail(MSHGNN_ERR_ARG, "plan is NULL");
+    int rc;
+    if ((rc = check_plan_mode(plan, mode))) return rc;
     const Plan& p = plan->p;
-    if (mode != MSHGNN_MODE_FP32 && mode != MSHGNN_MODE_TC && mode != MSHGNN_MODE_TC_1X) return fail(MSHGNN_ERR_ARG, "unknown mode %d", mode);
     if (x_dtype != MSHGNN_F32 && x_dtype != MSHGNN_F64 && x_dtype != MSHGNN_F16) return fail(MSHGNN_ERR_ARG, "x_dtype must be F32, F64 or F16");
     if (!x || !params || !dout) return fail(MSHGNN_ERR_ARG, "NULL argument");
     const bool want_dw = grads != nullptr;      // NULL: input-only backward (the dX chain for mshgnn_input_grad, no weight gradient)
-    const WsLayout w = ws_layout(p, B, 1, mode);
-    int rc = check_common(plan, B, workspace, workspace_bytes, w);
-    if (rc) return rc;
-    if ((rc = ensure_uploaded(p))) return rc;
+    Call c;
+    if ((rc = open_call(c, plan, B, 1, mode, workspace, workspace_bytes))) return rc;
+    if ((rc = bind_call(c, params, grads, x))) return rc;
+    float* const grads_out = grads;             // padded plans: the caller's gradients, compacted from c.grads
+    grads = c.grads;
+    params = c.params;
     cudaStream_t st = (cudaStream_t)stream;
-    float* const grads_out = grads;
-    if (p.padded) {     // the forward's 128-wide parameter copy; gradients go to the 128-wide buffer, then compacted into grads_out
-        params = (const float*)((char*)workspace + w.pad_params);
-        if (grads) grads = (float*)((char*)workspace + w.pad_grads);
-    }
-    BufTable bt;
-    fill_bufs(p, w, (char*)workspace, bt);
-    bt.p[BUF_PARAMS] = (void*)params;
-    bt.p[BUF_GRADS] = grads;
-    for (int t = 0; t < p.n_types; ++t) { if (!x[t]) return fail(MSHGNN_ERR_ARG, "x[%d] is NULL", t); bt.p[BUF_X0 + t] = (void*)x[t]; }
+    const WsLayout& w = c.w;
+    const BufTable& bt = c.bt;
+    const BufRows& br = c.br;
+    const WsMaps& wm = c.wm;
+    char* ws = c.ws;
+    const bool tc = c.tc;
+    const int split = c.split;
+    const float G = c.G;
     const int xf64 = x_dtype == MSHGNN_F64 ? 1 : (x_dtype == MSHGNN_F16 ? 2 : 0);      // element-type code of the kernels (ld_x)
-    char* ws = (char*)workspace;
     float* part_w = (float*)(ws + w.part_w);
     float* part_b = (float*)(ws + w.part_b);
     float* dec_part = (float*)(ws + w.dec_part);
-    const bool tc = mode != MSHGNN_MODE_FP32;
-    const int split = mode == MSHGNN_MODE_TC;
-    BufTable16 bh;
-    fill_bufs16(p, w, ws, bh);
-    WsMaps wm;
-    if (tc && (rc = make_ws_maps(&wm, workspace, w))) return rc;
-    // tensor-core modes carry every backward quantity multiplied by a power of two G ~ #output rows so that the
-    // fp16 (hi, lo) images of dL/dh stay in the normal range; the final reductions multiply by 1/G (exact).
-    BufRows br;
-    fill_rows16(p, w, br);
-    float G = 1.f;
-    if (tc) { int e = 0; std::frexp((double)(B * p.dec.n_dec), &e); G = (float)std::ldexp(1.0, e - 1); }
 
     if (!want_dw) {
-        if (tc && (rc = stack_sync_reset(w, ws, st))) return rc;
-    } else if (tc && w.stack && (reinterpret_cast<uintptr_t>(grads) & 15) == 0) {
+        if ((rc = stack_sync_reset(w, ws, st))) return rc;
+    } else if (w.stack && (reinterpret_cast<uintptr_t>(grads) & 15) == 0) {
         ProfScope ps(K_MEMSET, st);
         const int64_t n4 = p.n_params / 4;
         k_bwd_prologue<<<296, 256, 0, st>>>((float4*)grads, n4, grads + n4 * 4, (int)(p.n_params - n4 * 4), (uint32_t*)(ws + w.stack_sync), w.stack_sync_bytes / 4);
         LAUNCH_CHECK();
     } else {
         { ProfScope ps(K_MEMSET, st); CUDA_TRY(cudaMemsetAsync(grads, 0, (size_t)p.n_params * 4, st)); }
-        if (tc && (rc = stack_sync_reset(w, ws, st))) return rc;
+        if ((rc = stack_sync_reset(w, ws, st))) return rc;
     }
 
     {   // decoder backward: dH_L on the decoded slots (+ masked copy = dc_{L-1}), dW_dec, db_dec
         const int L = p.L;
-        float* dh = nullptr; float* dc = nullptr; int mk = MK_NONE; const void* mbuf = nullptr;
-        if (p.morph_sym) {
-            dh = (float*)bt.p[BUF_DHL0 + L];
-            if (p.dec_type != p.mlp_type) { dc = (float*)bt.p[BUF_DCL0 + L - 1]; mk = MK_BITS; mbuf = bt.p[BUF_MASK0 + L - 1]; }
-        } else {
-            dc = (float*)bt.p[BUF_DCL0 + L - 1]; mk = MK_BITS; mbuf = bt.p[BUF_MASK0 + L - 1];
-        }
-        ProfScope ps(K_DEC_BWD, st);
-        const int dhb = BUF_DHL0 + L, dcb = BUF_DCL0 + L - 1;
         const bool want_dh = p.morph_sym, want_dc = !p.morph_sym || p.dec_type != p.mlp_type;
-#define MSHGNN_DEC_BWD(CM) k_decoder_bwd<CM><<<DEC_BLOCKS, 256, 0, st>>>(p.dec, tc ? nullptr : (const float*)bt.p[BUF_H0 + L], tc ? bh.hi[BUF_H0 + L] : nullptr, \
-                                                  tc ? bh.lo[BUF_H0 + L] : nullptr, params, p.d_signs, dout, tc ? nullptr : dh, tc ? nullptr : dc, mk, mbuf, \
-                                                  dec_part, B, w.Bp, G, (tc && want_dh) ? bh.hi[dhb] : nullptr, (tc && want_dh) ? bh.lo[dhb] : nullptr, \
-                                                  (tc && want_dc) ? bh.hi[dcb] : nullptr, (tc && want_dc) ? bh.lo[dcb] : nullptr)
+        const int dhb = BUF_DHL0 + L, dcb = BUF_DCL0 + L - 1;
+        // fp32 mode writes the slabs, the tensor-core modes the (hi, lo) images (the layout has only one of them)
+        float* dh = want_dh ? (float*)bt.p[dhb] : nullptr;
+        float* dc = want_dc ? (float*)bt.p[dcb] : nullptr;
+        const int mk = want_dc ? MK_BITS : MK_NONE;
+        const void* mbuf = want_dc ? bt.p[BUF_MASK0 + L - 1] : nullptr;
+        ProfScope ps(K_DEC_BWD, st);
+#define MSHGNN_DEC_BWD(CM) k_decoder_bwd<CM><<<DEC_BLOCKS, 256, 0, st>>>(p.dec, (const float*)bt.p[BUF_H0 + L], image16(ws, w, BUF_H0 + L, 0), \
+                                                  image16(ws, w, BUF_H0 + L, 1), params, p.d_signs, dout, dh, dc, mk, mbuf, dec_part, B, w.Bp, G, \
+                                                  want_dh ? image16(ws, w, dhb, 0) : nullptr, want_dh ? image16(ws, w, dhb, 1) : nullptr, \
+                                                  want_dc ? image16(ws, w, dcb, 0) : nullptr, want_dc ? image16(ws, w, dcb, 1) : nullptr)
         if (p.dec.C <= 2) MSHGNN_DEC_BWD(2); else if (p.dec.C <= 4) MSHGNN_DEC_BWD(4); else MSHGNN_DEC_BWD(8);
 #undef MSHGNN_DEC_BWD
         LAUNCH_CHECK();
         if (want_dw) {
             k_decoder_bwd_reduce<<<p.dec.C * H + p.dec.C, 256, 0, st>>>(p.dec, dec_part, DEC_BLOCKS, grads, 1.f / G);
             LAUNCH_CHECK();
-        }
-    }
-    auto launch_dw = [&](int kind, const Launch& L) -> int {
-        if (L.count == 0 || !want_dw) return 0;
-        ProfScope ps(kind, st);
-        dim3 grid((unsigned)L.count, (unsigned)w.n_splits);
-        k_reducegemm<<<grid, 256, 0, st>>>(p.d_rtasks, p.d_rpairs, L.begin, bt, B, w.Bp, xf64, w.n_splits, part_w, part_b);
-        LAUNCH_CHECK();
-        return 0;
-    };
-    if (tc && w.stack) {
-        // the whole dX chain (with the base_transform backward chained on chip) in one launch over per-layer dh / dc / du
-        // images, then the weight gradients of every layer (they only read what the chain and the forward pass stored)
-        if ((rc = launch_stack(K_STACK_BWD, p, p.stack_bwd, w, bt, br, wm, ws, B, split, st))) return rc;
-        if (want_dw && w.dw_merged) {
-            // tasks are laid out layer L-1 first, contiguously: one launch covers them all (ws_layout fitted one split count)
-            Launch all{p.dw_layer[p.L - 1].begin, 0};
-            for (int l = 0; l < p.L; ++l) all.count += p.dw_layer[l].count;
-            if ((rc = launch_tc_dw(K_DW_LAYER, p, p.L - 1, all, w, br, wm, B, split, part_w, part_b, st))) return rc;
-        } else if (want_dw) {
-            for (int l = p.L - 1; l >= 0; --l)
-                if ((rc = launch_tc_dw(K_DW_LAYER, p, l, p.dw_layer[l], w, br, wm, B, split, part_w, part_b, st))) return rc;
-        }
-    } else
-    for (int l = p.L - 1; l >= 0; --l) {
-        if (tc) {
-            if ((rc = launch_tc_rowgemm(K_MLP_BWD, p, p.bwd_m1[l], bt, br, wm, B, w.Bp, split, st))) return rc;
-            if ((rc = launch_tc_rowgemm(K_MLP_BWD, p, p.bwd_m2[l], bt, br, wm, B, w.Bp, split, st))) return rc;
-            if (want_dw && (rc = launch_tc_dw(K_DW_LAYER, p, l, p.dw_layer[l], w, br, wm, B, split, part_w, part_b, st))) return rc;
-            if ((rc = launch_tc_rowgemm(K_DX_BWD, p, p.bwd_dx[l], bt, br, wm, B, w.Bp, split, st))) return rc;
-        } else {
-            if ((rc = launch_rowgemm(K_MLP_BWD, p, p.bwd_m1[l], bt, B, w.Bp, 0, st))) return rc;
-            if ((rc = launch_rowgemm(K_MLP_BWD, p, p.bwd_m2[l], bt, B, w.Bp, 0, st))) return rc;
-            if ((rc = launch_dw(K_DW_LAYER, p.dw_layer[l]))) return rc;
-            if ((rc = launch_rowgemm(K_DX_BWD, p, p.bwd_dx[l], bt, B, w.Bp, 0, st))) return rc;
         }
     }
     // layer-stack groups were produced with the split count of the kernel that ran them, encoder groups with the SIMT one
@@ -913,73 +909,71 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         return 0;
     };
     if (tc) {
+        if (w.stack) {
+            // the whole dX chain (with the base_transform backward chained on chip) in one launch over per-layer dh / dc / du
+            // images, then the weight gradients of every layer (they only read what the chain and the forward pass stored)
+            if ((rc = launch_stack(K_STACK_BWD, p, p.stack_bwd, w, bt, br, wm, ws, B, split, st))) return rc;
+            if (want_dw && w.dw_merged) {
+                // tasks are laid out layer L-1 first, contiguously: one launch covers them all (ws_layout fitted one split count)
+                Launch all{p.dw_layer[p.L - 1].begin, 0};
+                for (int l = 0; l < p.L; ++l) all.count += p.dw_layer[l].count;
+                if ((rc = launch_tc_dw(K_DW_LAYER, p, p.L - 1, all, w, br, wm, B, split, part_w, part_b, st))) return rc;
+            } else if (want_dw) {
+                for (int l = p.L - 1; l >= 0; --l)
+                    if ((rc = launch_tc_dw(K_DW_LAYER, p, l, p.dw_layer[l], w, br, wm, B, split, part_w, part_b, st))) return rc;
+            }
+        } else {
+            for (int l = p.L - 1; l >= 0; --l) {
+                if ((rc = launch_tc_rowgemm(K_MLP_BWD, p, p.bwd_m1[l], bt, br, wm, B, w.Bp, split, st))) return rc;
+                if ((rc = launch_tc_rowgemm(K_MLP_BWD, p, p.bwd_m2[l], bt, br, wm, B, w.Bp, split, st))) return rc;
+                if (want_dw && (rc = launch_tc_dw(K_DW_LAYER, p, l, p.dw_layer[l], w, br, wm, B, split, part_w, part_b, st))) return rc;
+                if ((rc = launch_tc_rowgemm(K_DX_BWD, p, p.bwd_dx[l], bt, br, wm, B, w.Bp, split, st))) return rc;
+            }
+        }
         // Every gradient outside the encoder is final here - before the encoder weight gradient, the last 8 % of the step, has
         // even started: the caller's event lets a data-parallel trainer all-reduce that 7.5 MB segment underneath it.
         if ((rc = reduce_layers())) return rc;
         if (p.padded && want_dw && (rc = compact_grads(p, p.n_pad_enc, (int)p.pad_segs.size() - p.n_pad_enc, grads, grads_out, st))) return rc;
         if (layers_ready_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)layers_ready_event, st));
-        if (!p.enc_units.empty() && want_dw) {
-            static std::atomic<bool> attr_set[64];
-            if (first_on_device(attr_set)) {
-                CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder_dw<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, EDW_SMEM_BYTES));
-                CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder_dw<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, EDW_SMEM_BYTES));
-            }
-            // x rows by TMA (raw fp32 into the X operand area, converted in place) when every feature tensor allows it: fp32, 16-byte rows
-            // (measured, same box: 0.258-0.270 ms against 0.246-0.251 ms for the register-staged loaders - here the loads of a step are issued
-            // BEFORE its stage is free and nothing is pipelined across register sets, so the scoreboard effect of kernels_enc.cuh costs
-            // little, while a landing zone inside the stage serialises copy -> conversion -> MMA per stage.  Off unless MSHGNN_ENC_DW=tma.)
-            static const bool want_xt = [] { const char* e = getenv("MSHGNN_ENC_DW"); return e && !strcmp(e, "tma"); }();
-            bool xt = xf64 == 0 && (g_encoder_dw_tma.load() >= 0 ? g_encoder_dw_tma.load() != 0 : want_xt);
-            for (const EncDwUnit& eu : p.enc_units)
-                if (xt) xt = eu.x_buf >= BUF_X0 && eu.x_buf < BUF_X0 + p.n_types && enq_rows_ok(bt.p[eu.x_buf], eu.K, 0);
-            EncXMaps xm;
-            for (int t = 0; t < 4; ++t) {
-                if (xt && t < p.n_types && p.in_w[t] % 4 == 0 && (reinterpret_cast<uintptr_t>(bt.p[BUF_X0 + t]) & 15) == 0) {
-                    if ((rc = make_map_x3d(&xm.x[t], bt.p[BUF_X0 + t], B, p.nodes[t], p.in_w[t], 64))) return rc;
-                } else xm.x[t] = wm.dw;
-            }
-            float* pe_w = (float*)(ws + w.part_enc_w);
-            float* pe_b = (float*)(ws + w.part_enc_b);
-            {
-                ProfScope ps(K_DW_ENC, st);
-                dim3 grid((unsigned)p.enc_units.size(), (unsigned)w.n_splits_enc);
-                if (xt) k_tc_encoder_dw<true><<<grid, ENC_THREADS, EDW_SMEM_BYTES, st>>>(wm.dw, xm, (int)BUF_X0, p.d_enc_units, bt, br, B, w.Bp, w.rows_per_enc, w.n_splits_enc, xf64,
-                                                                                         split, pe_w, pe_b);
-                else k_tc_encoder_dw<false><<<grid, ENC_THREADS, EDW_SMEM_BYTES, st>>>(wm.dw, xm, (int)BUF_X0, p.d_enc_units, bt, br, B, w.Bp, w.rows_per_enc, w.n_splits_enc, xf64,
-                                                                                       split, pe_w, pe_b);
-                LAUNCH_CHECK();
-            }
-            {
-                ProfScope ps(K_REDUCE, st);
-                dim3 grid((unsigned)p.enc_groups.size(), 48);
-                k_reduce_enc<<<grid, 256, 0, st>>>(p.d_enc_groups, pe_w, pe_b, w.n_splits_enc, grads, 1.f / G);
-                LAUNCH_CHECK();
-            }
-        }
+        if (!p.enc_units.empty() && want_dw && (rc = launch_tc_encoder_dw(c, B, xf64, st))) return rc;
         if (p.padded && want_dw && (rc = compact_grads(p, 0, p.n_pad_enc, grads, grads_out, st))) return rc;
-    } else if ((rc = launch_dw(K_DW_ENC, p.dw_enc))) return rc;
-    if (!tc && (rc = reduce_layers())) return rc;
-    if (nge > 0 && !tc && want_dw) {
-        dim3 grid((unsigned)nge, 32);
-        ProfScope ps(K_REDUCE, st);
-        k_reduce_partials<<<grid, 256, 0, st>>>(p.d_groups + ngl, part_w, part_b, w.segs, grads, 1.f / G);
-        LAUNCH_CHECK();
+    } else {
+        auto launch_dw = [&](int kind, const Launch& L) -> int {
+            if (L.count == 0 || !want_dw) return 0;
+            ProfScope ps(kind, st);
+            dim3 grid((unsigned)L.count, (unsigned)w.n_splits);
+            k_reducegemm<<<grid, 256, 0, st>>>(p.d_rtasks, p.d_rpairs, L.begin, bt, B, w.Bp, xf64, w.n_splits, part_w, part_b);
+            LAUNCH_CHECK();
+            return 0;
+        };
+        for (int l = p.L - 1; l >= 0; --l) {
+            if ((rc = launch_rowgemm(K_MLP_BWD, p, p.bwd_m1[l], bt, B, w.Bp, 0, st))) return rc;
+            if ((rc = launch_rowgemm(K_MLP_BWD, p, p.bwd_m2[l], bt, B, w.Bp, 0, st))) return rc;
+            if ((rc = launch_dw(K_DW_LAYER, p.dw_layer[l]))) return rc;
+            if ((rc = launch_rowgemm(K_DX_BWD, p, p.bwd_dx[l], bt, B, w.Bp, 0, st))) return rc;
+        }
+        if ((rc = launch_dw(K_DW_ENC, p.dw_enc))) return rc;
+        if ((rc = reduce_layers())) return rc;
+        if (nge > 0 && want_dw) {
+            dim3 grid((unsigned)nge, 32);
+            ProfScope ps(K_REDUCE, st);
+            k_reduce_partials<<<grid, 256, 0, st>>>(p.d_groups + ngl, part_w, part_b, w.segs, grads, 1.f / G);
+            LAUNCH_CHECK();
+        }
+        if (p.padded && want_dw && (rc = compact_grads(p, 0, (int)p.pad_segs.size(), grads, grads_out, st))) return rc;
+        if (layers_ready_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)layers_ready_event, st));
     }
-    if (!tc && p.padded && want_dw && (rc = compact_grads(p, 0, (int)p.pad_segs.size(), grads, grads_out, st))) return rc;
-    if (!tc && layers_ready_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)layers_ready_event, st));
     return 0;
 }
 
 int mshgnn_input_grad(const mshgnn_plan* plan, int64_t B, const float* params, float* const* dx, void* workspace, int64_t workspace_bytes,
                       int32_t mode, void* stream) {
-    if (!plan) return fail(MSHGNN_ERR_ARG, "plan is NULL");
+    int rc;
+    if ((rc = check_plan_mode(plan, mode))) return rc;
     const Plan& p = plan->p;
-    if (mode != MSHGNN_MODE_FP32 && mode != MSHGNN_MODE_TC && mode != MSHGNN_MODE_TC_1X) return fail(MSHGNN_ERR_ARG, "unknown mode %d", mode);
     if (!params || !dx) return fail(MSHGNN_ERR_ARG, "NULL argument");
-    if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1 (got %lld)", (long long)B);
-    const WsLayout w = ws_layout(p, B, 1, mode);
-    int rc = check_common(plan, B, workspace, workspace_bytes, w);
-    if (rc) return rc;
+    Call c;
+    if ((rc = open_call(c, plan, B, 1, mode, workspace, workspace_bytes))) return rc;
     DxOut o;
     memset(&o, 0, sizeof o);
     unsigned n_kb = 1;
@@ -991,43 +985,34 @@ int mshgnn_input_grad(const mshgnn_plan* plan, int64_t B, const float* params, f
         any = any || dx[t];
     }
     if (!any) return 0;
-    if ((rc = ensure_uploaded(p))) return rc;
+    if ((rc = bind_call(c, params, nullptr, nullptr))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    char* ws = (char*)workspace;
+    const WsLayout& w = c.w;
     const unsigned n_units = (unsigned)p.dx_units.size();
-    if (mode == MSHGNN_MODE_FP32) {
-        if (p.padded) params = (const float*)(ws + w.pad_params);      // the forward's 128-wide copy (o.w_off is in that layout)
-        BufTable bt;
-        fill_bufs(p, w, ws, bt);
+    if (!c.tc) {      // c.params: a padded plan's 128-wide copy (o.w_off is in that layout)
         ProfScope ps(K_DX_ENC, st);
-        k_encoder_dx<<<dim3((unsigned)((B + 15) / 16), n_units, n_kb), 256, 0, st>>>(p.d_dx_units, o, (const float*)bt.p[BUF_DCL0 - 1], params, p.d_signs, B, w.Bp);
+        k_encoder_dx<<<dim3((unsigned)((B + 15) / 16), n_units, n_kb), 256, 0, st>>>(p.d_dx_units, o, (const float*)c.bt.p[BUF_DCL0 - 1], c.params, p.d_signs, B, w.Bp);
         LAUNCH_CHECK();
         return 0;
     }
     // tensor-core modes: dpre0 as (hi, lo) images, the encoder weight image of the forward prologue (x 2^8), G of the backward
     static std::atomic<bool> attr_set[64];
     if (first_on_device(attr_set)) CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder_dx, cudaFuncAttributeMaxDynamicSharedMemorySize, DX_SMEM_BYTES));
-    WsMaps wm;
-    if ((rc = make_ws_maps(&wm, workspace, w))) return rc;
-    BufRows br;
-    fill_rows16(p, w, br);
     DxMaps maps;
-    maps.a = wm.tc.o;
-    if ((rc = make_map_2d(&maps.w_hi, ws + w.wenc16[0], (int64_t)p.n_types * H, p.enc_kmax, 64, 64, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-    if ((rc = make_map_2d(&maps.w_lo, ws + w.wenc16[1], (int64_t)p.n_types * H, p.enc_kmax, 64, 64, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+    maps.a = c.wm.tc.o;
+    if ((rc = make_map_2d(&maps.w_hi, c.ws + w.wenc16[0], (int64_t)p.n_types * H, p.enc_kmax, 64, 64, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+    if ((rc = make_map_2d(&maps.w_lo, c.ws + w.wenc16[1], (int64_t)p.n_types * H, p.enc_kmax, 64, 64, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
     for (int t = 0; t < 4; ++t) {
-        maps.x[t] = wm.tc.o;
+        maps.x[t] = c.wm.tc.o;
         if (t < p.n_types && dx[t] && enq_rows_ok(dx[t], p.in_w[t], -1)) {
             if ((rc = make_map_x3d(&maps.x[t], dx[t], B, p.nodes[t], p.in_w[t], 128, 32, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
             o.tma |= 1 << t;
         }
     }
-    int e = 0;
-    std::frexp((double)(B * p.dec.n_dec), &e);
-    const float scale = (float)std::ldexp(1.0, -(e - 1)) * TC_W_UNSCALE;      // 1 / (G 2^8)
+    const float scale = TC_W_UNSCALE / c.G;      // 1 / (G 2^8)
     ProfScope ps(K_DX_ENC, st);
-    k_tc_encoder_dx<<<dim3((unsigned)(w.Bp / TILE_M), n_units), DX_THREADS, DX_SMEM_BYTES, st>>>(maps, p.d_dx_units, o, p.d_signs, br.hi[BUF_DC1_ID],
-                                                                                               br.lo[BUF_DC1_ID], B, w.Bp, mode == MSHGNN_MODE_TC, scale);
+    k_tc_encoder_dx<<<dim3((unsigned)(w.Bp / TILE_M), n_units), DX_THREADS, DX_SMEM_BYTES, st>>>(maps, p.d_dx_units, o, p.d_signs, c.br.hi[BUF_DC1_ID],
+                                                                                               c.br.lo[BUF_DC1_ID], B, w.Bp, c.split, scale);
     LAUNCH_CHECK();
     return 0;
 }
@@ -1178,7 +1163,7 @@ int mshgnn_relu_mask_offset(const mshgnn_plan* plan, int64_t B, int32_t mode, in
     const Plan& p = plan->p;
     if (layer < -1 || layer >= p.L) return fail(MSHGNN_ERR_ARG, "layer out of range");
     const WsLayout w = ws_layout(p, B, 1, mode);
-    *byte_off = layer < 0 ? w.maske : w.mask[layer];
+    *byte_off = w.buf[layer < 0 ? BUF_MASKE : BUF_MASK0 + layer];
     *n_slots = layer < 0 ? p.S : p.S + p.nm;
     *rows_padded = w.Bp;
     return 0;

@@ -29,12 +29,6 @@ struct BufTable {
     void* p[MAX_BUFS];
 };
 
-// fp16 (hi, lo) images of the slab buffers (tensor-core modes): v ~= hi + lo with ~22 significant bits
-struct BufTable16 {
-    __half* hi[MAX_BUFS];
-    __half* lo[MAX_BUFS];
-};
-
 // One K-chunk of a row-GEMM: D[rows,128] += A[rows,K] * Wt[K,128]
 struct Chunk {
     int a_kind;      // A_SLAB: fp32 slab tile; A_EXT: caller's x tensor (strided rows, f32/f64)

@@ -106,8 +106,7 @@ __device__ __forceinline__ void rg_load(const Tile& t, const BufTable& bt, int c
 }
 
 __global__ void __launch_bounds__(256, 2)
-k_rowgemm(const Tile* __restrict__ tiles, const BufTable bt, const int64_t B, const int64_t Bp, const int x_f64,
-          const BufTable16 bh, const int write16) {
+k_rowgemm(const Tile* __restrict__ tiles, const BufTable bt, const int64_t B, const int64_t Bp, const int x_f64) {
     __shared__ Tile t;
     __shared__ __align__(16) float As[RG_BK][RG_AS];
     __shared__ __align__(16) float Ws[RG_BK][H];
@@ -205,14 +204,7 @@ k_rowgemm(const Tile* __restrict__ tiles, const BufTable bt, const int64_t B, co
                     *mp = word;
                 }
             }
-            if (!live) {
-                if (write16) {   // rows [B, Bp) of the fp16 images stay zero (read in whole 64-row blocks by k_tc_reducegemm)
-                    const float z[4] = {0.f, 0.f, 0.f, 0.f};
-                    if (t.out_buf >= 0) split_store4(bh.hi[t.out_buf], bh.lo[t.out_buf], ((int64_t)t.out_slot * Bp + row) * H + col, z);
-                    if (t.out2_buf >= 0) split_store4(bh.hi[t.out2_buf], bh.lo[t.out2_buf], ((int64_t)t.out2_slot * Bp + row) * H + col, z);
-                }
-                continue;
-            }
+            if (!live) continue;
             if (t.posmask_buf >= 0) {
                 const unsigned w = *((const unsigned*)bt.p[t.posmask_buf] +
                                      ((int64_t)t.posmask_slot * Bp + row) * 4 + hh * 2 + (tx >> 3));
@@ -228,7 +220,6 @@ k_rowgemm(const Tile* __restrict__ tiles, const BufTable bt, const int64_t B, co
             if (t.out_buf >= 0) {
                 const int64_t off = ((int64_t)t.out_slot * Bp + row) * H + col;
                 *reinterpret_cast<float4*>((float*)bt.p[t.out_buf] + off) = make_float4(v[0], v[1], v[2], v[3]);
-                if (write16) split_store4(bh.hi[t.out_buf], bh.lo[t.out_buf], off, v);
             }
             if (t.out2_buf >= 0) {
                 if (t.out2_mask_kind == MK_BITS) {
@@ -240,7 +231,6 @@ k_rowgemm(const Tile* __restrict__ tiles, const BufTable bt, const int64_t B, co
                 }
                 const int64_t off2 = ((int64_t)t.out2_slot * Bp + row) * H + col;
                 *reinterpret_cast<float4*>((float*)bt.p[t.out2_buf] + off2) = make_float4(v[0], v[1], v[2], v[3]);
-                if (write16) split_store4(bh.hi[t.out2_buf], bh.lo[t.out2_buf], off2, v);
             }
         }
     }

@@ -801,60 +801,64 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode) {
     auto take = [&](int64_t bytes) { int64_t at = o; o += round_up(bytes, 256); return at; };
     const int64_t slab = (int64_t)p.S * w.Bp * H * 4;
     const int64_t ctb = (int64_t)2 * p.nm * w.Bp * H * 4;
-    w.derived = take(p.n_derived * 4);
-    for (int l = 0; l <= MAX_LAYERS; ++l) w.h[l] = -1;
-    for (int l = 0; l < MAX_LAYERS; ++l) { w.ct[l] = -1; w.mask[l] = -1; }
-    w.dh[0] = w.dh[1] = w.dc[0] = w.dc[1] = w.du = w.part_w = w.part_b = w.dec_part = -1;
+    for (int id = 0; id < MAX_BUFS; ++id) w.buf[id] = w.buf16[id][0] = w.buf16[id][1] = -1;
+    w.part_w = w.part_b = w.dec_part = -1;
+    w.buf[BUF_DERIVED] = take(p.n_derived * 4);
     // fp32 slabs exist in MODE_FP32 only: the tensor-core modes keep every activation / gradient as (hi, lo) fp16 images
     if (train) {
         if (!tc) {
-            for (int l = 0; l <= p.L; ++l) w.h[l] = take(slab);
+            for (int l = 0; l <= p.L; ++l) w.buf[BUF_H0 + l] = take(slab);
             if (p.morph_sym)
-                for (int l = 0; l < p.L; ++l) w.ct[l] = take(ctb);
+                for (int l = 0; l < p.L; ++l) w.buf[BUF_CT0 + l] = take(ctb);
         }
-        for (int l = 0; l < p.L; ++l) w.mask[l] = take((int64_t)(p.S + p.nm) * w.Bp * 16);
-        w.maske = take((int64_t)p.S * w.Bp * 16);
-        if (!tc) {
-            w.dh[0] = take(slab); w.dh[1] = take(slab); w.dc[0] = take(slab); w.dc[1] = take(slab);
-            if (p.morph_sym) w.du = take((int64_t)p.nm * w.Bp * H * 4);
+        for (int l = 0; l < p.L; ++l) w.buf[BUF_MASK0 + l] = take((int64_t)(p.S + p.nm) * w.Bp * 16);
+        w.buf[BUF_MASKE] = take((int64_t)p.S * w.Bp * 16);
+        if (!tc) {      // the per-layer backward ids alias two ping-pong slabs
+            int64_t dh[2], dc[2], du = -1;
+            dh[0] = take(slab); dh[1] = take(slab); dc[0] = take(slab); dc[1] = take(slab);
+            if (p.morph_sym) du = take((int64_t)p.nm * w.Bp * H * 4);
+            for (int l = 0; l <= p.L; ++l) w.buf[BUF_DHL0 + l] = dh[l & 1];
+            for (int l = -1; l < p.L; ++l) w.buf[BUF_DCL0 + l] = dc[(l + 2) & 1];
+            for (int l = 0; l < p.L; ++l) w.buf[BUF_DUL0 + l] = du;
         }
         w.part_w = take(w.part_slots * H * H * 4);
         w.part_b = take(w.part_slots * H * 4);
         w.dec_part = take((int64_t)DEC_BLOCKS * (DEC_MAXC * H + DEC_MAXC) * 4);
     } else if (!tc) {
         const int64_t a = take(slab), b = take(slab);
-        for (int l = 0; l <= p.L; ++l) w.h[l] = (l & 1) ? b : a;
-        if (p.morph_sym) { const int64_t c = take(ctb); for (int l = 0; l < p.L; ++l) w.ct[l] = c; }
+        for (int l = 0; l <= p.L; ++l) w.buf[BUF_H0 + l] = (l & 1) ? b : a;
+        if (p.morph_sym) { const int64_t c = take(ctb); for (int l = 0; l < p.L; ++l) w.buf[BUF_CT0 + l] = c; }
     }
-    for (int l = 0; l <= MAX_LAYERS; ++l) w.h16[l][0] = w.h16[l][1] = -1;
-    for (int l = 0; l < MAX_LAYERS; ++l) w.ct16[l][0] = w.ct16[l][1] = -1;
-    for (int i = 0; i < 2; ++i) { w.dh16[i][0] = w.dh16[i][1] = w.dc16[i][0] = w.dc16[i][1] = -1; w.du16[i] = -1; w.w16[i] = -1; }
-    for (int l = 0; l <= MAX_LAYERS; ++l) for (int i = 0; i < 2; ++i) { w.dhL16[l][i] = -1; w.dcL16[l][i] = -1; }
-    for (int l = 0; l < MAX_LAYERS; ++l) for (int i = 0; i < 2; ++i) w.duL16[l][i] = -1;
     if (tc) {
         for (int i = 0; i < 2; ++i) w.w16[i] = take((int64_t)p.n_mats16 * H * H * 2);
         if (train) {
-            for (int l = 0; l <= p.L; ++l) for (int i = 0; i < 2; ++i) w.h16[l][i] = take(slab / 2);
+            for (int l = 0; l <= p.L; ++l) for (int i = 0; i < 2; ++i) w.buf16[BUF_H0 + l][i] = take(slab / 2);
             if (p.morph_sym)
-                for (int l = 0; l < p.L; ++l) for (int i = 0; i < 2; ++i) w.ct16[l][i] = take(ctb / 2);
-            if (!w.stack) {
-                for (int b = 0; b < 2; ++b) for (int i = 0; i < 2; ++i) { w.dh16[b][i] = take(slab / 2); w.dc16[b][i] = take(slab / 2); }
-                if (p.morph_sym) for (int i = 0; i < 2; ++i) w.du16[i] = take((int64_t)p.nm * w.Bp * H * 2);
+                for (int l = 0; l < p.L; ++l) for (int i = 0; i < 2; ++i) w.buf16[BUF_CT0 + l][i] = take(ctb / 2);
+            if (!w.stack) {      // the per-layer launch sequence: backward ids alias two ping-pong images, as in MODE_FP32
+                int64_t dh[2][2], dc[2][2], du[2] = {-1, -1};
+                for (int b = 0; b < 2; ++b) for (int i = 0; i < 2; ++i) { dh[b][i] = take(slab / 2); dc[b][i] = take(slab / 2); }
+                if (p.morph_sym) for (int i = 0; i < 2; ++i) du[i] = take((int64_t)p.nm * w.Bp * H * 2);
+                for (int i = 0; i < 2; ++i) {
+                    for (int l = 0; l <= p.L; ++l) w.buf16[BUF_DHL0 + l][i] = dh[l & 1][i];
+                    for (int l = -1; l < p.L; ++l) w.buf16[BUF_DCL0 + l][i] = dc[(l + 2) & 1][i];
+                    for (int l = 0; l < p.L; ++l) w.buf16[BUF_DUL0 + l][i] = du[i];
+                }
             } else {
                 // the dX chain of all layers runs in ONE launch ahead of the weight-gradient kernels: every layer keeps its own
                 // dh / dc / du images (dh_l only where a residual or base_transform reads it: MS-HGNN models)
                 for (int l = 0; l <= p.L; ++l) for (int i = 0; i < 2; ++i) {
-                    if (p.morph_sym && l >= 1) w.dhL16[l][i] = take(slab / 2);
-                    w.dcL16[l][i] = take(slab / 2);                       // index l + 1: dc_{-1} (encoder dpre) .. dc_{L-1}
+                    if (p.morph_sym && l >= 1) w.buf16[BUF_DHL0 + l][i] = take(slab / 2);
+                    w.buf16[BUF_DCL0 + l - 1][i] = take(slab / 2);       // dc_{-1} (encoder dpre) .. dc_{L-1}
                 }
-                if (p.morph_sym) for (int l = 0; l < p.L; ++l) for (int i = 0; i < 2; ++i) w.duL16[l][i] = take((int64_t)p.nm * w.Bp * H * 2);
+                if (p.morph_sym) for (int l = 0; l < p.L; ++l) for (int i = 0; i < 2; ++i) w.buf16[BUF_DUL0 + l][i] = take((int64_t)p.nm * w.Bp * H * 2);
             }
         } else {
             int64_t a[2], b[2], c[2] = {-1, -1};
             for (int i = 0; i < 2; ++i) { a[i] = take(slab / 2); b[i] = take(slab / 2); }
             if (p.morph_sym) for (int i = 0; i < 2; ++i) c[i] = take(ctb / 2);
-            for (int l = 0; l <= p.L; ++l) for (int i = 0; i < 2; ++i) w.h16[l][i] = (l & 1) ? b[i] : a[i];
-            for (int l = 0; l < p.L; ++l) for (int i = 0; i < 2; ++i) w.ct16[l][i] = c[i];
+            for (int l = 0; l <= p.L; ++l) for (int i = 0; i < 2; ++i) w.buf16[BUF_H0 + l][i] = (l & 1) ? b[i] : a[i];
+            for (int l = 0; l < p.L; ++l) for (int i = 0; i < 2; ++i) w.buf16[BUF_CT0 + l][i] = c[i];
         }
     }
     if (tc) {

@@ -10,7 +10,7 @@
 
 namespace mshgnn {
 
-// buffer ids (BufTable slots)
+// buffer ids (BufTable / BufRows slots; ws_layout places each one in WsLayout::buf / buf16)
 enum : int {
     BUF_PARAMS = 0, BUF_DERIVED = 1, BUF_SIGNS = 2, BUF_GRADS = 3,
     BUF_X0 = 4,                       // +type
@@ -19,9 +19,9 @@ enum : int {
     BUF_H0 = 16,                      // +layer (0..L)
     BUF_CT0 = 32,                     // +layer
     BUF_MASK0 = 48,                   // +layer: ReLU bitmasks, slots [0,S) conv outputs, [S,S+nm) base-MLP hidden
-    // backward quantities, one id per layer.  The per-layer launch sequence aliases them onto two ping-pong buffers
-    // (dh_l -> dh[l & 1], dc_l -> dc[l & 1], du_l -> du); the cross-layer stack kernel runs the whole dX chain in one
-    // launch, before the weight-gradient kernels, so there every layer keeps its own buffer.
+    // backward quantities, one id per layer.  Under the per-layer launch sequence ws_layout aliases them onto two ping-pong
+    // buffers (dh_l -> dh[l & 1], dc_l -> dc[(l + 2) & 1], du_l -> du); the cross-layer stack kernel runs the whole dX chain
+    // in one launch, before the weight-gradient kernels, so there every layer keeps its own buffer.
     BUF_DHL0 = 64,                    // +l (0..L):  dL/dh_l
     BUF_DCL0 = 81,                    // +l (-1..L-1, i.e. BUF_DCL0 - 1 = dpre of the encoder): dL/dc_l (pre-activation gradients)
     BUF_DUL0 = 96                     // +l (0..L-1): gradient at the hidden ReLU of base_transform
@@ -126,6 +126,7 @@ struct Plan {
     mutable EncDwGroup* d_enc_groups = nullptr;
     mutable DxUnit* d_dx_units = nullptr;
     mutable PadSeg* d_pad_segs = nullptr;
+    mutable std::vector<void*> d_allocs;   // every device table above, freed by mshgnn_plan_destroy
 
     int slot_of(int type, int local) const { return type_base[type] + local; }
 };
@@ -139,22 +140,17 @@ struct WsLayout {
     int dw_slot0[MAX_LAYERS];          // first partial slot of each layer launch
     int dw_merged = 0;                 // stack mode: one weight-gradient launch for all layers (uniform row splits)
     int64_t part_slots = 0;            // total slots ([128][128] fp32 weight partial + [128] bias partial each)
-    int64_t derived = 0;
-    int64_t h[MAX_LAYERS + 1];
-    int64_t ct[MAX_LAYERS];
-    int64_t mask[MAX_LAYERS];
-    int64_t maske = -1;
-    int64_t dh[2], dc[2], du = 0;
+    // Where every buffer id lives (byte offsets into the workspace, -1 when the call has no such buffer).  ws_layout makes
+    // every aliasing decision here: several ids may name one buffer (the ping-pong slabs and images).
+    int64_t buf[MAX_BUFS];             // fp32: derived weights, slabs (MODE_FP32) and ReLU bitmasks
+    int64_t buf16[MAX_BUFS][2];        // tensor-core modes: (hi, lo) fp16 images, index [0] = hi, [1] = lo
+    int64_t w16[2] = {-1, -1};         // 128x128 weight images (hi, lo) of the tensor-core modes
     int64_t part_w = 0, part_b = 0, dec_part = 0, loss_part = 0;
     int n_splits_enc = 1, rows_per_enc = 512;          // row splits of the tensor-core encoder weight gradient
     int64_t part_enc_w = -1, part_enc_b = -1;          // [unit][split][128][192] fp32 / [unit][split][128]
     int64_t wenc16[2] = {-1, -1};                      // encoder weight images [n_types*128][enc_kmax] fp16 (hi, lo)
-    // tensor-core modes: (hi, lo) fp16 images; index [0] = hi, [1] = lo; -1 when absent
-    int64_t h16[MAX_LAYERS + 1][2], ct16[MAX_LAYERS][2], dh16[2][2], dc16[2][2], du16[2], w16[2];
-    // stack mode (training, tensor-core modes): per-layer backward images, -1 when the ping-pong layout is used
-    int stack = 0;
+    int stack = 0;                     // the layer loop runs as the cross-layer stack kernel (tensor-core modes)
     int stack_pair = 0;                // the stack launches use the CTA-pair kernel (Bp is a multiple of 256)
-    int64_t dhL16[MAX_LAYERS + 1][2], dcL16[MAX_LAYERS + 1][2] /* index l + 1 */, duL16[MAX_LAYERS][2];
     int64_t enc_sync = -1;             // work counter of the persistent encoder (k_tc_encoder_stream), zeroed by the forward prologue
     int64_t stack_sync = -1;           // dependency counters of the stack kernel (uint32 [phases][row tiles]) + error word
     int64_t stack_sync_bytes = 0;
