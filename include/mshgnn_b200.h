@@ -222,6 +222,33 @@ int mshgnn_build_windows(const mshgnn_window_desc* desc, const void* seq, const 
 int mshgnn_step_metrics(int32_t loss_kind, int64_t n, int32_t feet, const float* out, const void* labels, int32_t label_dtype,
                         double* batch, double* epoch, double* scratch, void* stream);
 
+/* Two more metric kinds, through mshgnn_step_metrics_ex (same batch / epoch / scratch contract as above; n = graphs):
+ *   MSHGNN_METRIC_COM: COM_Base_Lightning.calculate_losses_step (gnnLightning_com.py:L70-95).  out, labels [n, n_base*6]
+ *     (standardised, per base lin[3] then ang[3]); args: n_base, y_mean[6], y_std[6] (fp64, device).
+ *     slots 0 sum sq. err, 1 elements, 2 sum sq. err of the lin halves, 3 of the ang halves, 4 elements of one half,
+ *     5 sum over rows of the cosine similarity of the un-standardised (y * std + mean) lin 3-vectors of base 0, 6 the same
+ *     for ang, 7 rows; 20 MSE, 21 RMSE, 22 MSE lin, 23 MSE ang, 24 cos_sim_lin, 25 cos_sim_ang, 26 (cos_sim_lin + cos_sim_ang) / 2.
+ *     Cosine similarity is torch.nn.functional.cosine_similarity(pred, label, dim=1, eps=1e-8): each vector divided by
+ *     max(norm, eps), so a zero vector scores 0.
+ *   MSHGNN_METRIC_GRF_WORLD: HGNN_C2_Lightning_Reg.calculate_losses_step_worldframe (gnnLightning.py:L287-311).  out, labels
+ *     [n, 12] (4 feet x 3, body frame); args: quat [n, 4] (x, y, z, w; normalised here), quat_dtype MSHGNN_F32 | MSHGNN_F64, z_only.
+ *     slots 0 sum sq. err, 1 sum abs. err, 2 elements (body frame, as MSHGNN_LOSS_MSE), 3, 4, 5 the same after rotating each
+ *     foot's force by R(q)^T (with z_only: over the z components 2, 5, 8, 11 only); 20 MSE, 21 RMSE, 22 L1 (body frame),
+ *     23 MSE, 24 RMSE, 25 L1 (world frame).
+ * Arithmetic is fp64.  MSHGNN_ERR_ARG: n_base outside 1..4 or a NULL stat for COM, NULL quaternions for world frame. */
+#define MSHGNN_METRIC_COM       2
+#define MSHGNN_METRIC_GRF_WORLD 3
+typedef struct {
+    int32_t n_base;          /* COM: bases per graph, 1..4                              */
+    const double* y_mean;    /* COM: [6] standardiser mean (device)                     */
+    const double* y_std;     /* COM: [6] standardiser std (device)                      */
+    const void* quat;        /* GRF world frame: [n, 4] body orientation (device)       */
+    int32_t quat_dtype;      /* GRF world frame: MSHGNN_F32 or MSHGNN_F64               */
+    int32_t z_only;          /* GRF world frame: world-frame sums over z components only */
+} mshgnn_metric_args;
+int mshgnn_step_metrics_ex(int32_t kind, const mshgnn_metric_args* args, int64_t n, const float* out, const void* labels,
+                           int32_t label_dtype, double* batch, double* epoch, double* scratch, void* stream);
+
 /* JSON summary of the compiled tables (slots, liveness, gather lists); returns the bytes needed
  * (including the terminating NUL).  Host-only: usable without a GPU. */
 int64_t mshgnn_plan_describe(const mshgnn_plan* plan, char* buf, int64_t cap);

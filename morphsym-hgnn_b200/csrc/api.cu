@@ -1128,6 +1128,29 @@ int mshgnn_step_metrics(int32_t loss_kind, int64_t n, int32_t feet, const float*
     return 0;
 }
 
+int mshgnn_step_metrics_ex(int32_t kind, const mshgnn_metric_args* args, int64_t n, const float* out, const void* labels,
+                           int32_t label_dtype, double* batch, double* epoch, double* scratch, void* stream) {
+    if (!args || !out || !labels || !batch || !scratch || n < 1) return fail(MSHGNN_ERR_ARG, "bad argument");
+    if (kind != MSHGNN_METRIC_COM && kind != MSHGNN_METRIC_GRF_WORLD) return fail(MSHGNN_ERR_ARG, "bad metric kind");
+    if (label_dtype < 0 || label_dtype > 2) return fail(MSHGNN_ERR_ARG, "bad label_dtype");
+    if (kind == MSHGNN_METRIC_COM) {
+        if (args->n_base < 1 || args->n_base > 4) return fail(MSHGNN_ERR_ARG, "COM metrics need n_base in 1..4");
+        if (!args->y_mean || !args->y_std) return fail(MSHGNN_ERR_ARG, "COM metrics need y_mean and y_std");
+    } else {
+        if (!args->quat) return fail(MSHGNN_ERR_ARG, "world-frame GRF metrics need the quaternions");
+        if (args->quat_dtype != MSHGNN_F32 && args->quat_dtype != MSHGNN_F64) return fail(MSHGNN_ERR_ARG, "bad quat_dtype");
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    int blocks = (int)((n + 255) / 256);
+    if (blocks > MET_BLOCKS) blocks = MET_BLOCKS;
+    ProfScope ps(K_METRICS, st);
+    k_metrics_partial_ex<<<blocks, 256, 0, st>>>(kind, *args, out, labels, label_dtype, n, scratch);
+    LAUNCH_CHECK();
+    k_metrics_final<<<1, 32, 0, st>>>(kind, scratch, blocks, batch, epoch);
+    LAUNCH_CHECK();
+    return 0;
+}
+
 int mshgnn_profile_enable(int32_t on) {
     std::lock_guard<std::mutex> lk(g_prof_mu);
     g_prof_on = on != 0;

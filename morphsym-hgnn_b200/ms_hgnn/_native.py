@@ -21,6 +21,12 @@ F32, F64, I64, F16 = 0, 1, 2, 3
 MODE_FP32, MODE_TC, MODE_TC_1X = 0, 1, 2
 PLAN_PAD_HIDDEN = 1
 LOSS_MSE, LOSS_CE2 = 0, 1
+METRIC_COM, METRIC_GRF_WORLD = 2, 3
+# slots of mshgnn_step_metrics_ex (include/mshgnn_b200.h): 0..19 additive states (also added into epoch), 20+ derived values
+COM_SSE, COM_N, COM_SSE_LIN, COM_SSE_ANG, COM_N_HALF, COM_COS_LIN, COM_COS_ANG, COM_ROWS = range(8)
+COM_MSE, COM_RMSE, COM_MSE_LIN, COM_MSE_ANG, COM_COS_SIM_LIN, COM_COS_SIM_ANG, COM_AVG_COS_SIM = range(20, 27)
+GRF_SSE, GRF_SAE, GRF_N, GRF_SSE_WORLD, GRF_SAE_WORLD, GRF_N_WORLD = range(6)
+GRF_MSE, GRF_RMSE, GRF_L1, GRF_MSE_WORLD, GRF_RMSE_WORLD, GRF_L1_WORLD = range(20, 26)
 P_ENC_W, P_ENC_B, P_REL_W, P_REL_B, P_ROOT_W, P_MLP_W, P_MLP_B, P_DEC_W, P_DEC_B = range(9)
 
 # every symbol include/mshgnn_b200.h declares
@@ -31,7 +37,7 @@ EXPORTS = (
     "mshgnn_last_error", "mshgnn_version", "mshgnn_profile_enable", "mshgnn_profile_read", "mshgnn_kernel_kind_name",
     "mshgnn_relu_mask_offset", "mshgnn_build_windows", "mshgnn_step_metrics", "mshgnn_dw_layout",
     "mshgnn_check_edges", "mshgnn_set_option", "mshgnn_get_option", "mshgnn_stack_status", "mshgnn_stack_timing_offset",
-    "mshgnn_backward_staged", "mshgnn_input_grad", "mshgnn_plan_create_ex",
+    "mshgnn_backward_staged", "mshgnn_input_grad", "mshgnn_plan_create_ex", "mshgnn_step_metrics_ex",
 )
 
 
@@ -68,6 +74,12 @@ class WindowDesc(C.Structure):
         ("block_col", C.POINTER(C.c_int32)), ("block_sign", C.POINTER(C.c_int32)),
         ("label_col", C.POINTER(C.c_int32)), ("label_sign", C.POINTER(C.c_int32)),
     ]
+
+
+class MetricArgs(C.Structure):
+    """mshgnn_metric_args (include/mshgnn_b200.h)."""
+    _fields_ = [("n_base", C.c_int32), ("y_mean", C.c_void_p), ("y_std", C.c_void_p), ("quat", C.c_void_p),
+                ("quat_dtype", C.c_int32), ("z_only", C.c_int32)]
 
 
 _lib: Optional[C.CDLL] = None
@@ -128,6 +140,9 @@ def lib() -> C.CDLL:
     L.mshgnn_build_windows.argtypes = [C.POINTER(WindowDesc), vp, vp, i32, i64, vp, i64, C.POINTER(vp), vp, vp]
     L.mshgnn_build_windows.restype = C.c_int
     L.mshgnn_step_metrics.argtypes = [i32, i64, i32, vp, vp, i32, vp, vp, vp, vp]; L.mshgnn_step_metrics.restype = C.c_int
+    if hasattr(L, "mshgnn_step_metrics_ex"):     # absent from builds before it (MSHGNN_LIB A/B runs against an older commit)
+        L.mshgnn_step_metrics_ex.argtypes = [i32, C.POINTER(MetricArgs), i64, vp, vp, i32, vp, vp, vp, vp]
+        L.mshgnn_step_metrics_ex.restype = C.c_int
     L.mshgnn_check_edges.argtypes = [vp, i64, C.POINTER(vp), vp, vp]; L.mshgnn_check_edges.restype = C.c_int
     L.mshgnn_set_option.argtypes = [C.c_char_p, i32]; L.mshgnn_set_option.restype = C.c_int
     L.mshgnn_get_option.argtypes = [C.c_char_p]; L.mshgnn_get_option.restype = i32
@@ -302,6 +317,12 @@ METRIC_SLOTS, METRIC_SCRATCH = 32, 296 * 32
 def step_metrics(kind, n, feet, out_ptr, labels_ptr, label_dtype, batch_ptr, epoch_ptr, scratch_ptr, stream):
     check(lib().mshgnn_step_metrics(kind, n, feet, out_ptr, labels_ptr, label_dtype, batch_ptr, epoch_ptr, scratch_ptr, stream),
           "mshgnn_step_metrics")
+
+
+def step_metrics_ex(kind, args: MetricArgs, n, out_ptr, labels_ptr, label_dtype, batch_ptr, epoch_ptr, scratch_ptr, stream):
+    """METRIC_COM / METRIC_GRF_WORLD: ``n`` = graphs, ``args`` the kind's inputs (n_base and stats, or quaternions)."""
+    check(lib().mshgnn_step_metrics_ex(kind, C.byref(args), n, out_ptr, labels_ptr, label_dtype, batch_ptr, epoch_ptr, scratch_ptr,
+                                       stream), "mshgnn_step_metrics_ex")
 
 
 def adam_step(params_ptr, grads_ptr, m_ptr, v_ptr, n, step, lr, b1, b2, eps, wd, stream):

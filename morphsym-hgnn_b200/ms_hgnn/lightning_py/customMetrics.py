@@ -11,7 +11,7 @@ from torch import nn
 
 
 class FusedStepMetrics:
-    """Device-side accumulators of ``mshgnn_step_metrics`` (include/mshgnn_b200.h): one native call per step produces this
+    """Device-side accumulators of ``mshgnn_step_metrics`` / ``mshgnn_step_metrics_ex`` (include/mshgnn_b200.h): one native call per step produces this
     batch's values (``batch``) and adds the counts to the epoch states (``epoch``), replacing ~80 small torch launches of
     the op-by-op path below (and the reference's host-side sklearn / python loop, gnnLightning.py:L285-348)."""
 
@@ -19,7 +19,7 @@ class FusedStepMetrics:
         self.batch = self.epoch = self.scratch = None
         self.dirty = False
 
-    def update(self, kind: int, out2d: torch.Tensor, labels: torch.Tensor, n: int, feet: int) -> torch.Tensor:
+    def _operands(self, out2d: torch.Tensor, labels: torch.Tensor):
         from .. import _native as N
         dev = out2d.device
         if self.batch is None or self.batch.device != dev:
@@ -32,11 +32,55 @@ class FusedStepMetrics:
         code = {torch.float32: N.F32, torch.float64: N.F64, torch.int64: N.I64}.get(labels.dtype)
         if code is None:
             labels, code = labels.double(), N.F64
+        return out2d, labels, code
+
+    def update(self, kind: int, out2d: torch.Tensor, labels: torch.Tensor, n: int, feet: int) -> torch.Tensor:
+        from .. import _native as N
+        out2d, labels, code = self._operands(out2d, labels)
+        dev = out2d.device
         with torch.cuda.device(dev):
             N.step_metrics(kind, n, feet, out2d.data_ptr(), labels.data_ptr(), code, self.batch.data_ptr(), self.epoch.data_ptr(),
                            self.scratch.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
         self.dirty = True
         return self.batch
+
+    def _update_ex(self, kind: int, out2d: torch.Tensor, labels: torch.Tensor, n: int, args) -> torch.Tensor:
+        from .. import _native as N
+        out2d, labels, code = self._operands(out2d, labels)
+        dev = out2d.device
+        with torch.cuda.device(dev):
+            N.step_metrics_ex(kind, args, n, out2d.data_ptr(), labels.data_ptr(), code, self.batch.data_ptr(),
+                              self.epoch.data_ptr(), self.scratch.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+        self.dirty = True
+        return self.batch
+
+    def update_com(self, pred: torch.Tensor, labels: torch.Tensor, n_base: int, y_mean: torch.Tensor, y_std: torch.Tensor) -> torch.Tensor:
+        """COM momentum metrics (``METRIC_COM``): ``pred`` / ``labels`` [B, n_base*6] standardised, ``y_mean`` / ``y_std`` contiguous
+        fp64 [6] tensors on the same device (the standardiser's stats).  Returns the slot buffer (batch values at 20..26)."""
+        from .. import _native as N
+        B = pred.shape[0]
+        if pred.numel() != B * n_base * 6 or labels.numel() != pred.numel():
+            raise ValueError(f"COM metrics need predictions and labels of [B, {n_base * 6}]")
+        for t in (y_mean, y_std):
+            if t.dtype != torch.float64 or t.numel() != 6 or not t.is_contiguous() or t.device != pred.device:
+                raise ValueError("COM metrics need y_mean / y_std as contiguous float64 [6] tensors on the predictions' device")
+        args = N.MetricArgs(n_base=n_base, y_mean=y_mean.data_ptr(), y_std=y_std.data_ptr())
+        return self._update_ex(N.METRIC_COM, pred, labels, B, args)
+
+    def update_grf_world(self, pred: torch.Tensor, labels: torch.Tensor, quat: torch.Tensor, z_only: bool = False) -> torch.Tensor:
+        """Body- and world-frame GRF metrics (``METRIC_GRF_WORLD``): ``pred`` / ``labels`` [B, 12] body frame, ``quat`` [B, 4]
+        (x, y, z, w).  Slots 0..2 are those of the MSE kind, so this call also feeds metrics bound to the body-frame states."""
+        from .. import _native as N
+        B = pred.shape[0]
+        if pred.numel() != B * 12 or labels.numel() != B * 12 or quat.numel() != B * 4:
+            raise ValueError("world-frame GRF metrics need predictions and labels of [B, 12] and quaternions of [B, 4]")
+        if quat.device != pred.device:
+            raise ValueError("the quaternions must be on the predictions' device")
+        quat = quat.reshape(-1).contiguous()
+        if quat.dtype not in (torch.float32, torch.float64):
+            quat = quat.double()
+        args = N.MetricArgs(quat=quat.data_ptr(), quat_dtype=N.F64 if quat.dtype == torch.float64 else N.F32, z_only=int(bool(z_only)))
+        return self._update_ex(N.METRIC_GRF_WORLD, pred, labels, B, args)
 
     def reset(self):
         if self.epoch is not None:
@@ -168,4 +212,6 @@ class CosineSimilarityMetric(_Metric):
         return sim.mean()
 
     def compute(self):
+        if self._from_fused():
+            return self._fused_fn(self._fused.epoch)
         return self._state["sum"] / self._state["n"]

@@ -275,6 +275,10 @@ class HGNN_C2_Lightning_Reg(Base_Lightning):
             self.metric_rmse_worldframe = MeanSquaredError(squared=False)
             self.metric_l1_worldframe = MeanAbsoluteError()
             self.mse_loss_worldframe = self.rmse_loss_worldframe = self.l1_loss_worldframe = None
+            # the world-frame call (METRIC_GRF_WORLD) fills the body-frame states 0..2 too: the bindings above still hold
+            self.metric_mse_worldframe.bind(self._fused, lambda e: e[N.GRF_SSE_WORLD] / e[N.GRF_N_WORLD])
+            self.metric_rmse_worldframe.bind(self._fused, lambda e: torch.sqrt(e[N.GRF_SSE_WORLD] / e[N.GRF_N_WORLD]))
+            self.metric_l1_worldframe.bind(self._fused, lambda e: e[N.GRF_SAE_WORLD] / e[N.GRF_N_WORLD])
 
     def calculate_losses_step_original(self, y, y_pred):
         Base_Lightning.calculate_losses_step(self, y, y_pred)
@@ -285,16 +289,30 @@ class HGNN_C2_Lightning_Reg(Base_Lightning):
         return self.calculate_losses_step_original(y, y_pred)
 
     def calculate_losses_step_worldframe(self, y, y_pred, batch_r_quat, test_only_on_z: bool = False):
+        if y_pred.is_cuda and y_pred.shape[1] == 12:
+            self.mse_loss = native_loss(self.model, y_pred, y, N.LOSS_MSE)
+            with torch.no_grad():
+                self._worldframe_metrics_fused(y, y_pred.detach(), batch_r_quat, test_only_on_z)
+            return
         self.calculate_losses_step_original(y, y_pred)
         with torch.no_grad():
-            y_world = self.body_frame_to_world_frame(batch_r_quat, y)
-            y_pred_world = self.body_frame_to_world_frame(batch_r_quat, y_pred.detach())
-            if test_only_on_z:
-                z_index = [2, 5, 8, 11]
-                y_world, y_pred_world = y_world[:, z_index], y_pred_world[:, z_index]
-            self.mse_loss_worldframe = self.metric_mse_worldframe(y_pred_world, y_world)
-            self.rmse_loss_worldframe = self.metric_rmse_worldframe(y_pred_world, y_world)
-            self.l1_loss_worldframe = self.metric_l1_worldframe(y_pred_world, y_world)
+            self._worldframe_metrics_op_by_op(y, y_pred.detach(), batch_r_quat, test_only_on_z)
+
+    def _worldframe_metrics_fused(self, y, y_pred, batch_r_quat, test_only_on_z):
+        """Body- and world-frame metrics from ONE mshgnn_step_metrics_ex call (METRIC_GRF_WORLD, fp64)."""
+        b = self._fused.update_grf_world(y_pred, y, batch_r_quat, test_only_on_z)
+        b = b[N.GRF_RMSE:N.GRF_L1_WORLD + 1].clone()           # the fused buffer is overwritten by the next step
+        self.rmse_loss, self.l1_loss, self.mse_loss_worldframe, self.rmse_loss_worldframe, self.l1_loss_worldframe = b.unbind()
+
+    def _worldframe_metrics_op_by_op(self, y, y_pred, batch_r_quat, test_only_on_z):
+        y_world = self.body_frame_to_world_frame(batch_r_quat, y)
+        y_pred_world = self.body_frame_to_world_frame(batch_r_quat, y_pred)
+        if test_only_on_z:
+            z_index = [2, 5, 8, 11]
+            y_world, y_pred_world = y_world[:, z_index], y_pred_world[:, z_index]
+        self.mse_loss_worldframe = self.metric_mse_worldframe(y_pred_world, y_world)
+        self.rmse_loss_worldframe = self.metric_rmse_worldframe(y_pred_world, y_world)
+        self.l1_loss_worldframe = self.metric_l1_worldframe(y_pred_world, y_world)
 
     def body_frame_to_world_frame(self, batch_r_quat, grf_bodyFrame):
         """Rotate per-foot forces by the inverse of the (x, y, z, w) body quaternion, on the device

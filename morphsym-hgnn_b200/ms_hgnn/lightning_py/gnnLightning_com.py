@@ -2,7 +2,9 @@
 
 Drop-in for the hot-path part of the reference's ``gnnLightning_com.py``: ``COM_Base_Lightning``
 (L28-231), ``COM_HGNN_Lightning`` (L290-341), ``COM_HGNN_SYM_Lightning`` (L343-410).  The loss is the
-native fused MSE over ``[B, n_base*6]``; lin/ang MSE and cosine similarity are metrics only.
+native fused MSE over ``[B, n_base*6]``; lin/ang MSE and cosine similarity are metrics only.  On CUDA
+batches every metric of a step comes from one ``mshgnn_step_metrics_ex`` call (``METRIC_COM``, fp64);
+other inputs take the op-by-op metric classes of ``customMetrics.py``.
 ``rss_stats.npz`` is optional here (identity standardiser when absent); the reference hard-codes
 ``device='cuda:0'`` for it (L52-57), we follow the tensors' device.
 """
@@ -15,7 +17,7 @@ from torch import nn, optim
 from .. import _native as N
 from ..modules import native_loss
 from ._lightning_shim import LightningModule
-from .customMetrics import CosineSimilarityMetric, MeanSquaredError
+from .customMetrics import CosineSimilarityMetric, FusedStepMetrics, MeanSquaredError
 from .gnnLightning import _dims_of
 from .hgnn import COM_HGNN
 from .hgnn_c2_com import COM_HGNN_C2
@@ -57,6 +59,14 @@ class COM_Base_Lightning(LightningModule):
         self.metric_mse_ang = MeanSquaredError(squared=True)
         self.metric_cos_sim_lin = CosineSimilarityMetric()
         self.metric_cos_sim_ang = CosineSimilarityMetric()
+        # CUDA batches: one fused native call per step feeds every metric (mshgnn_step_metrics_ex, METRIC_COM)
+        self._fused = FusedStepMetrics()
+        self.metric_mse.bind(self._fused, lambda e: e[N.COM_SSE] / e[N.COM_N])
+        self.metric_rmse.bind(self._fused, lambda e: torch.sqrt(e[N.COM_SSE] / e[N.COM_N]))
+        self.metric_mse_lin.bind(self._fused, lambda e: e[N.COM_SSE_LIN] / e[N.COM_N_HALF])
+        self.metric_mse_ang.bind(self._fused, lambda e: e[N.COM_SSE_ANG] / e[N.COM_N_HALF])
+        self.metric_cos_sim_lin.bind(self._fused, lambda e: e[N.COM_COS_LIN] / e[N.COM_ROWS])
+        self.metric_cos_sim_ang.bind(self._fused, lambda e: e[N.COM_COS_ANG] / e[N.COM_ROWS])
         self.mse_loss = self.rmse_loss = self.mse_loss_lin = self.mse_loss_ang = None
         self.cos_sim_lin = self.cos_sim_ang = self.avg_cos_sim = self.loss = None
 
@@ -70,19 +80,34 @@ class COM_Base_Lightning(LightningModule):
     def calculate_losses_step(self, y: torch.Tensor, y_pred: torch.Tensor):
         self.mse_loss = native_loss(self.model, y_pred, y, N.LOSS_MSE)
         with torch.no_grad():
-            nb, nd = self.model.num_bases, self.model.num_dimensions_per_base
-            yd, pd = y, y_pred.detach()
-            self.metric_mse(pd.flatten(), yd.flatten())
-            self.rmse_loss = self.metric_rmse(pd.flatten(), yd.flatten())
-            yv = yd.view(yd.shape[0], nb, nd); pv = pd.view(pd.shape[0], nb, nd)
-            self.mse_loss_lin = self.metric_mse_lin(pv[:, :, :3].flatten(), yv[:, :, :3].flatten())
-            self.mse_loss_ang = self.metric_mse_ang(pv[:, :, 3:].flatten(), yv[:, :, 3:].flatten())
-            self.standarizer.to(yd.device)
-            yu = self.standarizer.unstandarize(yv); pu = self.standarizer.unstandarize(pv)
-            self.cos_sim_lin = self.metric_cos_sim_lin(pu[:, 0, :3], yu[:, 0, :3])
-            self.cos_sim_ang = self.metric_cos_sim_ang(pu[:, 0, 3:], yu[:, 0, 3:])
-            self.avg_cos_sim = (self.cos_sim_lin + self.cos_sim_ang) / 2
+            if y_pred.is_cuda and self.model.num_dimensions_per_base == 6:
+                self._metrics_step_fused(y, y_pred.detach())
+            else:
+                self._metrics_step_op_by_op(y, y_pred.detach())
         self.loss = self.mse_loss
+
+    def _metrics_step_fused(self, y, y_pred):
+        """Every metric of the step from one mshgnn_step_metrics_ex call (METRIC_COM, fp64)."""
+        st = self.standarizer
+        if st.y_mean.device != y_pred.device:           # the stats move to the device once
+            st.to(y_pred.device)
+        b = self._fused.update_com(y_pred, y, self.model.num_bases, st.y_mean, st.y_std)
+        b = b[N.COM_RMSE:N.COM_AVG_COS_SIM + 1].clone()         # the fused buffer is overwritten by the next step
+        self.rmse_loss, self.mse_loss_lin, self.mse_loss_ang, self.cos_sim_lin, self.cos_sim_ang, self.avg_cos_sim = b.unbind()
+
+    def _metrics_step_op_by_op(self, yd, pd):
+        """gnnLightning_com.py:L70-95 with the metric classes of customMetrics.py (CPU inputs and other widths)."""
+        nb, nd = self.model.num_bases, self.model.num_dimensions_per_base
+        self.metric_mse(pd.flatten(), yd.flatten())
+        self.rmse_loss = self.metric_rmse(pd.flatten(), yd.flatten())
+        yv = yd.view(yd.shape[0], nb, nd); pv = pd.view(pd.shape[0], nb, nd)
+        self.mse_loss_lin = self.metric_mse_lin(pv[:, :, :3].flatten(), yv[:, :, :3].flatten())
+        self.mse_loss_ang = self.metric_mse_ang(pv[:, :, 3:].flatten(), yv[:, :, 3:].flatten())
+        self.standarizer.to(yd.device)
+        yu = self.standarizer.unstandarize(yv); pu = self.standarizer.unstandarize(pv)
+        self.cos_sim_lin = self.metric_cos_sim_lin(pu[:, 0, :3], yu[:, 0, :3])
+        self.cos_sim_ang = self.metric_cos_sim_ang(pu[:, 0, 3:], yu[:, 0, 3:])
+        self.avg_cos_sim = (self.cos_sim_lin + self.cos_sim_ang) / 2
 
     def calculate_losses_epoch(self) -> None:
         self.mse_loss = self.metric_mse.compute()

@@ -12,6 +12,13 @@ arguments, same return values, the reference's checkpoint policy (``ModelCheckpo
 * datasets are ``WindowSubset``s of a ``DeviceSequence`` (ms_hgnn.windows) instead of ``torch.utils.data.Subset``s of a
   ``FlexibleDataset``: a batch is a tensor of window indices and is collated on the GPU.
 * the optimisation step is the fused native step (``FusedTrainer``), not autograd + ``torch.optim``.
+
+Centre-of-mass momentum (the Solo12 formats ``heterogeneous_gnn_{k4,c2,s4}_com``) goes through the same loops with
+``COM_HGNN_SYM_Lightning(model_type=<format>, data_path=data_path)``; ``data_path/processed/rss_stats.npz`` supplies the
+label standardiser when it exists.  Three choices for COM could not be checked against the reference's own code and follow
+the regression branch of these loops: the monitor ``val_MSE_loss``, the checkpoint name ``epoch=E-val_MSE_loss=x.xxxxx.ckpt``
+(no second metric: COM logs no ``val_L1_loss``) and ``evaluate_model``'s return tuple ``(pred, labels, mse, rmse, mse_lin,
+mse_ang, cos_sim_lin, cos_sim_ang)``, in the order ``COM_Base_Lightning`` computes them.
 """
 from __future__ import annotations
 
@@ -28,6 +35,7 @@ from ..synthetic import HeteroBatch
 from ..train import FusedTrainer
 
 _HGNN_FORMATS = ("heterogeneous_gnn", "heterogeneous_gnn_k4", "heterogeneous_gnn_c2")
+_COM_FORMATS = ("heterogeneous_gnn_k4_com", "heterogeneous_gnn_c2_com", "heterogeneous_gnn_s4_com")
 
 
 class WindowSubset:
@@ -53,8 +61,13 @@ def _loader(subset: WindowSubset, batch_size: int, shuffle: bool, generator: Opt
 
 
 def _build_module(model_type, hidden_size, num_layers, data_metadata, dummy_batch, optimizer, lr, regression, symmetry_mode,
-                  group_operator_path, grf_body_to_world_frame, grf_dimension):
+                  group_operator_path, grf_body_to_world_frame, grf_dimension, data_path):
     from . import gnnLightning as G
+    if model_type in _COM_FORMATS:
+        from .gnnLightning_com import COM_HGNN_SYM_Lightning
+        return COM_HGNN_SYM_Lightning(hidden_channels=hidden_size, num_layers=num_layers, data_metadata=data_metadata,
+                                      dummy_batch=dummy_batch, optimizer=optimizer, lr=lr, symmetry_mode=symmetry_mode,
+                                      group_operator_path=group_operator_path, model_type=model_type, data_path=data_path)
     if model_type == "heterogeneous_gnn":
         return G.Heterogeneous_GNN_Lightning(hidden_channels=hidden_size, num_layers=num_layers, data_metadata=data_metadata,
                                              dummy_batch=dummy_batch, optimizer=optimizer, lr=lr, regression=regression,
@@ -147,15 +160,20 @@ def train_model(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dat
                 train_percentage_to_log=None, symmetry_mode: str = None, group_operator_path: str = None,
                 subfoler_name: str = "default", data_path: Path = None, wandb_api_key: str = None,
                 grf_body_to_world_frame: bool = True, grf_dimension: int = 3, ckpt_path: str = None) -> str:
-    """Train with the reference's ``train_model`` contract (gnnLightning.py:L1099-1421).  Returns the checkpoint folder."""
+    """Train with the reference's ``train_model`` contract (gnnLightning.py:L1099-1421).  Returns the checkpoint folder.
+
+    COM formats build ``COM_HGNN_SYM_Lightning`` (a regression model whatever ``regression`` says) and monitor ``val_MSE_loss``;
+    ``data_path`` is where its standardiser statistics are looked up (module docstring: what is not checked against the
+    reference)."""
     fmts = [train_dataset.dataset.get_data_format(), val_dataset.dataset.get_data_format()]
     if not disable_test:
         fmts.append(test_dataset.dataset.get_data_format())
     if len(set(fmts)) != 1:
         raise ValueError("Data formats of datasets don't match")
     model_type = fmts[0]
-    if model_type not in _HGNN_FORMATS:
+    if model_type not in _HGNN_FORMATS + _COM_FORMATS:
         raise ValueError("Invalid model type.")
+    com = model_type in _COM_FORMATS
     if not 1 <= hidden_size <= 128:
         # narrower models run zero-padded on the 128-channel kernels; wider ones have no kernels
         raise ValueError(f"hidden_size={hidden_size}: the B200-native path supports hidden_size 1..128")
@@ -170,7 +188,7 @@ def train_model(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dat
     dummy_idx = _loader(train_dataset, batch_size, True, gen, 1)[0]
     dummy_batch = ds.batch(dummy_idx)
     module = _build_module(model_type, hidden_size, num_layers, data_metadata, dummy_batch, optimizer, lr, regression, symmetry_mode,
-                           group_operator_path, grf_body_to_world_frame, grf_dimension).to(ds.device)
+                           group_operator_path, grf_body_to_world_frame, grf_dimension, data_path).to(ds.device)
     module.model.validate_edges = "cached"
     n_params = sum(p.numel() for p in module.model.parameters() if p.requires_grad)
 
@@ -189,7 +207,7 @@ def train_model(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dat
     log_f.write(json.dumps({"config": {"batch_size": batch_size, "normalize": normalize, "num_parameters": n_params, "seed": seed,
                                        "train_percentage": train_percentage_to_log, "model_type": model_type}}) + "\n")
 
-    if regression:
+    if regression or com:
         monitor, second = "val_MSE_loss", "val_L1_loss"
     else:
         monitor, second = "val_CE_loss", "val_F1_Score_Leg_Avg"
@@ -257,7 +275,9 @@ def evaluate_model(path_to_checkpoint: Path, predict_dataset: WindowSubset, enab
                    batch_size: int = 100, task_type: str = "regression"):
     """Run a checkpoint over ``predict_dataset`` (gnnLightning.py:L913-1095): returns ``(pred, labels, *metrics)`` -
     classification: 16-class predictions / labels, accuracy, F1 of the four legs and their average; regression: predictions,
-    labels, MSE, RMSE, L1.  Works on reference checkpoints (``epoch=..ckpt`` from Lightning) and on ``train_model``'s."""
+    labels, MSE, RMSE, L1; COM: predictions, labels, MSE, RMSE, lin MSE, ang MSE, lin and ang cosine similarity.  Works on
+    reference checkpoints (``epoch=..ckpt`` from Lightning) and on ``train_model``'s.  For COM, ``data_path`` (when given)
+    replaces the one stored in the checkpoint as the place of ``processed/rss_stats.npz``."""
     from . import gnnLightning as G
     ds = predict_dataset.dataset
     model_type = ds.get_data_format()
@@ -266,6 +286,12 @@ def evaluate_model(path_to_checkpoint: Path, predict_dataset: WindowSubset, enab
     elif model_type == "heterogeneous_gnn_k4":
         model = G.HGNN_K4_Lightning.load_from_checkpoint(str(path_to_checkpoint), symmetry_mode=symmetry_mode,
                                                          group_operator_path=group_operator_path, strict=False)
+    elif model_type in _COM_FORMATS:
+        from .gnnLightning_com import COM_HGNN_SYM_Lightning
+        kw = {"data_path": data_path} if data_path is not None else {}
+        model = COM_HGNN_SYM_Lightning.load_from_checkpoint(str(path_to_checkpoint), symmetry_mode=symmetry_mode,
+                                                            group_operator_path=group_operator_path, model_type=model_type,
+                                                            strict=False, **kw)
     elif model_type == "heterogeneous_gnn_c2":
         cls = G.HGNN_C2_Lightning_Reg if task_type == "regression" else G.HGNN_C2_Lightning_Cls
         kw = dict(grf_body_to_world_frame=grf_body_to_world_frame, grf_dimension=grf_dimension) if task_type == "regression" else {}
@@ -317,4 +343,6 @@ def evaluate_model(path_to_checkpoint: Path, predict_dataset: WindowSubset, enab
         return pred, lab, model.acc, model.f1_leg0, model.f1_leg1, model.f1_leg2, model.f1_leg3, avg
     if world:
         return pred, lab, model.mse_loss_worldframe, model.rmse_loss_worldframe, model.l1_loss_worldframe
+    if model_type in _COM_FORMATS:
+        return pred, lab, model.mse_loss, model.rmse_loss, model.mse_loss_lin, model.mse_loss_ang, model.cos_sim_lin, model.cos_sim_ang
     return pred, lab, model.mse_loss, model.rmse_loss, model.l1_loss
