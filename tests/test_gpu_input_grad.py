@@ -4,13 +4,11 @@ The oracle's x.grad (fp64 autograd through the reference ops) is the checker.  L
 is discontinuous in the forward numerics (ReLU), so the strict bound (1e-4 norm-wise per node type) holds under the ReLU sign
 pattern the native forward took; the plain (unforced) error is printed next to it.
 """
-import contextlib
-
 import pytest
 import torch
 
-import mshgnn_oracle as O
-from helpers import TOL_FP32, native_relu_pattern, oracle_loss, oracle_model, rel_err
+from helpers import (TOL_FP32, forced_native_pattern, native_relu_pattern, oracle_grads_with_forced, oracle_model, oracle_run,
+                     rel_err)
 from ms_hgnn import _native as N
 from ms_hgnn.synthetic import CONFIGS, build_model, make_batch
 
@@ -24,36 +22,6 @@ CASES = [
     ("mini_cheetah-k4-contact", 2400, 8), ("mini_cheetah-c2-contact", 96, 8), ("a1-c2-grf", 64, 8), ("k4-grf-regression", 130, 8),
     ("solo12-k4-com", 257, 8), ("solo-c2-com", 33, 4), ("mi-grf", 20, 8), ("mi-contact", 30, 8), ("mi-com", 77, 2),
 ]
-
-
-def oracle_x_grads(cfg, model, batch, forced=None):
-    leaves = {k: v.double().clone().requires_grad_() for k, v in batch.x_dict.items()}
-    model.zero_grad()
-    with (O.ReluTap(forced=forced) if forced is not None else contextlib.nullcontext()):
-        out = model(dict(leaves), batch.edge_index_dict)
-        loss = oracle_loss(cfg, out, batch.y.double(), batch.batch_size)
-        loss.backward()
-    return out.detach(), {k: (v.grad if v.grad is not None else torch.zeros_like(v)) for k, v in leaves.items()}
-
-
-def forced_native_pattern(model, batch, native_model, fwd_err):
-    """The native forward's ReLU signs where they differ from the oracle's (only at numerically ambiguous pre-activations),
-    in the form O.ReluTap(forced=...) takes (the construction of helpers.gradient_check_under_native_pattern)."""
-    pattern = native_relu_pattern(native_model, batch.batch_size)
-    with torch.no_grad(), O.ReluTap(record=True) as tap:
-        model({k: v.double() for k, v in batch.x_dict.items()}, batch.edge_index_dict)
-    forced, flips = {}, 0
-    for i, (pre, tag) in enumerate(zip(tap.pre, tap.tags)):
-        bits, live = pattern[tag]
-        v = pre.detach()
-        diff = ((v > 0) != bits) & live[:, None]
-        if diff.any():
-            thr = 16.0 * max(fwd_err, 1e-7) * v.pow(2).mean().sqrt().item()
-            assert v.abs()[diff].max().item() <= thr, f"native ReLU pattern differs from the oracle at a non-ambiguous pre-activation ({tag})"
-            idx = torch.nonzero(diff.reshape(-1)).reshape(-1)
-            forced[i] = (idx, bits.reshape(-1)[idx])
-            flips += int(idx.numel())
-    return forced, flips
 
 
 def native_step(cfg, nm, batch, x_dtype=torch.float32, which=None, freeze=False):
@@ -84,11 +52,12 @@ def check_input_grads(cfg, B, layers, mode, x_dtype=torch.float32, freeze=False)
     om, nm = models(cfg, layers)
     nm = nm.set_mode(mode).to("cuda:0")
     out_n, dx_n = native_step(cfg, nm, batch, x_dtype, freeze=freeze)
-    out_o, dx_plain = oracle_x_grads(cfg, om, batch)
+    out_o, _, _, dx_plain = oracle_run(cfg, om, batch, x_grad=True)
     e_out = rel_err(out_n, out_o)
     assert e_out <= TOL_FP32
-    forced, flips = forced_native_pattern(om, batch, nm, e_out)
-    _, dx_o = oracle_x_grads(cfg, om, batch, forced)
+    forced, flips, ratio, error = forced_native_pattern(om, batch, native_relu_pattern(nm, B), e_out)
+    assert error is None and ratio <= 1.0, (error, "native ReLU pattern differs from the oracle at a non-ambiguous pre-activation", ratio)
+    _, dx_o = oracle_grads_with_forced(cfg, om, batch, forced, x_grad=True)
     worst, plain = 0.0, 0.0
     for k in dx_o:
         assert dx_n[k] is not None and dx_n[k].dtype == x_dtype and dx_n[k].shape == batch.x_dict[k].shape, k
@@ -232,7 +201,8 @@ def test_input_grad_across_stack_kernels_and_steps(name, B, restore_options):
 @pytest.mark.parametrize("mode", ["tc", "fp32"])
 def test_full_size_properties_16384_graphs(mode):
     """16384 K4 Mini Cheetah graphs: shard invariance (the full batch's dx x 2 against its two shards', mean loss), K4
-    equivariance of dx, and the first 64 graphs against the fp64 oracle."""
+    equivariance of dx, and every graph against the fp64 oracle (test_gpu_large_batch.check_training_batch: x.grad and every
+    parameter gradient under the native ReLU pattern, and every row tile of 128 graphs on its own)."""
     from ms_hgnn import morphology as M
     from ms_hgnn.synthetic import HeteroBatch
     cfg = CONFIGS["mini_cheetah-k4-contact"]
@@ -275,11 +245,6 @@ def test_full_size_properties_16384_graphs(mode):
     for k in dx_g:
         e = rel_err(dx_g[k], want[k])
         assert e <= TOL_FP32, (k, e)
-    # the full batch's rows of the first 64 graphs against the fp64 oracle on those graphs alone (mean loss: x B / 64)
-    head = batch.shard(0, 256)
-    _, do = oracle_x_grads(cfg, om, head)
-    for t, k in enumerate(nm.node_types):
-        rows = 64 * nm._last_engine.spec["nodes_per_graph"][t]
-        e = rel_err(dx[k][:rows] * (B // 64), do[k])
-        print(f"input grad, first 64 graphs [{mode}] {k}: {e:.2e}")
-        assert e <= PLAIN_BOUND, (k, e)
+    # every graph against the fp64 oracle
+    from test_gpu_large_batch import check_training_batch
+    check_training_batch(cfg, nm, om, batch.to("cuda:0"), mode, "input grad full-size properties")

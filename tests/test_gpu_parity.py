@@ -191,15 +191,15 @@ def test_equivariance_k4_contact():
 
 @pytest.mark.parametrize("mode", ["tc", "fp32"])
 def test_full_size_properties_16384_graphs(mode):
-    """BASELINE.json's full batch (16384 K4 Mini Cheetah graphs, L = 8) through size-independent properties, because the fp64
-    oracle takes minutes at this size:
+    """BASELINE.json's full batch (16384 K4 Mini Cheetah graphs, L = 8) through size-independent properties and the oracle:
       (i)   shard invariance - graphs are independent, so the predictions of the full batch equal, bit for bit, the predictions
             of its two data-parallel shards (different tile / CTA assignment, same per-row arithmetic);
       (ii)  gradient additivity - the flat gradient of the mean loss over the batch equals the shard gradients weighted by the
             shard sizes (what the one all-reduce of SURVEY 8e relies on), to 2e-5 norm-wise per tensor (the sums over graphs are
             split differently);
       (iii) K4 equivariance of the predictions under gs (LinTzuYaunDataset_Morph.py:L349-408) at the mode's tolerance;
-      (iv)  the first 64 graphs against the fp64 oracle run on those 64 graphs alone."""
+      (iv)  every graph against the fp64 oracle (run on the GPU in chunks): outputs, loss, every gradient and x.grad under the
+            native ReLU pattern, and every row tile of 128 graphs on its own (test_gpu_large_batch.check_training_batch)."""
     from ms_hgnn import morphology as M
     cfg = CONFIGS["mini_cheetah-k4-contact"]
     B = 16384
@@ -252,8 +252,6 @@ def test_full_size_properties_16384_graphs(mode):
         y_g = nm(gb.x_dict, gb.edge_index_dict).reshape(B, 4, 2)
     y_ref = out_full.reshape(B, 4, 2)[:, g["permutation_Q_ls"][0]]
     assert rel_err(y_g, y_ref) <= TOL_FP32
-    # (iv) oracle on the first 64 graphs
-    from helpers import oracle_run
-    head = batch.shard(0, 256)
-    out_o, _, _ = oracle_run(cfg, om, head)
-    assert rel_err(out_full[: 64 * 4], out_o) <= TOL_FP32
+    # (iv) every graph against the oracle
+    from test_gpu_large_batch import check_training_batch
+    check_training_batch(cfg, nm, om, batch.to("cuda:0"), mode, "full-size properties")

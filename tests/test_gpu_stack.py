@@ -193,14 +193,16 @@ def test_cached_validation_checks_a_tensor_once():
         assert N.launch_count() - n0 == a + 1
 
 
-@pytest.mark.parametrize("name,B", [("mini_cheetah-k4-contact", 2400), ("mini_cheetah-c2-contact", 1100), ("mini_cheetah-k4-contact", 96)])
+@pytest.mark.parametrize("name,B", [("mini_cheetah-k4-contact", 2400), ("mini_cheetah-c2-contact", 1100), ("mini_cheetah-k4-contact", 96),
+                                    ("mini_cheetah-k4-contact", 70001)])
 def test_encoder_kernels_are_bit_identical(name, B):
     """Encoder forward: persistent TMA-fed kernel (one / two row tiles per item; 2400 and 1100 graphs end on a one-tile item and give
-    some CTAs several items) against the one-item-per-CTA kernels, and the encoder weight gradient with TMA-fed against register-staged
-    feature rows: same bits in the predictions, the loss and EVERY gradient (all variants accumulate the same products in the same
-    order; hgnn_k4.py:L159-160 and its autograd)."""
+    some CTAs several items; 70001 graphs give every CTA many items and take the CTA-pair stack kernel) against the one-item-per-CTA
+    kernels, and the encoder weight gradient with TMA-fed against register-staged feature rows: same bits in the predictions, the loss
+    and EVERY gradient (all variants accumulate the same products in the same order; hgnn_k4.py:L159-160 and its autograd)."""
+    from test_gpu_large_batch import device_batch
     cfg = CONFIGS[name]
-    b = make_batch(cfg, B, seed=B + 7).to("cuda:0")
+    b = device_batch(cfg, B, seed=B + 7) if B > 16384 else make_batch(cfg, B, seed=B + 7).to("cuda:0")
     nm = build_model(cfg, layers=8, seed=5).set_mode("tc").to("cuda:0")
     ref = None
     try:
