@@ -164,6 +164,33 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B,
 int mshgnn_input_grad(const mshgnn_plan* plan, int64_t B, const float* params, float* const* dx,
                       void* workspace, int64_t workspace_bytes, int32_t mode, void* stream);
 
+/* ---- model batches: M >= 1 independent models of one plan in every launch of a step -----------------------------------
+ * Model m has its own parameters (row m of params / grads [M, param_count]), its own B graphs (rows [m*B, (m+1)*B) of
+ * x[t] [M*B*nodes_per_graph[t], in_width[t]], i.e. model-major), its own outputs (rows [m*out_rows(B), (m+1)*out_rows(B))
+ * of out) and labels, and its own loss: loss_out[m] is the mean over its outputs and its dout is scaled by
+ * loss_scale / n_m, exactly as mshgnn_loss on its rows.  Everything model m gets is bit for bit what the single-model calls
+ * give for its parameters and graphs: the per-model reductions keep the splits of a B-graph call.  The single-model entry
+ * points above are M = 1.  M > 1 needs a tensor-core mode (MSHGNN_MODE_TC / MODE_TC_1X) and the cross-layer stack kernel
+ * (option "stack" on); otherwise, and for M < 1, these return MSHGNN_ERR_ARG (-1 for the workspace query) before any
+ * device work; M is at most 1023.  mshgnn_input_grad has no model-batch form and must not follow a model-batch backward on the
+ * same workspace (it would read that workspace with the single-model layout).  mshgnn_adam_step / mshgnn_sgd_step on M*param_count elements
+ * are M independent optimizers. */
+int64_t mshgnn_workspace_bytes_models(const mshgnn_plan* plan, int64_t M, int64_t B, int32_t train, int32_t mode);
+int mshgnn_forward_models(const mshgnn_plan* plan, int64_t M, int64_t B,
+                          const void* const* x, int32_t x_dtype,
+                          const float* params, float* out,
+                          void* workspace, int64_t workspace_bytes,
+                          int32_t train, int32_t mode, void* stream);
+int mshgnn_loss_models(const mshgnn_plan* plan, int64_t M, int64_t B, int32_t loss_kind,
+                       const float* out, const void* labels, int32_t label_dtype,
+                       float loss_scale, float* loss_out, float* dout,
+                       void* workspace, int64_t workspace_bytes, void* stream);
+int mshgnn_backward_models(const mshgnn_plan* plan, int64_t M, int64_t B,
+                           const void* const* x, int32_t x_dtype,
+                           const float* params, const float* dout, float* grads,
+                           void* workspace, int64_t workspace_bytes,
+                           int32_t mode, void* stream, void* layers_ready_event);
+
 /* Fused Adam on flat buffers (torch.optim.Adam defaults semantics, gnnLightning.py:L258-265):
  * step is the 1-based step count after this update. */
 int mshgnn_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq,

@@ -248,7 +248,8 @@ int launch_tc_encoder(const Plan& p, const Launch& L, const WsLayout& w, const B
     if (L.count == 0) return 0;
     static std::atomic<bool> attr_set[64];
     static const int which_env = [] { const char* e = getenv("MSHGNN_ENCODER"); return !e ? 0 : (!strcmp(e, "v1") ? 1 : (!strcmp(e, "pair") ? 2 : 0)); }();   // default: k_tc_encoder_pair; "stream": persistent bulk-copy kernel (kernels_enc.cuh), "v1": one tile per CTA
-    const int which = g_encoder_kernel.load() >= 0 ? g_encoder_kernel.load() : which_env;
+    // a model batch runs the two-tile kernel, the one that knows which model a row tile belongs to (the kernels give identical bits)
+    const int which = w.M > 1 ? 2 : (g_encoder_kernel.load() >= 0 ? g_encoder_kernel.load() : which_env);
     if (first_on_device(attr_set)) {
         CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder, cudaFuncAttributeMaxDynamicSharedMemorySize, ENC_SMEM_BYTES));
         CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder_pair, cudaFuncAttributeMaxDynamicSharedMemorySize, ENCP_SMEM_BYTES));
@@ -258,8 +259,8 @@ int launch_tc_encoder(const Plan& p, const Launch& L, const WsLayout& w, const B
     __half* e_lo = (__half*)(ws + w.wenc16[1]);
     EncMaps maps;
     int rc;
-    if ((rc = make_map_2d(&maps.w_hi, e_hi, (int64_t)p.n_types * H, p.enc_kmax, 64, 128, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-    if ((rc = make_map_2d(&maps.w_lo, e_lo, (int64_t)p.n_types * H, p.enc_kmax, 64, 128, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+    if ((rc = make_map_2d(&maps.w_hi, e_hi, (int64_t)w.M * p.n_types * H, p.enc_kmax, 64, 128, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+    if ((rc = make_map_2d(&maps.w_lo, e_lo, (int64_t)w.M * p.n_types * H, p.enc_kmax, 64, 128, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
     maps.o = wm.tc.o;
     // the persistent kernel copies row fragments with cp.async.bulk: fp32 features, every 64-column fragment 16-byte aligned
     bool stream_ok = xf64 == 0 && L.count <= ENQ_MAX_SLOTS;
@@ -272,7 +273,9 @@ int launch_tc_encoder(const Plan& p, const Launch& L, const WsLayout& w, const B
     if (which == 1) k_tc_encoder<<<dim3(n_row_tiles, (unsigned)L.count), ENC_THREADS, ENC_SMEM_BYTES, st>>>(maps, p.d_tiles + L.begin, bt, br, B, w.Bp, xf64, split);
     else if (which == 2 || !stream_ok) {
         static const int pf = [] { const char* e = getenv("MSHGNN_ENC_PREFETCH"); return e ? atoi(e) : 0; }();     // 1: whole-row L2 prefetch of the feature rows (measured +12 % time: off)
-        k_tc_encoder_pair<<<dim3((n_row_tiles + 1) / 2, (unsigned)L.count), ENC_THREADS, ENCP_SMEM_BYTES, st>>>(maps, p.d_tiles + L.begin, bt, br, B, w.Bp, xf64, split, pf);
+        const unsigned pairs = (unsigned)(w.M * ((w.Bm / TILE_M + 1) / 2));     // per model: its row-tile pairs
+        k_tc_encoder_pair<<<dim3(pairs, (unsigned)L.count), ENC_THREADS, ENCP_SMEM_BYTES, st>>>(maps, p.d_tiles + L.begin, bt, br, B, w.Bp, xf64, split, pf,
+                                                                                          w.Bm, p.n_types * H, p.n_params);
     } else {
         // persistent kernel: one CTA per SM draws (node slot, row-tile pair) items from the counter the forward prologue zeroed
         int n_sm = 0;
@@ -356,9 +359,9 @@ int launch_tc_dw(int kind, const Plan& p, int layer, const Launch& L, const WsLa
             if (p.rpairs[T.pair_begin + j].a_kind != A_SLAB) return fail(MSHGNN_ERR_ARG, "internal: tensor-core weight-gradient task must read slabs");
     }
     ProfScope ps(kind, st);
-    dim3 grid((unsigned)L.count, (unsigned)w.dw_ns[layer]);          // wave-fitted row splits of this layer (ws_layout)
+    dim3 grid((unsigned)L.count, (unsigned)(w.M * w.dw_ns[layer]));          // per model: the wave-fitted row splits of this layer (ws_layout)
     k_tc_reducegemm<<<grid, TC_THREADS, DW_SMEM_BYTES, st>>>(wm.dw, p.d_rtasks, p.d_rpairs, L.begin, br, B, w.Bp, w.dw_rows[layer], w.dw_slot0[layer],
-                                                             split, part_w, part_b);
+                                                             split, part_w, part_b, w.Bm, w.dw_ns[layer], w.part_slots);
     LAUNCH_CHECK();
     return 0;
 }
@@ -429,6 +432,7 @@ int launch_stack(int kind, const Plan& p, const Plan::Stack& sp, const WsLayout&
     if (n_total > 0x7fffffffLL) return fail(MSHGNN_ERR_ARG, "batch too large for one stack launch");
     a.n_total = (int)n_total;
     a.split = split; a.B = B; a.Bp = w.Bp; a.n_slots = p.S;
+    a.tiles_m = (int)(w.Bm / TILE_M); a.w16_rows = p.n_mats16 * H; a.n_params = (int)p.n_params; a.n_derived = (int)p.n_derived;
     a.sync = (uint32_t*)(ws + w.stack_sync);
     a.err = (uint32_t*)(ws + w.stack_sync + w.stack_sync_bytes - 4);
     a.next = (uint32_t*)(ws + w.stack_sync + w.stack_sync_bytes - 8);
@@ -503,10 +507,10 @@ int launch_stack(int kind, const Plan& p, const Plan::Stack& sp, const WsLayout&
 }
 
 // padded plans: caller's gradients of the tensors segs [first, first + count) from the internal 128-wide gradient buffer
-int compact_grads(const Plan& p, int first, int count, const float* in, float* ext, cudaStream_t st) {
+int compact_grads(const Plan& p, int M, int first, int count, const float* in, float* ext, cudaStream_t st) {
     if (count == 0) return 0;
     ProfScope ps(K_PAD, st);
-    k_compact_grads<<<dim3(PAD_BLOCKS_X, (unsigned)count), 256, 0, st>>>(p.d_pad_segs + first, in, ext);
+    k_compact_grads<<<dim3(PAD_BLOCKS_X, (unsigned)count, (unsigned)M), 256, 0, st>>>(p.d_pad_segs + first, in, ext, p.n_params, p.ext.n);
     LAUNCH_CHECK();
     return 0;
 }
@@ -541,11 +545,26 @@ struct Call {
     WsMaps wm;                         // tensor-core modes
 };
 
-int open_call(Call& c, const mshgnn_plan* plan, int64_t B, int train, int32_t mode, void* ws, int64_t ws_bytes) {
-    if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1 (got %lld)", (long long)B);      // before ws_layout, which needs B >= 1
+// What a model batch of M models supports; checked before the device is touched
+int check_models(const Plan& p, int64_t M, int64_t B, int32_t mode) {
+    if (M < 1) return fail(MSHGNN_ERR_ARG, "M must be >= 1 (got %lld)", (long long)M);
+    if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1 (got %lld)", (long long)B);
+    if (M == 1) return 0;
+    if (mode == MSHGNN_MODE_FP32) return fail(MSHGNN_ERR_ARG, "model batches (M = %lld) run in the tensor-core modes only", (long long)M);
+    if (!stack_enabled() || p.stack_infer.prog.n_phases == 0) return fail(MSHGNN_ERR_ARG, "model batches (M = %lld) need the cross-layer stack kernel (option 'stack')", (long long)M);
+    if (M * std::max(p.n_params, p.n_derived) > 0x7fffffffLL || M * p.n_mats16 * H > 0x7fffffffLL || M * B > 0x7fffffffLL)
+        return fail(MSHGNN_ERR_ARG, "model batch of %lld models too large", (long long)M);
+    // grid.y / grid.z of the per-model launches: M x (up to 64 row splits) for the weight-gradient kernels, M elsewhere
+    if (M > 65535 / 64) return fail(MSHGNN_ERR_ARG, "model batch of %lld models: at most %d models per call", (long long)M, 65535 / 64);
+    return 0;
+}
+
+int open_call(Call& c, const mshgnn_plan* plan, int64_t M, int64_t B, int train, int32_t mode, void* ws, int64_t ws_bytes) {
     const Plan& p = plan->p;
+    int rc;
+    if ((rc = check_models(p, M, B, mode))) return rc;      // before ws_layout, which needs B >= 1
     c.p = &p;
-    c.w = ws_layout(p, B, train, mode);
+    c.w = ws_layout(p, B, train, mode, (int)M);
     if (!ws) return fail(MSHGNN_ERR_ARG, "workspace is NULL");
     if (ws_bytes < c.w.total) return fail(MSHGNN_ERR_WORKSPACE, "workspace too small: %lld < %lld bytes", (long long)ws_bytes, (long long)c.w.total);
     if (reinterpret_cast<uintptr_t>(ws) & 255) return fail(MSHGNN_ERR_ARG, "workspace must be 256-byte aligned");
@@ -594,7 +613,7 @@ int launch_tc_encoder_dw(const Call& c, int64_t B, int xf64, cudaStream_t st) {
     // BEFORE its stage is free and nothing is pipelined across register sets, so the scoreboard effect of kernels_enc.cuh costs
     // little, while a landing zone inside the stage serialises copy -> conversion -> MMA per stage.  Off unless MSHGNN_ENC_DW=tma.)
     static const bool want_xt = [] { const char* e = getenv("MSHGNN_ENC_DW"); return e && !strcmp(e, "tma"); }();
-    bool xt = xf64 == 0 && (g_encoder_dw_tma.load() >= 0 ? g_encoder_dw_tma.load() != 0 : want_xt);
+    bool xt = xf64 == 0 && w.M == 1 && (g_encoder_dw_tma.load() >= 0 ? g_encoder_dw_tma.load() != 0 : want_xt);
     for (const EncDwUnit& eu : p.enc_units)
         if (xt) xt = eu.x_buf >= BUF_X0 && eu.x_buf < BUF_X0 + p.n_types && enq_rows_ok(bt.p[eu.x_buf], eu.K, 0);
     EncXMaps xm;
@@ -608,17 +627,17 @@ int launch_tc_encoder_dw(const Call& c, int64_t B, int xf64, cudaStream_t st) {
     float* pe_b = (float*)(c.ws + w.part_enc_b);
     {
         ProfScope ps(K_DW_ENC, st);
-        dim3 grid((unsigned)p.enc_units.size(), (unsigned)w.n_splits_enc);
+        dim3 grid((unsigned)p.enc_units.size(), (unsigned)(w.M * w.n_splits_enc));
         if (xt) k_tc_encoder_dw<true><<<grid, ENC_THREADS, EDW_SMEM_BYTES, st>>>(c.wm.dw, xm, (int)BUF_X0, p.d_enc_units, bt, c.br, B, w.Bp, w.rows_per_enc, w.n_splits_enc, xf64,
-                                                                                 c.split, pe_w, pe_b);
+                                                                                 c.split, pe_w, pe_b, w.Bm);
         else k_tc_encoder_dw<false><<<grid, ENC_THREADS, EDW_SMEM_BYTES, st>>>(c.wm.dw, xm, (int)BUF_X0, p.d_enc_units, bt, c.br, B, w.Bp, w.rows_per_enc, w.n_splits_enc, xf64,
-                                                                               c.split, pe_w, pe_b);
+                                                                               c.split, pe_w, pe_b, w.Bm);
         LAUNCH_CHECK();
     }
     {
         ProfScope ps(K_REDUCE, st);
-        dim3 grid((unsigned)p.enc_groups.size(), 48);
-        k_reduce_enc<<<grid, 256, 0, st>>>(p.d_enc_groups, pe_w, pe_b, w.n_splits_enc, c.grads, 1.f / c.G);
+        dim3 grid((unsigned)p.enc_groups.size(), 48, (unsigned)w.M);
+        k_reduce_enc<<<grid, 256, 0, st>>>(p.d_enc_groups, pe_w, pe_b, w.n_splits_enc, c.grads, 1.f / c.G, (int)p.enc_units.size(), p.n_params);
         LAUNCH_CHECK();
     }
     return 0;
@@ -672,10 +691,16 @@ int mshgnn_param_offset(const mshgnn_plan* plan, int32_t kind, int32_t layer, in
 }
 
 int64_t mshgnn_workspace_bytes(const mshgnn_plan* plan, int64_t B, int32_t train, int32_t mode) {
-    if (!plan || B < 1) return -1;
-    const WsLayout w = ws_layout(plan->p, B, train, mode);
+    return mshgnn_workspace_bytes_models(plan, 1, B, train, mode);
+}
+
+int64_t mshgnn_workspace_bytes_models(const mshgnn_plan* plan, int64_t M, int64_t B, int32_t train, int32_t mode) {
+    if (!plan || M < 1 || B < 1) return -1;
+    if (M > 1 && (check_plan_mode(plan, mode) || check_models(plan->p, M, B, mode))) return -1;
+    const WsLayout w = ws_layout(plan->p, B, train, mode, (int)M);
     if (train && mode != MSHGNN_MODE_FP32 && getenv("MSHGNN_DEBUG_LAYOUT")) {   // weight-gradient row splits per layer launch
-        fprintf(stderr, "mshgnn layout B=%lld: dW default %d x %d rows, %lld partial slots;", (long long)B, w.n_splits_tc, w.rows_per_tc, (long long)w.part_slots);
+        fprintf(stderr, "mshgnn layout M=%d B=%lld Bm=%lld: dW default %d x %d rows, %lld partial slots;", w.M, (long long)B, (long long)w.Bm,
+                w.n_splits_tc, w.rows_per_tc, (long long)w.part_slots);
         for (size_t l = 0; l < plan->p.dw_layer.size(); ++l) fprintf(stderr, " L%zu[%d tasks]: %d x %d", l, plan->p.dw_layer[l].count, w.dw_ns[l], w.dw_rows[l]);
         fprintf(stderr, "; segments");
         for (int i = 0; i < w.segs.n; ++i) fprintf(stderr, " [tasks %d..%d) x %d @ slot %d", w.segs.begin[i], w.segs.begin[i + 1], w.segs.ns[i], w.segs.base[i]);
@@ -713,13 +738,18 @@ int64_t mshgnn_plan_describe(const mshgnn_plan* plan, char* buf, int64_t cap) {
 
 int mshgnn_forward(const mshgnn_plan* plan, int64_t B, const void* const* x, int32_t x_dtype, const float* params,
                    float* out, void* workspace, int64_t workspace_bytes, int32_t train, int32_t mode, void* stream) {
+    return mshgnn_forward_models(plan, 1, B, x, x_dtype, params, out, workspace, workspace_bytes, train, mode, stream);
+}
+
+int mshgnn_forward_models(const mshgnn_plan* plan, int64_t M, int64_t B, const void* const* x, int32_t x_dtype, const float* params,
+                          float* out, void* workspace, int64_t workspace_bytes, int32_t train, int32_t mode, void* stream) {
     int rc;
     if ((rc = check_plan_mode(plan, mode))) return rc;
     const Plan& p = plan->p;
     if (x_dtype != MSHGNN_F32 && x_dtype != MSHGNN_F64 && x_dtype != MSHGNN_F16) return fail(MSHGNN_ERR_ARG, "x_dtype must be F32, F64 or F16");
     if (!x || !params || !out) return fail(MSHGNN_ERR_ARG, "NULL argument");
     Call c;
-    if ((rc = open_call(c, plan, B, train, mode, workspace, workspace_bytes))) return rc;
+    if ((rc = open_call(c, plan, M, B, train, mode, workspace, workspace_bytes))) return rc;
     for (int t = 0; t < p.n_types; ++t)      // before the device is touched
         if (!x[t]) return fail(MSHGNN_ERR_ARG, "x[%d] is NULL", t);
     if ((rc = bind_call(c, params, nullptr, x))) return rc;
@@ -728,7 +758,7 @@ int mshgnn_forward(const mshgnn_plan* plan, int64_t B, const void* const* x, int
     const BufTable& bt = c.bt;
     if (p.padded) {     // every kernel below reads the 128-wide zero-padded copy
         ProfScope ps(K_PAD, st);
-        k_pad_params<<<dim3(PAD_BLOCKS_X, (unsigned)p.pad_segs.size()), 256, 0, st>>>(p.d_pad_segs, params, (float*)c.params);
+        k_pad_params<<<dim3(PAD_BLOCKS_X, (unsigned)p.pad_segs.size(), (unsigned)w.M), 256, 0, st>>>(p.d_pad_segs, params, (float*)c.params, p.ext.n, p.n_params);
         LAUNCH_CHECK();
     }
     params = c.params;
@@ -769,8 +799,9 @@ int mshgnn_forward(const mshgnn_plan* plan, int64_t B, const void* const* x, int
             fp.zero_words = w.stack ? w.stack_sync_bytes / 4 : 0;
             fp.zero_blocks = w.stack ? 16 : 0;
             fp.enc_sync = (uint32_t*)((char*)workspace + w.enc_sync);
+            fp.n_params = p.n_params; fp.n_derived = p.n_derived;
             const unsigned blocks = (unsigned)(fp.n_bias + 8 * fp.n16 + 64 * p.n_types + fp.zero_blocks);
-            k_fwd_prologue<<<blocks, 256, 0, st>>>(fp, params, (float*)bt.p[BUF_DERIVED], w_hi, w_lo, (__half*)((char*)workspace + w.wenc16[0]),
+            k_fwd_prologue<<<dim3(blocks, (unsigned)w.M), 256, 0, st>>>(fp, params, (float*)bt.p[BUF_DERIVED], w_hi, w_lo, (__half*)((char*)workspace + w.wenc16[0]),
                                                     (__half*)((char*)workspace + w.wenc16[1]));
             LAUNCH_CHECK();
         }
@@ -790,8 +821,8 @@ int mshgnn_forward(const mshgnn_plan* plan, int64_t B, const void* const* x, int
         int blocks = (int)((rows + 7) / 8);
         if (blocks > 148 * 8) blocks = 148 * 8;
         ProfScope ps(K_DEC_FWD, st);
-#define MSHGNN_DEC_FWD(CM) k_decoder_fwd<CM><<<blocks, 256, 0, st>>>(p.dec, (const float*)bt.p[BUF_H0 + p.L], image16(c.ws, w, BUF_H0 + p.L, 0), \
-                                              image16(c.ws, w, BUF_H0 + p.L, 1), params, p.d_signs, out, B, w.Bp)
+#define MSHGNN_DEC_FWD(CM) k_decoder_fwd<CM><<<dim3(blocks, (unsigned)w.M), 256, 0, st>>>(p.dec, (const float*)bt.p[BUF_H0 + p.L], image16(c.ws, w, BUF_H0 + p.L, 0), \
+                                              image16(c.ws, w, BUF_H0 + p.L, 1), params, p.d_signs, out, B, w.Bp, w.Bm, p.n_params)
         if (p.dec.C <= 2) MSHGNN_DEC_FWD(2); else if (p.dec.C <= 4) MSHGNN_DEC_FWD(4); else MSHGNN_DEC_FWD(8);
 #undef MSHGNN_DEC_FWD
         LAUNCH_CHECK();
@@ -802,25 +833,32 @@ int mshgnn_forward(const mshgnn_plan* plan, int64_t B, const void* const* x, int
 int mshgnn_loss(const mshgnn_plan* plan, int64_t B, int32_t loss_kind, const float* out, const void* labels,
                 int32_t label_dtype, float loss_scale, float* loss_out, float* dout, void* workspace,
                 int64_t workspace_bytes, void* stream) {
+    return mshgnn_loss_models(plan, 1, B, loss_kind, out, labels, label_dtype, loss_scale, loss_out, dout, workspace, workspace_bytes, stream);
+}
+
+int mshgnn_loss_models(const mshgnn_plan* plan, int64_t M, int64_t B, int32_t loss_kind, const float* out, const void* labels,
+                       int32_t label_dtype, float loss_scale, float* loss_out, float* dout, void* workspace,
+                       int64_t workspace_bytes, void* stream) {
     if (!plan) return fail(MSHGNN_ERR_ARG, "plan is NULL");
     const Plan& p = plan->p;
     if (!out || !labels || !loss_out || !workspace) return fail(MSHGNN_ERR_ARG, "NULL argument");
     if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1");
+    if (M < 1 || M > 65535) return fail(MSHGNN_ERR_ARG, "M must be in 1..65535 (got %lld)", (long long)M);
     if (label_dtype < 0 || label_dtype > 2) return fail(MSHGNN_ERR_ARG, "bad label_dtype");
     if (loss_kind == MSHGNN_LOSS_CE2 && p.C != 2) return fail(MSHGNN_ERR_ARG, "CE2 loss needs out_channels == 2");
     if (loss_kind != MSHGNN_LOSS_CE2 && loss_kind != MSHGNN_LOSS_MSE) return fail(MSHGNN_ERR_ARG, "bad loss_kind");
-    if (workspace_bytes < LOSS_BLOCKS * 8) return fail(MSHGNN_ERR_WORKSPACE, "workspace too small for the loss partials");
+    if (workspace_bytes < M * LOSS_BLOCKS * 8) return fail(MSHGNN_ERR_WORKSPACE, "workspace too small for the loss partials");
     cudaStream_t st = (cudaStream_t)stream;
-    // the loss partials live in the last 256-aligned LOSS_BLOCKS*8 bytes of the workspace
-    double* partial = (double*)((char*)workspace + ((workspace_bytes - LOSS_BLOCKS * 8) & ~(int64_t)255));
+    // the loss partials (LOSS_BLOCKS per model) live in the last 256-aligned M*LOSS_BLOCKS*8 bytes of the workspace
+    double* partial = (double*)((char*)workspace + ((workspace_bytes - M * LOSS_BLOCKS * 8) & ~(int64_t)255));
     const int64_t rows = B * p.dec.n_dec;
     const int64_t n = loss_kind == MSHGNN_LOSS_MSE ? rows * p.C : rows;
     int blocks = (int)((n + 255) / 256);
     if (blocks > LOSS_BLOCKS) blocks = LOSS_BLOCKS;
     ProfScope ps(K_LOSS, st);
-    k_loss_partial<<<blocks, 256, 0, st>>>(loss_kind, out, labels, label_dtype, n, loss_scale / (float)n, dout, partial);
+    k_loss_partial<<<dim3(blocks, (unsigned)M), 256, 0, st>>>(loss_kind, out, labels, label_dtype, n, loss_scale / (float)n, dout, partial);
     LAUNCH_CHECK();
-    k_loss_final<<<1, 32, 0, st>>>(partial, blocks, 1.0 / (double)n, loss_kind == MSHGNN_LOSS_CE2, loss_out);
+    k_loss_final<<<(unsigned)M, 32, 0, st>>>(partial, blocks, 1.0 / (double)n, loss_kind == MSHGNN_LOSS_CE2, loss_out);
     LAUNCH_CHECK();
     return 0;
 }
@@ -833,6 +871,12 @@ int mshgnn_backward(const mshgnn_plan* plan, int64_t B, const void* const* x, in
 int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const* x, int32_t x_dtype, const float* params,
                            const float* dout, float* grads, void* workspace, int64_t workspace_bytes, int32_t mode, void* stream,
                            void* layers_ready_event) {
+    return mshgnn_backward_models(plan, 1, B, x, x_dtype, params, dout, grads, workspace, workspace_bytes, mode, stream, layers_ready_event);
+}
+
+int mshgnn_backward_models(const mshgnn_plan* plan, int64_t M, int64_t B, const void* const* x, int32_t x_dtype, const float* params,
+                           const float* dout, float* grads, void* workspace, int64_t workspace_bytes, int32_t mode, void* stream,
+                           void* layers_ready_event) {
     int rc;
     if ((rc = check_plan_mode(plan, mode))) return rc;
     const Plan& p = plan->p;
@@ -840,7 +884,7 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
     if (!x || !params || !dout) return fail(MSHGNN_ERR_ARG, "NULL argument");
     const bool want_dw = grads != nullptr;      // NULL: input-only backward (the dX chain for mshgnn_input_grad, no weight gradient)
     Call c;
-    if ((rc = open_call(c, plan, B, 1, mode, workspace, workspace_bytes))) return rc;
+    if ((rc = open_call(c, plan, M, B, 1, mode, workspace, workspace_bytes))) return rc;
     if ((rc = bind_call(c, params, grads, x))) return rc;
     float* const grads_out = grads;             // padded plans: the caller's gradients, compacted from c.grads
     grads = c.grads;
@@ -863,11 +907,11 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         if ((rc = stack_sync_reset(w, ws, st))) return rc;
     } else if (w.stack && (reinterpret_cast<uintptr_t>(grads) & 15) == 0) {
         ProfScope ps(K_MEMSET, st);
-        const int64_t n4 = p.n_params / 4;
-        k_bwd_prologue<<<296, 256, 0, st>>>((float4*)grads, n4, grads + n4 * 4, (int)(p.n_params - n4 * 4), (uint32_t*)(ws + w.stack_sync), w.stack_sync_bytes / 4);
+        const int64_t n_all = w.M * p.n_params, n4 = n_all / 4;
+        k_bwd_prologue<<<296, 256, 0, st>>>((float4*)grads, n4, grads + n4 * 4, (int)(n_all - n4 * 4), (uint32_t*)(ws + w.stack_sync), w.stack_sync_bytes / 4);
         LAUNCH_CHECK();
     } else {
-        { ProfScope ps(K_MEMSET, st); CUDA_TRY(cudaMemsetAsync(grads, 0, (size_t)p.n_params * 4, st)); }
+        { ProfScope ps(K_MEMSET, st); CUDA_TRY(cudaMemsetAsync(grads, 0, (size_t)w.M * p.n_params * 4, st)); }
         if ((rc = stack_sync_reset(w, ws, st))) return rc;
     }
 
@@ -881,15 +925,15 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         const int mk = want_dc ? MK_BITS : MK_NONE;
         const void* mbuf = want_dc ? bt.p[BUF_MASK0 + L - 1] : nullptr;
         ProfScope ps(K_DEC_BWD, st);
-#define MSHGNN_DEC_BWD(CM) k_decoder_bwd<CM><<<DEC_BLOCKS, 256, 0, st>>>(p.dec, (const float*)bt.p[BUF_H0 + L], image16(ws, w, BUF_H0 + L, 0), \
+#define MSHGNN_DEC_BWD(CM) k_decoder_bwd<CM><<<dim3(DEC_BLOCKS, (unsigned)w.M), 256, 0, st>>>(p.dec, (const float*)bt.p[BUF_H0 + L], image16(ws, w, BUF_H0 + L, 0), \
                                                   image16(ws, w, BUF_H0 + L, 1), params, p.d_signs, dout, dh, dc, mk, mbuf, dec_part, B, w.Bp, G, \
                                                   want_dh ? image16(ws, w, dhb, 0) : nullptr, want_dh ? image16(ws, w, dhb, 1) : nullptr, \
-                                                  want_dc ? image16(ws, w, dcb, 0) : nullptr, want_dc ? image16(ws, w, dcb, 1) : nullptr)
+                                                  want_dc ? image16(ws, w, dcb, 0) : nullptr, want_dc ? image16(ws, w, dcb, 1) : nullptr, w.Bm, p.n_params)
         if (p.dec.C <= 2) MSHGNN_DEC_BWD(2); else if (p.dec.C <= 4) MSHGNN_DEC_BWD(4); else MSHGNN_DEC_BWD(8);
 #undef MSHGNN_DEC_BWD
         LAUNCH_CHECK();
         if (want_dw) {
-            k_decoder_bwd_reduce<<<p.dec.C * H + p.dec.C, 256, 0, st>>>(p.dec, dec_part, DEC_BLOCKS, grads, 1.f / G);
+            k_decoder_bwd_reduce<<<dim3(p.dec.C * H + p.dec.C, (unsigned)w.M), 256, 0, st>>>(p.dec, dec_part, DEC_BLOCKS, grads, 1.f / G, p.n_params);
             LAUNCH_CHECK();
         }
     }
@@ -901,9 +945,9 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
             // 16..64 splits per element, and that serial chain (not the 117 MB of partials) sets the launch time.  (Four lanes per
             // element over the splits of a task, combined through shared memory, was measured: 2x SLOWER - the chain that matters is
             // the one over the TASKS of a group, one load round trip each.)
-            dim3 grid((unsigned)ngl, 64);
+            dim3 grid((unsigned)ngl, 64, (unsigned)w.M);
             ProfScope ps(K_REDUCE, st);
-            k_reduce_partials<<<grid, 256, 0, st>>>(p.d_groups, part_w, part_b, w.segs, grads, 1.f / G);
+            k_reduce_partials<<<grid, 256, 0, st>>>(p.d_groups, part_w, part_b, w.segs, grads, 1.f / G, w.part_slots, p.n_params);
             LAUNCH_CHECK();
         }
         return 0;
@@ -933,10 +977,10 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         // Every gradient outside the encoder is final here - before the encoder weight gradient, the last 8 % of the step, has
         // even started: the caller's event lets a data-parallel trainer all-reduce that 7.5 MB segment underneath it.
         if ((rc = reduce_layers())) return rc;
-        if (p.padded && want_dw && (rc = compact_grads(p, p.n_pad_enc, (int)p.pad_segs.size() - p.n_pad_enc, grads, grads_out, st))) return rc;
+        if (p.padded && want_dw && (rc = compact_grads(p, w.M, p.n_pad_enc, (int)p.pad_segs.size() - p.n_pad_enc, grads, grads_out, st))) return rc;
         if (layers_ready_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)layers_ready_event, st));
         if (!p.enc_units.empty() && want_dw && (rc = launch_tc_encoder_dw(c, B, xf64, st))) return rc;
-        if (p.padded && want_dw && (rc = compact_grads(p, 0, p.n_pad_enc, grads, grads_out, st))) return rc;
+        if (p.padded && want_dw && (rc = compact_grads(p, w.M, 0, p.n_pad_enc, grads, grads_out, st))) return rc;
     } else {
         auto launch_dw = [&](int kind, const Launch& L) -> int {
             if (L.count == 0 || !want_dw) return 0;
@@ -957,10 +1001,10 @@ int mshgnn_backward_staged(const mshgnn_plan* plan, int64_t B, const void* const
         if (nge > 0 && want_dw) {
             dim3 grid((unsigned)nge, 32);
             ProfScope ps(K_REDUCE, st);
-            k_reduce_partials<<<grid, 256, 0, st>>>(p.d_groups + ngl, part_w, part_b, w.segs, grads, 1.f / G);
+            k_reduce_partials<<<grid, 256, 0, st>>>(p.d_groups + ngl, part_w, part_b, w.segs, grads, 1.f / G, w.part_slots, p.n_params);
             LAUNCH_CHECK();
         }
-        if (p.padded && want_dw && (rc = compact_grads(p, 0, (int)p.pad_segs.size(), grads, grads_out, st))) return rc;
+        if (p.padded && want_dw && (rc = compact_grads(p, w.M, 0, (int)p.pad_segs.size(), grads, grads_out, st))) return rc;
         if (layers_ready_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)layers_ready_event, st));
     }
     return 0;
@@ -973,7 +1017,7 @@ int mshgnn_input_grad(const mshgnn_plan* plan, int64_t B, const float* params, f
     const Plan& p = plan->p;
     if (!params || !dx) return fail(MSHGNN_ERR_ARG, "NULL argument");
     Call c;
-    if ((rc = open_call(c, plan, B, 1, mode, workspace, workspace_bytes))) return rc;
+    if ((rc = open_call(c, plan, 1, B, 1, mode, workspace, workspace_bytes))) return rc;
     DxOut o;
     memset(&o, 0, sizeof o);
     unsigned n_kb = 1;

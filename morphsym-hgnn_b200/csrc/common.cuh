@@ -19,6 +19,7 @@ constexpr int MAX_CHUNKS = 8;
 constexpr int MAX_BUFS = 128;
 constexpr int TILE_M = 128;
 constexpr int DEC_MAXC = 8;     // max decoder width
+constexpr int LOSS_PARTIALS = 592;   // block partials per model of the loss head (plan.cuh LOSS_BLOCKS)
 constexpr float LO_SCALE = 1.f; // scale of the low half of a (hi, lo) fp16 pair: lo = fp16((v - hi) * LO_SCALE)
 
 enum AKind : int { A_SLAB = 0, A_EXT = 1 };

@@ -15,15 +15,17 @@ __device__ __forceinline__ float pad_at(const PadSeg& s, const float* __restrict
 }
 
 // internal[seg] = zero-padded external[seg] for every tensor: every internal element is written, zeros included, so the
-// result does not depend on what an earlier call left in the workspace
+// result does not depend on what an earlier call left in the workspace.  blockIdx.z = model of a model batch (row z of both).
 __global__ void __launch_bounds__(256)
-k_pad_params(const PadSeg* __restrict__ segs, const float* __restrict__ ext, float* __restrict__ in) {
+k_pad_params(const PadSeg* __restrict__ segs, const float* __restrict__ ext, float* __restrict__ in, const int64_t ext_n, const int64_t in_n) {
     const PadSeg s = segs[blockIdx.y];
+    ext += blockIdx.z * ext_n;
+    in += blockIdx.z * in_n;
     const int n = s.rows_i * s.cols_i;                            // < 2^30 (build_plan)
     float* dst = in + s.int_off;
     const int stride = gridDim.x * blockDim.x;
     const int t0 = blockIdx.x * blockDim.x + threadIdx.x;
-    if ((s.cols_i & 3) == 0 && (s.int_off & 3) == 0) {          // four consecutive elements share a row: one 16-byte store
+    if ((s.cols_i & 3) == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {     // four consecutive elements share a row: one 16-byte store
         for (int q = t0; q < n / 4; q += stride) {
             const int r = q * 4 / s.cols_i, c = q * 4 - r * s.cols_i;
             reinterpret_cast<float4*>(dst)[q] = make_float4(pad_at(s, ext, r, c), pad_at(s, ext, r, c + 1), pad_at(s, ext, r, c + 2),
@@ -39,8 +41,10 @@ k_pad_params(const PadSeg* __restrict__ segs, const float* __restrict__ ext, flo
 
 // external[seg] = top-left block of internal[seg] for the tensors segs[0 .. gridDim.y): every external element is written
 __global__ void __launch_bounds__(256)
-k_compact_grads(const PadSeg* __restrict__ segs, const float* __restrict__ in, float* __restrict__ ext) {
+k_compact_grads(const PadSeg* __restrict__ segs, const float* __restrict__ in, float* __restrict__ ext, const int64_t in_n, const int64_t ext_n) {
     const PadSeg s = segs[blockIdx.y];
+    in += blockIdx.z * in_n;
+    ext += blockIdx.z * ext_n;
     const int n = s.rows * s.cols;
     const int stride = gridDim.x * blockDim.x;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {

@@ -356,12 +356,16 @@ k_reducegemm(const RTask* __restrict__ tasks, const RPair* __restrict__ pairs, c
     if (t.want_colsum && tid < H) part_b[((int64_t)task * n_splits + split) * H + tid] = cs;
 }
 
-// sum the split partials of a group of tasks into the flat gradient buffer (fixed order => deterministic)
+// sum the split partials of a group of tasks into the flat gradient buffer (fixed order => deterministic).  blockIdx.z = model of a
+// model batch: its partials start part_slots slots further, its gradients n_params elements further.
 __global__ void __launch_bounds__(256)
 k_reduce_partials(const OutGroup* __restrict__ groups, const float* __restrict__ part_w,
                   const float* __restrict__ part_b, const __grid_constant__ PartSegs segs,
-                  float* __restrict__ grads, const float rscale) {
+                  float* __restrict__ grads, const float rscale, const int64_t part_slots, const int64_t n_params) {
     const OutGroup g = groups[blockIdx.x];
+    part_w += blockIdx.z * part_slots * (H * H);
+    part_b += blockIdx.z * part_slots * H;
+    grads += blockIdx.z * n_params;
     if (g.kind == 0) {
         const int per = (H * H) / gridDim.y;
         for (int e = blockIdx.y * per + threadIdx.x; e < (blockIdx.y + 1) * per; e += 256) {
@@ -428,12 +432,25 @@ k_derive(const DeriveOp* __restrict__ ops, const float* __restrict__ params, flo
 // ------------------------------------------------------------------------------------------
 // decoder: out[g*n_dec + j, c] = (h[slot_j][g] . Wdec[c] + b[c]) * sign[j*C + c]
 // ------------------------------------------------------------------------------------------
+// 4 consecutive weights: one 16-byte load where aligned.  Row m of a model batch's [M, n_params] buffer starts 4 m n_params bytes in,
+// which is 16-byte aligned only when n_params is a multiple of 4.
+__device__ __forceinline__ float4 ld_w4(const float* p) {
+    if ((reinterpret_cast<uintptr_t>(p) & 15) == 0) return __ldg(reinterpret_cast<const float4*>(p));
+    return make_float4(__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3));
+}
+
 // CMAX: compile-time bound of the decoder width (2 / 4 / 8): the weight rows are register arrays, and sized for 8 channels they cost the
 // 2-channel contact head 48 registers it never uses
 template <int CMAX>
 __global__ void __launch_bounds__(256)
 k_decoder_fwd(const DecoderDesc dd, const float* __restrict__ hslab, const __half* __restrict__ h_hi, const __half* __restrict__ h_lo,
-              const float* __restrict__ params, const float* __restrict__ signs, float* __restrict__ out, const int64_t B, const int64_t Bp) {
+              const float* __restrict__ params, const float* __restrict__ signs, float* __restrict__ out, const int64_t B, const int64_t Bp,
+              const int64_t Bm, const int64_t n_params) {
+    // blockIdx.y = model of a model batch: its parameters, its row block [y Bm, y Bm + B) of the slabs, its output rows
+    params += blockIdx.y * n_params;
+    out += blockIdx.y * B * dd.n_dec * dd.C;
+    if (hslab) hslab += blockIdx.y * Bm * H;
+    if (h_hi) { h_hi += blockIdx.y * Bm * H; h_lo += blockIdx.y * Bm * H; }
     const int lane = threadIdx.x & 31;
     const int64_t warp = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
     const int64_t n_rows = B * dd.n_dec;
@@ -441,7 +458,7 @@ k_decoder_fwd(const DecoderDesc dd, const float* __restrict__ hslab, const __hal
     float4 w[CMAX];
 #pragma unroll
     for (int c = 0; c < CMAX; ++c)
-        w[c] = (c < dd.C) ? __ldg(reinterpret_cast<const float4*>(params + dd.w_off + c * H + lane * 4))
+        w[c] = (c < dd.C) ? ld_w4(params + dd.w_off + c * H + lane * 4)
                           : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll 2
     for (int64_t row = warp; row < n_rows; row += stride) {
@@ -472,9 +489,24 @@ k_decoder_bwd(const DecoderDesc dd, const float* __restrict__ hslab, const __hal
               const float* __restrict__ signs, const float* __restrict__ dout,
               float* __restrict__ dh, float* __restrict__ dc, const int mask_kind, const void* __restrict__ mask_buf,
               float* __restrict__ part, const int64_t B, const int64_t Bp, const float gscale,
-              __half* __restrict__ dh_hi, __half* __restrict__ dh_lo, __half* __restrict__ dc_hi, __half* __restrict__ dc_lo) {
+              __half* __restrict__ dh_hi, __half* __restrict__ dh_lo, __half* __restrict__ dc_hi, __half* __restrict__ dc_lo,
+              const int64_t Bm, const int64_t n_params) {
     __shared__ float red[8][CMAX][H + 1];
     __shared__ float redb[8][CMAX];
+    // blockIdx.y = model of a model batch (see k_decoder_fwd); its partials are the next gridDim.x blocks
+    {
+        const int64_t r0 = blockIdx.y * Bm * H;      // the model's first row of every slab / image
+        params += blockIdx.y * n_params;
+        dout += blockIdx.y * B * dd.n_dec * dd.C;
+        part += (int64_t)blockIdx.y * gridDim.x * (DEC_MAXC * H + DEC_MAXC);
+        if (hslab) hslab += r0;
+        if (h_hi) { h_hi += r0; h_lo += r0; }
+        if (dh) dh += r0;
+        if (dc) dc += r0;
+        if (dh_hi) { dh_hi += r0; dh_lo += r0; }
+        if (dc_hi) { dc_hi += r0; dc_lo += r0; }
+        if (mask_buf) mask_buf = (const unsigned*)mask_buf + blockIdx.y * Bm * 4;
+    }
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int64_t warp = (int64_t)blockIdx.x * 8 + wid;
     const int64_t n_rows = B * dd.n_dec;
@@ -483,7 +515,7 @@ k_decoder_bwd(const DecoderDesc dd, const float* __restrict__ hslab, const __hal
     float gb[CMAX];
 #pragma unroll
     for (int c = 0; c < CMAX; ++c) {
-        w[c] = (c < dd.C) ? __ldg(reinterpret_cast<const float4*>(params + dd.w_off + c * H + lane * 4))
+        w[c] = (c < dd.C) ? ld_w4(params + dd.w_off + c * H + lane * 4)
                           : make_float4(0.f, 0.f, 0.f, 0.f);
         gw[c] = make_float4(0.f, 0.f, 0.f, 0.f);
         gb[c] = 0.f;
@@ -519,8 +551,8 @@ k_decoder_bwd(const DecoderDesc dd, const float* __restrict__ hslab, const __hal
             if (dc_hi) { const float vv[4] = {d.x, d.y, d.z, d.w}; split_store4(dc_hi, dc_lo, off, vv); }
         }
     }
-    if (dh_hi || dc_hi) {   // rows [B, Bp) of the decoded slots' fp16 images stay zero
-        const int64_t pad = Bp - B;
+    if (dh_hi || dc_hi) {   // rows [B, Bm) of the model's block of the decoded slots' fp16 images stay zero
+        const int64_t pad = Bm - B;
         const float z[4] = {0.f, 0.f, 0.f, 0.f};
         for (int64_t r = warp; r < pad * dd.n_dec; r += stride) {
             const int64_t off = ((int64_t)dd.slots[r / pad] * Bp + B + r % pad) * H + lane * 4;
@@ -554,9 +586,12 @@ k_decoder_bwd(const DecoderDesc dd, const float* __restrict__ hslab, const __hal
 
 __global__ void __launch_bounds__(256)
 k_decoder_bwd_reduce(const DecoderDesc dd, const float* __restrict__ part, const int n_blocks, float* __restrict__ grads,
-                     const float scale) {
-    // one CTA per output element: thread t sums the partials of blocks t, t + 256, ... (fixed order), then a fixed tree
+                     const float scale, const int64_t n_params) {
+    // one CTA per output element: thread t sums the partials of blocks t, t + 256, ... (fixed order), then a fixed tree;
+    // blockIdx.y = model of a model batch
     __shared__ float sh[256];
+    part += (int64_t)blockIdx.y * n_blocks * (DEC_MAXC * H + DEC_MAXC);
+    grads += blockIdx.y * n_params;
     const int e = blockIdx.x;
     const int src = (e < dd.C * H) ? e : (DEC_MAXC * H + (e - dd.C * H));
     float s = 0.f;
@@ -637,12 +672,20 @@ __device__ __forceinline__ double block_sum(double v, double* sh) {
     return s;   // valid in thread 0
 }
 
-// MSE: n elements; CE2: n rows of 2 logits.  partial[blockIdx.x] = block sum (double)
+// MSE: n elements; CE2: n rows of 2 logits.  partial[blockIdx.x] = block sum (double).  blockIdx.y = model of a model batch:
+// its n elements / rows follow those of the models before it, its partials start LOSS_PARTIALS further.
 __global__ void __launch_bounds__(256)
 k_loss_partial(const int kind, const float* __restrict__ out, const void* __restrict__ labels, const int label_dtype,
                const int64_t n, const float dscale, float* __restrict__ dout, double* __restrict__ partial) {
     __shared__ double sh[8];
     double acc = 0.0;
+    {
+        const int64_t first = blockIdx.y * n;       // the model's first element (MSE) / row (CE2)
+        partial += blockIdx.y * LOSS_PARTIALS;
+        out += kind == 0 ? first : 2 * first;
+        if (dout) dout += kind == 0 ? first : 2 * first;
+        labels = (const char*)labels + first * (label_dtype == 0 ? 4 : 8);
+    }
     for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256) {
         if (kind == 0) {
             const float d = out[i] - (float)ld_label(labels, label_dtype, i);
@@ -668,7 +711,9 @@ k_loss_partial(const int kind, const float* __restrict__ out, const void* __rest
 
 __global__ void k_loss_final(const double* __restrict__ partial, const int n_blocks, const double inv_n,
                              const int round_f32, float* __restrict__ loss_out) {
-    // one warp: lane l sums the partials l, l + 32, ... (fixed order), then a fixed shuffle tree
+    // one warp: lane l sums the partials l, l + 32, ... (fixed order), then a fixed shuffle tree; blockIdx.x = model
+    partial += blockIdx.x * LOSS_PARTIALS;
+    loss_out += blockIdx.x;
     double s = 0.0;
     for (int i = threadIdx.x; i < n_blocks; i += 32) s += partial[i];
 #pragma unroll

@@ -59,6 +59,9 @@ struct StackArgs {
     int n_total;                 // n_row_tiles * prog.items_per_row
     int split;                   // 1: (hi, lo) operands, 3 MMAs per product; 0: hi only
     int64_t B, Bp;
+    // model batch: row tile r belongs to model r / tiles_m, which reads its own weight-image rows (w16_rows per model) and biases
+    // (n_params / n_derived per model); the scheduler warp resolves both, and the model's bound on live rows, once per item
+    int tiles_m, w16_rows, n_params, n_derived;
     uint32_t* sync;              // [n_phases][n_row_tiles][n_slots] completion counters (4 = the four epilogue groups of the producing item)
     uint32_t* err;               // error word (a dependency wait timed out)
     uint32_t* next;              // work counter: the next item index to hand out (zeroed with the completion counters)
@@ -203,7 +206,7 @@ __device__ __forceinline__ void tma_store_wait_pending() { asm volatile("cp.asyn
 // that the single-thread TMA producer never waits for a descriptor load: {first row of the A hi image of the node slot,
 // same for the lo image, first row of the weight image, -}.  `meta` holds one byte per step: chunks | a_stage << 4.
 __device__ __forceinline__ int4 stack_chunk_desc(const Tile* tiles, const int first_tile, const int n_steps, const int meta, const int lane,
-                                                 const BufRows& br, const int64_t Bp) {
+                                                 const BufRows& br, const int64_t Bp, const int w16_add) {
     int cum = 0;
     int4 d = make_int4(0, 0, 0, 0);
     for (int s = 0; s < n_steps && s < 4; ++s) {
@@ -211,7 +214,7 @@ __device__ __forceinline__ int4 stack_chunk_desc(const Tile* tiles, const int fi
         if (lane >= cum && lane < cum + nc) {
             const Chunk* c = &tiles[first_tile + s].chunks[lane - cum];
             const int a_buf = __ldg(&c->a_buf), a_slot = __ldg(&c->a_slot);
-            d = make_int4(br.hi[a_buf] + (int)((int64_t)a_slot * Bp), br.lo[a_buf] + (int)((int64_t)a_slot * Bp), __ldg(&c->w16_row), 0);
+            d = make_int4(br.hi[a_buf] + (int)((int64_t)a_slot * Bp), br.lo[a_buf] + (int)((int64_t)a_slot * Bp), __ldg(&c->w16_row) + w16_add, 0);
         }
         cum += nc;
     }
@@ -233,6 +236,20 @@ __device__ __forceinline__ TileHdr load_hdr(const Tile* t) {
     return h;
 }
 static_assert(sizeof(TileHdr) == 16 * SK_HDR16, "queue header slots must hold a TileHdr");
+static_assert(offsetof(TileHdr, bias_off) == 16, "stack_model_hdr patches bias_off as word x of header vector 1");
+
+// Model of a model batch that row tile `row_tile` (of 128 rows) belongs to
+__device__ __forceinline__ int stack_model(const StackArgs& a, const int row_tile) { return row_tile / a.tiles_m; }
+// Rows of the workspace below this bound are live for an item of model `mdl` (its graphs end there; the rest of its block is padding)
+__device__ __forceinline__ int stack_live_end(const StackArgs& a, const int mdl) { return mdl * a.tiles_m * TILE_M + (int)a.B; }
+// Header vector `v` of a step of model `mdl`: its bias offset moved to that model's parameters / derived bias sums
+__device__ __forceinline__ int4 stack_model_hdr(int4 h, const int v, const Tile* tile, const int mdl, const StackArgs& a) {
+    if (mdl && v == 1) {
+        const int bb = __ldg(&tile->bias_buf);
+        h.x += bb == BUF_PARAMS_ID ? mdl * a.n_params : (bb == BUF_DERIVED_ID ? mdl * a.n_derived : 0);
+    }
+    return h;
+}
 static_assert(sizeof(TileHdr) % 16 == 0 && sizeof(Tile) % 16 == 0, "Tile entries are read with 128-bit loads");
 
 struct StackEpi {
@@ -557,7 +574,7 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
     const long long t_begin = TIMING ? clock64() : 0;
     const StackProg& pg = args.prog;
     const int NT = args.n_row_tiles, RC = args.delay, n_total = args.n_total, split = args.split;
-    const int64_t B = args.B, Bp = args.Bp;
+    const int64_t Bp = args.Bp;
     uint32_t* const err = args.err;
     // Programmatic dependent launch: everything above ran while the previous kernel of the stream was still draining
     asm volatile("griddepcontrol.wait;" ::: "memory");
@@ -584,9 +601,12 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
             if (cur < n_total) {
                 const ItemRef ir = args.chunked ? stack_decode_chunked(pg, NT, RC, cur) : stack_decode(pg, NT, RC, cur);
                 const StackItem it = items[ir.item];
+                const int mdl = stack_model(args, ir.row_tile);
                 // descriptor loads first, dependency wait second: the two global round trips overlap
-                if (lane < SK_QCHUNKS) cd = stack_chunk_desc(tiles, it.tile, it.n_steps, it.meta, lane, br, Bp);
-                if (lane < it.n_steps * SK_HDR16) hd = __ldg(reinterpret_cast<const int4*>(tiles + it.tile + lane / SK_HDR16) + lane % SK_HDR16);
+                if (lane < SK_QCHUNKS) cd = stack_chunk_desc(tiles, it.tile, it.n_steps, it.meta, lane, br, Bp, mdl * args.w16_rows);
+                if (lane < it.n_steps * SK_HDR16)
+                    hd = stack_model_hdr(__ldg(reinterpret_cast<const int4*>(tiles + it.tile + lane / SK_HDR16) + lane % SK_HDR16), lane % SK_HDR16,
+                                         tiles + it.tile + lane / SK_HDR16, mdl, args);
                 if (ir.phase > 0 && it.dep_mask)
                     SK_TIMED(1, stack_wait(args.sync + ((size_t)(ir.phase - 1) * NT + ir.row_tile) * args.n_slots, it.dep_mask, lane, err));
                 a = make_int4(ir.row_tile, ir.phase, it.tile, it.n_steps);
@@ -731,7 +751,8 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
                 const uint32_t a = k % SK_ACCS;
                 es.accum_bar = acc_full0 + 8 * a; es.free_bar = acc_free0 + 8 * a;
                 es.acc_parity = (k / SK_ACCS) & 1;
-                stack_epilogue<PRIV>(t, bt, br, &maps.k, tmem_base + a * 128, qa.x * TILE_M, B, Bp, warp, lane, grp, es, n_res,
+                const int live_end = stack_live_end(args, stack_model(args, qa.x));
+                stack_epilogue<PRIV>(t, bt, br, &maps.k, tmem_base + a * 128, qa.x * TILE_M, live_end, Bp, warp, lane, grp, es, n_res,
                                      s == qa.w - 1 ? ctr : nullptr, pending, args.ws, (TIMING && warp == 2 && lane == 0) ? &tim[5] : nullptr);
             }
         }

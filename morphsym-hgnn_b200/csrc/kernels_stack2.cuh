@@ -151,7 +151,7 @@ k_tc_stack2(const __grid_constant__ TcMaps maps, const __grid_constant__ CUtenso
     constexpr int SPC = H / SK_KB;
     const StackProg& pg = args.prog;
     const int NT = args.n_row_tiles, NP = NT >> 1, RC2 = args.delay, n_total = args.n_total, split = args.split;
-    const int64_t B = args.B, Bp = args.Bp;
+    const int64_t Bp = args.Bp;
     uint32_t* const err = args.err;
     const bool dbg_no_a = args.debug & 1, dbg_no_w = args.debug & 2, dbg_no_mma = args.debug & 4, dbg_bare_epi = args.debug & 8;
     asm volatile("griddepcontrol.wait;" ::: "memory");
@@ -179,16 +179,18 @@ k_tc_stack2(const __grid_constant__ TcMaps maps, const __grid_constant__ CUtenso
                 if (cur < n_total) {
                     const ItemRef ir = args.chunked ? stack_decode_chunked(pg, NP, RC2, cur) : stack_decode(pg, NP, RC2, cur);
                     const StackItem it = items[ir.item];
+                    const int mdl = stack_model(args, 2 * ir.row_tile);      // Bm is a multiple of 256: both row tiles are the model's
                     // descriptors first (they do not depend on the dependency; the slot is invisible until q_count moves),
                     // dependency wait second: the global round trips and the remote stores overlap
                     if (lane < SK_QCHUNKS) {
-                        const int4 d = stack_chunk_desc(tiles, it.tile, it.n_steps, it.meta, lane, br, Bp);
+                        const int4 d = stack_chunk_desc(tiles, it.tile, it.n_steps, it.meta, lane, br, Bp, mdl * args.w16_rows);
                         const uint32_t qc = smem_u32(&q_chunk[slot][lane]);
                         st_cluster_v4(map_to_cta(qc, 0), d);
                         st_cluster_v4(map_to_cta(qc, 1), d);
                     }
                     if (lane < it.n_steps * SK_HDR16) {
-                        const int4 h = __ldg(reinterpret_cast<const int4*>(tiles + it.tile + lane / SK_HDR16) + lane % SK_HDR16);
+                        const int4 h = stack_model_hdr(__ldg(reinterpret_cast<const int4*>(tiles + it.tile + lane / SK_HDR16) + lane % SK_HDR16), lane % SK_HDR16,
+                                                       tiles + it.tile + lane / SK_HDR16, mdl, args);
                         const uint32_t qh = smem_u32(&q_hdr[slot][lane / SK_HDR16][lane % SK_HDR16]);
                         st_cluster_v4(map_to_cta(qh, 0), h);
                         st_cluster_v4(map_to_cta(qh, 1), h);
@@ -355,7 +357,8 @@ k_tc_stack2(const __grid_constant__ TcMaps maps, const __grid_constant__ CUtenso
                 const uint32_t a = k % SK_ACCS;
                 es.accum_bar = acc_full0 + 8 * a; es.free_bar = acc_free0 + 8 * a;
                 es.acc_parity = (k / SK_ACCS) & 1;
-                    stack_epilogue<PRIV>(t, bt, br, &maps.k, tmem_base + a * 128, qa.x * TILE_M, B, Bp, warp, lane, grp, es, n_res, s == qa.w - 1 ? ctr : nullptr,
+                    const int live_end = stack_live_end(args, stack_model(args, qa.x));
+                    stack_epilogue<PRIV>(t, bt, br, &maps.k, tmem_base + a * 128, qa.x * TILE_M, live_end, Bp, warp, lane, grp, es, n_res, s == qa.w - 1 ? ctr : nullptr,
                                    pending, args.ws, nullptr, dbg_bare_epi, args.debug);
             }
         }

@@ -1013,6 +1013,7 @@ k_tc_rowgemm_pair(const __grid_constant__ TcMaps maps, const Tile* __restrict__ 
 //  Accumulators (TMEM columns): D0 [0,128) hi*hi, D1 [128,256) cross terms (x 2^11), D2 [256,272) colsum hi,
 //  D3 [288,304) colsum lo (x 2^11).  One CTA = one task (<= 4 pairs) x one row split; fp32 partials go to part_w /
 //  part_b and are summed in double by k_reduce_partials (deterministic, no atomics).
+constexpr int BUF_PARAMS_ID = 0, BUF_DERIVED_ID = 1;     // plan.cuh BUF_PARAMS, BUF_DERIVED
 constexpr int BUF_DC1_ID = 80;     // plan.cuh BUF_DCL0 - 1: dpre of the encoder (dc_{-1}), written by the layer-0 dX tiles
 
 constexpr int DW_STAGES = 3;
@@ -1038,7 +1039,7 @@ constexpr uint32_t DW_IDESC_CS = (1u << 4) | (1u << 15) | ((16u >> 3) << 17) | (
 __global__ void __launch_bounds__(TC_THREADS, 1)
 k_tc_reducegemm(const __grid_constant__ CUtensorMap map, const RTask* __restrict__ tasks, const RPair* __restrict__ pairs,
                 const int task0, const BufRows br, const int64_t B, const int64_t Bp, const int rows_per, const int slot0 /*first partial slot of this launch*/,
-                const int split, float* __restrict__ part_w, float* __restrict__ part_b) {
+                const int split, float* __restrict__ part_w, float* __restrict__ part_b, const int64_t Bm, const int n_splits, const int64_t part_slots) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ RTask t;
     __shared__ RPair prs[DW_MAX_PAIRS];
@@ -1074,9 +1075,11 @@ k_tc_reducegemm(const __grid_constant__ CUtensorMap map, const RTask* __restrict
     __syncthreads();
     const uint32_t tmem_base = tmem_base_s;
 
-    const int sp = blockIdx.y;
-    const int64_t r_begin = (int64_t)sp * rows_per;
-    const int64_t r_end = (r_begin + rows_per < B) ? (r_begin + rows_per) : B;
+    // blockIdx.y = model x row split: model m reduces its rows [m Bm, m Bm + B) in the splits of a single-model call, into its own partials
+    const int mdl = blockIdx.y / n_splits, sp = blockIdx.y - mdl * n_splits;
+    const int64_t r_first = (int64_t)mdl * Bm;
+    const int64_t r_begin = r_first + (int64_t)sp * rows_per;
+    const int64_t r_end = (r_begin + rows_per < r_first + B) ? (r_begin + rows_per) : r_first + B;
     const int n_kb = r_end > r_begin ? (int)((r_end - r_begin + DW_KB - 1) / DW_KB) : 0;
     const int n_pairs = t.n_pairs < DW_MAX_PAIRS ? t.n_pairs : DW_MAX_PAIRS;
     const int n_steps = n_kb * n_pairs;
@@ -1141,7 +1144,7 @@ k_tc_reducegemm(const __grid_constant__ CUtensorMap map, const RTask* __restrict
         tc_fence_after();
         const int q = warp & 3;
         const int o = q * 32 + lane;
-        const int64_t slot = (int64_t)slot0 + (int64_t)blockIdx.x * gridDim.y + sp;      // gridDim.y = row splits of this launch
+        const int64_t slot = mdl * part_slots + slot0 + (int64_t)blockIdx.x * n_splits + sp;
         float* pw = part_w + slot * (H * H) + (int64_t)o * H;
 #pragma unroll 1
         for (int cc = 0; cc < 4; ++cc) {
@@ -1493,7 +1496,8 @@ constexpr int ENC_PF_BYTES = 1536;                      // first L2 prefetch req
 
 __global__ void __launch_bounds__(ENC_THREADS, 1)
 k_tc_encoder_pair(const __grid_constant__ EncMaps maps, const Tile* __restrict__ tiles, const BufTable bt, const BufRows br,
-                  const int64_t B, const int64_t Bp, const int x_f64, const int split, const int enc_prefetch) {
+                  const int64_t B, const int64_t Bp, const int x_f64, const int split, const int enc_prefetch, const int64_t Bm,
+                  const int enc_rows /*weight-image rows of one model*/, const int64_t n_params) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ Tile t;
     __shared__ __align__(16) float bias_s[H];
@@ -1506,13 +1510,21 @@ k_tc_encoder_pair(const __grid_constant__ EncMaps maps, const Tile* __restrict__
     const uint32_t full0 = smem_u32(bars), empty0 = smem_u32(bars + ENCP_STAGES), accum_bar = smem_u32(bars + 2 * ENCP_STAGES),
                    res_bar = smem_u32(bars + 2 * ENCP_STAGES + 1);
     const uint32_t smem_base = smem_u32(smem);
+    // model of a model batch: blockIdx.x walks the row-tile pairs of model 0's block [0, Bm), then model 1's, ...  Its tile reads
+    // that model's weight-image rows and bias; its graphs are rows [mdl B, mdl B + B) of the caller's feature tensors.
+    const int pairs_m = (int)((Bm / TILE_M + 1) / 2);
+    const int mdl = blockIdx.x / pairs_m;
+    const int64_t m_row0 = (int64_t)mdl * Bm;
     {
         const int* src = reinterpret_cast<const int*>(tiles + blockIdx.y);
         int* dst = reinterpret_cast<int*>(&t);
-        for (int i = tid; i < (int)(sizeof(Tile) / 4); i += ENC_THREADS) dst[i] = src[i];
+        for (int i = tid; i < (int)(sizeof(Tile) / 4); i += ENC_THREADS)
+            dst[i] = src[i] + (i == (int)(offsetof(Tile, bias_off) / 4) ? mdl * (int)n_params : 0)
+                            + (i == (int)((offsetof(Tile, chunks) + offsetof(Chunk, w16_row)) / 4) ? mdl * enc_rows : 0);
     }
-    const int row0 = blockIdx.x * (2 * TILE_M);
-    const int n_tiles = (int64_t)row0 + TILE_M < Bp ? 2 : 1;     // Bp is a multiple of 128, not of 256
+    const int row0 = (int)(m_row0 + (int64_t)(blockIdx.x - mdl * pairs_m) * (2 * TILE_M));
+    const int n_tiles = (int64_t)row0 + TILE_M < m_row0 + Bm ? 2 : 1;     // Bm is a multiple of 128, not of 256
+    const int64_t B_end = m_row0 + B;                                    // rows [B_end, m_row0 + Bm) are padding
     if (tid == 0) {
         // a stage is full when the weight TMA and the four loader warps of every live row tile have arrived
         for (int s = 0; s < ENCP_STAGES; ++s) { mbar_init(full0 + 8 * s, 1 + ENC_LOADER_WARPS * n_tiles); mbar_init(empty0 + 8 * s, 1); }
@@ -1543,8 +1555,8 @@ k_tc_encoder_pair(const __grid_constant__ EncMaps maps, const Tile* __restrict__
             if (byte1 <= byte0) return;
             for (int r = l0; r < n_tiles * TILE_M; r += lstep) {
                 const int64_t row = (int64_t)row0 + r;
-                if (row >= B) break;
-                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<const char*>(xb + row * ch0.lda) + byte0), "r"(byte1 - byte0) : "memory");
+                if (row >= B_end) break;
+                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<const char*>(xb + (row - m_row0 + mdl * B) * ch0.lda) + byte0), "r"(byte1 - byte0) : "memory");
             }
         };
         if (pf_ok) prefetch_rows(0, row_bytes < ENC_PF_BYTES ? row_bytes : ENC_PF_BYTES, lane, 32);
@@ -1595,7 +1607,9 @@ k_tc_encoder_pair(const __grid_constant__ EncMaps maps, const Tile* __restrict__
         const int g = (warp - 2) / ENC_LOADER_WARPS;
         const int gt = tid - 64 - g * (ENC_LOADER_WARPS * 32);
         const Chunk& ch = t.chunks[0];
-        const XRows xr = make_xrows(bt.p[ch.a_buf], x_f64, ch.lda, ch.a_off, K);
+        // workspace row r of this model is the caller's graph r - mdl (Bm - B): shift the base by that many graphs
+        const int esz = x_f64 == 1 ? 8 : (x_f64 == 2 ? 2 : 4);
+        const XRows xr = make_xrows((const char*)bt.p[ch.a_buf] - (int64_t)mdl * (Bm - B) * ch.lda * esz, x_f64, ch.lda, ch.a_off, K);
         const float* signs = (const float*)bt.p[2];
         const int kq = gt & 15;                                   // which 4-column group of the 64-column block
         const int rsub = gt >> 4;                                 // 0..7
@@ -1605,7 +1619,7 @@ k_tc_encoder_pair(const __grid_constant__ EncMaps maps, const Tile* __restrict__
         const int n_units = g < n_tiles ? n_kb * 2 : 0;
         float4 v[ENC_SETS][8];
         auto load = [&](float4 (&v)[8], const int n) {
-            if (n < n_units) load_x_block<8>(v, xr, row_first + (n & 1) * 64, B - 1, (n >> 1) * 64 + kq * 4);
+            if (n < n_units) load_x_block<8>(v, xr, row_first + (n & 1) * 64, B_end - 1, (n >> 1) * 64 + kq * 4);
         };
         auto convert = [&](const float4 (&v)[8], const int n) {
             if (n >= n_units) return;
@@ -1640,7 +1654,7 @@ k_tc_encoder_pair(const __grid_constant__ EncMaps maps, const Tile* __restrict__
             EpiSmem es;
             es.stg = smem_base + (uint32_t)tl * 65536u; es.bias = smem_u32(bias_s); es.res_bar = res_bar; es.accum_bar = accum_bar;
             es.free_bar = 0; es.acc_parity = 0; es.res_parity = 0; es.persistent = 0; es.n_groups = 2;
-            tc_epilogue(t, bt, br, &maps.o, tmem_base + (uint32_t)tl * 128u, row0 + tl * TILE_M, B, Bp, split, warp, lane, es);
+            tc_epilogue(t, bt, br, &maps.o, tmem_base + (uint32_t)tl * 128u, row0 + tl * TILE_M, B_end, Bp, split, warp, lane, es);
         }
     }
     tc_fence_before();
@@ -1684,7 +1698,7 @@ __global__ void __launch_bounds__(ENC_THREADS, 1)
 k_tc_encoder_dw(const __grid_constant__ CUtensorMap map, const __grid_constant__ EncXMaps xmaps, const int x_buf0, const EncDwUnit* __restrict__ units,
                 const BufTable bt, const BufRows br,
                 const int64_t B, const int64_t Bp, const int rows_per, const int n_splits, const int x_f64, const int split,
-                float* __restrict__ part_w, float* __restrict__ part_b) {
+                float* __restrict__ part_w, float* __restrict__ part_b, const int64_t Bm) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ EncDwUnit u;
     __shared__ uint32_t tmem_base_s;
@@ -1718,9 +1732,11 @@ k_tc_encoder_dw(const __grid_constant__ CUtensorMap map, const __grid_constant__
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_s;
 
-    const int sp = blockIdx.y;
-    const int64_t r_begin = (int64_t)sp * rows_per;
-    const int64_t r_end = (r_begin + rows_per < B) ? (r_begin + rows_per) : B;
+    // blockIdx.y = model x row split (as in k_tc_reducegemm); partials of model m follow those of every unit of model m - 1
+    const int mdl = blockIdx.y / n_splits, sp = blockIdx.y - mdl * n_splits;
+    const int64_t r_first = (int64_t)mdl * Bm;
+    const int64_t r_begin = r_first + (int64_t)sp * rows_per;
+    const int64_t r_end = (r_begin + rows_per < r_first + B) ? (r_begin + rows_per) : r_first + B;
     const int n_rb = r_end > r_begin ? (int)((r_end - r_begin + DW_KB - 1) / DW_KB) : 0;
     const int n_steps = n_rb * u.n_slots;
     const int nkb = u.nkb;
@@ -1790,10 +1806,12 @@ k_tc_encoder_dw(const __grid_constant__ CUtensorMap map, const __grid_constant__
         const int gt = tid - 64 - g * (ENC_LOADER_WARPS * 32);
         const float* signs = (const float*)bt.p[2];
         const int kq = gt & 15, rsub = gt >> 4;
+        const int esz = x_f64 == 1 ? 8 : (x_f64 == 2 ? 2 : 4);
+        const char* xbase = (const char*)bt.p[u.x_buf] - (int64_t)mdl * (Bm - B) * u.lda * esz;     // workspace row r -> caller's graph r - mdl (Bm - B)
         for (int i = g; i < n_steps; i += 2) {
             const int s = i % EDW_STAGES;
             const int j = i / n_rb;
-            const XRows xr = make_xrows(bt.p[u.x_buf], x_f64, u.lda, u.a_off[j], u.K);
+            const XRows xr = make_xrows(xbase, x_f64, u.lda, u.a_off[j], u.K);
             const int64_t r0 = r_begin + (int64_t)(i % n_rb) * DW_KB + rsub;
             const uint32_t st = smem_base + s * EDW_STAGE_BYTES + 2 * EDW_DC_BYTES;
             float4 v[3][8];
@@ -1813,7 +1831,7 @@ k_tc_encoder_dw(const __grid_constant__ CUtensorMap map, const __grid_constant__
             } else {
 #pragma unroll
                 for (int jb = 0; jb < 3; ++jb)
-                    if (jb < nkb) load_x_block<8>(v[jb], xr, r0, B - 1, u.k0 + jb * 64 + kq * 4);
+                    if (jb < nkb) load_x_block<8>(v[jb], xr, r0, r_first + B - 1, u.k0 + jb * 64 + kq * 4);
                 mbar_wait(empty0 + 8 * s, ((i / EDW_STAGES) & 1) ^ 1);
             }
 #pragma unroll
@@ -1837,7 +1855,7 @@ k_tc_encoder_dw(const __grid_constant__ CUtensorMap map, const __grid_constant__
             tc_fence_after();
             const int q = warp & 3;
             const int o = q * 32 + lane;
-            const int64_t slot = (int64_t)blockIdx.x * n_splits + sp;
+            const int64_t slot = ((int64_t)mdl * gridDim.x + blockIdx.x) * n_splits + sp;
             float* pw = part_w + slot * (H * EDW_NMAX) + (int64_t)o * EDW_NMAX;
             for (int cc = 0; cc < nkb * 2; ++cc) {
                 uint32_t raw[32];
@@ -1873,8 +1891,12 @@ k_tc_encoder_dw(const __grid_constant__ CUtensorMap map, const __grid_constant__
 // sum the encoder partials of one (type, 192-column range) group into the flat gradient buffer (fixed order, double)
 __global__ void __launch_bounds__(256)
 k_reduce_enc(const EncDwGroup* __restrict__ groups, const float* __restrict__ part_w, const float* __restrict__ part_b,
-             const int n_splits, float* __restrict__ grads, const float rscale) {
+             const int n_splits, float* __restrict__ grads, const float rscale, const int n_units, const int64_t n_params) {
     const EncDwGroup g = groups[blockIdx.x];
+    // blockIdx.z = model of a model batch
+    part_w += (int64_t)blockIdx.z * n_units * n_splits * (H * EDW_NMAX);
+    part_b += (int64_t)blockIdx.z * n_units * n_splits * H;
+    grads += blockIdx.z * n_params;
     const int n = H * g.width;
     for (int e = blockIdx.y * 256 + threadIdx.x; e < n; e += gridDim.y * 256) {
         const int o = e / g.width, i = e % g.width;
@@ -1950,12 +1972,18 @@ struct FwdPrologue {
     EncImgDesc ed; int kmax;
     uint32_t* zero; int64_t zero_words; int zero_blocks;
     uint32_t* enc_sync;          // work counter of k_tc_encoder_stream
-};
+    int64_t n_params, n_derived; // per-model strides of a model batch (blockIdx.y = model); the weight images of a model are n16 x 128
+};                               // rows, its encoder images ed.n_types x 128 rows
 __global__ void __launch_bounds__(256)
 k_fwd_prologue(const FwdPrologue a, const float* __restrict__ params, float* __restrict__ derived, __half* __restrict__ w_hi, __half* __restrict__ w_lo,
                __half* __restrict__ e_hi, __half* __restrict__ e_lo) {
     int b = blockIdx.x;
-    if (b == 0 && threadIdx.x == 0 && a.enc_sync) *a.enc_sync = 0u;
+    const int mdl = blockIdx.y;
+    params += mdl * a.n_params;
+    derived += mdl * a.n_derived;
+    w_hi += (int64_t)mdl * a.n16 * H * H; w_lo += (int64_t)mdl * a.n16 * H * H;
+    e_hi += (int64_t)mdl * a.ed.n_types * H * a.kmax; e_lo += (int64_t)mdl * a.ed.n_types * H * a.kmax;
+    if (b == 0 && mdl == 0 && threadIdx.x == 0 && a.enc_sync) *a.enc_sync = 0u;
     if (b < a.n_bias) {
         const DeriveOp op = a.ops[b];
         const int n = op.rows * op.cols;
@@ -1997,6 +2025,7 @@ k_fwd_prologue(const FwdPrologue a, const float* __restrict__ params, float* __r
         return;
     }
     b -= 64 * a.ed.n_types;
+    if (mdl) return;
     for (int64_t i = (int64_t)b * 256 + threadIdx.x; i < a.zero_words; i += (int64_t)a.zero_blocks * 256) a.zero[i] = 0u;
 }
 

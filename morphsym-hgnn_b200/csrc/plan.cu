@@ -704,12 +704,16 @@ int stack_pair_mode() {
 }
 void set_stack_pair_mode(int v) { g_stack_pair.store(v < 0 ? 0 : (v > 2 ? 2 : v), std::memory_order_relaxed); }
 
-WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode) {
+// Every split below is a function of the per-model batch B alone: model m of a model batch reduces its rows exactly as a
+// single-model call on its B graphs does, so its gradients are bit for bit the same.
+WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode, int M) {
     const bool tc = mode != MSHGNN_MODE_FP32;
     WsLayout w{};
+    w.M = M < 1 ? 1 : M;
     w.stack = tc && stack_enabled() && p.stack_infer.prog.n_phases > 0;
-    w.stack_pair = w.stack && (stack_pair_mode() == 2 || (stack_pair_mode() == 1 && B >= STACK_PAIR_MIN_GRAPHS));
-    w.Bp = round_up(B < 1 ? 1 : B, w.stack_pair ? 2 * TILE_M : TILE_M);      // the CTA-pair kernel walks row tiles two at a time
+    w.stack_pair = w.stack && (stack_pair_mode() == 2 || (stack_pair_mode() == 1 && (int64_t)w.M * B >= STACK_PAIR_MIN_GRAPHS));
+    w.Bm = round_up(B < 1 ? 1 : B, w.stack_pair ? 2 * TILE_M : TILE_M);      // the CTA-pair kernel walks row tiles two at a time
+    w.Bp = (int64_t)w.M * w.Bm;
     int ns = (int)((B + 511) / 512);
     w.n_splits = ns < 1 ? 1 : (ns > 64 ? 64 : ns);
     {   // tcgen05 reduce-GEMM: ~1024 rows per split (MSHGNN_DW_ROWS overrides for A/B runs) (fp32 accumulation in TMEM, splits summed in double), no empty split.
@@ -803,7 +807,7 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode) {
     const int64_t ctb = (int64_t)2 * p.nm * w.Bp * H * 4;
     for (int id = 0; id < MAX_BUFS; ++id) w.buf[id] = w.buf16[id][0] = w.buf16[id][1] = -1;
     w.part_w = w.part_b = w.dec_part = -1;
-    w.buf[BUF_DERIVED] = take(p.n_derived * 4);
+    w.buf[BUF_DERIVED] = take(w.M * p.n_derived * 4);
     // fp32 slabs exist in MODE_FP32 only: the tensor-core modes keep every activation / gradient as (hi, lo) fp16 images
     if (train) {
         if (!tc) {
@@ -821,16 +825,16 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode) {
             for (int l = -1; l < p.L; ++l) w.buf[BUF_DCL0 + l] = dc[(l + 2) & 1];
             for (int l = 0; l < p.L; ++l) w.buf[BUF_DUL0 + l] = du;
         }
-        w.part_w = take(w.part_slots * H * H * 4);
-        w.part_b = take(w.part_slots * H * 4);
-        w.dec_part = take((int64_t)DEC_BLOCKS * (DEC_MAXC * H + DEC_MAXC) * 4);
+        w.part_w = take(w.M * w.part_slots * H * H * 4);
+        w.part_b = take(w.M * w.part_slots * H * 4);
+        w.dec_part = take((int64_t)w.M * DEC_BLOCKS * (DEC_MAXC * H + DEC_MAXC) * 4);
     } else if (!tc) {
         const int64_t a = take(slab), b = take(slab);
         for (int l = 0; l <= p.L; ++l) w.buf[BUF_H0 + l] = (l & 1) ? b : a;
         if (p.morph_sym) { const int64_t c = take(ctb); for (int l = 0; l < p.L; ++l) w.buf[BUF_CT0 + l] = c; }
     }
     if (tc) {
-        for (int i = 0; i < 2; ++i) w.w16[i] = take((int64_t)p.n_mats16 * H * H * 2);
+        for (int i = 0; i < 2; ++i) w.w16[i] = take((int64_t)w.M * p.n_mats16 * H * H * 2);
         if (train) {
             for (int l = 0; l <= p.L; ++l) for (int i = 0; i < 2; ++i) w.buf16[BUF_H0 + l][i] = take(slab / 2);
             if (p.morph_sym)
@@ -862,7 +866,7 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode) {
         }
     }
     if (tc) {
-        for (int i = 0; i < 2; ++i) w.wenc16[i] = take((int64_t)p.n_types * H * p.enc_kmax * 2);
+        for (int i = 0; i < 2; ++i) w.wenc16[i] = take((int64_t)w.M * p.n_types * H * p.enc_kmax * 2);
         w.enc_sync = take(256);
         if (train) {
             // row splits of the encoder weight gradient, fitted to whole waves like the layer-stack ones (16 units for the K4 model:
@@ -882,8 +886,8 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode) {
                 }
             }
             w.n_splits_enc = (int)((B + w.rows_per_enc - 1) / w.rows_per_enc);
-            w.part_enc_w = take((int64_t)p.enc_units.size() * w.n_splits_enc * H * 192 * 4);
-            w.part_enc_b = take((int64_t)p.enc_units.size() * w.n_splits_enc * H * 4);
+            w.part_enc_w = take((int64_t)w.M * p.enc_units.size() * w.n_splits_enc * H * 192 * 4);
+            w.part_enc_b = take((int64_t)w.M * p.enc_units.size() * w.n_splits_enc * H * 4);
         }
     }
     if (w.stack) {
@@ -892,10 +896,10 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode) {
         w.stack_timing = take(256 * 16 * 8);
     }
     if (p.padded) {
-        w.pad_params = take(p.n_params * 4);
-        if (train) w.pad_grads = take(p.n_params * 4);
+        w.pad_params = take(w.M * p.n_params * 4);
+        if (train) w.pad_grads = take(w.M * p.n_params * 4);
     }
-    w.loss_part = take(LOSS_BLOCKS * 8);      // last: mshgnn_loss finds its partials at the end of the caller's workspace
+    w.loss_part = take((int64_t)w.M * LOSS_BLOCKS * 8);      // last: mshgnn_loss finds its partials at the end of the caller's workspace
     w.total = o;
     return w;
 }
@@ -904,7 +908,8 @@ std::string describe_plan(const Plan& p) {
     std::ostringstream os;
     os << "{\"S\":" << p.S << ",\"L\":" << p.L << ",\"hidden\":" << p.hidden << ",\"kernel_hidden\":" << H << ",\"n_params\":" << p.ext.n << ",\"n_derived\":" << p.n_derived
        << ",\"n_tiles\":" << p.tiles.size() << ",\"n_rtasks\":" << p.rtasks.size() << ",\"n_rpairs\":" << p.rpairs.size()
-       << ",\"n_groups\":" << p.groups.size() << ",\"need\":[";
+       << ",\"n_groups\":" << p.groups.size() << ",\"n_mats16\":" << p.n_mats16 << ",\"enc_kmax\":" << p.enc_kmax
+       << ",\"n_types\":" << p.n_types << ",\"need\":[";
     for (int l = 0; l <= p.L; ++l) {
         os << (l ? "," : "") << "[";
         for (int s = 0; s < p.S; ++s) os << (s ? "," : "") << (int)p.need[l][s];

@@ -28,6 +28,7 @@ enum : int {
 };
 constexpr int MAX_LAYERS = 15;
 static_assert(BUF_DCL0 - 1 == 80, "kernels_tc.cuh BUF_DC1_ID names the encoder dpre buffer by number");
+static_assert(BUF_PARAMS == 0 && BUF_DERIVED == 1, "kernels_tc.cuh BUF_PARAMS_ID / BUF_DERIVED_ID name these buffers by number");
 
 struct Launch { int begin = 0, count = 0; };
 
@@ -132,6 +133,10 @@ struct Plan {
 };
 
 struct WsLayout {
+    // A model batch of M models keeps model m's graphs in rows [m Bm, m Bm + B) of every slab, Bm = B padded to the row-tile
+    // granularity of the stack kernel (128, 256 for the CTA-pair kernel), so no row tile belongs to two models.  Bp = M Bm.
+    int M = 1;
+    int64_t Bm = 0;
     int64_t Bp = 0;
     int n_splits = 1;                  // row splits of the SIMT reduce-GEMM (<= 512 rows each)
     int n_splits_tc = 1, rows_per_tc = 64;   // default row splits of the tcgen05 reduce-GEMM (multiples of 64 rows)
@@ -139,7 +144,7 @@ struct WsLayout {
     PartSegs segs;                     // packed partial slots of the weight-gradient tasks (common.cuh)
     int dw_slot0[MAX_LAYERS];          // first partial slot of each layer launch
     int dw_merged = 0;                 // stack mode: one weight-gradient launch for all layers (uniform row splits)
-    int64_t part_slots = 0;            // total slots ([128][128] fp32 weight partial + [128] bias partial each)
+    int64_t part_slots = 0;            // slots of one model ([128][128] fp32 weight partial + [128] bias partial each); model m's follow model m-1's
     // Where every buffer id lives (byte offsets into the workspace, -1 when the call has no such buffer).  ws_layout makes
     // every aliasing decision here: several ids may name one buffer (the ping-pong slabs and images).
     int64_t buf[MAX_BUFS];             // fp32: derived weights, slabs (MODE_FP32) and ReLU bitmasks
@@ -160,10 +165,10 @@ struct WsLayout {
 };
 
 constexpr int DEC_BLOCKS = 1184;     // 148 SMs x 8 resident CTAs of the 2-channel instantiation (48 registers, 8 KB of shared memory; the 8-channel one: 2 per SM): one load in flight per warp, so latency is hidden by warps
-constexpr int LOSS_BLOCKS = 592;
+constexpr int LOSS_BLOCKS = LOSS_PARTIALS;
 
 std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p);   // returns error text ("" = ok)
-WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode);
+WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode, int M = 1);   // B graphs per model
 bool stack_enabled();                 // cross-layer stack kernel on (default) / off (MSHGNN_STACK=0 or mshgnn_set_option)
 void set_stack_enabled(int on);
 int stack_pair_mode();                // CTA-pair (cta_group::2) stack kernel: 1 = by batch size (default), 2 = always, 0 = never (MSHGNN_STACK_2CTA)

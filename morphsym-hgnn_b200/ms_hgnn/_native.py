@@ -38,6 +38,7 @@ EXPORTS = (
     "mshgnn_relu_mask_offset", "mshgnn_build_windows", "mshgnn_step_metrics", "mshgnn_dw_layout",
     "mshgnn_check_edges", "mshgnn_set_option", "mshgnn_get_option", "mshgnn_stack_status", "mshgnn_stack_timing_offset",
     "mshgnn_backward_staged", "mshgnn_input_grad", "mshgnn_plan_create_ex", "mshgnn_step_metrics_ex",
+    "mshgnn_workspace_bytes_models", "mshgnn_forward_models", "mshgnn_loss_models", "mshgnn_backward_models",
 )
 
 
@@ -126,6 +127,12 @@ def lib() -> C.CDLL:
     L.mshgnn_backward_staged.argtypes = [vp, i64, C.POINTER(vp), i32, vp, vp, vp, vp, i64, i32, vp, vp]; L.mshgnn_backward_staged.restype = C.c_int
     if hasattr(L, "mshgnn_input_grad"):          # absent from builds before it (MSHGNN_LIB A/B runs against an older commit)
         L.mshgnn_input_grad.argtypes = [vp, i64, vp, C.POINTER(vp), vp, i64, i32, vp]; L.mshgnn_input_grad.restype = C.c_int
+    if hasattr(L, "mshgnn_forward_models"):      # absent from builds before it (MSHGNN_LIB A/B runs against an older commit)
+        L.mshgnn_workspace_bytes_models.argtypes = [vp, i64, i64, i32, i32]; L.mshgnn_workspace_bytes_models.restype = i64
+        L.mshgnn_forward_models.argtypes = [vp, i64, i64, C.POINTER(vp), i32, vp, vp, vp, i64, i32, i32, vp]; L.mshgnn_forward_models.restype = C.c_int
+        L.mshgnn_loss_models.argtypes = [vp, i64, i64, i32, vp, vp, i32, f32, vp, vp, vp, i64, vp]; L.mshgnn_loss_models.restype = C.c_int
+        L.mshgnn_backward_models.argtypes = [vp, i64, i64, C.POINTER(vp), i32, vp, vp, vp, vp, i64, i32, vp, vp]
+        L.mshgnn_backward_models.restype = C.c_int
     L.mshgnn_adam_step.argtypes = [vp, vp, vp, vp, i64, i64, f32, f32, f32, f32, f32, vp]; L.mshgnn_adam_step.restype = C.c_int
     L.mshgnn_sgd_step.argtypes = [vp, vp, i64, f32, vp]; L.mshgnn_sgd_step.restype = C.c_int
     L.mshgnn_plan_describe.argtypes = [vp, C.c_char_p, i64]; L.mshgnn_plan_describe.restype = i64
@@ -251,6 +258,14 @@ class NativePlan:
             raise RuntimeError("mshgnn_workspace_bytes failed")
         return n
 
+    def workspace_bytes_models(self, M: int, B: int, train: bool, mode: int) -> int:
+        """Workspace of a model batch of M models with B graphs each (mshgnn_workspace_bytes_models)."""
+        n = int(lib().mshgnn_workspace_bytes_models(self.handle, M, B, int(train), mode))
+        if n < 0:
+            raise RuntimeError(f"mshgnn_workspace_bytes_models failed: no model batch of {M} x {B} graphs in mode {mode} "
+                               "(M > 1 needs a tensor-core mode and the stack kernel)")
+        return n
+
     def dw_layout(self, B: int, mode: int = MODE_TC):
         """Per layer launch of the weight-gradient GEMM: (tasks, row splits, rows per split, first partial slot)."""
         buf = (C.c_int32 * 64)()
@@ -304,6 +319,21 @@ class NativePlan:
         arr = (C.c_void_p * len(x_ptrs))(*x_ptrs)
         check(lib().mshgnn_backward_staged(self.handle, B, arr, x_dtype, params_ptr, dout_ptr, grads_ptr, ws_ptr, ws_bytes, mode, stream,
                                            layers_ready_event), "mshgnn_backward")
+
+    # ---- model batches: M models of this plan, B graphs each (include/mshgnn_b200.h) ----
+    def forward_models(self, M, B, x_ptrs, x_dtype, params_ptr, out_ptr, ws_ptr, ws_bytes, train, mode, stream):
+        arr = (C.c_void_p * len(x_ptrs))(*x_ptrs)
+        check(lib().mshgnn_forward_models(self.handle, M, B, arr, x_dtype, params_ptr, out_ptr, ws_ptr, ws_bytes, int(train), mode, stream),
+              "mshgnn_forward_models")
+
+    def loss_models(self, M, B, kind, out_ptr, labels_ptr, label_dtype, loss_scale, loss_ptr, dout_ptr, ws_ptr, ws_bytes, stream):
+        check(lib().mshgnn_loss_models(self.handle, M, B, kind, out_ptr, labels_ptr, label_dtype, loss_scale, loss_ptr, dout_ptr,
+                                       ws_ptr, ws_bytes, stream), "mshgnn_loss_models")
+
+    def backward_models(self, M, B, x_ptrs, x_dtype, params_ptr, dout_ptr, grads_ptr, ws_ptr, ws_bytes, mode, stream, layers_ready_event=None):
+        arr = (C.c_void_p * len(x_ptrs))(*x_ptrs)
+        check(lib().mshgnn_backward_models(self.handle, M, B, arr, x_dtype, params_ptr, dout_ptr, grads_ptr, ws_ptr, ws_bytes, mode, stream,
+                                           layers_ready_event), "mshgnn_backward_models")
 
     def input_grad(self, B, params_ptr, dx_ptrs, ws_ptr, ws_bytes, mode, stream):
         """d loss / d x[t] into the fp32 buffers dx_ptrs[t] (None: skip type t), after backward on the same workspace."""

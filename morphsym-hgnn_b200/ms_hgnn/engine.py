@@ -62,7 +62,7 @@ class Engine:
         self.n_params = self.plan.n_params
         self._ws: Optional[torch.Tensor] = None
         self._ws_key = None
-        self._train_ctx = None        # (B, x tensors) of the last train-mode forward
+        self._train_ctx = None        # (B, x tensors, x dtype code, models) of the last train-mode forward
 
     # ---- parameter layout ------------------------------------------------------------
     def param_layout(self) -> List[Tuple[str, int, Tuple[int, ...]]]:
@@ -88,8 +88,9 @@ class Engine:
         return out
 
     # ---- workspace --------------------------------------------------------------------
-    def workspace(self, B: int, train: bool, device) -> torch.Tensor:
-        need = self.plan.workspace_bytes(B, train, self.mode)
+    def workspace(self, B: int, train: bool, device, n_models: int = 1) -> torch.Tensor:
+        """B: graphs per model of a model batch of ``n_models`` models (1: a single model)."""
+        need = self.plan.workspace_bytes(B, train, self.mode) if n_models == 1 else self.plan.workspace_bytes_models(n_models, B, train, self.mode)
         if self._ws is None or self._ws.numel() < need or self._ws.device != device:
             self._ws = None
             self._ws = torch.empty(need, dtype=torch.uint8, device=device)
@@ -122,38 +123,65 @@ class Engine:
             raise ValueError("empty batch")
         return B, _dtype_code(x[0])
 
-    def forward(self, x: Sequence[torch.Tensor], flat_params: torch.Tensor, train: bool) -> torch.Tensor:
+    @staticmethod
+    def _check_models(n_models: int) -> int:
+        if int(n_models) != n_models or n_models < 1:
+            raise ValueError(f"n_models must be a positive integer, got {n_models}")
+        return int(n_models)
+
+    def forward(self, x: Sequence[torch.Tensor], flat_params: torch.Tensor, train: bool, n_models: int = 1) -> torch.Tensor:
+        """``n_models`` > 1: a model batch - x[t] holds the graphs of model 0, then those of model 1, ... (equal counts),
+        ``flat_params`` is [n_models, n_params] (or its flattening) and the output rows follow the same model-major order."""
+        M = self._check_models(n_models)
         B, xd = self._check_inputs(x)
+        if B % M:
+            raise ValueError(f"{B} graphs cannot be split evenly over {M} models")
+        B //= M
         x = [t.contiguous() for t in x]
         dev = x[0].device
-        if flat_params.device != dev or flat_params.dtype != torch.float32 or flat_params.numel() != self.n_params:
+        if flat_params.device != dev or flat_params.dtype != torch.float32 or flat_params.numel() != M * self.n_params \
+                or (M > 1 and not flat_params.is_contiguous()):
             raise RuntimeError("flat parameter buffer mismatch")
-        ws = self.workspace(B, train, dev)
-        out = torch.empty(self.plan.out_rows(B), self.spec["out_channels"], dtype=torch.float32, device=dev)
+        ws = self.workspace(B, train, dev, M)
+        out = torch.empty(M * self.plan.out_rows(B), self.spec["out_channels"], dtype=torch.float32, device=dev)
         stream = torch.cuda.current_stream(dev).cuda_stream
         with torch.cuda.device(dev):
-            self.plan.forward(B, [t.data_ptr() for t in x], xd, flat_params.data_ptr(), out.data_ptr(), ws.data_ptr(),
-                              ws.numel(), train, self.mode, stream)
-        self._train_ctx = (B, x, xd) if train else None
+            if M == 1:
+                self.plan.forward(B, [t.data_ptr() for t in x], xd, flat_params.data_ptr(), out.data_ptr(), ws.data_ptr(),
+                                  ws.numel(), train, self.mode, stream)
+            else:
+                self.plan.forward_models(M, B, [t.data_ptr() for t in x], xd, flat_params.data_ptr(), out.data_ptr(), ws.data_ptr(),
+                                         ws.numel(), train, self.mode, stream)
+        self._train_ctx = (B, x, xd, M) if train else None
         return out
 
-    def loss(self, out: torch.Tensor, labels: torch.Tensor, kind: int, want_grad: bool = True, loss_scale: float = 1.0):
-        """Returns (loss [1] fp32 device tensor, dout or None)."""
+    def loss(self, out: torch.Tensor, labels: torch.Tensor, kind: int, want_grad: bool = True, loss_scale: float = 1.0,
+             n_models: int = 1):
+        """Returns (loss [n_models] fp32 device tensor, dout or None).  ``n_models`` > 1: the rows of ``out`` and ``labels`` are
+        model-major; loss[m] is model m's mean loss and its rows of dout are scaled by loss_scale / (its element count)."""
+        M = self._check_models(n_models)
         dev = out.device
-        B = out.shape[0] // self.spec["nodes_per_graph"][self.spec["decode_type"]]
+        rows = self.spec["nodes_per_graph"][self.spec["decode_type"]]
+        if out.shape[0] % (rows * M):
+            raise ValueError(f"{out.shape[0]} output rows are not {M} models x whole graphs")
+        B = out.shape[0] // (rows * M)
         labels = labels.contiguous()
         n_expected = out.numel() if kind == N.LOSS_MSE else out.shape[0]
         if labels.numel() != n_expected:
             raise ValueError(f"labels have {labels.numel()} elements, expected {n_expected}")
         if labels.device != dev:
             raise ValueError("labels must live on the same device as the predictions")
-        ws = self.workspace(B, self._train_ctx is not None, dev)
-        loss = torch.empty(1, dtype=torch.float32, device=dev)
+        ws = self.workspace(B, self._train_ctx is not None, dev, M)
+        loss = torch.empty(M, dtype=torch.float32, device=dev)
         dout = torch.empty_like(out) if want_grad else None
         stream = torch.cuda.current_stream(dev).cuda_stream
         with torch.cuda.device(dev):
-            self.plan.loss(B, kind, out.data_ptr(), labels.data_ptr(), _dtype_code(labels), float(loss_scale), loss.data_ptr(),
-                           dout.data_ptr() if want_grad else None, ws.data_ptr(), ws.numel(), stream)
+            if M == 1:
+                self.plan.loss(B, kind, out.data_ptr(), labels.data_ptr(), _dtype_code(labels), float(loss_scale), loss.data_ptr(),
+                               dout.data_ptr() if want_grad else None, ws.data_ptr(), ws.numel(), stream)
+            else:
+                self.plan.loss_models(M, B, kind, out.data_ptr(), labels.data_ptr(), _dtype_code(labels), float(loss_scale), loss.data_ptr(),
+                                      dout.data_ptr() if want_grad else None, ws.data_ptr(), ws.numel(), stream)
         return loss, dout
 
     def encoder_param_end(self) -> int:
@@ -163,31 +191,36 @@ class Engine:
     def backward(self, dout: torch.Tensor, flat_params: torch.Tensor, grads: Optional[torch.Tensor] = None,
                  layers_ready: Optional[torch.cuda.Event] = None, param_grads: bool = True) -> Optional[torch.Tensor]:
         """d loss / d params into ``grads`` (allocated when None) and returned.  ``param_grads=False`` runs the input-only
-        backward of a frozen model: no weight gradient is computed and None is returned; input_grad() may follow."""
+        backward of a frozen model: no weight gradient is computed and None is returned; input_grad() may follow.
+        After a model-batch forward the gradients are [n_models * n_params], model-major."""
         if self._train_ctx is None:
             raise RuntimeError("backward() needs a preceding forward(train=True) on the same engine")
-        B, x, xd = self._train_ctx
+        B, x, xd, M = self._train_ctx
         dev = x[0].device
         dout = dout.contiguous()
         if dout.dtype != torch.float32:
             dout = dout.float()
-        if dout.numel() != self.plan.out_rows(B) * self.spec["out_channels"]:
+        if dout.numel() != M * self.plan.out_rows(B) * self.spec["out_channels"]:
             raise ValueError("dout has the wrong number of elements")
         if not param_grads:
             grads = None
         elif grads is None:
-            grads = torch.empty(self.n_params, dtype=torch.float32, device=dev)
-        ws = self.workspace(B, True, dev)
+            grads = torch.empty(M * self.n_params, dtype=torch.float32, device=dev)
+        elif M > 1 and (grads.numel() != M * self.n_params or not grads.is_contiguous()):
+            raise ValueError("gradient buffer mismatch")
+        ws = self.workspace(B, True, dev, M)
         stream = torch.cuda.current_stream(dev).cuda_stream
         with torch.cuda.device(dev):
             if layers_ready is not None:
                 # torch creates the CUDA event lazily at its first record(): make sure the handle exists
                 if layers_ready.cuda_event == 0:
                     layers_ready.record(torch.cuda.current_stream(dev))
-            self.plan.backward(B, [t.data_ptr() for t in x], xd, flat_params.data_ptr(), dout.data_ptr(),
-                               grads.data_ptr() if grads is not None else None,
-                               ws.data_ptr(), ws.numel(), self.mode, stream,
-                               layers_ready.cuda_event if layers_ready is not None else None)
+            args = ([t.data_ptr() for t in x], xd, flat_params.data_ptr(), dout.data_ptr(), grads.data_ptr() if grads is not None else None,
+                    ws.data_ptr(), ws.numel(), self.mode, stream, layers_ready.cuda_event if layers_ready is not None else None)
+            if M == 1:
+                self.plan.backward(B, *args)
+            else:
+                self.plan.backward_models(M, B, *args)
         return grads
 
     def input_grad(self, which: Sequence[bool], flat_params: torch.Tensor) -> List[Optional[torch.Tensor]]:
@@ -195,7 +228,9 @@ class Engine:
         backward() of the last train-mode forward, on the same workspace."""
         if self._train_ctx is None:
             raise RuntimeError("input_grad() needs a preceding forward(train=True) and backward() on the same engine")
-        B, x, _ = self._train_ctx
+        B, x, _, M = self._train_ctx
+        if M != 1:
+            raise ValueError("input gradients are not available for a model batch (n_models > 1)")
         dev = x[0].device
         out = [torch.empty(t.shape, dtype=torch.float32, device=dev) if w else None for t, w in zip(x, which)]
         ws = self.workspace(B, True, dev)

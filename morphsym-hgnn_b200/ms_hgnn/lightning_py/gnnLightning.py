@@ -404,4 +404,4 @@ class HGNN_C2_Lightning_Reg(Base_Lightning):
 
 
 # train_model / evaluate_model live next to the modules in the reference (gnnLightning.py:L913-1421)
-from .trainer import WindowSubset, evaluate_model, train_model  # noqa: E402,F401
+from .trainer import WindowSubset, evaluate_model, train_model, train_models  # noqa: E402,F401

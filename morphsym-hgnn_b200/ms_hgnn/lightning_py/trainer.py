@@ -153,18 +153,93 @@ def _run_epoch(module, dataset, batches, kind: str):
     return {k: _value(v) for k, v in module.logged.items() if k.startswith(("val_" if kind == "validation" else kind + "_"))}
 
 
-def train_model(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dataset: Optional[WindowSubset], normalize: bool,
-                testing_mode: bool = False, disable_logger: bool = False, logger_project_name: str = None, batch_size: int = 100,
-                num_layers: int = 8, optimizer: str = "adam", lr: float = 0.003, epochs: int = 30, hidden_size: int = 10,
-                regression: bool = True, seed: int = 0, devices: int = 1, early_stopping: bool = False, disable_test: bool = False,
-                train_percentage_to_log=None, symmetry_mode: str = None, group_operator_path: str = None,
-                subfoler_name: str = "default", data_path: Path = None, wandb_api_key: str = None,
-                grf_body_to_world_frame: bool = True, grf_dimension: int = 3, ckpt_path: str = None) -> str:
-    """Train with the reference's ``train_model`` contract (gnnLightning.py:L1099-1421).  Returns the checkpoint folder.
+class _Run:
+    """One seed's training run: its module, shuffle generator, checkpoint folder, metrics log and the early-stopping / top-k
+    bookkeeping of the reference's callbacks."""
 
-    COM formats build ``COM_HGNN_SYM_Lightning`` (a regression model whatever ``regression`` says) and monitor ``val_MSE_loss``;
-    ``data_path`` is where its standardiser statistics are looked up (module docstring: what is not checked against the
-    reference)."""
+    def __init__(self, train_dataset, model_type, com, data_metadata, seed, batch_size, normalize, hidden_size, num_layers, optimizer, lr,
+                 regression, symmetry_mode, group_operator_path, grf_body_to_world_frame, grf_dimension, data_path,
+                 disable_logger, logger_project_name, subfoler_name, train_percentage_to_log):
+        torch.manual_seed(seed)                                    # seed_everything(seed)
+        self.gen = torch.Generator().manual_seed(seed)
+        self.ds = ds = train_dataset.dataset
+        dummy_idx = _loader(train_dataset, batch_size, True, self.gen, 1)[0]
+        dummy_batch = ds.batch(dummy_idx)
+        self.module = module = _build_module(model_type, hidden_size, num_layers, data_metadata, dummy_batch, optimizer, lr, regression,
+                                             symmetry_mode, group_operator_path, grf_body_to_world_frame, grf_dimension, data_path).to(ds.device)
+        module.model.validate_edges = "cached"
+        n_params = sum(p.numel() for p in module.model.parameters() if p.requires_grad)
+
+        if not disable_logger:
+            if logger_project_name is None:
+                raise ValueError("Need to define \"logger_project_name\" if logger is enabled.")
+            path_to_save = Path("models", subfoler_name, f"{logger_project_name}-seed{seed}-{time.strftime('%Y%m%d-%H%M%S')}")
+        else:
+            path_to_save = Path("models", f"{model_type}_run-seed{seed}-{time.strftime('%Y%m%d-%H%M%S')}")
+        base, k = path_to_save, 0
+        while path_to_save.exists():                               # two runs inside the same second
+            k += 1
+            path_to_save = Path(str(base) + f"-{k}")
+        path_to_save.mkdir(parents=True)
+        self.path = path_to_save
+        self.log_f = open(path_to_save / "metrics.jsonl", "a")
+        self.log_f.write(json.dumps({"config": {"batch_size": batch_size, "normalize": normalize, "num_parameters": n_params, "seed": seed,
+                                                "train_percentage": train_percentage_to_log, "model_type": model_type}}) + "\n")
+        if regression or com:
+            self.monitor, self.second = "val_MSE_loss", "val_L1_loss"
+        else:
+            self.monitor, self.second = "val_CE_loss", "val_F1_Score_Leg_Avg"
+        self.dummy_idx = dummy_idx
+        self.saved: List[tuple] = []        # (epoch, monitor value, path)
+        self.best_seen, self.bad_epochs = float("inf"), 0
+        self.stopped = False
+
+    def start(self):
+        self.dummy_plain = _plain_batch(self.ds.batch(self.dummy_idx[:min(20, self.dummy_idx.numel())]))
+
+    def resume(self, resumed) -> None:
+        """early stopping, the top-k policy and the shuffle order continue where the run stopped"""
+        self.best_seen, self.bad_epochs = float(resumed["best_seen"]), int(resumed["bad_epochs"])
+        self.saved = [(int(e), float(v), Path(pth)) for e, v, pth in resumed["saved"] if Path(pth).exists()]
+        self.gen.set_state(resumed["generator_state"])
+
+    def end_epoch(self, trainer, val_dataset, batch_size, lim_val, epoch, global_step, loss, early_stopping) -> None:
+        """Validation, metrics line, checkpoint and the top-k / early-stopping policy after a training epoch."""
+        module, monitor, second = self.module, self.monitor, self.second
+        module.eval()
+        _run_epoch(module, val_dataset.dataset, _loader(val_dataset, batch_size, False, None, lim_val), "validation")
+        logged = {k: _value(v) for k, v in module.logged.items() if k.startswith("val_")}
+        logged.update(epoch=epoch, global_step=global_step, train_loss_last_step=_value(loss))
+        self.log_f.write(json.dumps(logged) + "\n"); self.log_f.flush()
+        name = f"epoch={epoch}-{monitor}={logged[monitor]:.5f}" + (f"-{second}={logged[second]:.5f}" if second in logged else "") + ".ckpt"
+        saved = self.saved
+        saved.append((epoch, logged[monitor], self.path / name))
+        better = logged[monitor] < self.best_seen
+        _save_checkpoint(self.path / name, module, trainer, epoch, global_step, self.dummy_plain,
+                         {"best_seen": min(self.best_seen, logged[monitor]), "bad_epochs": 0 if better else self.bad_epochs + 1,
+                          "saved": [(e, v, str(pth)) for e, v, pth in saved], "generator_state": self.gen.get_state()})
+        # ModelCheckpoint(save_top_k=7, mode='min', monitor=monitor) + ModelCheckpoint(save_top_k=3, mode='max', monitor='epoch')
+        keep = {s[2] for s in sorted(saved, key=lambda s: s[1])[:7]} | {s[2] for s in sorted(saved, key=lambda s: s[0])[-3:]}
+        for s in saved:
+            if s[2] not in keep and s[2].exists():
+                s[2].unlink()
+        self.saved = [s for s in saved if s[2] in keep]
+        if logged[monitor] < self.best_seen:
+            self.best_seen, self.bad_epochs = logged[monitor], 0
+        else:
+            self.bad_epochs += 1
+        if early_stopping and self.bad_epochs >= 10:                # EarlyStopping(monitor, patience=10, mode='min')
+            self.stopped = True
+
+    def finish(self, test_dataset, batch_size, lim_test, disable_test) -> str:
+        if not disable_test:
+            logged = _run_epoch(self.module, test_dataset.dataset, _loader(test_dataset, batch_size, False, None, lim_test), "test")
+            self.log_f.write(json.dumps(logged) + "\n")
+        self.log_f.close()
+        return str(self.path)
+
+
+def _check_run_args(train_dataset, val_dataset, test_dataset, disable_test, hidden_size, devices):
     fmts = [train_dataset.dataset.get_data_format(), val_dataset.dataset.get_data_format()]
     if not disable_test:
         fmts.append(test_dataset.dataset.get_data_format())
@@ -173,44 +248,35 @@ def train_model(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dat
     model_type = fmts[0]
     if model_type not in _HGNN_FORMATS + _COM_FORMATS:
         raise ValueError("Invalid model type.")
-    com = model_type in _COM_FORMATS
     if not 1 <= hidden_size <= 128:
         # narrower models run zero-padded on the 128-channel kernels; wider ones have no kernels
         raise ValueError(f"hidden_size={hidden_size}: the B200-native path supports hidden_size 1..128")
     if devices != 1:
         raise ValueError("train_model drives one GPU; launch one process per GPU and pass a process group to FusedTrainer for data parallelism")
+    return model_type, model_type in _COM_FORMATS
+
+
+def train_model(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dataset: Optional[WindowSubset], normalize: bool,
+                testing_mode: bool = False, disable_logger: bool = False, logger_project_name: str = None, batch_size: int = 100,
+                num_layers: int = 8, optimizer: str = "adam", lr: float = 0.003, epochs: int = 30, hidden_size: int = 10,
+                regression: bool = True, seed: int = 0, devices: int = 1, early_stopping: bool = False, disable_test: bool = False,
+                train_percentage_to_log=None, symmetry_mode: str = None, group_operator_path: str = None,
+                subfoler_name: str = "default", data_path: Path = None, wandb_api_key: str = None,
+                grf_body_to_world_frame: bool = True, grf_dimension: int = 3, ckpt_path: str = None, mode: str = "fp32") -> str:
+    """Train with the reference's ``train_model`` contract (gnnLightning.py:L1099-1421).  Returns the checkpoint folder.
+    ``mode``: arithmetic mode of the native kernels ('fp32', 'tc' or 'tc1x', ``NativeHGNN.set_mode``).
+
+    COM formats build ``COM_HGNN_SYM_Lightning`` (a regression model whatever ``regression`` says) and monitor ``val_MSE_loss``;
+    ``data_path`` is where its standardiser statistics are looked up (module docstring: what is not checked against the
+    reference)."""
+    model_type, com = _check_run_args(train_dataset, val_dataset, test_dataset, disable_test, hidden_size, devices)
     data_metadata = train_dataset.dataset.get_data_metadata()
     lim_train, lim_val, lim_test = (10, 5, 5) if testing_mode else (None, None, None)
-
-    torch.manual_seed(seed)                                        # seed_everything(seed)
-    gen = torch.Generator().manual_seed(seed)
-    ds = train_dataset.dataset
-    dummy_idx = _loader(train_dataset, batch_size, True, gen, 1)[0]
-    dummy_batch = ds.batch(dummy_idx)
-    module = _build_module(model_type, hidden_size, num_layers, data_metadata, dummy_batch, optimizer, lr, regression, symmetry_mode,
-                           group_operator_path, grf_body_to_world_frame, grf_dimension, data_path).to(ds.device)
-    module.model.validate_edges = "cached"
-    n_params = sum(p.numel() for p in module.model.parameters() if p.requires_grad)
-
-    if not disable_logger:
-        if logger_project_name is None:
-            raise ValueError("Need to define \"logger_project_name\" if logger is enabled.")
-        path_to_save = Path("models", subfoler_name, f"{logger_project_name}-seed{seed}-{time.strftime('%Y%m%d-%H%M%S')}")
-    else:
-        path_to_save = Path("models", f"{model_type}_run-seed{seed}-{time.strftime('%Y%m%d-%H%M%S')}")
-    base, k = path_to_save, 0
-    while path_to_save.exists():                                   # two runs inside the same second
-        k += 1
-        path_to_save = Path(str(base) + f"-{k}")
-    path_to_save.mkdir(parents=True)
-    log_f = open(path_to_save / "metrics.jsonl", "a")
-    log_f.write(json.dumps({"config": {"batch_size": batch_size, "normalize": normalize, "num_parameters": n_params, "seed": seed,
-                                       "train_percentage": train_percentage_to_log, "model_type": model_type}}) + "\n")
-
-    if regression or com:
-        monitor, second = "val_MSE_loss", "val_L1_loss"
-    else:
-        monitor, second = "val_CE_loss", "val_F1_Score_Leg_Avg"
+    run = _Run(train_dataset, model_type, com, data_metadata, seed, batch_size, normalize, hidden_size, num_layers, optimizer, lr,
+               regression, symmetry_mode, group_operator_path, grf_body_to_world_frame, grf_dimension, data_path,
+               disable_logger, logger_project_name, subfoler_name, train_percentage_to_log)
+    module, ds = run.module, run.ds
+    module.model.set_mode(mode)
 
     trainer = FusedTrainer(module)
     start_epoch, global_step = 0, 0
@@ -226,47 +292,80 @@ def train_model(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dat
     else:
         resumed = None
 
-    dummy_plain = _plain_batch(ds.batch(dummy_idx[:min(20, dummy_idx.numel())]))
-    saved: List[tuple] = []         # (epoch, monitor value, path)
-    best_seen, bad_epochs = float("inf"), 0
-    if resumed:                     # early stopping, the top-k policy and the shuffle order continue where the run stopped
-        best_seen, bad_epochs = float(resumed["best_seen"]), int(resumed["bad_epochs"])
-        saved = [(int(e), float(v), Path(pth)) for e, v, pth in resumed["saved"] if Path(pth).exists()]
-        gen.set_state(resumed["generator_state"])
+    run.start()
+    if resumed:
+        run.resume(resumed)
     loss = torch.zeros(())
     for epoch in range(start_epoch, epochs):
         module.train()
-        for idx in _loader(train_dataset, batch_size, True, gen, lim_train):
+        for idx in _loader(train_dataset, batch_size, True, run.gen, lim_train):
             loss = trainer.train_step(ds.batch(idx))
             global_step += 1
-        module.eval()
-        _run_epoch(module, val_dataset.dataset, _loader(val_dataset, batch_size, False, None, lim_val), "validation")
-        logged = {k: _value(v) for k, v in module.logged.items() if k.startswith("val_")}
-        logged.update(epoch=epoch, global_step=global_step, train_loss_last_step=_value(loss))
-        log_f.write(json.dumps(logged) + "\n"); log_f.flush()
-        name = f"epoch={epoch}-{monitor}={logged[monitor]:.5f}" + (f"-{second}={logged[second]:.5f}" if second in logged else "") + ".ckpt"
-        saved.append((epoch, logged[monitor], path_to_save / name))
-        better = logged[monitor] < best_seen
-        _save_checkpoint(path_to_save / name, module, trainer, epoch, global_step, dummy_plain,
-                         {"best_seen": min(best_seen, logged[monitor]), "bad_epochs": 0 if better else bad_epochs + 1,
-                          "saved": [(e, v, str(pth)) for e, v, pth in saved], "generator_state": gen.get_state()})
-        # ModelCheckpoint(save_top_k=7, mode='min', monitor=monitor) + ModelCheckpoint(save_top_k=3, mode='max', monitor='epoch')
-        keep = {s[2] for s in sorted(saved, key=lambda s: s[1])[:7]} | {s[2] for s in sorted(saved, key=lambda s: s[0])[-3:]}
-        for s in saved:
-            if s[2] not in keep and s[2].exists():
-                s[2].unlink()
-        saved = [s for s in saved if s[2] in keep]
-        if logged[monitor] < best_seen:
-            best_seen, bad_epochs = logged[monitor], 0
-        else:
-            bad_epochs += 1
-        if early_stopping and bad_epochs >= 10:                    # EarlyStopping(monitor, patience=10, mode='min')
+        run.end_epoch(trainer, val_dataset, batch_size, lim_val, epoch, global_step, loss, early_stopping)
+        if run.stopped:
             break
-    if not disable_test:
-        logged = _run_epoch(module, test_dataset.dataset, _loader(test_dataset, batch_size, False, None, lim_test), "test")
-        log_f.write(json.dumps(logged) + "\n")
-    log_f.close()
-    return str(path_to_save)
+    return run.finish(test_dataset, batch_size, lim_test, disable_test)
+
+
+class _SeedOptimizerView:
+    """Model ``i`` of a ModelBatchTrainer seen as a FusedTrainer by the checkpoint writer (its moments, step count, settings)."""
+
+    def __init__(self, tr, i):
+        self.exp_avg, self.exp_avg_sq = tr.exp_avg[i], tr.exp_avg_sq[i]
+        self.step_count = tr.step_count[i]
+        self.lr, self.betas, self.eps, self.weight_decay = tr.lr, tr.betas, tr.eps, tr.weight_decay
+
+
+def train_models(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dataset: Optional[WindowSubset], normalize: bool,
+                 testing_mode: bool = False, disable_logger: bool = False, logger_project_name: str = None, batch_size: int = 100,
+                 num_layers: int = 8, optimizer: str = "adam", lr: float = 0.003, epochs: int = 30, hidden_size: int = 10,
+                 regression: bool = True, seeds=(0,), devices: int = 1, early_stopping: bool = False, disable_test: bool = False,
+                 train_percentage_to_log=None, symmetry_mode: str = None, group_operator_path: str = None,
+                 subfoler_name: str = "default", data_path: Path = None, wandb_api_key: str = None,
+                 grf_body_to_world_frame: bool = True, grf_dimension: int = 3, mode: str = "tc") -> List[str]:
+    """``train_model`` for several seeds at once: returns one checkpoint folder per seed, each with what ``train_model(seed=s)``
+    writes for that seed - bit for bit the same checkpoints (parameters and optimizer state) and metrics.
+
+    Every seed is built exactly as ``train_model`` builds it (global seed, its own shuffle generator, dummy batch, module); the
+    training steps of all seeds run as one model batch (``ModelBatchTrainer``, arithmetic ``mode`` 'tc' or 'tc1x', which every
+    seed's module uses for validation and test too); validation, test, checkpoints, top-k and early stopping stay per seed.  A
+    seed that has stopped early still rides along in the batched step but gets no optimizer update and writes nothing more.
+    Resuming (``ckpt_path`` of ``train_model``) is not offered."""
+    from ..model_batch import ModelBatch, ModelBatchTrainer
+    seeds = list(seeds)
+    if not seeds:
+        raise ValueError("train_models needs at least one seed")
+    model_type, com = _check_run_args(train_dataset, val_dataset, test_dataset, disable_test, hidden_size, devices)
+    data_metadata = train_dataset.dataset.get_data_metadata()
+    lim_train, lim_val, lim_test = (10, 5, 5) if testing_mode else (None, None, None)
+    runs = [_Run(train_dataset, model_type, com, data_metadata, seed, batch_size, normalize, hidden_size, num_layers, optimizer, lr,
+                 regression, symmetry_mode, group_operator_path, grf_body_to_world_frame, grf_dimension, data_path,
+                 disable_logger, logger_project_name, subfoler_name, train_percentage_to_log) for seed in seeds]
+    for r in runs:
+        r.module.model.set_mode(mode)
+        r.start()
+    m0 = runs[0].module
+    # the settings FusedTrainer(module) takes from the module
+    tr = ModelBatchTrainer(ModelBatch([r.module.model for r in runs]), optimizer=getattr(m0, "optimizer", "adam"), lr=float(getattr(m0, "lr", 1e-3)),
+                           regression=getattr(m0, "regression", getattr(m0.model, "regression", True)))
+    ds = runs[0].ds
+    global_step = 0
+    losses = [torch.zeros(())] * len(runs)
+    for epoch in range(epochs):
+        live = [not r.stopped for r in runs]
+        if not any(live):
+            break
+        for r in runs:
+            r.module.train()
+        loaders = [_loader(train_dataset, batch_size, True, r.gen, lim_train) for r in runs]
+        for step in range(len(loaders[0])):
+            loss = tr.train_step([ds.batch(ld[step]) for ld in loaders], active=live)
+            losses = [loss[i] if live[i] else losses[i] for i in range(len(runs))]
+            global_step += 1
+        for i, r in enumerate(runs):
+            if live[i]:
+                r.end_epoch(_SeedOptimizerView(tr, i), val_dataset, batch_size, lim_val, epoch, global_step, losses[i], early_stopping)
+    return [r.finish(test_dataset, batch_size, lim_test, disable_test) for r in runs]
 
 
 def evaluate_model(path_to_checkpoint: Path, predict_dataset: WindowSubset, enable_testing_mode: bool = False,
