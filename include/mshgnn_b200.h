@@ -191,6 +191,23 @@ int mshgnn_backward_models(const mshgnn_plan* plan, int64_t M, int64_t B,
                            void* workspace, int64_t workspace_bytes,
                            int32_t mode, void* stream, void* layers_ready_event);
 
+/* ---- model batches of different hidden widths (hyperparameter sweeps) -----------------------------------------------------
+ * mshgnn_plan_create_models: one plan for M models (1..1023) that differ only in hidden width, hidden[m] in 1..128 (host array;
+ * desc->hidden is ignored).  params / grads are the models' own flat layouts laid end to end ("ragged"): model m's layout at
+ * width hidden[m] (the layout mshgnn_param_offset reports for a plan of that width) starts where model m-1's ends, and
+ * mshgnn_param_count returns the total.  mshgnn_param_offset_model returns the absolute offset of a tensor of model m;
+ * mshgnn_param_offset refuses a plan of M > 1 models.  Every model runs zero-padded on the 128-wide kernels as with
+ * MSHGNN_PLAN_PAD_HIDDEN and gets bit for bit the outputs, loss and gradients of the single-model calls on a plan of its own
+ * width.  With every width at 128 the plan runs exactly the launches of a model batch of a plain plan.
+ * The *_models entry points above take such a plan only with M equal to the plan's M, the single-model ones only when M = 1;
+ * otherwise they return MSHGNN_ERR_ARG (-1 for the workspace query) before any device work.  Staged backward: every model's
+ * gradients outside its encoder block are final when layers_ready_event is recorded; the encoder blocks (each model's first
+ * tensors, so one range per model, not one prefix of the buffer) follow.  All per-model tables are uploaded once, at the
+ * first compute call on a device: forward, loss and backward may be captured in a CUDA graph after one eager call. */
+int mshgnn_plan_create_models(const mshgnn_desc* desc, int32_t M, const int32_t* hidden, mshgnn_plan** plan_out);
+int mshgnn_param_offset_model(const mshgnn_plan* plan, int32_t m, int32_t kind, int32_t layer, int32_t idx,
+                              int64_t* offset_out, int64_t* numel_out);
+
 /* Fused Adam on flat buffers (torch.optim.Adam defaults semantics, gnnLightning.py:L258-265):
  * step is the 1-based step count after this update. */
 int mshgnn_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq,
@@ -198,6 +215,16 @@ int mshgnn_adam_step(float* params, const float* grads, float* exp_avg, float* e
                      float weight_decay, void* stream);
 /* plain SGD: p -= lr * g */
 int mshgnn_sgd_step(float* params, const float* grads, int64_t n, float lr, void* stream);
+/* Per-model optimizers in one launch (M in 1..1023): model m owns elements [offsets[m], offsets[m+1]) of every buffer and is
+ * updated with its own step count and learning rate; each model's result is bit for bit mshgnn_adam_step / mshgnn_sgd_step
+ * on its range.  offsets [M+1], step [M], lr [M] and active [M] are host arrays, read during the call: the values are
+ * passed to the kernel by value, so a captured launch replays with them.  step[m] = 0 (Adam) or active[m] = 0 (SGD; NULL =
+ * every model active) leaves model m's parameters and moments untouched.  beta1, beta2, eps and weight_decay are shared. */
+int mshgnn_adam_step_models(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int32_t M,
+                            const int64_t* offsets, const int64_t* step, const float* lr, float beta1, float beta2,
+                            float eps, float weight_decay, void* stream);
+int mshgnn_sgd_step_models(float* params, const float* grads, int32_t M, const int64_t* offsets, const float* lr,
+                           const int32_t* active, void* stream);
 
 /* ---- device-side window builder (SURVEY 8f-3) ---------------------------------------------
  * Replaces, batched on the GPU, the reference's per-sample dataset path

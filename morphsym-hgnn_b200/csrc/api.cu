@@ -506,11 +506,21 @@ int launch_stack(int kind, const Plan& p, const Plan::Stack& sp, const WsLayout&
     return 0;
 }
 
+// Grid z and per-model strides of the pad / compaction kernels for a call on M models: a plan of one model repeats its table
+// for every model (z = M), a mixed plan's table already covers every model with absolute offsets (z = 1, strides 0).
+struct PadGrid { unsigned z; int64_t ext_n, in_n; };
+PadGrid pad_grid(const Plan& p, int M) {
+    if (p.n_models > 1) return {1u, 0, 0};
+    return {(unsigned)M, p.ext_base.back(), p.n_params};
+}
+unsigned pad_grid_y(int count) { return (unsigned)std::min(count, PAD_MAX_GRID_Y); }
+
 // padded plans: caller's gradients of the tensors segs [first, first + count) from the internal 128-wide gradient buffer
 int compact_grads(const Plan& p, int M, int first, int count, const float* in, float* ext, cudaStream_t st) {
     if (count == 0) return 0;
+    const PadGrid g = pad_grid(p, M);
     ProfScope ps(K_PAD, st);
-    k_compact_grads<<<dim3(PAD_BLOCKS_X, (unsigned)count, (unsigned)M), 256, 0, st>>>(p.d_pad_segs + first, in, ext, p.n_params, p.ext.n);
+    k_compact_grads<<<dim3(PAD_BLOCKS_X, pad_grid_y(count), g.z), 256, 0, st>>>(p.d_pad_segs + first, count, in, ext, g.in_n, g.ext_n);
     LAUNCH_CHECK();
     return 0;
 }
@@ -548,6 +558,8 @@ struct Call {
 // What a model batch of M models supports; checked before the device is touched
 int check_models(const Plan& p, int64_t M, int64_t B, int32_t mode) {
     if (M < 1) return fail(MSHGNN_ERR_ARG, "M must be >= 1 (got %lld)", (long long)M);
+    if (p.n_models > 1 && M != p.n_models)
+        return fail(MSHGNN_ERR_ARG, "the plan describes a model batch of %d models: M must be %d (got %lld)", p.n_models, p.n_models, (long long)M);
     if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1 (got %lld)", (long long)B);
     if (M == 1) return 0;
     if (mode == MSHGNN_MODE_FP32) return fail(MSHGNN_ERR_ARG, "model batches (M = %lld) run in the tensor-core modes only", (long long)M);
@@ -643,6 +655,28 @@ int launch_tc_encoder_dw(const Call& c, int64_t B, int xf64, cudaStream_t st) {
     return 0;
 }
 
+// What the per-model optimizer entry points share: argument checks and the per-model table (lr, ranges, active flags).
+int opt_models_table(const float* params, const float* grads, int32_t M, const int64_t* offsets, const float* lr, OptModels& t, int64_t* most) {
+    if (!params || !grads || !offsets || !lr) return fail(MSHGNN_ERR_ARG, "NULL argument");
+    if (M < 1 || M > OPT_MAX_MODELS) return fail(MSHGNN_ERR_ARG, "M must be in 1..%d (got %d)", OPT_MAX_MODELS, M);
+    if (offsets[0] < 0) return fail(MSHGNN_ERR_ARG, "offsets[0] must be >= 0");
+    memset(&t, 0, sizeof t);
+    *most = 0;
+    for (int m = 0; m <= M; ++m) {
+        if (m > 0 && offsets[m] < offsets[m - 1]) return fail(MSHGNN_ERR_ARG, "offsets must not decrease (model %d)", m - 1);
+        t.off[m] = offsets[m];
+        if (m > 0) *most = std::max(*most, offsets[m] - offsets[m - 1]);
+    }
+    for (int m = 0; m < M; ++m) t.lr[m] = lr[m];
+    return 0;
+}
+
+// grid of the per-model optimizer kernels: one row of CTAs per model, together about as many CTAs as k_adam's launch
+dim3 opt_models_grid(int32_t M, int64_t most) {
+    int64_t bx = std::min<int64_t>((most + 255) / 256, (148 * 8 + M - 1) / M);
+    return dim3((unsigned)std::max<int64_t>(bx, 1), (unsigned)M);
+}
+
 }  // namespace
 
 extern "C" {
@@ -660,6 +694,19 @@ int mshgnn_plan_create_ex(const mshgnn_desc* desc, int32_t flags, mshgnn_plan** 
 
 int mshgnn_plan_create(const mshgnn_desc* desc, mshgnn_plan** plan_out) { return mshgnn_plan_create_ex(desc, 0, plan_out); }
 
+int mshgnn_plan_create_models(const mshgnn_desc* desc, int32_t M, const int32_t* hidden, mshgnn_plan** plan_out) {
+    if (!plan_out) return fail(MSHGNN_ERR_ARG, "plan_out is NULL");
+    *plan_out = nullptr;
+    if (M < 1 || M > OPT_MAX_MODELS) return fail(MSHGNN_ERR_ARG, "M must be in 1..%d (got %d)", OPT_MAX_MODELS, M);
+    if (!hidden) return fail(MSHGNN_ERR_ARG, "hidden is NULL");
+    mshgnn_plan* pl = new (std::nothrow) mshgnn_plan();
+    if (!pl) return fail(MSHGNN_ERR_ARG, "out of host memory");
+    std::string e = build_plan(desc, 0, pl->p, std::vector<int>(hidden, hidden + M));
+    if (!e.empty()) { delete pl; return fail(MSHGNN_ERR_ARG, "%s", e.c_str()); }
+    *plan_out = pl;
+    return 0;
+}
+
 void mshgnn_plan_destroy(mshgnn_plan* plan) {
     if (!plan) return;
     Plan& p = plan->p;
@@ -667,24 +714,32 @@ void mshgnn_plan_destroy(mshgnn_plan* plan) {
     delete plan;
 }
 
-int64_t mshgnn_param_count(const mshgnn_plan* plan) { return plan ? plan->p.ext.n : -1; }
+int64_t mshgnn_param_count(const mshgnn_plan* plan) { return plan ? plan->p.ext_base.back() : -1; }
 
 int mshgnn_param_offset(const mshgnn_plan* plan, int32_t kind, int32_t layer, int32_t idx, int64_t* off, int64_t* numel) {
+    if (plan && plan->p.n_models > 1)
+        return fail(MSHGNN_ERR_ARG, "the plan describes %d models: use mshgnn_param_offset_model", plan->p.n_models);
+    return mshgnn_param_offset_model(plan, 0, kind, layer, idx, off, numel);
+}
+
+int mshgnn_param_offset_model(const mshgnn_plan* plan, int32_t m, int32_t kind, int32_t layer, int32_t idx, int64_t* off, int64_t* numel) {
     if (!plan || !off || !numel) return fail(MSHGNN_ERR_ARG, "NULL argument");
     const Plan& p = plan->p;
-    const ParamLayout& y = p.ext;      // the caller's layout, at the model's width h
-    const int64_t h = p.hidden;
+    if (m < 0 || m >= p.n_models) return fail(MSHGNN_ERR_ARG, "model %d out of range (the plan describes %d)", m, p.n_models);
+    const ParamLayout& y = p.ext[m];      // the caller's layout of model m, at its width h, from the model's start
+    const int64_t h = p.hidden[m];
+    const int64_t base = p.ext_base[m];
     auto lay_ok = [&]() { return layer >= 0 && layer < p.L && idx >= 0 && idx < p.n_etypes; };
     switch (kind) {
-        case MSHGNN_P_ENC_W: if (idx < 0 || idx >= p.n_types) break; *off = y.enc_w[idx]; *numel = h * p.in_w[idx]; return 0;
-        case MSHGNN_P_ENC_B: if (idx < 0 || idx >= p.n_types) break; *off = y.enc_b[idx]; *numel = h; return 0;
-        case MSHGNN_P_REL_W: if (!lay_ok()) break; *off = y.rel_w[layer * p.n_etypes + idx]; *numel = h * h; return 0;
-        case MSHGNN_P_REL_B: if (!lay_ok()) break; *off = y.rel_b[layer * p.n_etypes + idx]; *numel = h; return 0;
-        case MSHGNN_P_ROOT_W: if (!lay_ok()) break; *off = y.root_w[layer * p.n_etypes + idx]; *numel = h * h; return 0;
-        case MSHGNN_P_MLP_W: if (!p.morph_sym || idx < 0 || idx > 1) break; *off = y.mlp_w[idx]; *numel = h * h; return 0;
-        case MSHGNN_P_MLP_B: if (!p.morph_sym || idx < 0 || idx > 1) break; *off = y.mlp_b[idx]; *numel = h; return 0;
-        case MSHGNN_P_DEC_W: *off = y.dec_w; *numel = p.C * h; return 0;
-        case MSHGNN_P_DEC_B: *off = y.dec_b; *numel = p.C; return 0;
+        case MSHGNN_P_ENC_W: if (idx < 0 || idx >= p.n_types) break; *off = base + y.enc_w[idx]; *numel = h * p.in_w[idx]; return 0;
+        case MSHGNN_P_ENC_B: if (idx < 0 || idx >= p.n_types) break; *off = base + y.enc_b[idx]; *numel = h; return 0;
+        case MSHGNN_P_REL_W: if (!lay_ok()) break; *off = base + y.rel_w[layer * p.n_etypes + idx]; *numel = h * h; return 0;
+        case MSHGNN_P_REL_B: if (!lay_ok()) break; *off = base + y.rel_b[layer * p.n_etypes + idx]; *numel = h; return 0;
+        case MSHGNN_P_ROOT_W: if (!lay_ok()) break; *off = base + y.root_w[layer * p.n_etypes + idx]; *numel = h * h; return 0;
+        case MSHGNN_P_MLP_W: if (!p.morph_sym || idx < 0 || idx > 1) break; *off = base + y.mlp_w[idx]; *numel = h * h; return 0;
+        case MSHGNN_P_MLP_B: if (!p.morph_sym || idx < 0 || idx > 1) break; *off = base + y.mlp_b[idx]; *numel = h; return 0;
+        case MSHGNN_P_DEC_W: *off = base + y.dec_w; *numel = p.C * h; return 0;
+        case MSHGNN_P_DEC_B: *off = base + y.dec_b; *numel = p.C; return 0;
         default: break;
     }
     return fail(MSHGNN_ERR_ARG, "no such parameter (kind=%d layer=%d idx=%d)", kind, layer, idx);
@@ -696,7 +751,7 @@ int64_t mshgnn_workspace_bytes(const mshgnn_plan* plan, int64_t B, int32_t train
 
 int64_t mshgnn_workspace_bytes_models(const mshgnn_plan* plan, int64_t M, int64_t B, int32_t train, int32_t mode) {
     if (!plan || M < 1 || B < 1) return -1;
-    if (M > 1 && (check_plan_mode(plan, mode) || check_models(plan->p, M, B, mode))) return -1;
+    if ((M > 1 || plan->p.n_models > 1) && (check_plan_mode(plan, mode) || check_models(plan->p, M, B, mode))) return -1;
     const WsLayout w = ws_layout(plan->p, B, train, mode, (int)M);
     if (train && mode != MSHGNN_MODE_FP32 && getenv("MSHGNN_DEBUG_LAYOUT")) {   // weight-gradient row splits per layer launch
         fprintf(stderr, "mshgnn layout M=%d B=%lld Bm=%lld: dW default %d x %d rows, %lld partial slots;", w.M, (long long)B, (long long)w.Bm,
@@ -757,8 +812,10 @@ int mshgnn_forward_models(const mshgnn_plan* plan, int64_t M, int64_t B, const v
     const WsLayout& w = c.w;
     const BufTable& bt = c.bt;
     if (p.padded) {     // every kernel below reads the 128-wide zero-padded copy
+        const PadGrid g = pad_grid(p, w.M);
+        const int n_segs = (int)p.pad_segs.size();
         ProfScope ps(K_PAD, st);
-        k_pad_params<<<dim3(PAD_BLOCKS_X, (unsigned)p.pad_segs.size(), (unsigned)w.M), 256, 0, st>>>(p.d_pad_segs, params, (float*)c.params, p.ext.n, p.n_params);
+        k_pad_params<<<dim3(PAD_BLOCKS_X, pad_grid_y(n_segs), g.z), 256, 0, st>>>(p.d_pad_segs, n_segs, params, (float*)c.params, g.ext_n, g.in_n);
         LAUNCH_CHECK();
     }
     params = c.params;
@@ -844,6 +901,8 @@ int mshgnn_loss_models(const mshgnn_plan* plan, int64_t M, int64_t B, int32_t lo
     if (!out || !labels || !loss_out || !workspace) return fail(MSHGNN_ERR_ARG, "NULL argument");
     if (B < 1) return fail(MSHGNN_ERR_ARG, "B must be >= 1");
     if (M < 1 || M > 65535) return fail(MSHGNN_ERR_ARG, "M must be in 1..65535 (got %lld)", (long long)M);
+    if (p.n_models > 1 && M != p.n_models)
+        return fail(MSHGNN_ERR_ARG, "the plan describes a model batch of %d models: M must be %d (got %lld)", p.n_models, p.n_models, (long long)M);
     if (label_dtype < 0 || label_dtype > 2) return fail(MSHGNN_ERR_ARG, "bad label_dtype");
     if (loss_kind == MSHGNN_LOSS_CE2 && p.C != 2) return fail(MSHGNN_ERR_ARG, "CE2 loss needs out_channels == 2");
     if (loss_kind != MSHGNN_LOSS_CE2 && loss_kind != MSHGNN_LOSS_MSE) return fail(MSHGNN_ERR_ARG, "bad loss_kind");
@@ -1080,6 +1139,39 @@ int mshgnn_sgd_step(float* params, const float* grads, int64_t n, float lr, void
     if (blocks > 148 * 8) blocks = 148 * 8;
     ProfScope ps(K_OPTIM, (cudaStream_t)stream);
     k_sgd<<<blocks, 256, 0, (cudaStream_t)stream>>>(params, grads, n, lr);
+    LAUNCH_CHECK();
+    return 0;
+}
+
+int mshgnn_adam_step_models(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int32_t M, const int64_t* offsets,
+                            const int64_t* step, const float* lr, float beta1, float beta2, float eps, float weight_decay, void* stream) {
+    OptModels t;
+    int64_t most = 0;
+    int rc;
+    if ((rc = opt_models_table(params, grads, M, offsets, lr, t, &most))) return rc;
+    if (!exp_avg || !exp_avg_sq || !step) return fail(MSHGNN_ERR_ARG, "NULL argument");
+    for (int m = 0; m < M; ++m) {
+        if (step[m] < 0) return fail(MSHGNN_ERR_ARG, "step[%d] must be >= 0 (got %lld)", m, (long long)step[m]);
+        t.active[m] = step[m] > 0;
+        if (!t.active[m]) continue;
+        t.bc1[m] = 1.f - (float)std::pow((double)beta1, (double)step[m]);           // as mshgnn_adam_step
+        t.bc2s[m] = (float)std::sqrt(1.0 - std::pow((double)beta2, (double)step[m]));
+    }
+    ProfScope ps(K_OPTIM, (cudaStream_t)stream);
+    k_adam_models<<<opt_models_grid(M, most), 256, 0, (cudaStream_t)stream>>>(params, grads, exp_avg, exp_avg_sq, t, beta1, beta2, eps, weight_decay);
+    LAUNCH_CHECK();
+    return 0;
+}
+
+int mshgnn_sgd_step_models(float* params, const float* grads, int32_t M, const int64_t* offsets, const float* lr, const int32_t* active,
+                           void* stream) {
+    OptModels t;
+    int64_t most = 0;
+    int rc;
+    if ((rc = opt_models_table(params, grads, M, offsets, lr, t, &most))) return rc;
+    for (int m = 0; m < M; ++m) t.active[m] = !active || active[m] != 0;
+    ProfScope ps(K_OPTIM, (cudaStream_t)stream);
+    k_sgd_models<<<opt_models_grid(M, most), 256, 0, (cudaStream_t)stream>>>(params, grads, t);
     LAUNCH_CHECK();
     return 0;
 }

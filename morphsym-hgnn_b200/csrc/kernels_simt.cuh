@@ -725,24 +725,66 @@ __global__ void k_loss_final(const double* __restrict__ partial, const int n_blo
 // ------------------------------------------------------------------------------------------
 // optimizers on the flat buffers
 // ------------------------------------------------------------------------------------------
+// One element of the Adam / SGD updates.  k_adam / k_sgd and their per-model forms call the same function, so the compiler
+// contracts the same products into FMAs and model m of a per-model launch gets the bits of a launch on its range alone.
+__device__ __forceinline__ void adam_update(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                            const int64_t i, const float lr, const float b1, const float b2, const float eps, const float wd,
+                                            const float bc1, const float bc2s) {
+    float gi = g[i];
+    const float pi = p[i];
+    if (wd != 0.f) gi = fmaf(wd, pi, gi);
+    const float mi = m[i] + (1.f - b1) * (gi - m[i]);      // torch: exp_avg.lerp_(grad, 1-beta1)
+    const float vi = b2 * v[i] + (1.f - b2) * gi * gi;
+    m[i] = mi; v[i] = vi;
+    const float denom = sqrtf(vi) / bc2s + eps;
+    p[i] = pi - (lr / bc1) * (mi / denom);
+}
+
+__device__ __forceinline__ void sgd_update(float* __restrict__ p, const float* __restrict__ g, const int64_t i, const float lr) { p[i] -= lr * g[i]; }
+
 __global__ void __launch_bounds__(256)
 k_adam(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, const int64_t n,
        const float lr, const float b1, const float b2, const float eps, const float wd, const float bc1, const float bc2s) {
-    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256) {
-        float gi = g[i];
-        const float pi = p[i];
-        if (wd != 0.f) gi = fmaf(wd, pi, gi);
-        const float mi = m[i] + (1.f - b1) * (gi - m[i]);      // torch: exp_avg.lerp_(grad, 1-beta1)
-        const float vi = b2 * v[i] + (1.f - b2) * gi * gi;
-        m[i] = mi; v[i] = vi;
-        const float denom = sqrtf(vi) / bc2s + eps;
-        p[i] = pi - (lr / bc1) * (mi / denom);
-    }
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256)
+        adam_update(p, g, m, v, i, lr, b1, b2, eps, wd, bc1, bc2s);
 }
 
 __global__ void __launch_bounds__(256)
 k_sgd(float* __restrict__ p, const float* __restrict__ g, const int64_t n, const float lr) {
-    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256) p[i] -= lr * g[i];
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256) sgd_update(p, g, i, lr);
+}
+
+// Per-model optimizer table of mshgnn_adam_step_models / mshgnn_sgd_step_models, passed by value: a launch captured in a CUDA
+// graph keeps the values it was captured with, like the scalars of k_adam, and no host-to-device copy is needed.
+constexpr int OPT_MAX_MODELS = 1023;
+struct OptModels {
+    int64_t off[OPT_MAX_MODELS + 1];   // model m owns elements [off[m], off[m + 1]) of every buffer
+    float lr[OPT_MAX_MODELS];
+    float bc1[OPT_MAX_MODELS];         // Adam bias corrections of the model's step (host-computed as mshgnn_adam_step does)
+    float bc2s[OPT_MAX_MODELS];
+    uint8_t active[OPT_MAX_MODELS];    // 0: the model's elements are not touched
+};
+static_assert(sizeof(OptModels) + 64 <= 32764, "the per-model optimizer table must fit the kernel-parameter limit");
+
+// grid.y = model; grid.x strides over that model's range
+__global__ void __launch_bounds__(256)
+k_adam_models(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, const __grid_constant__ OptModels t,
+              const float b1, const float b2, const float eps, const float wd) {
+    const int mo = blockIdx.y;
+    if (!t.active[mo]) return;
+    const float lr = t.lr[mo], bc1 = t.bc1[mo], bc2s = t.bc2s[mo];
+    const int64_t end = t.off[mo + 1];
+    for (int64_t i = t.off[mo] + (int64_t)blockIdx.x * 256 + threadIdx.x; i < end; i += (int64_t)gridDim.x * 256)
+        adam_update(p, g, m, v, i, lr, b1, b2, eps, wd, bc1, bc2s);
+}
+
+__global__ void __launch_bounds__(256)
+k_sgd_models(float* __restrict__ p, const float* __restrict__ g, const __grid_constant__ OptModels t) {
+    const int mo = blockIdx.y;
+    if (!t.active[mo]) return;
+    const float lr = t.lr[mo];
+    const int64_t end = t.off[mo + 1];
+    for (int64_t i = t.off[mo] + (int64_t)blockIdx.x * 256 + threadIdx.x; i < end; i += (int64_t)gridDim.x * 256) sgd_update(p, g, i, lr);
 }
 
 // ------------------------------------------------------------------------------------------

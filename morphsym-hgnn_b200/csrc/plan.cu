@@ -257,17 +257,28 @@ static ParamLayout param_layout(const Plan& p, int64_t h) {
     return y;
 }
 
-std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p) {
+std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p, const std::vector<int>& widths) {
     char err[256];
     if (!d) return "desc is NULL";
     if (flags & ~MSHGNN_PLAN_PAD_HIDDEN) { snprintf(err, sizeof err, "unknown plan flags 0x%x", (unsigned)flags); return err; }
-    if (!(flags & MSHGNN_PLAN_PAD_HIDDEN) && d->hidden != H) {
-        snprintf(err, sizeof err, "hidden=%d unsupported: this build is specialised for H=128 (MSHGNN_PLAN_PAD_HIDDEN runs 1..128)", d->hidden);
-        return err;
+    if (widths.empty()) {
+        if (!(flags & MSHGNN_PLAN_PAD_HIDDEN) && d->hidden != H) {
+            snprintf(err, sizeof err, "hidden=%d unsupported: this build is specialised for H=128 (MSHGNN_PLAN_PAD_HIDDEN runs 1..128)", d->hidden);
+            return err;
+        }
+        if (d->hidden < 1 || d->hidden > H) { snprintf(err, sizeof err, "hidden=%d unsupported: padded plans take 1..128 hidden channels", d->hidden); return err; }
+        p.hidden.assign(1, d->hidden);
+    } else {
+        for (size_t m = 0; m < widths.size(); ++m)
+            if (widths[m] < 1 || widths[m] > H) {
+                snprintf(err, sizeof err, "model %zu: hidden=%d unsupported: model batches take 1..128 hidden channels", m, widths[m]);
+                return err;
+            }
+        p.hidden = widths;
     }
-    if (d->hidden < 1 || d->hidden > H) { snprintf(err, sizeof err, "hidden=%d unsupported: padded plans take 1..128 hidden channels", d->hidden); return err; }
-    p.hidden = d->hidden;
-    p.padded = p.hidden != H;
+    p.n_models = (int)p.hidden.size();
+    p.padded = false;
+    for (int h : p.hidden) p.padded = p.padded || h != H;
     if (d->n_node_types < 1 || d->n_node_types > MSHGNN_MAX_NODE_TYPES) return "n_node_types out of range";
     if (d->n_edge_types < 1 || d->n_edge_types > MSHGNN_MAX_EDGE_TYPES) return "n_edge_types out of range";
     if (d->num_layers < 1 || d->num_layers > MAX_LAYERS) return "num_layers out of range (1..15)";
@@ -324,26 +335,40 @@ std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p) {
         p.off_dec_w = in.dec_w; p.off_dec_b = in.dec_b;
         p.n_params = in.n;
         if (in.n > (int64_t)1 << 30) return "parameter count too large";
-        p.ext = p.padded ? param_layout(p, p.hidden) : in;
+        p.ext_base.assign(1, 0);
+        for (int m = 0; m < p.n_models; ++m) {
+            p.ext.push_back(p.hidden[m] != H ? param_layout(p, p.hidden[m]) : in);
+            p.ext_base.push_back(p.ext_base.back() + p.ext.back().n);
+        }
     }
     if (p.padded) {
-        // the caller's [h, in], [h], [h, h], [C, h] tensors are the top-left blocks of the 128-wide ones
-        const int h = p.hidden;
+        // The caller's [h, in], [h], [h, h], [C, h] tensors are the top-left blocks of the 128-wide ones.  Every model's encoder
+        // segments come first: the backward compacts the rest before the encoder weight gradient runs, then the encoder block.
         auto seg = [&](int64_t e, int64_t i, int rows, int cols, int rows_i, int cols_i) { p.pad_segs.push_back(PadSeg{e, i, rows, cols, rows_i, cols_i}); };
-        for (int t = 0; t < p.n_types; ++t) {
-            seg(p.ext.enc_w[t], p.off_enc_w[t], h, p.in_w[t], H, p.in_w[t]);
-            seg(p.ext.enc_b[t], p.off_enc_b[t], 1, h, 1, H);
+        for (int m = 0; m < p.n_models; ++m) {
+            const ParamLayout& y = p.ext[m];
+            const int64_t e0 = p.ext_base[m], i0 = m * p.n_params;
+            const int h = p.hidden[m];
+            for (int t = 0; t < p.n_types; ++t) {
+                seg(e0 + y.enc_w[t], i0 + p.off_enc_w[t], h, p.in_w[t], H, p.in_w[t]);
+                seg(e0 + y.enc_b[t], i0 + p.off_enc_b[t], 1, h, 1, H);
+            }
         }
         p.n_pad_enc = (int)p.pad_segs.size();
-        for (int i = 0; i < p.L * p.n_etypes; ++i) {
-            seg(p.ext.rel_w[i], p.off_rel_w[i], h, h, H, H);
-            seg(p.ext.rel_b[i], p.off_rel_b[i], 1, h, 1, H);
-            seg(p.ext.root_w[i], p.off_root_w[i], h, h, H, H);
+        for (int m = 0; m < p.n_models; ++m) {
+            const ParamLayout& y = p.ext[m];
+            const int64_t e0 = p.ext_base[m], i0 = m * p.n_params;
+            const int h = p.hidden[m];
+            for (int i = 0; i < p.L * p.n_etypes; ++i) {
+                seg(e0 + y.rel_w[i], i0 + p.off_rel_w[i], h, h, H, H);
+                seg(e0 + y.rel_b[i], i0 + p.off_rel_b[i], 1, h, 1, H);
+                seg(e0 + y.root_w[i], i0 + p.off_root_w[i], h, h, H, H);
+            }
+            if (p.morph_sym)
+                for (int i = 0; i < 2; ++i) { seg(e0 + y.mlp_w[i], i0 + p.off_mlp_w[i], h, h, H, H); seg(e0 + y.mlp_b[i], i0 + p.off_mlp_b[i], 1, h, 1, H); }
+            seg(e0 + y.dec_w, i0 + p.off_dec_w, p.C, h, p.C, H);
+            seg(e0 + y.dec_b, i0 + p.off_dec_b, 1, p.C, 1, p.C);
         }
-        if (p.morph_sym)
-            for (int i = 0; i < 2; ++i) { seg(p.ext.mlp_w[i], p.off_mlp_w[i], h, h, H, H); seg(p.ext.mlp_b[i], p.off_mlp_b[i], 1, h, 1, H); }
-        seg(p.ext.dec_w, p.off_dec_w, p.C, h, p.C, H);
-        seg(p.ext.dec_b, p.off_dec_b, 1, p.C, 1, p.C);
     }
 
     // ---------------- derived weights ----------------
@@ -906,7 +931,13 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode, int M) {
 
 std::string describe_plan(const Plan& p) {
     std::ostringstream os;
-    os << "{\"S\":" << p.S << ",\"L\":" << p.L << ",\"hidden\":" << p.hidden << ",\"kernel_hidden\":" << H << ",\"n_params\":" << p.ext.n << ",\"n_derived\":" << p.n_derived
+    os << "{\"S\":" << p.S << ",\"L\":" << p.L << ",\"hidden\":" << p.hidden[0];
+    if (p.n_models > 1) {
+        os << ",\"hidden_models\":[";
+        for (int m = 0; m < p.n_models; ++m) os << (m ? "," : "") << p.hidden[m];
+        os << "]";
+    }
+    os << ",\"kernel_hidden\":" << H << ",\"n_params\":" << p.ext_base.back() << ",\"n_derived\":" << p.n_derived
        << ",\"n_tiles\":" << p.tiles.size() << ",\"n_rtasks\":" << p.rtasks.size() << ",\"n_rpairs\":" << p.rpairs.size()
        << ",\"n_groups\":" << p.groups.size() << ",\"n_mats16\":" << p.n_mats16 << ",\"enc_kmax\":" << p.enc_kmax
        << ",\"n_types\":" << p.n_types << ",\"need\":[";

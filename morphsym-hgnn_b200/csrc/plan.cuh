@@ -44,14 +44,21 @@ struct ParamLayout {
 struct Plan {
     // ---- description (deep copy) ----
     int n_types = 0, n_etypes = 0, L = 0, morph_sym = 0, mlp_type = -1, dec_type = 0, C = 0;
-    // Hidden width of the model.  The kernels are H = 128 wide: a padded plan (hidden < H, MSHGNN_PLAN_PAD_HIDDEN) runs the
-    // model as the 128-wide one whose weights are its zero-padded copy.  Every table below except `ext` refers to that
-    // 128-wide internal layout; the caller's params / grads are in `ext`, copied by k_pad_params / k_compact_grads.
-    int hidden = H;
+    // Hidden widths.  The kernels are H = 128 wide: a padded plan (a width < H: MSHGNN_PLAN_PAD_HIDDEN or
+    // mshgnn_plan_create_models) runs each model as the 128-wide one whose weights are its zero-padded copy.  Every table
+    // below except `ext` refers to that 128-wide internal layout; the caller's params / grads are in `ext`, copied by
+    // k_pad_params / k_compact_grads.
+    // A plan of mshgnn_plan_create_models with M > 1 describes n_models = M models that differ only in width (a "mixed" plan):
+    // model m's layout ext[m] starts at ext_base[m] of the caller's buffer (the layouts laid end to end), its 128-wide
+    // internal copy at m * n_params, and the PadSeg table holds absolute offsets for all of them.  Other plans have
+    // n_models = 1 and serve a model batch of any M through per-model strides (blockIdx.z of the pad kernels).
+    int n_models = 1;
+    std::vector<int> hidden;           // [n_models]
     bool padded = false;
-    ParamLayout ext;
-    std::vector<PadSeg> pad_segs;      // one per parameter tensor, in flat order
-    int n_pad_enc = 0;                 // segments [0, n_pad_enc) are the encoder block
+    std::vector<ParamLayout> ext;      // [n_models], offsets from the model's own start
+    std::vector<int64_t> ext_base;     // [n_models + 1]; ext_base[n_models] = mshgnn_param_count
+    std::vector<PadSeg> pad_segs;      // one per parameter tensor and model: every model's encoder block, then every model's rest
+    int n_pad_enc = 0;                 // segments [0, n_pad_enc) are the encoder blocks
     int nodes[MSHGNN_MAX_NODE_TYPES] = {0}, in_w[MSHGNN_MAX_NODE_TYPES] = {0};
     int e_src_t[MSHGNN_MAX_EDGE_TYPES] = {0}, e_dst_t[MSHGNN_MAX_EDGE_TYPES] = {0}, e_mean[MSHGNN_MAX_EDGE_TYPES] = {0};
     std::vector<int> e_src[MSHGNN_MAX_EDGE_TYPES], e_dst[MSHGNN_MAX_EDGE_TYPES];
@@ -167,7 +174,8 @@ struct WsLayout {
 constexpr int DEC_BLOCKS = 1184;     // 148 SMs x 8 resident CTAs of the 2-channel instantiation (48 registers, 8 KB of shared memory; the 8-channel one: 2 per SM): one load in flight per warp, so latency is hidden by warps
 constexpr int LOSS_BLOCKS = LOSS_PARTIALS;
 
-std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p);   // returns error text ("" = ok)
+// returns error text ("" = ok).  widths empty: one model of width d->hidden; otherwise one model per width (d->hidden ignored)
+std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p, const std::vector<int>& widths = {});
 WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode, int M = 1);   // B graphs per model
 bool stack_enabled();                 // cross-layer stack kernel on (default) / off (MSHGNN_STACK=0 or mshgnn_set_option)
 void set_stack_enabled(int on);

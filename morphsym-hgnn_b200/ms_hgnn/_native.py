@@ -39,7 +39,9 @@ EXPORTS = (
     "mshgnn_check_edges", "mshgnn_set_option", "mshgnn_get_option", "mshgnn_stack_status", "mshgnn_stack_timing_offset",
     "mshgnn_backward_staged", "mshgnn_input_grad", "mshgnn_plan_create_ex", "mshgnn_step_metrics_ex",
     "mshgnn_workspace_bytes_models", "mshgnn_forward_models", "mshgnn_loss_models", "mshgnn_backward_models",
+    "mshgnn_plan_create_models", "mshgnn_param_offset_model", "mshgnn_adam_step_models", "mshgnn_sgd_step_models",
 )
+MAX_MODELS = 1023
 
 
 class Desc(C.Structure):
@@ -133,6 +135,15 @@ def lib() -> C.CDLL:
         L.mshgnn_loss_models.argtypes = [vp, i64, i64, i32, vp, vp, i32, f32, vp, vp, vp, i64, vp]; L.mshgnn_loss_models.restype = C.c_int
         L.mshgnn_backward_models.argtypes = [vp, i64, i64, C.POINTER(vp), i32, vp, vp, vp, vp, i64, i32, vp, vp]
         L.mshgnn_backward_models.restype = C.c_int
+    if hasattr(L, "mshgnn_plan_create_models"):  # absent from builds before it (MSHGNN_LIB A/B runs against an older commit)
+        L.mshgnn_plan_create_models.argtypes = [C.POINTER(Desc), i32, C.POINTER(i32), C.POINTER(vp)]
+        L.mshgnn_plan_create_models.restype = C.c_int
+        L.mshgnn_param_offset_model.argtypes = [vp, i32, i32, i32, i32, C.POINTER(i64), C.POINTER(i64)]
+        L.mshgnn_param_offset_model.restype = C.c_int
+        L.mshgnn_adam_step_models.argtypes = [vp, vp, vp, vp, i32, C.POINTER(i64), C.POINTER(i64), C.POINTER(f32), f32, f32, f32, f32, vp]
+        L.mshgnn_adam_step_models.restype = C.c_int
+        L.mshgnn_sgd_step_models.argtypes = [vp, vp, i32, C.POINTER(i64), C.POINTER(f32), C.POINTER(i32), vp]
+        L.mshgnn_sgd_step_models.restype = C.c_int
     L.mshgnn_adam_step.argtypes = [vp, vp, vp, vp, i64, i64, f32, f32, f32, f32, f32, vp]; L.mshgnn_adam_step.restype = C.c_int
     L.mshgnn_sgd_step.argtypes = [vp, vp, i64, f32, vp]; L.mshgnn_sgd_step.restype = C.c_int
     L.mshgnn_plan_describe.argtypes = [vp, C.c_char_p, i64]; L.mshgnn_plan_describe.restype = i64
@@ -200,7 +211,9 @@ def get_option(name: str) -> int:
 
 class NativePlan:
     """Owns a mshgnn_plan*.  ``spec`` is a plain dict (see engine.build_spec); ``spec["pad_hidden"]`` true creates the plan
-    with MSHGNN_PLAN_PAD_HIDDEN (hidden 1..128, run zero-padded on the 128-wide kernels)."""
+    with MSHGNN_PLAN_PAD_HIDDEN (hidden 1..128, run zero-padded on the 128-wide kernels).  ``spec["widths"]`` (a list of M
+    widths) creates the plan of a model batch of M models of those widths (mshgnn_plan_create_models); ``models`` is then M,
+    and None for other plans."""
 
     def __init__(self, spec: dict):
         L = lib()
@@ -231,7 +244,13 @@ class NativePlan:
             self._keep.append(arr)
             d.out_sign = C.cast(arr, C.POINTER(C.c_float))
         h = C.c_void_p()
-        if spec.get("pad_hidden") and hasattr(L, "mshgnn_plan_create_ex"):     # older builds (MSHGNN_LIB): 128 wide only
+        self.models = None
+        if spec.get("widths") is not None:
+            w = [int(v) for v in spec["widths"]]
+            arr = (C.c_int32 * max(len(w), 1))(*w)
+            check(L.mshgnn_plan_create_models(C.byref(d), len(w), arr, C.byref(h)), "mshgnn_plan_create_models")
+            self.models = len(w)
+        elif spec.get("pad_hidden") and hasattr(L, "mshgnn_plan_create_ex"):     # older builds (MSHGNN_LIB): 128 wide only
             check(L.mshgnn_plan_create_ex(C.byref(d), PLAN_PAD_HIDDEN, C.byref(h)), "mshgnn_plan_create_ex")
         else:
             check(L.mshgnn_plan_create(C.byref(d), C.byref(h)), "mshgnn_plan_create")
@@ -247,9 +266,14 @@ class NativePlan:
         except Exception:
             pass
 
-    def param_offset(self, kind: int, layer: int = 0, idx: int = 0):
+    def param_offset(self, kind: int, layer: int = 0, idx: int = 0, model: Optional[int] = None):
+        """(offset, numel) of one parameter tensor; ``model``: of model m of a model-batch plan (absolute offset)."""
         off, n = C.c_int64(), C.c_int64()
-        check(lib().mshgnn_param_offset(self.handle, kind, layer, idx, C.byref(off), C.byref(n)), "mshgnn_param_offset")
+        if model is None:
+            check(lib().mshgnn_param_offset(self.handle, kind, layer, idx, C.byref(off), C.byref(n)), "mshgnn_param_offset")
+        else:
+            check(lib().mshgnn_param_offset_model(self.handle, model, kind, layer, idx, C.byref(off), C.byref(n)),
+                  "mshgnn_param_offset_model")
         return off.value, n.value
 
     def workspace_bytes(self, B: int, train: bool, mode: int = MODE_FP32) -> int:
@@ -361,3 +385,22 @@ def adam_step(params_ptr, grads_ptr, m_ptr, v_ptr, n, step, lr, b1, b2, eps, wd,
 
 def sgd_step(params_ptr, grads_ptr, n, lr, stream):
     check(lib().mshgnn_sgd_step(params_ptr, grads_ptr, n, lr, stream), "mshgnn_sgd_step")
+
+
+def adam_step_models(params_ptr, grads_ptr, m_ptr, v_ptr, offsets: Sequence[int], steps: Sequence[int], lrs: Sequence[float],
+                     b1, b2, eps, wd, stream):
+    """One Adam launch for M models: model m owns [offsets[m], offsets[m+1]), takes step steps[m] (0: untouched) at lr lrs[m]."""
+    M = len(steps)
+    if len(offsets) != M + 1 or len(lrs) != M:
+        raise ValueError(f"{M} models need {M + 1} offsets and {M} learning rates")
+    check(lib().mshgnn_adam_step_models(params_ptr, grads_ptr, m_ptr, v_ptr, M, (C.c_int64 * (M + 1))(*offsets), (C.c_int64 * M)(*steps),
+                                        (C.c_float * M)(*lrs), b1, b2, eps, wd, stream), "mshgnn_adam_step_models")
+
+
+def sgd_step_models(params_ptr, grads_ptr, offsets: Sequence[int], lrs: Sequence[float], active: Sequence[bool], stream):
+    """One SGD launch for M models (model m: [offsets[m], offsets[m+1]) at lr lrs[m], untouched when not active[m])."""
+    M = len(lrs)
+    if len(offsets) != M + 1 or len(active) != M:
+        raise ValueError(f"{M} models need {M + 1} offsets and {M} active flags")
+    check(lib().mshgnn_sgd_step_models(params_ptr, grads_ptr, M, (C.c_int64 * (M + 1))(*offsets), (C.c_float * M)(*lrs),
+                                       (C.c_int32 * M)(*[int(bool(a)) for a in active]), stream), "mshgnn_sgd_step_models")

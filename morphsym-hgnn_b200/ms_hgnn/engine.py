@@ -65,27 +65,42 @@ class Engine:
         self._train_ctx = None        # (B, x tensors, x dtype code, models) of the last train-mode forward
 
     # ---- parameter layout ------------------------------------------------------------
-    def param_layout(self) -> List[Tuple[str, int, Tuple[int, ...]]]:
-        """[(reference state-dict name, flat offset, shape)] in named_parameters() order."""
+    def param_layout(self, model: int = 0) -> List[Tuple[str, int, Tuple[int, ...]]]:
+        """[(reference state-dict name, flat offset, shape)] in named_parameters() order.  On the plan of a model batch of
+        several widths (spec["widths"]): the tensors of model ``model``, at their absolute offsets in the batch's buffer."""
         s = self.spec
-        H = s["hidden"]
+        ragged = self.plan.models is not None
+        H = s["widths"][model] if ragged else s["hidden"]
+
+        def at(kind, layer=0, idx=0):
+            return self.plan.param_offset(kind, layer, idx, model if ragged else None)[0]
         out = []
         for i, t in enumerate(s["node_types"]):
-            o, _ = self.plan.param_offset(N.P_ENC_W, 0, i); out.append((f"encoder.lins.{t}.weight", o, (H, s["in_width"][i])))
-            o, _ = self.plan.param_offset(N.P_ENC_B, 0, i); out.append((f"encoder.lins.{t}.bias", o, (H,)))
+            out.append((f"encoder.lins.{t}.weight", at(N.P_ENC_W, 0, i), (H, s["in_width"][i])))
+            out.append((f"encoder.lins.{t}.bias", at(N.P_ENC_B, 0, i), (H,)))
         for l in range(s["num_layers"]):
             for e, et in enumerate(s["edge_types"]):
                 key = "<" + "___".join(et) + ">"
-                o, _ = self.plan.param_offset(N.P_REL_W, l, e); out.append((f"convs.{l}.convs.{key}.lin_rel.weight", o, (H, H)))
-                o, _ = self.plan.param_offset(N.P_REL_B, l, e); out.append((f"convs.{l}.convs.{key}.lin_rel.bias", o, (H,)))
-                o, _ = self.plan.param_offset(N.P_ROOT_W, l, e); out.append((f"convs.{l}.convs.{key}.lin_root.weight", o, (H, H)))
+                out.append((f"convs.{l}.convs.{key}.lin_rel.weight", at(N.P_REL_W, l, e), (H, H)))
+                out.append((f"convs.{l}.convs.{key}.lin_rel.bias", at(N.P_REL_B, l, e), (H,)))
+                out.append((f"convs.{l}.convs.{key}.lin_root.weight", at(N.P_ROOT_W, l, e), (H, H)))
         if s["morph_sym"]:
             for i, j in ((0, 0), (1, 2)):
-                o, _ = self.plan.param_offset(N.P_MLP_W, 0, i); out.append((f"base_transform.{j}.weight", o, (H, H)))
-                o, _ = self.plan.param_offset(N.P_MLP_B, 0, i); out.append((f"base_transform.{j}.bias", o, (H,)))
-        o, _ = self.plan.param_offset(N.P_DEC_W); out.append(("decoder.weight", o, (s["out_channels"], H)))
-        o, _ = self.plan.param_offset(N.P_DEC_B); out.append(("decoder.bias", o, (s["out_channels"],)))
+                out.append((f"base_transform.{j}.weight", at(N.P_MLP_W, 0, i), (H, H)))
+                out.append((f"base_transform.{j}.bias", at(N.P_MLP_B, 0, i), (H,)))
+        out.append(("decoder.weight", at(N.P_DEC_W), (s["out_channels"], H)))
+        out.append(("decoder.bias", at(N.P_DEC_B), (s["out_channels"],)))
         return out
+
+    def model_offsets(self) -> List[int]:
+        """Model m of a model-batch plan (spec["widths"]) owns elements [offsets[m], offsets[m + 1]) of the flat buffers: its
+        first tensor is its encoder weight of node type 0."""
+        return [self.plan.param_offset(N.P_ENC_W, 0, 0, m)[0] for m in range(self.plan.models)] + [self.n_params]
+
+    def _params_total(self, M: int) -> int:
+        """Elements of the flat parameter (and gradient) buffer of a call on M models: a model-batch plan's count is already
+        the total of its models."""
+        return self.n_params if self.plan.models is not None else M * self.n_params
 
     # ---- workspace --------------------------------------------------------------------
     def workspace(self, B: int, train: bool, device, n_models: int = 1) -> torch.Tensor:
@@ -131,7 +146,8 @@ class Engine:
 
     def forward(self, x: Sequence[torch.Tensor], flat_params: torch.Tensor, train: bool, n_models: int = 1) -> torch.Tensor:
         """``n_models`` > 1: a model batch - x[t] holds the graphs of model 0, then those of model 1, ... (equal counts),
-        ``flat_params`` is [n_models, n_params] (or its flattening) and the output rows follow the same model-major order."""
+        ``flat_params`` is [n_models, n_params] (or its flattening; on a plan of several widths, the models' layouts end to end)
+        and the output rows follow the same model-major order."""
         M = self._check_models(n_models)
         B, xd = self._check_inputs(x)
         if B % M:
@@ -139,7 +155,7 @@ class Engine:
         B //= M
         x = [t.contiguous() for t in x]
         dev = x[0].device
-        if flat_params.device != dev or flat_params.dtype != torch.float32 or flat_params.numel() != M * self.n_params \
+        if flat_params.device != dev or flat_params.dtype != torch.float32 or flat_params.numel() != self._params_total(M) \
                 or (M > 1 and not flat_params.is_contiguous()):
             raise RuntimeError("flat parameter buffer mismatch")
         ws = self.workspace(B, train, dev, M)
@@ -205,8 +221,8 @@ class Engine:
         if not param_grads:
             grads = None
         elif grads is None:
-            grads = torch.empty(M * self.n_params, dtype=torch.float32, device=dev)
-        elif M > 1 and (grads.numel() != M * self.n_params or not grads.is_contiguous()):
+            grads = torch.empty(self._params_total(M), dtype=torch.float32, device=dev)
+        elif M > 1 and (grads.numel() != self._params_total(M) or not grads.is_contiguous()):
             raise ValueError("gradient buffer mismatch")
         ws = self.workspace(B, True, dev, M)
         stream = torch.cuda.current_stream(dev).cuda_stream

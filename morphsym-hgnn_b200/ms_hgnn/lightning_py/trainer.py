@@ -313,40 +313,57 @@ class _SeedOptimizerView:
     def __init__(self, tr, i):
         self.exp_avg, self.exp_avg_sq = tr.exp_avg[i], tr.exp_avg_sq[i]
         self.step_count = tr.step_count[i]
-        self.lr, self.betas, self.eps, self.weight_decay = tr.lr, tr.betas, tr.eps, tr.weight_decay
+        self.lr, self.betas, self.eps, self.weight_decay = tr.lr[i], tr.betas, tr.eps, tr.weight_decay
+
+
+def _per_run(value, name: str, n: int) -> list:
+    """A scalar for every run, or a sequence of one value per run."""
+    if isinstance(value, (str, bytes)) or not hasattr(value, "__len__"):
+        return [value] * n
+    values = list(value)
+    if len(values) != n:
+        raise ValueError(f"{name} has {len(values)} entries for {n} runs (one per seed expected)")
+    return values
 
 
 def train_models(train_dataset: WindowSubset, val_dataset: WindowSubset, test_dataset: Optional[WindowSubset], normalize: bool,
                  testing_mode: bool = False, disable_logger: bool = False, logger_project_name: str = None, batch_size: int = 100,
-                 num_layers: int = 8, optimizer: str = "adam", lr: float = 0.003, epochs: int = 30, hidden_size: int = 10,
+                 num_layers: int = 8, optimizer: str = "adam", lr=0.003, epochs: int = 30, hidden_size=10,
                  regression: bool = True, seeds=(0,), devices: int = 1, early_stopping: bool = False, disable_test: bool = False,
                  train_percentage_to_log=None, symmetry_mode: str = None, group_operator_path: str = None,
                  subfoler_name: str = "default", data_path: Path = None, wandb_api_key: str = None,
                  grf_body_to_world_frame: bool = True, grf_dimension: int = 3, mode: str = "tc") -> List[str]:
-    """``train_model`` for several seeds at once: returns one checkpoint folder per seed, each with what ``train_model(seed=s)``
-    writes for that seed - bit for bit the same checkpoints (parameters and optimizer state) and metrics.
+    """``train_model`` for several runs at once: returns one checkpoint folder per run, each with what
+    ``train_model(seed=s, hidden_size=h, lr=l)`` writes for that run - bit for bit the same checkpoints (parameters and
+    optimizer state) and metrics.
 
-    Every seed is built exactly as ``train_model`` builds it (global seed, its own shuffle generator, dummy batch, module); the
-    training steps of all seeds run as one model batch (``ModelBatchTrainer``, arithmetic ``mode`` 'tc' or 'tc1x', which every
-    seed's module uses for validation and test too); validation, test, checkpoints, top-k and early stopping stay per seed.  A
-    seed that has stopped early still rides along in the batched step but gets no optimizer update and writes nothing more.
-    Resuming (``ckpt_path`` of ``train_model``) is not offered."""
+    Run i is ``(seeds[i], hidden_size[i], lr[i])``: ``hidden_size`` and ``lr`` are a value for every run or a sequence as long
+    as ``seeds`` (a seed may repeat), so one call trains a sweep over widths and learning rates.  Every run is built exactly as
+    ``train_model`` builds it (global seed, its own shuffle generator, dummy batch, module); the training steps of all runs run
+    as one model batch (``ModelBatchTrainer``, arithmetic ``mode`` 'tc' or 'tc1x', which every run's module uses for
+    validation and test too); validation, test, checkpoints, top-k and early stopping stay per run.  A run that has stopped
+    early still rides along in the batched step but gets no optimizer update and writes nothing more.  Resuming
+    (``ckpt_path`` of ``train_model``) is not offered."""
     from ..model_batch import ModelBatch, ModelBatchTrainer
     seeds = list(seeds)
     if not seeds:
         raise ValueError("train_models needs at least one seed")
-    model_type, com = _check_run_args(train_dataset, val_dataset, test_dataset, disable_test, hidden_size, devices)
+    hidden_sizes = _per_run(hidden_size, "hidden_size", len(seeds))
+    lrs = _per_run(lr, "lr", len(seeds))
+    for h in hidden_sizes:
+        model_type, com = _check_run_args(train_dataset, val_dataset, test_dataset, disable_test, h, devices)
     data_metadata = train_dataset.dataset.get_data_metadata()
     lim_train, lim_val, lim_test = (10, 5, 5) if testing_mode else (None, None, None)
-    runs = [_Run(train_dataset, model_type, com, data_metadata, seed, batch_size, normalize, hidden_size, num_layers, optimizer, lr,
+    runs = [_Run(train_dataset, model_type, com, data_metadata, seed, batch_size, normalize, h, num_layers, optimizer, l,
                  regression, symmetry_mode, group_operator_path, grf_body_to_world_frame, grf_dimension, data_path,
-                 disable_logger, logger_project_name, subfoler_name, train_percentage_to_log) for seed in seeds]
+                 disable_logger, logger_project_name, subfoler_name, train_percentage_to_log) for seed, h, l in zip(seeds, hidden_sizes, lrs)]
     for r in runs:
         r.module.model.set_mode(mode)
         r.start()
     m0 = runs[0].module
-    # the settings FusedTrainer(module) takes from the module
-    tr = ModelBatchTrainer(ModelBatch([r.module.model for r in runs]), optimizer=getattr(m0, "optimizer", "adam"), lr=float(getattr(m0, "lr", 1e-3)),
+    # the settings FusedTrainer(module) takes from each module
+    tr = ModelBatchTrainer(ModelBatch([r.module.model for r in runs], mixed_hidden=True), optimizer=getattr(m0, "optimizer", "adam"),
+                           lr=[float(getattr(r.module, "lr", 1e-3)) for r in runs],
                            regression=getattr(m0, "regression", getattr(m0.model, "regression", True)))
     ds = runs[0].ds
     global_step = 0
