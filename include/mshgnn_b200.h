@@ -341,29 +341,26 @@ int64_t mshgnn_dw_layout(const mshgnn_plan* plan, int64_t B, int32_t mode, int32
  * it is the guard that makes "no edge_index on the device" safe. */
 int mshgnn_check_edges(const mshgnn_plan* plan, int64_t B, const int64_t* const* edge_index, int32_t* flag, void* stream);
 
-/* ---- switches and status --------------------------------------------------------------------
- * Option "stack" (default 1, environment MSHGNN_STACK=0 turns it off): run the layer loop of the tensor-core modes
+/* ---- options and status ---------------------------------------------------------------------
+ * Kernel choices are process-wide options, set by mshgnn_set_option and read back by mshgnn_get_option (-1 for an unknown
+ * name).  The library reads no environment variable to choose a kernel.
+ * Option "stack" (default 1; 0 turns it off): run the layer loop of the tensor-core modes
  * (hgnn_k4.py:L170-186 and its backward) as ONE persistent cross-layer kernel over L2-resident row chunks instead of one
  * launch per layer.  It changes the workspace layout: query mshgnn_workspace_bytes again after switching.
- * Option "stack_pair" (MSHGNN_STACK_2CTA): the stack launches use the CTA-pair kernel (clusters of two CTAs,
+ * Option "stack_pair": the stack launches use the CTA-pair kernel (clusters of two CTAs,
  * tcgen05.mma.cta_group::2 on two row tiles at once; rows are then padded to a multiple of 256 - query the workspace size
  * again after switching): 1 (default) = for batches of >= 6144 graphs, 2 = always, 0 = never (the one-CTA stack kernel).
  * Both choose between implementations that produce identical bits (tests/test_gpu_stack.py).
- * Option "encoder" (MSHGNN_ENCODER=stream|v1|pair): kernel of the encoder forward: -1 (default) = the persistent TMA-fed kernel
+ * Option "encoder": kernel of the encoder forward: -1 (default) = the persistent TMA-fed kernel
  * whenever the feature tensors allow it (fp32, 16-byte rows), 0 = the same, 1 = one row tile per CTA, 2 = two row tiles per CTA;
- * "encoder_tpi" (MSHGNN_ENC_TPI): row tiles per work item of the persistent kernel, 0 = by batch size, 1, 2;
- * "encoder_dw_tma" (MSHGNN_ENC_DW=tma): feature rows of the encoder weight gradient by TMA (1) or register-staged loads (0, default).
+ * "encoder_tpi": row tiles per work item of the persistent kernel, 0 (default) = by batch size, 1, 2;
+ * "encoder_dw_tma": feature rows of the encoder weight gradient by TMA (1) or register-staged loads (-1 = default, 0).
  * All of them produce identical bits (tests/test_gpu_stack.py::test_encoder_kernels_are_bit_identical).
  * mshgnn_stack_status copies one word back (synchronising): *status_out = 1 when a dependency wait inside the last stack
  * launch on this workspace timed out (its results are then invalid); used by the tests. */
 int mshgnn_set_option(const char* name, int32_t value);
 int32_t mshgnn_get_option(const char* name);
 int mshgnn_stack_status(const mshgnn_plan* plan, int64_t B, int32_t train, int32_t mode, const void* workspace, int32_t* status_out);
-/* Diagnostics (MSHGNN_STACK_TIMING=1 selects an instrumented build of the stack kernel): byte offset in the workspace of
- * uint64 [CTA][16] cycle counters of the LAST stack launch - producer waiting for a ring slot / for a dependency, MMA
- * issuer waiting for operands / a free accumulator / a staged operand, epilogue group 0 waiting for an accumulator,
- * kernel cycles, steps.  -1 when the stack kernel is off. */
-int64_t mshgnn_stack_timing_offset(const mshgnn_plan* plan, int64_t B, int32_t train, int32_t mode);
 
 int64_t mshgnn_launch_count(void);
 const char* mshgnn_last_error(void);

@@ -239,7 +239,7 @@ bool first_on_device(std::atomic<bool> (&flags)[MAX_DEVICES]) {
     return !flags[dev].exchange(true);
 }
 
-// encoder kernel choice: -1 = environment / default (persistent TMA-fed kernel when the inputs allow it), 0 persistent, 1 one tile per CTA, 2 two tiles per CTA;
+// encoder kernel choice: -1 = default (persistent TMA-fed kernel when the inputs allow it), 0 persistent, 1 one tile per CTA, 2 two tiles per CTA;
 // rows tiles per item of the persistent kernel: 0 = by batch size, 1, 2 (mshgnn_set_option "encoder" / "encoder_tpi"; same-process A/B and bit-identity tests)
 static std::atomic<int> g_encoder_kernel{-1}, g_encoder_tpi{0}, g_encoder_dw_tma{-1};
 
@@ -247,9 +247,9 @@ int launch_tc_encoder(const Plan& p, const Launch& L, const WsLayout& w, const B
                       const float* params, int64_t B, int xf64, int split, cudaStream_t st) {
     if (L.count == 0) return 0;
     static std::atomic<bool> attr_set[64];
-    static const int which_env = [] { const char* e = getenv("MSHGNN_ENCODER"); return !e ? 0 : (!strcmp(e, "v1") ? 1 : (!strcmp(e, "pair") ? 2 : 0)); }();   // default: k_tc_encoder_pair; "stream": persistent bulk-copy kernel (kernels_enc.cuh), "v1": one tile per CTA
     // a model batch runs the two-tile kernel, the one that knows which model a row tile belongs to (the kernels give identical bits)
-    const int which = w.M > 1 ? 2 : (g_encoder_kernel.load() >= 0 ? g_encoder_kernel.load() : which_env);
+    const int opt = g_encoder_kernel.load();
+    const int which = w.M > 1 ? 2 : (opt >= 0 ? opt : 0);
     if (first_on_device(attr_set)) {
         CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder, cudaFuncAttributeMaxDynamicSharedMemorySize, ENC_SMEM_BYTES));
         CUDA_TRY(cudaFuncSetAttribute(k_tc_encoder_pair, cudaFuncAttributeMaxDynamicSharedMemorySize, ENCP_SMEM_BYTES));
@@ -272,9 +272,8 @@ int launch_tc_encoder(const Plan& p, const Launch& L, const WsLayout& w, const B
     const unsigned n_row_tiles = (unsigned)(w.Bp / TILE_M);
     if (which == 1) k_tc_encoder<<<dim3(n_row_tiles, (unsigned)L.count), ENC_THREADS, ENC_SMEM_BYTES, st>>>(maps, p.d_tiles + L.begin, bt, br, B, w.Bp, xf64, split);
     else if (which == 2 || !stream_ok) {
-        static const int pf = [] { const char* e = getenv("MSHGNN_ENC_PREFETCH"); return e ? atoi(e) : 0; }();     // 1: whole-row L2 prefetch of the feature rows (measured +12 % time: off)
         const unsigned pairs = (unsigned)(w.M * ((w.Bm / TILE_M + 1) / 2));     // per model: its row-tile pairs
-        k_tc_encoder_pair<<<dim3(pairs, (unsigned)L.count), ENC_THREADS, ENCP_SMEM_BYTES, st>>>(maps, p.d_tiles + L.begin, bt, br, B, w.Bp, xf64, split, pf,
+        k_tc_encoder_pair<<<dim3(pairs, (unsigned)L.count), ENC_THREADS, ENCP_SMEM_BYTES, st>>>(maps, p.d_tiles + L.begin, bt, br, B, w.Bp, xf64, split, /*enc_prefetch*/ 0,
                                                                                           w.Bm, p.n_types * H, p.n_params);
     } else {
         // persistent kernel: one CTA per SM draws (node slot, row-tile pair) items from the counter the forward prologue zeroed
@@ -282,13 +281,10 @@ int launch_tc_encoder(const Plan& p, const Launch& L, const WsLayout& w, const B
         if ((rc = sm_count(&n_sm))) return rc;
         // two row tiles per item (they share every weight stage) only when that leaves every SM several items: at 2048 graphs 64 long and
         // 96 short pair items on 148 SMs would make two long items the critical path (1.5 x the balanced time); single tiles balance
-        static const int force_tpi = [] { const char* e = getenv("MSHGNN_ENC_TPI"); return e ? atoi(e) : 0; }();
-        const int opt_tpi = g_encoder_tpi.load() ? g_encoder_tpi.load() : force_tpi;
-        const int tpi = opt_tpi == 1 || opt_tpi == 2 ? opt_tpi : ((int64_t)L.count * ((n_row_tiles + 1) / 2) >= 4 * (int64_t)n_sm ? 2 : 1);
+        const int opt_tpi = g_encoder_tpi.load();
+        const int tpi = opt_tpi ? opt_tpi : ((int64_t)L.count * ((n_row_tiles + 1) / 2) >= 4 * (int64_t)n_sm ? 2 : 1);
         const int64_t n_items = (int64_t)L.count * ((n_row_tiles + tpi - 1) / tpi);
         const unsigned grid = (unsigned)(n_items < n_sm ? n_items : n_sm);
-        static const int pf_kb = [] { const char* e = getenv("MSHGNN_ENC_PF"); return e ? atoi(e) : 0; }();                 // L2 prefetch distance of the feature boxes in K blocks; measured 2: no change, 4: +10 %, 8: +25 % time -> off
-        static const int dbg = [] { const char* e = getenv("MSHGNN_ENC_DEBUG"); return e ? atoi(e) : 0; }();               // measurement switches (results are wrong when set)
         EnqMaps em;
         em.w_hi = maps.w_hi; em.w_lo = maps.w_lo; em.o = maps.o;
         for (int t = 0; t < p.n_types; ++t) {
@@ -296,7 +292,8 @@ int launch_tc_encoder(const Plan& p, const Launch& L, const WsLayout& w, const B
             if ((rc = make_map_x3d(&em.x[t], bt.p[BUF_X0 + t], B, p.nodes[t], p.in_w[t]))) return rc;
         }
         for (int t = p.n_types; t < 4; ++t) em.x[t] = maps.o;
-        k_tc_encoder_stream<<<grid, ENQ_THREADS, ENQ_SMEM_BYTES, st>>>(em, p.d_tiles + L.begin, L.count, (int)BUF_X0, bt, br, B, w.Bp, split, (uint32_t*)(ws + w.enc_sync), tpi, pf_kb, dbg);
+        k_tc_encoder_stream<<<grid, ENQ_THREADS, ENQ_SMEM_BYTES, st>>>(em, p.d_tiles + L.begin, L.count, (int)BUF_X0, bt, br, B, w.Bp, split, (uint32_t*)(ws + w.enc_sync), tpi,
+                                                                       /*pf*/ 0, /*dbg*/ 0);
     }
     LAUNCH_CHECK();
     return 0;
@@ -306,8 +303,6 @@ int launch_tc_rowgemm(int kind, const Plan& p, const Launch& L, const BufTable& 
                       int64_t B, int64_t Bp, int split, cudaStream_t st) {
     if (L.count == 0) return 0;
     static std::atomic<bool> attr_set[64];
-    static const bool use_v2 = [] { const char* e = getenv("MSHGNN_ROWGEMM"); return e && !strcmp(e, "tile"); }();       // one-tile-per-CTA kernel (A/B measurements)
-    static const bool use_single = [] { const char* e = getenv("MSHGNN_ROWGEMM"); return e && !strcmp(e, "single"); }(); // persistent kernel, one row tile per item
     if (first_on_device(attr_set)) {
         CUDA_TRY(cudaFuncSetAttribute(k_tc_rowgemm, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES));
         CUDA_TRY(cudaFuncSetAttribute(k_tc_rowgemm_persistent, cudaFuncAttributeMaxDynamicSharedMemorySize, PK_SMEM_BYTES));
@@ -318,7 +313,7 @@ int launch_tc_rowgemm(int kind, const Plan& p, const Launch& L, const BufTable& 
             if (p.tiles[L.begin + i].chunks[c].a_kind != A_SLAB)
                 return fail(MSHGNN_ERR_ARG, "internal: a tensor-core row-GEMM launch must read slab buffers");
     ProfScope ps(kind, st);
-    if (use_v2 || L.count > PK_MAX_TILES) {
+    if (L.count > PK_MAX_TILES) {
         dim3 grid((unsigned)L.count, (unsigned)(Bp / TILE_M));
         k_tc_rowgemm<<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(wm.tc, p.d_tiles + L.begin, bt, br, B, Bp, split);
     } else {
@@ -326,7 +321,7 @@ int launch_tc_rowgemm(int kind, const Plan& p, const Launch& L, const BufTable& 
         if ((rc = sm_count(&n_sm))) return rc;
         // two row tiles per item (shared weight stages) only when that still leaves every SM >= 4 items: short launches
         // (base MLP: 4-8 output tiles) lose more to wave quantisation than they gain from the smaller operand stream
-        const bool pair = !use_single && Bp >= 2 * TILE_M && (int64_t)L.count * ((Bp / TILE_M + 1) / 2) >= 4 * (int64_t)n_sm;
+        const bool pair = Bp >= 2 * TILE_M && (int64_t)L.count * ((Bp / TILE_M + 1) / 2) >= 4 * (int64_t)n_sm;
         const int64_t n_items = (int64_t)L.count * (pair ? (Bp / TILE_M + 1) / 2 : Bp / TILE_M);
         if (n_items > 0x7fffffffLL) return fail(MSHGNN_ERR_ARG, "batch too large for one row-GEMM launch");
         const unsigned grid = (unsigned)(n_items < n_sm ? n_items : n_sm);
@@ -367,29 +362,18 @@ int launch_tc_dw(int kind, const Plan& p, int layer, const Launch& L, const WsLa
 }
 
 // ---- cross-layer stack kernel (kernels_stack.cuh) ----
-// Item order of the stack kernel (kernels_stack.cuh).  Default: CHUNKED - row chunks of RC row tiles, walked phase by phase.
-// RC trades the two things the kernel is sensitive to (tools/stack_timing.py, 16384 graphs, K4 Mini Cheetah):
+// Item order of the stack kernel (kernels_stack.cuh): row chunks of RC row tiles, walked phase by phase.
+// RC trades the two things the kernel is sensitive to (cycle counters of an instrumented build, profiles/r2_stack_timing.txt, 16384 graphs, K4 Mini Cheetah):
 //   * dependency distance: the items of layer l + 1 of a row tile are handed out RC x (items per row tile and layer) items
 //     after those of layer l; below ~2 x 148 items in flight + the latency of the slowest item (a base_transform chain) the
 //     scheduler warps wait (RC = 24: 22 % of the kernel in queue waits, RC = 32: 9 %, RC = 48: 7 %);
 //   * L2 residency: a chunk's input and output slabs of one layer are RC x 2 x S x 128 x 512 B (RC = 32: 84 MB of 126 MB).
-// MSHGNN_STACK_ORDER=diag selects the diagonal wavefront (uniform distance D x items per slot, MSHGNN_STACK_DELAY); measured
-// 5 % slower at equal footprint (all layers' weights and buffers are live at once).
+// The diagonal wavefront (uniform distance D x items per slot) was measured 5 % slower at equal footprint (all layers'
+// weights and buffers are live at once); the host always selects the chunked order.
 int stack_rows_per_chunk(const Plan& p) {
-    static const int env = [] { const char* e = getenv("MSHGNN_STACK_RC"); return e ? atoi(e) : 0; }();
-    if (env > 0) return env;
     const int64_t per_row_tile = (int64_t)2 * p.S * TILE_M * H * 4;
     int rc = (int)((int64_t)84 * 1024 * 1024 / per_row_tile);
     return rc < 16 ? 16 : (rc > 64 ? 64 : rc);
-}
-int stack_delay(const Plan::Stack& sp, int n_row_tiles, int n_sm) {
-    static const int env = [] { const char* e = getenv("MSHGNN_STACK_DELAY"); return e ? atoi(e) : 0; }();
-    if (env > 0) return env;
-    const int per_slot = sp.prog.items_per_row > 0 ? sp.prog.items_per_row : 1;
-    int d = (4 * n_sm + per_slot - 1) / per_slot;
-    const int most = n_row_tiles / (sp.prog.n_phases > 0 ? sp.prog.n_phases : 1);      // short batches: do not stretch the pipeline beyond the rows there are
-    if (d > most) d = most;
-    return d < 1 ? 1 : d;
 }
 
 int stack_sync_reset(const WsLayout& w, char* ws, cudaStream_t st) {
@@ -403,12 +387,9 @@ int launch_stack(int kind, const Plan& p, const Plan::Stack& sp, const WsLayout&
                  char* ws, int64_t B, int split, cudaStream_t st) {
     if (sp.prog.n_phases == 0) return 0;
     static std::atomic<bool> attr_set[64];
-    static const bool timing = [] { const char* e = getenv("MSHGNN_STACK_TIMING"); return e && !strcmp(e, "1"); }();
     if (first_on_device(attr_set)) {
-        CUDA_TRY(cudaFuncSetAttribute(k_tc_stack<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SK_SMEM_BYTES));
-        CUDA_TRY(cudaFuncSetAttribute(k_tc_stack<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SK_SMEM_BYTES));
-        CUDA_TRY(cudaFuncSetAttribute(k_tc_stack<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SK_SMEM_BYTES));
-        CUDA_TRY(cudaFuncSetAttribute(k_tc_stack<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SK_SMEM_BYTES));
+        CUDA_TRY(cudaFuncSetAttribute(k_tc_stack<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SK_SMEM_BYTES));
+        CUDA_TRY(cudaFuncSetAttribute(k_tc_stack<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SK_SMEM_BYTES));
     }
     bool has_priv = false;               // thread-private fp32 tensors in this program (kernels_stack.cuh): selects the PRIV instantiation
     for (int i = 0; i < sp.tiles.count; ++i) {
@@ -436,20 +417,16 @@ int launch_stack(int kind, const Plan& p, const Plan::Stack& sp, const WsLayout&
     a.sync = (uint32_t*)(ws + w.stack_sync);
     a.err = (uint32_t*)(ws + w.stack_sync + w.stack_sync_bytes - 4);
     a.next = (uint32_t*)(ws + w.stack_sync + w.stack_sync_bytes - 8);
-    a.timing = (unsigned long long*)(ws + w.stack_timing);
     a.ws = ws;
-    static const int env_dbg = [] { const char* e = getenv("MSHGNN_STACK_DEBUG"); return e ? atoi(e) : 0; }();
-    a.debug = env_dbg;
+    a.debug = 0;
     if ((int64_t)sp.prog.n_phases * a.n_row_tiles * p.S + 2 > w.stack_sync_bytes / 4) return fail(MSHGNN_ERR_WORKSPACE, "internal: stack counters do not fit");
     int n_sm = 0, rc;
     if ((rc = sm_count(&n_sm))) return rc;
-    static const bool chunked = [] { const char* e = getenv("MSHGNN_STACK_ORDER"); return !(e && !strcmp(e, "diag")); }();
     // an item drawn long before it runs delays its dependents: the scheduler warp stays one item ahead of the producer
-    static const int env_la = [] { const char* e = getenv("MSHGNN_STACK_LOOKAHEAD"); return e ? atoi(e) : 0; }();
-    a.lookahead = env_la > 0 ? (env_la > 4 ? 4 : env_la) : 1;
-    a.chunked = chunked ? 1 : 0;
-    a.delay = chunked ? stack_rows_per_chunk(p) : stack_delay(sp, a.n_row_tiles, n_sm);
-    if (w.stack_pair && !timing) {
+    a.lookahead = 1;
+    a.chunked = 1;
+    a.delay = stack_rows_per_chunk(p);
+    if (w.stack_pair) {
         // CTA-pair kernel: items are (phase, row-tile pair, node slot); one cluster of two CTAs per TPC
         if (a.n_row_tiles & 1) return fail(MSHGNN_ERR_ARG, "internal: the CTA-pair stack kernel needs an even number of row tiles");
         static std::atomic<bool> attr2_set[64];
@@ -462,8 +439,7 @@ int launch_stack(int kind, const Plan& p, const Plan::Stack& sp, const WsLayout&
         }
         const int64_t n_pairs_total = (int64_t)(a.n_row_tiles / 2) * sp.prog.items_per_row;
         a.n_total = (int)n_pairs_total;
-        if (a.chunked) { a.delay = a.delay / 2; if (a.delay < 1) a.delay = 1; }
-        else a.delay = stack_delay(sp, a.n_row_tiles / 2, n_sm / 2);
+        a.delay = std::max(a.delay / 2, 1);
         cudaLaunchConfig_t cfg = {};
         cfg.blockDim = dim3(SK_THREADS); cfg.dynamicSmemBytes = S2_SMEM_BYTES; cfg.stream = st;
         cudaLaunchAttribute at[2];
@@ -498,10 +474,8 @@ int launch_stack(int kind, const Plan& p, const Plan::Stack& sp, const WsLayout&
     cfg.attrs = at; cfg.numAttrs = 1;
     const Tile* d_tiles = p.d_tiles + sp.tiles.begin;
     const StackItem* d_items = p.d_stack_items + sp.item0;
-    if (timing && has_priv) CUDA_TRY(cudaLaunchKernelEx(&cfg, k_tc_stack<true, true>, wm.tc, d_tiles, d_items, a, bt, br));
-    else if (timing) CUDA_TRY(cudaLaunchKernelEx(&cfg, k_tc_stack<true, false>, wm.tc, d_tiles, d_items, a, bt, br));
-    else if (has_priv) CUDA_TRY(cudaLaunchKernelEx(&cfg, k_tc_stack<false, true>, wm.tc, d_tiles, d_items, a, bt, br));
-    else CUDA_TRY(cudaLaunchKernelEx(&cfg, k_tc_stack<false, false>, wm.tc, d_tiles, d_items, a, bt, br));
+    if (has_priv) CUDA_TRY(cudaLaunchKernelEx(&cfg, k_tc_stack<true>, wm.tc, d_tiles, d_items, a, bt, br));
+    else CUDA_TRY(cudaLaunchKernelEx(&cfg, k_tc_stack<false>, wm.tc, d_tiles, d_items, a, bt, br));
     LAUNCH_CHECK();
     return 0;
 }
@@ -623,9 +597,8 @@ int launch_tc_encoder_dw(const Call& c, int64_t B, int xf64, cudaStream_t st) {
     // x rows by TMA (raw fp32 into the X operand area, converted in place) when every feature tensor allows it: fp32, 16-byte rows
     // (measured, same box: 0.258-0.270 ms against 0.246-0.251 ms for the register-staged loaders - here the loads of a step are issued
     // BEFORE its stage is free and nothing is pipelined across register sets, so the scoreboard effect of kernels_enc.cuh costs
-    // little, while a landing zone inside the stage serialises copy -> conversion -> MMA per stage.  Off unless MSHGNN_ENC_DW=tma.)
-    static const bool want_xt = [] { const char* e = getenv("MSHGNN_ENC_DW"); return e && !strcmp(e, "tma"); }();
-    bool xt = xf64 == 0 && w.M == 1 && (g_encoder_dw_tma.load() >= 0 ? g_encoder_dw_tma.load() != 0 : want_xt);
+    // little, while a landing zone inside the stage serialises copy -> conversion -> MMA per stage.  Off unless option "encoder_dw_tma" is 1.)
+    bool xt = xf64 == 0 && w.M == 1 && g_encoder_dw_tma.load() > 0;
     for (const EncDwUnit& eu : p.enc_units)
         if (xt) xt = eu.x_buf >= BUF_X0 && eu.x_buf < BUF_X0 + p.n_types && enq_rows_ok(bt.p[eu.x_buf], eu.K, 0);
     EncXMaps xm;
@@ -1016,14 +989,11 @@ int mshgnn_backward_models(const mshgnn_plan* plan, int64_t M, int64_t B, const 
             // the whole dX chain (with the base_transform backward chained on chip) in one launch over per-layer dh / dc / du
             // images, then the weight gradients of every layer (they only read what the chain and the forward pass stored)
             if ((rc = launch_stack(K_STACK_BWD, p, p.stack_bwd, w, bt, br, wm, ws, B, split, st))) return rc;
-            if (want_dw && w.dw_merged) {
+            if (want_dw) {
                 // tasks are laid out layer L-1 first, contiguously: one launch covers them all (ws_layout fitted one split count)
                 Launch all{p.dw_layer[p.L - 1].begin, 0};
                 for (int l = 0; l < p.L; ++l) all.count += p.dw_layer[l].count;
                 if ((rc = launch_tc_dw(K_DW_LAYER, p, p.L - 1, all, w, br, wm, B, split, part_w, part_b, st))) return rc;
-            } else if (want_dw) {
-                for (int l = p.L - 1; l >= 0; --l)
-                    if ((rc = launch_tc_dw(K_DW_LAYER, p, l, p.dw_layer[l], w, br, wm, B, split, part_w, part_b, st))) return rc;
             }
         } else {
             for (int l = p.L - 1; l >= 0; --l) {
@@ -1383,12 +1353,6 @@ int mshgnn_stack_status(const mshgnn_plan* plan, int64_t B, int32_t train, int32
     CUDA_TRY(cudaMemcpy(&word, (const char*)workspace + w.stack_sync + w.stack_sync_bytes - 4, 4, cudaMemcpyDeviceToHost));
     *status_out = word ? 1 : 0;
     return 0;
-}
-
-int64_t mshgnn_stack_timing_offset(const mshgnn_plan* plan, int64_t B, int32_t train, int32_t mode) {
-    if (!plan || B < 1) return -1;
-    const WsLayout w = ws_layout(plan->p, B, train, mode);
-    return w.stack ? w.stack_timing : -1;
 }
 
 int64_t mshgnn_launch_count(void) { return g_launches.load(); }

@@ -1,5 +1,5 @@
 // Persistent, warp-specialised encoder (default of the tensor-core modes since round 2 for fp32 feature tensors with 16-byte aligned
-// rows; MSHGNN_ENCODER=pair / v1 select the one-item-per-CTA kernels of kernels_tc.cuh, which also serve fp64 / fp16 / unaligned inputs).
+// rows; option "encoder" = 2 / 1 selects the one-item-per-CTA kernels of kernels_tc.cuh, which also serve fp64 / fp16 / unaligned inputs).
 //
 //   h0[slot] = relu((x[slot] * sign[slot]) W_enc[type]^T + b)                    (hgnn_k4.py:L159-160, L198-237)
 //
@@ -89,7 +89,7 @@ __device__ __forceinline__ int enq_take(EnqCtl& ctl, const int m, const bool who
 __global__ void __launch_bounds__(ENQ_THREADS, 1)
 k_tc_encoder_stream(const __grid_constant__ EnqMaps maps, const Tile* __restrict__ tiles, const int n_slots, const int x_buf0 /*buffer id of the first feature tensor*/, const BufTable bt, const BufRows br,
                     const int64_t B, const int64_t Bp, const int split, uint32_t* __restrict__ counter, const int tpi /*row tiles per item: 1 or 2*/, const int pf /*L2 prefetch distance in K blocks, 0 = off*/,
-                    const int dbg /*measurement switches: 1 no conversion, 2 no MMAs, 4 no weight loads (results are wrong when set)*/) {
+                    const int dbg /*measurement switches: 1 no conversion, 2 no MMAs, 4 no weight loads (results are wrong when set; the host passes 0)*/) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     const int tid = threadIdx.x;
     const int warp = tid >> 5, lane = tid & 31;
@@ -173,8 +173,8 @@ k_tc_encoder_stream(const __grid_constant__ EnqMaps maps, const Tile* __restrict
                     for (int i = 0; i < n_kb; ++i, ++kbi) {
                         // optional L2 prefetch of the feature boxes pf K blocks ahead of the loads (through this item into the next one).  Idea: the
                         // landing zones are the two operand stages, so a stage that is being converted or multiplied requests nothing - a prefetch
-                        // would keep DRAM busy meanwhile.  Measured (MSHGNN_ENC_PF, same box): 2 K blocks ahead no change, 4: 0.21 -> 0.235 ms,
-                        // 8: 0.266 ms - the extra requests compete with the demand loads instead of preceding them.  Off by default.
+                        // would keep DRAM busy meanwhile.  Measured (same box): 2 K blocks ahead no change, 4: 0.21 -> 0.235 ms,
+                        // 8: 0.266 ms - the extra requests compete with the demand loads instead of preceding them.  The host passes pf = 0.
                         while (pf > 0 && pf_pos <= i + pf) {
                             if (pf_pos < n_kb) {
                                 tma_prefetch_3d(xm, pf_pos * 64, node, row0);

@@ -32,7 +32,7 @@ namespace mshgnn {
 
 // Operand K blocks are 64 fp16 wide (128-byte rows, SWIZZLE_128B): with the 32-column blocks of the per-layer kernels the
 // MMA warp spent 40-50 % of the kernel waiting for operands while the producer rarely waited for a ring slot - the
-// L2 -> SM stream of 64-byte row segments was the bottleneck (tools/stack_timing.py), not the bytes in flight.
+// L2 -> SM stream of 64-byte row segments was the bottleneck (profiles/r2_stack_timing.txt), not the bytes in flight.
 constexpr int SK_KB = 64;
 constexpr int SK_TILE_BYTES = 128 * SK_KB * 2;                            // 16 KB
 constexpr int SK_STAGE_BYTES = 4 * SK_TILE_BYTES;                         // A_hi, A_lo, W_hi, W_lo = 64 KB
@@ -65,9 +65,8 @@ struct StackArgs {
     uint32_t* sync;              // [n_phases][n_row_tiles][n_slots] completion counters (4 = the four epilogue groups of the producing item)
     uint32_t* err;               // error word (a dependency wait timed out)
     uint32_t* next;              // work counter: the next item index to hand out (zeroed with the completion counters)
-    unsigned long long* timing;  // TIMING instantiation only: per CTA 8 cycle counters (see k_tc_stack)
     char* ws;                    // workspace base (thread-private fp32 tensors live in the image area of their buffer)
-    int debug;                   // ablation switches for timing experiments (MSHGNN_STACK_DEBUG; results are then garbage): 1 no A loads,
+    int debug;                   // ablation switches for timing experiments (the host passes 0; results are garbage otherwise): 1 no A loads,
                                  // 2 no W loads, 4 no MMAs, 8 epilogue reduced to its handshakes, 16 completion signal at once, 32 barrier before every staging write,
                                  // 64 no L1 prefetch, 256 no second output of two-output tiles, 512 no residuals (CTA-pair kernel only)
 };
@@ -85,7 +84,7 @@ __device__ __forceinline__ int stack_count(const StackProg& pg, const int NT, co
     for (int p = 0; p < pg.n_phases; ++p) c += pg.n_items[p] * min(max(t - p * D, 0), NT);
     return c;
 }
-// chunked order: chunks of RC row tiles, phase-major inside a chunk (MSHGNN_STACK_ORDER=chunk, for A/B measurements)
+// chunked order: chunks of RC row tiles, phase-major inside a chunk (the order the host selects: StackArgs::chunked = 1)
 __device__ __forceinline__ ItemRef stack_decode_chunked(const StackProg& pg, const int NT, const int RC, const int i) {
     const int chunk_items = RC * pg.items_per_row;
     const int c = i / chunk_items;
@@ -337,8 +336,7 @@ template <bool PRIV>
 __device__ __forceinline__ void stack_epilogue(const TileHdr& t, const BufTable& bt, const BufRows& br, const CUtensorMap* map_k,
                                                const uint32_t tmem_acc, const int row0, const int64_t B, const int64_t Bp,
                                                const int warp, const int lane, const int grp, const StackEpi es, uint32_t& res_count,
-                                               uint32_t* sig, uint32_t*& pending, char* const ws, unsigned long long* t_wait_acc = nullptr,
-                                               const bool dbg_bare = false, const int dbg = 0) {
+                                               uint32_t* sig, uint32_t*& pending, char* const ws, const bool dbg_bare = false, const int dbg = 0) {
     const int q = warp & 3;                        // TMEM lane quarter this warp may access (hardware rule: warp index mod 4)
     const bool leader = q == 2 && lane == 0;       // first warp of the group (warps 2 + 4g .. 5 + 4g): warp index = 2 mod 4
     const int rl = q * 32 + lane;                  // row inside the tile
@@ -408,8 +406,7 @@ __device__ __forceinline__ void stack_epilogue(const TileHdr& t, const BufTable&
         m2 = __ldg(reinterpret_cast<const uint32_t*>(bt.p[t.out2_mask_buf]) + ((int64_t)t.out2_mask_slot * Bp + row) * 4 + grp);
     if (leader && pending && !mbar_test(es.accum_bar, es.acc_parity)) stack_flush_signal(pending);     // idle anyway
 
-    if (t_wait_acc) { const long long t0 = clock64(); mbar_wait(es.accum_bar, es.acc_parity); *t_wait_acc += (unsigned long long)(clock64() - t0); }
-    else mbar_wait(es.accum_bar, es.acc_parity);
+    mbar_wait(es.accum_bar, es.acc_parity);
     tc_fence_after();
     uint32_t raw[32];
     tmem_ld32(tmem_acc + ((uint32_t)(q * 32) << 16) + col0, raw);
@@ -525,11 +522,7 @@ __device__ __forceinline__ void stack_epilogue(const TileHdr& t, const BufTable&
     if (leader && (dbg & 16)) stack_flush_signal(pending);
 }
 
-// TIMING = true is a diagnostic instantiation (MSHGNN_STACK_TIMING=1): the single-thread roles accumulate the cycles they
-// spend in each kind of wait into args.timing[blockIdx.x * 8 + {0: producer/ring slot, 1: producer/dependency, 2: MMA/operands,
-// 3: MMA/accumulator free, 4: MMA/staged operand, 5: epilogue group 0/accumulator, 6: kernel, 7: steps}].
-#define SK_TIMED(slot, stmt) do { if (TIMING) { const long long t0_ = clock64(); stmt; tim[slot] += (unsigned long long)(clock64() - t0_); } else { stmt; } } while (0)
-template <bool TIMING, bool PRIV>
+template <bool PRIV>
 __global__ void __launch_bounds__(SK_THREADS, 1)
 k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, const StackItem* __restrict__ items,
            const __grid_constant__ StackArgs args, const BufTable bt, const BufRows br) {
@@ -570,8 +563,6 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_s;
     constexpr int SPC = H / SK_KB;                 // pipeline steps (K blocks) per chunk
-    unsigned long long tim[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-    const long long t_begin = TIMING ? clock64() : 0;
     const StackProg& pg = args.prog;
     const int NT = args.n_row_tiles, RC = args.delay, n_total = args.n_total, split = args.split;
     const int64_t Bp = args.Bp;
@@ -608,7 +599,7 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
                     hd = stack_model_hdr(__ldg(reinterpret_cast<const int4*>(tiles + it.tile + lane / SK_HDR16) + lane % SK_HDR16), lane % SK_HDR16,
                                          tiles + it.tile + lane / SK_HDR16, mdl, args);
                 if (ir.phase > 0 && it.dep_mask)
-                    SK_TIMED(1, stack_wait(args.sync + ((size_t)(ir.phase - 1) * NT + ir.row_tile) * args.n_slots, it.dep_mask, lane, err));
+                    stack_wait(args.sync + ((size_t)(ir.phase - 1) * NT + ir.row_tile) * args.n_slots, it.dep_mask, lane, err);
                 a = make_int4(ir.row_tile, ir.phase, it.tile, it.n_steps);
                 b = make_int4(it.meta, it.out_slot, 0, 0);
             }
@@ -625,12 +616,11 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
             ++n_pub;
             if (cur >= n_total) break;
         }
-        if (TIMING && lane == 0) args.timing[(size_t)blockIdx.x * 16 + 1] = tim[1];
     } else if (warp == 0) {
         uint32_t g = 0;                        // pipeline step counter, runs across items
         for (int n = 0;; ++n) {
             int4 qa, qb;
-            SK_TIMED(11, next_item(n, qa, qb));
+            next_item(n, qa, qb);
             if (qa.w == 0) break;
             if (lane == 0) {
                 q_prod = n + 1;
@@ -648,11 +638,10 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
                         const uint32_t tx_bytes = (uint32_t)((from_stage ? 1 : 2) * (split ? 2 : 1) * SK_TILE_BYTES);
                         for (int kb = 0; kb < SPC; ++kb, ++g) {
                             const uint32_t s4 = g % SK_STAGES;
-                            SK_TIMED(0, mbar_wait(empty0 + 8 * s4, ((g / SK_STAGES) & 1) ^ 1));
+                            mbar_wait(empty0 + 8 * s4, ((g / SK_STAGES) & 1) ^ 1);
                             const int kcol = kb * SK_KB;
                             const uint32_t st = smem_base + s4 * SK_STAGE_BYTES;
                             const uint32_t fb = full0 + 8 * s4;
-                            const long long t_tma = TIMING ? clock64() : 0;
                             mbar_expect_tx(fb, tx_bytes);
                             if (!from_stage) tma_load_2d(st, &maps.o, fb, kcol, arow_hi);
                             tma_load_2d(st + 2 * SK_TILE_BYTES, &maps.o, fb, kcol, br.w_hi + w16_row);
@@ -660,40 +649,36 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
                                 if (!from_stage) tma_load_2d(st + SK_TILE_BYTES, &maps.o, fb, kcol, arow_lo);
                                 tma_load_2d(st + 3 * SK_TILE_BYTES, &maps.o, fb, kcol, br.w_lo + w16_row);
                             }
-                            if (TIMING) tim[10] += (unsigned long long)(clock64() - t_tma);
                         }
                     }
                 }
             }
             __syncwarp();
         }
-        if (TIMING && lane == 0) { args.timing[(size_t)blockIdx.x * 16] = tim[0]; args.timing[(size_t)blockIdx.x * 16 + 10] = tim[10]; args.timing[(size_t)blockIdx.x * 16 + 11] = tim[11]; }
     } else if (warp == 1) {
         uint32_t g = 0, k = 0, n_staged = 0;
         for (int n = 0;; ++n) {
             int4 qa, qb;
-            SK_TIMED(8, next_item(n, qa, qb));
+            next_item(n, qa, qb);
             if (qa.w == 0) break;
             if (lane == 0) {
                 for (int s = 0; s < qa.w; ++s, ++k) {
                     const int n_chunks = (qb.x >> (8 * s)) & 0xf, a_stage = (qb.x >> (8 * s + 4)) & 1;
                     const uint32_t a = k % SK_ACCS;
-                    SK_TIMED(3, mbar_wait(acc_free0 + 8 * a, ((k / SK_ACCS) & 1) ^ 1));      // the epilogue has drained this accumulator
+                    mbar_wait(acc_free0 + 8 * a, ((k / SK_ACCS) & 1) ^ 1);      // the epilogue has drained this accumulator
                     tc_fence_after();
-                    if (TIMING) tim[7] += 1;
                     const uint32_t d0 = tmem_base + a * 128;
                     for (int c = 0; c < n_chunks; ++c) {
                         const bool from_stage = a_stage && c == 0;
                         if (from_stage) {
-                            SK_TIMED(4, mbar_wait(stage_bar, n_staged & 1));   // the four quarters of the previous step's result are staged
+                            mbar_wait(stage_bar, n_staged & 1);   // the four quarters of the previous step's result are staged
                             ++n_staged;
                             tc_fence_after();
                         }
                         for (int kb = 0; kb < SPC; ++kb, ++g) {
                             const uint32_t s4 = g % SK_STAGES;
-                            SK_TIMED(2, mbar_wait(full0 + 8 * s4, (g / SK_STAGES) & 1));
+                            mbar_wait(full0 + 8 * s4, (g / SK_STAGES) & 1);
                             tc_fence_after();
-                            const long long t_issue = TIMING ? clock64() : 0;
                             const uint32_t st = smem_base + s4 * SK_STAGE_BYTES;
                             const uint64_t w_hi = smem_desc_sw128(st + 2 * SK_TILE_BYTES), w_lo = smem_desc_sw128(st + 3 * SK_TILE_BYTES);
 #pragma unroll
@@ -716,17 +701,12 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
                                 }
                             }
                             umma_commit(empty0 + 8 * s4);
-                            if (TIMING) tim[9] += (unsigned long long)(clock64() - t_issue);
                         }
                     }
                     umma_commit(acc_full0 + 8 * a);
                 }
             }
             __syncwarp();
-        }
-        if (TIMING && lane == 0) {
-            tim[6] = (unsigned long long)(clock64() - t_begin);
-            for (int j = 2; j < 10; ++j) if (j != 5) args.timing[(size_t)blockIdx.x * 16 + j] = tim[j];
         }
     } else {
         // group g (warps 2 + 4g .. 5 + 4g) drains column quarter g of every step
@@ -753,11 +733,10 @@ k_tc_stack(const __grid_constant__ TcMaps maps, const Tile* __restrict__ tiles, 
                 es.acc_parity = (k / SK_ACCS) & 1;
                 const int live_end = stack_live_end(args, stack_model(args, qa.x));
                 stack_epilogue<PRIV>(t, bt, br, &maps.k, tmem_base + a * 128, qa.x * TILE_M, live_end, Bp, warp, lane, grp, es, n_res,
-                                     s == qa.w - 1 ? ctr : nullptr, pending, args.ws, (TIMING && warp == 2 && lane == 0) ? &tim[5] : nullptr);
+                                     s == qa.w - 1 ? ctr : nullptr, pending, args.ws);
             }
         }
         if (sig_leader) { stack_flush_signal(pending); tma_store_wait_all(); }
-        if (TIMING && warp == 2 && lane == 0) args.timing[(size_t)blockIdx.x * 16 + 5] = tim[5];
     }
     tc_fence_before();
     __syncthreads();

@@ -6,7 +6,7 @@
 //  writes the next operands into the same memory (83 B per tensor cycle: every product of the fp32-class mode streams a
 //  (hi, lo) activation tile and a (hi, lo) weight tile) and the epilogue stages residuals / results through it.  Per
 //  three-product step that is ~1.2 MB of shared-memory traffic against 4608 tensor cycles = 590 KB of bandwidth: the tensor
-//  pipe cannot be more than ~48 % busy (measured: 47-51 %, tools/stack_timing.py "mma:issue" = back-pressured MMA issue).
+//  pipe cannot be more than ~48 % busy (measured: 47-51 %, profiles/r2_stack_timing.txt "mma:issue" = back-pressured MMA issue).
 //  With a CTA pair each SM holds only ITS half of every weight K block (64 of the 128 output channels): the weight fill and
 //  the B-operand reads per SM halve (40 KB -> 30 KB per K = 16 step and SM), and one thread issues the MMAs of both SMs.
 //
@@ -359,7 +359,7 @@ k_tc_stack2(const __grid_constant__ TcMaps maps, const __grid_constant__ CUtenso
                 es.acc_parity = (k / SK_ACCS) & 1;
                     const int live_end = stack_live_end(args, stack_model(args, qa.x));
                     stack_epilogue<PRIV>(t, bt, br, &maps.k, tmem_base + a * 128, qa.x * TILE_M, live_end, Bp, warp, lane, grp, es, n_res, s == qa.w - 1 ? ctr : nullptr,
-                                   pending, args.ws, nullptr, dbg_bare_epi, args.debug);
+                                   pending, args.ws, dbg_bare_epi, args.debug);
             }
         }
         if (sig_leader) { stack_flush_signal(pending); tma_store_wait_all(); }

@@ -1477,7 +1477,7 @@ k_tc_encoder(const __grid_constant__ EncMaps maps, const Tile* __restrict__ tile
 }
 
 // ------------------------------------------------------------------------------------------
-// encoder, two row tiles per CTA (default; MSHGNN_ENCODER=v1 selects k_tc_encoder)
+// encoder, two row tiles per CTA (model batches, inputs the persistent kernel cannot read, option "encoder" = 2)
 // ------------------------------------------------------------------------------------------
 //  ncu of k_tc_encoder: 46.7 M L2->SM read sectors (1.49 GB) for 708 MB of features - a 128-row x 64-column fp32 block
 //  of x is 32 KB and so is the (hi, lo) weight K block it meets, i.e. every CTA pulls as many weight bytes out of L2 as
@@ -1543,7 +1543,7 @@ k_tc_encoder_pair(const __grid_constant__ EncMaps maps, const Tile* __restrict__
     const int n_kb = (K + 63) / 64;
 
     if (warp == 0) {
-        // Optional (MSHGNN_ENC_PREFETCH=1, off by default) L2 prefetch of this CTA's feature rows as WHOLE-ROW bulk requests (one per
+        // Optional (enc_prefetch; the host passes 0) L2 prefetch of this CTA's feature rows as WHOLE-ROW bulk requests (one per
         // graph row, up to 1.5 KB at a time).  Hypothesis tested in round 2: the loaders read the rows as 256-byte fragments, 14 KB
         // apart, K block by K block, and DRAM serves that pattern badly (the weight-gradient kernel reads the same rows in 768-byte
         // fragments at 3.8 TB/s).  Measured: 0.346 -> 0.388 ms, i.e. WORSE - fragment size is not what limits this kernel.

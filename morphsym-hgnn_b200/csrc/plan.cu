@@ -83,12 +83,6 @@ static bool is_phase_buffer(int buf) {
     return (buf >= BUF_H0 && buf < BUF_H0 + MAX_LAYERS + 1) || (buf >= BUF_DHL0 && buf < BUF_DUL0 + MAX_LAYERS);
 }
 
-// MSHGNN_STACK_PRIVATE_DH=0: keep dh of every node as (hi, lo) images (A/B runs; read when a plan is created)
-static bool stack_private_dh() {
-    static const bool on = [] { const char* e = getenv("MSHGNN_STACK_PRIVATE_DH"); return !(e && !strcmp(e, "0")); }();
-    return on;
-}
-
 static std::string build_stack_programs(Plan& p) {
     auto begin_prog = [&](Plan::Stack& st) { st.tiles.begin = (int)p.tiles.size(); st.item0 = (int)p.stack_items.size(); st.prog = StackProg{}; };
     auto begin_phase = [&](Plan::Stack& st) -> std::string {
@@ -217,7 +211,7 @@ static std::string build_stack_programs(Plan& p) {
                     // kept as fp32 in a thread-private layout (kernels_stack.cuh): written straight from the epilogue's registers,
                     // read back by one bulk copy - no (hi, lo) split, no second in-place pass through the staging tiles, and the
                     // tile is left with ONE staged output (dc).  dh_L comes from the decoder kernel as images.
-                    if (p.morph_sym && stack_private_dh()) {
+                    if (p.morph_sym) {
                         const int slot = T.out_buf >= 0 ? T.out_slot : T.out2_slot;
                         const bool base = p.slot_type[slot] == p.mlp_type;
                         if (!base && T.out_buf == BUF_DHL0 + l && T.out2_buf >= 0) T.priv |= TILE_OUT_PRIV;
@@ -700,34 +694,37 @@ std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p, const std::
     return "";
 }
 
-static std::atomic<int> g_stack_on{-1};
-bool stack_enabled() {
-    int v = g_stack_on.load(std::memory_order_relaxed);
-    if (v < 0) {
-        const char* e = getenv("MSHGNN_STACK");
-        v = !(e && !strcmp(e, "0"));
-        g_stack_on.store(v, std::memory_order_relaxed);
-    }
-    return v != 0;
-}
+static std::atomic<int> g_stack_on{1};
+bool stack_enabled() { return g_stack_on.load(std::memory_order_relaxed) != 0; }
 void set_stack_enabled(int on) { g_stack_on.store(on ? 1 : 0, std::memory_order_relaxed); }
 
 // CTA-pair variant of the stack kernel (kernels_stack2.cuh): 1 (default) = for batches of >= STACK_PAIR_MIN_GRAPHS graphs, 2 = always,
-// 0 = never (MSHGNN_STACK_2CTA / option "stack_pair").  Below ~6 K graphs a phase of a row chunk has fewer pair items than there are
+// 0 = never (option "stack_pair").  Below ~6 K graphs a phase of a row chunk has fewer pair items than there are
 // CTA pairs to feed (8 pairs x 20 items against 74 pairs at 2048 graphs) and the one-CTA kernel is 5-10 % faster
 // (2048 graphs: 0.155 / 0.155 ms against 0.159 / 0.171; 4096: 0.214 / 0.251 against 0.215 / 0.268; 16384: 0.81 / 1.03 against 0.77 / 0.975).
 constexpr int64_t STACK_PAIR_MIN_GRAPHS = 6144;
-static std::atomic<int> g_stack_pair{-1};
-int stack_pair_mode() {
-    int v = g_stack_pair.load(std::memory_order_relaxed);
-    if (v < 0) {
-        const char* e = getenv("MSHGNN_STACK_2CTA");
-        v = e ? (atoi(e) < 0 ? 0 : (atoi(e) > 2 ? 2 : atoi(e))) : 1;
-        g_stack_pair.store(v, std::memory_order_relaxed);
-    }
-    return v;
-}
+static std::atomic<int> g_stack_pair{1};
+int stack_pair_mode() { return g_stack_pair.load(std::memory_order_relaxed); }
 void set_stack_pair_mode(int v) { g_stack_pair.store(v < 0 ? 0 : (v > 2 ? 2 : v), std::memory_order_relaxed); }
+
+// Row split of a weight-gradient launch of `units` CTAs per split (one unit x one row split each, one CTA per SM): a CTA takes
+// time ~ rows + a fixed ~96 rows' worth, and the launch ceil(units x splits / 148) waves of that.  Starting from `rows0`, whose
+// cost counts `keep` times, a candidate of [lo, hi] rows (multiples of 64, at most 64 splits) is taken when its cost is below
+// `gain` times the best so far.
+static int64_t fit_split_rows(int64_t B, int64_t units, int64_t rows0, double keep, double gain, int64_t lo, int64_t hi) {
+    auto cost = [&](int64_t rows) {
+        const int64_t ns = (B + rows - 1) / rows;
+        return (double)((units * ns + 147) / 148) * (double)(rows + 96);
+    };
+    int64_t best = rows0;
+    double best_c = keep * cost(rows0);
+    for (int64_t rows = lo; rows <= hi; rows += 64) {
+        if ((B + rows - 1) / rows > 64) continue;
+        const double c = cost(rows);
+        if (c < gain * best_c) { best_c = c; best = rows; }
+    }
+    return best;
+}
 
 // Every split below is a function of the per-model batch B alone: model m of a model batch reduces its rows exactly as a
 // single-model call on its B graphs does, so its gradients are bit for bit the same.
@@ -741,11 +738,11 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode, int M) {
     w.Bp = (int64_t)w.M * w.Bm;
     int ns = (int)((B + 511) / 512);
     w.n_splits = ns < 1 ? 1 : (ns > 64 ? 64 : ns);
-    {   // tcgen05 reduce-GEMM: ~1024 rows per split (MSHGNN_DW_ROWS overrides for A/B runs) (fp32 accumulation in TMEM, splits summed in double), no empty split.
+    {   // tcgen05 reduce-GEMM: ~1024 rows per split (fp32 accumulation in TMEM, splits summed in double), no empty split.
         // Row range per CTA decides the L2 reuse: the CTAs resident together (148) cover 148 / n_tasks splits, and every
         // dC / A slot tile of those rows is read by ~3 pairs at different times.  With 2048-row splits that working set was
         // 336 MB (> 126 MB L2) and ncu counted 607 MB of DRAM reads per launch for 300 MB of operands.
-        static const int64_t dw_rows = [] { const char* e = getenv("MSHGNN_DW_ROWS"); const int64_t v = e ? atoll(e) : 1024; return v < 64 ? 64 : v; }();
+        const int64_t dw_rows = 1024;
         int64_t target = (B + dw_rows - 1) / dw_rows;
         // small batches: still give every SM a CTA (tasks x splits >= ~148), down to 64-row splits
         int tasks = 1;
@@ -755,54 +752,25 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode, int M) {
         target = target < 1 ? 1 : (target > 64 ? 64 : target);
         w.rows_per_tc = (int)round_up((B + target - 1) / target, 64);
         w.n_splits_tc = (int)((B + w.rows_per_tc - 1) / w.rows_per_tc);
-        // Per layer launch: a CTA (one task x one row split, one CTA per SM) takes time ~ rows + a fixed ~96 rows' worth, and a
-        // launch takes ceil(tasks x splits / 148) waves of that.  The pruned last layers have 2 / 5 / 8 / 11 tasks instead of
-        // 17 (dead branches), so the default 16 splits left them at 32 / 80 / 128 / 176 CTAs - a quarter-filled wave, or one
-        // full wave plus a 19 % one (ncu: 57 / 58 / 61 / 114 us against 121 us for the full 272-CTA layer).  Pick the split
-        // that minimises waves x (rows + 96) under the same row cap; keep the default unless the model gains > 10 %.
-        static const bool fit = [] { const char* e = getenv("MSHGNN_DW_FIT"); return !(e && !strcmp(e, "0")); }();
+        // Per layer launch: the pruned last layers have 2 / 5 / 8 / 11 tasks instead of 17 (dead branches), so the default 16
+        // splits left them at 32 / 80 / 128 / 176 CTAs - a quarter-filled wave, or one full wave plus a 19 % one (ncu: 57 / 58 /
+        // 61 / 114 us against 121 us for the full 272-CTA layer).  Fit each layer's split under the same row cap; keep the
+        // default unless the model gains > 10 %.
         const int64_t cap = dw_rows > w.rows_per_tc ? dw_rows : w.rows_per_tc;
         for (int l = 0; l < MAX_LAYERS; ++l) { w.dw_ns[l] = w.n_splits_tc; w.dw_rows[l] = w.rows_per_tc; }
+        int64_t all_tasks = 0;
         for (size_t l = 0; l < p.dw_layer.size() && l < (size_t)MAX_LAYERS; ++l) {
-            const int64_t count = p.dw_layer[l].count;
-            if (count < 1 || !fit) continue;
-            auto cost = [&](int64_t rows) {
-                const int64_t ns = (B + rows - 1) / rows;
-                return (double)((count * ns + 147) / 148) * (double)(rows + 96);
-            };
-            int64_t best = w.rows_per_tc;
-            double best_c = 0.9 * cost(best);
-            for (int64_t rows = 64; rows <= cap; rows += 64) {
-                if ((B + rows - 1) / rows > 64) continue;
-                const double c = cost(rows);
-                if (c < best_c) { best_c = c; best = rows; }
-            }
-            w.dw_rows[l] = (int)best;
-            w.dw_ns[l] = (int)((B + best - 1) / best);
+            all_tasks += p.dw_layer[l].count;
+            w.dw_rows[l] = (int)fit_split_rows(B, p.dw_layer[l].count, w.rows_per_tc, 0.9, 1.0, 64, cap);
+            w.dw_ns[l] = (int)((B + w.dw_rows[l] - 1) / w.dw_rows[l]);
         }
         // Stack mode: the dX chain of every layer has already run when the weight gradients start, so ALL layers' tasks go
         // into ONE launch (K4: 94 tasks) with one row split count fitted to whole waves by the same cost model - 8 launches
         // fewer, and at small batches (2048 graphs: 136 CTAs of 256 rows per layer launch) CTAs long enough to amortise
         // their fixed prologue / partial write-out (94 x 3 splits of 704 rows).
-        if (w.stack && train && fit) {
-            int64_t count = 0;
-            for (size_t l = 0; l < p.dw_layer.size(); ++l) count += p.dw_layer[l].count;
-            if (count > 0) {
-                auto cost = [&](int64_t rows) {
-                    const int64_t ns = (B + rows - 1) / rows;
-                    return (double)((count * ns + 147) / 148) * (double)(rows + 96);
-                };
-                int64_t best = w.rows_per_tc;
-                double best_c = cost(best);
-                const int64_t cap2 = round_up(B < 2048 ? B : 2048, 64);
-                for (int64_t rows = 64; rows <= cap2; rows += 64) {
-                    if ((B + rows - 1) / rows > 64) continue;
-                    const double c = cost(rows);
-                    if (c < best_c) { best_c = c; best = rows; }
-                }
-                for (size_t l = 0; l < p.dw_layer.size() && l < (size_t)MAX_LAYERS; ++l) { w.dw_rows[l] = (int)best; w.dw_ns[l] = (int)((B + best - 1) / best); }
-                w.dw_merged = 1;
-            }
+        if (w.stack && train) {
+            const int64_t best = fit_split_rows(B, all_tasks, w.rows_per_tc, 1.0, 1.0, 64, round_up(B < 2048 ? B : 2048, 64));
+            for (size_t l = 0; l < p.dw_layer.size() && l < (size_t)MAX_LAYERS; ++l) { w.dw_rows[l] = (int)best; w.dw_ns[l] = (int)((B + best - 1) / best); }
         }
     }
     {   // partial slots, packed launch by launch in task order (the SIMT kernels use one split count for every task)
@@ -895,21 +863,8 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode, int M) {
         w.enc_sync = take(256);
         if (train) {
             // row splits of the encoder weight gradient, fitted to whole waves like the layer-stack ones (16 units for the K4 model:
-            // 512-row splits gave 64 CTAs on 148 SMs at 2048 graphs)
-            w.rows_per_enc = 512;
-            {
-                const int64_t units = (int64_t)p.enc_units.size();
-                auto cost = [&](int64_t rows) {
-                    const int64_t ns = (B + rows - 1) / rows;
-                    return (double)((units * ns + 147) / 148) * (double)(rows + 96);
-                };
-                double best_c = cost(512);
-                for (int64_t rows = 128; rows <= 1024 && units > 0; rows += 64) {
-                    if ((B + rows - 1) / rows > 64) continue;
-                    const double c = cost(rows);
-                    if (c < 0.97 * best_c) { best_c = c; w.rows_per_enc = (int)rows; }
-                }
-            }
+            // 512-row splits gave 64 CTAs on 148 SMs at 2048 graphs); each step must gain 3 %
+            w.rows_per_enc = (int)fit_split_rows(B, (int64_t)p.enc_units.size(), 512, 1.0, 0.97, 128, 1024);
             w.n_splits_enc = (int)((B + w.rows_per_enc - 1) / w.rows_per_enc);
             w.part_enc_w = take((int64_t)w.M * p.enc_units.size() * w.n_splits_enc * H * 192 * 4);
             w.part_enc_b = take((int64_t)w.M * p.enc_units.size() * w.n_splits_enc * H * 4);
@@ -918,7 +873,6 @@ WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode, int M) {
     if (w.stack) {
         w.stack_sync_bytes = ((int64_t)(p.L + 2) * (w.Bp / TILE_M) * p.S + 64) * 4;      // per (phase, row tile, node slot) completion counters + work counter + error word
         w.stack_sync = take(w.stack_sync_bytes);
-        w.stack_timing = take(256 * 16 * 8);
     }
     if (p.padded) {
         w.pad_params = take(w.M * p.n_params * 4);

@@ -150,7 +150,6 @@ struct WsLayout {
     int dw_ns[MAX_LAYERS], dw_rows[MAX_LAYERS];   // per layer launch: row splits actually used (wave-fitted, see ws_layout)
     PartSegs segs;                     // packed partial slots of the weight-gradient tasks (common.cuh)
     int dw_slot0[MAX_LAYERS];          // first partial slot of each layer launch
-    int dw_merged = 0;                 // stack mode: one weight-gradient launch for all layers (uniform row splits)
     int64_t part_slots = 0;            // slots of one model ([128][128] fp32 weight partial + [128] bias partial each); model m's follow model m-1's
     // Where every buffer id lives (byte offsets into the workspace, -1 when the call has no such buffer).  ws_layout makes
     // every aliasing decision here: several ids may name one buffer (the ping-pong slabs and images).
@@ -166,7 +165,6 @@ struct WsLayout {
     int64_t enc_sync = -1;             // work counter of the persistent encoder (k_tc_encoder_stream), zeroed by the forward prologue
     int64_t stack_sync = -1;           // dependency counters of the stack kernel (uint32 [phases][row tiles]) + error word
     int64_t stack_sync_bytes = 0;
-    int64_t stack_timing = -1;         // diagnostic cycle counters of the TIMING instantiation: [CTA][8] uint64
     int64_t pad_params = -1, pad_grads = -1;   // padded plans: 128-wide fp32 parameters (every call) / gradients (training)
     int64_t total = 0;
 };
@@ -177,9 +175,9 @@ constexpr int LOSS_BLOCKS = LOSS_PARTIALS;
 // returns error text ("" = ok).  widths empty: one model of width d->hidden; otherwise one model per width (d->hidden ignored)
 std::string build_plan(const mshgnn_desc* d, int32_t flags, Plan& p, const std::vector<int>& widths = {});
 WsLayout ws_layout(const Plan& p, int64_t B, int train, int mode, int M = 1);   // B graphs per model
-bool stack_enabled();                 // cross-layer stack kernel on (default) / off (MSHGNN_STACK=0 or mshgnn_set_option)
+bool stack_enabled();                 // cross-layer stack kernel on (default) / off (option "stack")
 void set_stack_enabled(int on);
-int stack_pair_mode();                // CTA-pair (cta_group::2) stack kernel: 1 = by batch size (default), 2 = always, 0 = never (MSHGNN_STACK_2CTA)
+int stack_pair_mode();                // CTA-pair (cta_group::2) stack kernel: 1 = by batch size (default), 2 = always, 0 = never (option "stack_pair")
 void set_stack_pair_mode(int v);
 std::string describe_plan(const Plan& p);
 

@@ -36,7 +36,7 @@ EXPORTS = (
     "mshgnn_adam_step", "mshgnn_sgd_step", "mshgnn_plan_describe", "mshgnn_launch_count",
     "mshgnn_last_error", "mshgnn_version", "mshgnn_profile_enable", "mshgnn_profile_read", "mshgnn_kernel_kind_name",
     "mshgnn_relu_mask_offset", "mshgnn_build_windows", "mshgnn_step_metrics", "mshgnn_dw_layout",
-    "mshgnn_check_edges", "mshgnn_set_option", "mshgnn_get_option", "mshgnn_stack_status", "mshgnn_stack_timing_offset",
+    "mshgnn_check_edges", "mshgnn_set_option", "mshgnn_get_option", "mshgnn_stack_status",
     "mshgnn_backward_staged", "mshgnn_input_grad", "mshgnn_plan_create_ex", "mshgnn_step_metrics_ex",
     "mshgnn_workspace_bytes_models", "mshgnn_forward_models", "mshgnn_loss_models", "mshgnn_backward_models",
     "mshgnn_plan_create_models", "mshgnn_param_offset_model", "mshgnn_adam_step_models", "mshgnn_sgd_step_models",
@@ -165,7 +165,6 @@ def lib() -> C.CDLL:
     L.mshgnn_set_option.argtypes = [C.c_char_p, i32]; L.mshgnn_set_option.restype = C.c_int
     L.mshgnn_get_option.argtypes = [C.c_char_p]; L.mshgnn_get_option.restype = i32
     L.mshgnn_stack_status.argtypes = [vp, i64, i32, i32, vp, C.POINTER(i32)]; L.mshgnn_stack_status.restype = C.c_int
-    L.mshgnn_stack_timing_offset.argtypes = [vp, i64, i32, i32]; L.mshgnn_stack_timing_offset.restype = i64
     _lib = L
     return L
 
@@ -324,9 +323,6 @@ class NativePlan:
         out = C.c_int32()
         check(lib().mshgnn_stack_status(self.handle, B, int(train), mode, ws_ptr, C.byref(out)), "mshgnn_stack_status")
         return out.value
-
-    def stack_timing_offset(self, B, train, mode) -> int:
-        return int(lib().mshgnn_stack_timing_offset(self.handle, B, int(train), mode))
 
     # ---- compute (raw device pointers) ----
     def forward(self, B, x_ptrs: Sequence[int], x_dtype, params_ptr, out_ptr, ws_ptr, ws_bytes, train, mode, stream):

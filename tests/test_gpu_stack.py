@@ -122,7 +122,7 @@ def test_stack_kernel_single_pass_mode_is_bit_identical_too(restore_stack_option
 
 @pytest.mark.parametrize("name,B,layers", [("mini_cheetah-k4-contact", 200, 8), ("solo12-k4-com", 257, 8), ("mi-grf", 20, 8)])
 def test_per_layer_launch_path_still_matches_the_oracle(name, B, layers, restore_stack_option):
-    """MSHGNN_STACK=0 keeps the round-1 launch sequence alive for A/B measurements: same 1e-4 bound."""
+    """Option "stack" = 0 keeps the round-1 launch sequence alive for A/B measurements: same 1e-4 bound."""
     from test_gpu_parity import check_gradients
     N.set_option("stack", 0)
     check_gradients(CONFIGS[name], B, layers, mode="tc")
