@@ -14,8 +14,8 @@ import time
 import pytest
 import torch
 
-from helpers import (TOL_FP32, gradient_check_under_native_pattern, graph_slice, oracle_model, oracle_outputs, oracle_run,
-                     rel_err)
+from helpers import (TOL_FP32, gradient_check_under_native_pattern, graph_slice, in_x_grad_dtype, oracle_model, oracle_outputs,
+                     oracle_run, rel_err)
 from ms_hgnn import _native as N
 from ms_hgnn import morphology as M
 from ms_hgnn.synthetic import CONFIGS, HeteroBatch, build_model
@@ -196,7 +196,7 @@ def check_training_batch(cfg, nm, om, batch, mode, label, sel=None, t0=None):
     dx_o = info.pop("forced_dx", None)
     tiles = {"out": (out_n, out_o)}
     if dx_o is not None:
-        tiles.update({f"x.grad[{k}]": (dx_n[k], dx_o[k]) for k in dx_o})
+        tiles.update({f"x.grad[{k}]": (dx_n[k], in_x_grad_dtype(dx_o[k], dx_n[k])) for k in dx_o})
     wt = worst_tile(tiles, B)
     torch.cuda.synchronize()
     res = {"B": B, "mode": mode, "out": e_out, "loss": e_loss, "grad": info.get("err"), "grad_tensor": info.get("tensor"),

@@ -40,7 +40,8 @@ def _step(nm, cfg, b):
 # 5000 / 7000 graphs = 40 / 55 row tiles: two and three L2 chunks (24 row tiles each for the 20-slot templates), the last one short
 STACK_CASES = [("mini_cheetah-k4-contact", 1, 3), ("mini_cheetah-k4-contact", 200, 8), ("mini_cheetah-k4-contact", 5000, 8),
                ("mini_cheetah-c2-contact", 1100, 8), ("a1-c2-grf", 300, 8), ("solo12-k4-com", 7000, 8), ("solo-c2-com", 33, 4),
-               ("mi-contact", 400, 8), ("mi-com", 77, 2)]
+               ("mi-contact", 400, 8), ("mi-com", 77, 2),
+               ("mini_cheetah-k4-contact", 300, 15), ("solo12-k4-com", 257, 15)]           # MAX_LAYERS: the longest stack programs
 
 
 @pytest.mark.parametrize("name,B,layers", STACK_CASES)
@@ -83,7 +84,8 @@ def test_stack_kernel_is_bit_identical_to_the_per_layer_launches(name, B, layers
 @pytest.mark.parametrize("name,B,layers,mode", [("mini_cheetah-k4-contact", 1, 3, "tc"), ("mini_cheetah-k4-contact", 129, 8, "tc"),
                                                 ("mini_cheetah-k4-contact", 5000, 8, "tc"), ("mini_cheetah-c2-contact", 385, 8, "tc"),
                                                 ("solo12-k4-com", 2100, 8, "tc"), ("mi-contact", 400, 8, "tc"),
-                                                ("mini_cheetah-k4-contact", 3300, 8, "tc1x")])
+                                                ("mini_cheetah-k4-contact", 3300, 8, "tc1x"), ("mini_cheetah-k4-contact", 385, 15, "tc"),
+                                                ("mi-contact", 400, 15, "tc")])
 def test_cta_pair_stack_kernel_is_bit_identical_to_the_one_cta_kernel(name, B, layers, mode, restore_stack_option):
     cfg = CONFIGS[name]
     b = make_batch(cfg, B, seed=B + 2).to("cuda:0")
